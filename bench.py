@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- byte-mix embedding fwd+bwd throughput (tokens/s) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one forward + one backward of the fused byte-mix embedding over one
 synthetic batch (per GPU), plus -- for N > 1 -- the all-reduce(AVG) of the dense
@@ -78,7 +78,37 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-torch-gpu", action="store_true", help="skip the PyTorch-on-the-same-GPU arm (eager + torch.compile)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (output, gradients) as DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return a
+
+
+DUMP_BYTES = 60 << 20   # data of all files; leaves room for the .npy headers under 64 MB
+
+
+def dump_outputs(path, arrays, seed=0):
+    """Write each tensor of `arrays` as <path>/<name>.npy in float32 (float64 stays float64), DUMP_BYTES in all.  The
+    smallest go first and are written whole; a tensor larger than an even share of what is left keeps a sample of its
+    rows (leading dimension), the same sorted rows on every run, so two builds can be compared output for output."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    left, items = DUMP_BYTES, sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    for i, (name, t) in enumerate(items):
+        t = t.detach().reshape(-1) if t.dim() == 0 else t.detach()
+        dt = torch.float64 if t.dtype == torch.float64 else torch.float32
+        row_bytes = max(1, t[0].numel()) * dt.itemsize
+        keep = min(t.shape[0], left // (len(items) - i) // row_bytes)
+        if keep < t.shape[0]:
+            rows = np.sort(np.random.default_rng(seed).choice(t.shape[0], keep, replace=False))
+            t = t.index_select(0, torch.from_numpy(rows).to(t.device))
+        a = t.to(dt).cpu().numpy()
+        np.save(os.path.join(path, f"{name}.npy"), a)
+        left -= a.nbytes
 
 
 def workload_config(args):
@@ -247,14 +277,14 @@ def cpu_reference_step_fn(w, n_sample, seed=12345):
 
 def time_cpu_reference(w, steps, warmup, budget_s=20.0, n_sample=None):
     """The oracle port on the host cores.  n_sample=None: the FULL per-GPU batch of the workload (same config as the GPU
-    arm); the number of timed steps is bounded by `budget_s` seconds."""
+    arm); the number of timed steps is bounded by `budget_s` seconds (budget_s=None: exactly `steps`)."""
     torch.set_num_threads(os.cpu_count() or 1)
     n_sample = w["N"] if n_sample is None else min(w["N"], n_sample)
     step = cpu_reference_step_fn(w, n_sample)
     for _ in range(max(1, min(warmup, 3))):
         step()
     t0 = time.perf_counter(); step(); one = time.perf_counter() - t0
-    reps = max(1, min(steps, int(budget_s / max(one, 1e-6))))
+    reps = steps if budget_s is None else max(1, min(steps, int(budget_s / max(one, 1e-6))))
     t0 = time.perf_counter()
     for _ in range(reps):
         step()
@@ -272,7 +302,7 @@ def run_reference(args):
     if rank != 0:
         return
     w = workload_config(args)
-    r = time_cpu_reference(w, args.steps, args.warmup, budget_s=90.0)
+    r = time_cpu_reference(w, args.steps, args.warmup, budget_s=None)
     cfg = main_config(w, args, world) if w["variant"] in ("V3", "V3d", "V4") else \
         {"workload": w["name"], "variant": w["variant"], "tokens_per_gpu_per_step": w["N"], "token_dim": w["Dt"],
          "byte_dim": w["bd"], "bytes_per_token": w["bpt"]}
@@ -367,10 +397,10 @@ def run_torch_gpu(args):
     dev = torch.device("cuda", int(os.environ.get("LOCAL_RANK", "0")))
     torch.cuda.set_device(dev)
     w = workload_config(args)
-    r = time_torch_gpu(w, dev, steps=max(5, min(args.steps, 50)), warmup=max(3, min(args.warmup, 10)))
+    r = time_torch_gpu(w, dev, steps=args.steps, warmup=max(3, min(args.warmup, 10)))
     best = min(v for k, v in r.items() if k.endswith("_ms_per_step"))
     line = {"impl": "torch-gpu", "metric": "byte-mix embedding fwd+bwd tokens/sec", "value": w["N"] / (best * 1e-3), "unit": "tokens/s",
-            "n_gpus": 1, "steps": max(5, min(args.steps, 50)), "warmup": max(3, min(args.warmup, 10)), "ms_per_step": best,
+            "n_gpus": 1, "steps": args.steps, "warmup": max(3, min(args.warmup, 10)), "ms_per_step": best,
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": w["dtype"], "data": "synthetic",
             "config": main_config(w, args, world), "torch_gpu": r, "gpu_launches": 0}
     print(json.dumps(line), flush=True)
@@ -489,6 +519,9 @@ def run_ours(args):
     e1.record()
     barrier()
     launches = mot_b200.launch_count()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"out": out, "grad_embed_tokens": gE_tok, "grad_embed_bytes": gE_byte,
+                                         **({"grad_lambdas": g_lam} if g_lam is not None else {})})
     ms_total = e0.elapsed_time(e1)
     t = torch.tensor([ms_total], device=dev)
     if world > 1:
@@ -866,6 +899,8 @@ def run_proj(args):
     e1.record()
     barrier()
     launches = mot_b200.launch_count()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"out": out, "grad_embed_tokens": gE_tok, "grad_embed_bytes": gE_byte, "grad_proj": gW})
     t = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -1000,6 +1035,9 @@ def run_value_embeds(args):
     e1.record()
     torch.cuda.synchronize()
     launches = mot_b200.launch_count()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {**{f"out_{i}": o for i, o in enumerate(outs)},
+                                         **{f"grad_value_embeds_{i}": gE for i, gE in enumerate(grads)}})
     ms_step = e0.elapsed_time(e1) / K
     # instrumented pass: event pairs around the main backward kernel of every scatter (3 per step -> the last one wins;
     # use one step per pair)
@@ -1070,6 +1108,7 @@ def run_mathblations(args):
     idx_host = torch.randint(0, 10000, (B, S), generator=g)
     idx_host[torch.rand(B, S, generator=g) < 0.2] = 10000
     idx_host = idx_host.pin_memory()
+    torch.manual_seed(12345)     # the module's initial weights and gout: the same inputs on every run
     m = mot_b200.DigitMixinEmbedding(V, w["Dt"], w["bd"], dpt).to(dev)
     gout = torch.randn(B, S, w["Do"], device=dev)
     res_host = torch.empty(14, w["bd"]).pin_memory()
@@ -1080,10 +1119,12 @@ def run_mathblations(args):
             p_.grad = None
         t = idx_host.to(dev, non_blocking=True) if e2e else idx
         digits = mot_b200.tokens_to_digits(t, dpt, 10000, 10001, 10002).view(B, S * dpt)
-        m(t, digits).backward(gout)
+        y = m(t, digits)
+        y.backward(gout)
         if e2e:
             res_host.copy_(m.dte.weight.grad, non_blocking=True)
             torch.cuda.current_stream().synchronize()
+        return y
 
     for _ in range(max(args.warmup, 3)):
         step()
@@ -1094,9 +1135,11 @@ def run_mathblations(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(K):
-        step()
+        y = step()
     e1.record(); torch.cuda.synchronize()
     launches = mot_b200.launch_count()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"out": y, **{"grad_" + n.replace(".", "_"): p_.grad for n, p_ in m.named_parameters()}})
     ms_step = e0.elapsed_time(e1) / K
     t0 = time.perf_counter()
     for _ in range(K):

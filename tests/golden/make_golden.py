@@ -281,7 +281,8 @@ def golden_runs():
                 out[f"{k}_gscalars"] = np_(scalars.grad)
             out[f"{k}_out"] = np_(x)
             out[f"{k}_gout"] = np_(gout)
-    np.savez_compressed(f"{HERE}/runs_float.npz", **out)
+    for dt in ("f32", "bf16"):     # one file per dtype keeps each fixture under 1 MB
+        np.savez_compressed(f"{HERE}/runs_float_{dt}.npz", **{k: v for k, v in out.items() if k.split("_")[2] == dt})
     print("runs float:", len(out), "arrays")
 
 

@@ -36,6 +36,30 @@ def test_reference_arm_other_ranks_stay_silent():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_steps_below_one_are_refused():
+    r = run(["--impl", "reference", "--steps", "0"])
+    assert r.returncode == 2 and "--steps must be at least 1" in r.stderr
+
+
+def test_dump_outputs_stays_in_budget_and_samples_the_same_rows(tmp_path, monkeypatch):
+    sys.path.insert(0, ROOT)
+    import numpy as np
+    import torch
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 40_000)
+    big = torch.arange(3000, dtype=torch.float32)[:, None].repeat(1, 8)     # every element holds its row number
+    small = torch.randn(5, 4, dtype=torch.float64)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"big": big, "small": small, "scalar": torch.tensor(2.5)})
+    a, b = np.load(tmp_path / "a" / "big.npy"), np.load(tmp_path / "b" / "big.npy")
+    assert a.dtype == np.float32 and np.array_equal(a, b)
+    rows = a[:, 0].astype(np.int64)
+    assert 0 < len(rows) < 3000 and np.all(np.diff(rows) > 0) and np.array_equal(a, big.float().numpy()[rows])
+    assert np.array_equal(np.load(tmp_path / "a" / "small.npy"), small.numpy())                  # float64 kept, whole
+    assert np.load(tmp_path / "a" / "scalar.npy").tolist() == [2.5]
+    assert sum(np.load(p).nbytes for p in (tmp_path / "a").iterdir()) <= 40_000
+
+
 def test_algorithmic_bytes_follow_survey_8d():
     sys.path.insert(0, ROOT)
     import bench

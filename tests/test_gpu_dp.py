@@ -141,7 +141,7 @@ def _worker(rank, world, port, q):
 def test_exchange_kernels_and_pipelined_step_multi_gpu():
     n = torch.cuda.device_count()
     if n < 2:
-        pytest.skip("needs >= 2 CUDA devices (the driver's 1-GPU box skips; run under gpurun --gpus 2)")
+        pytest.skip("needs >= 2 CUDA devices with NVLink peers; a 1-GPU machine skips it")
     world = 8 if n >= 8 else (4 if n >= 4 else 2)
     import torch.multiprocessing as mp
     ctx = mp.get_context("spawn")

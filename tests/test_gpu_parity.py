@@ -194,9 +194,9 @@ def test_ids_from_ttb_token_major_and_scramble(golden_dir):
 
 
 def test_reference_golden_runs_through_cuda(golden_dir):
-    """The reference's own outputs (tests/golden/runs_float.npz, fp32 runs) reproduced by the CUDA path."""
+    """The reference's own outputs (tests/golden/runs_float_f32.npz, fp32 runs) reproduced by the CUDA path."""
     import mot_b200
-    g = np.load(os.path.join(golden_dir, "runs_float.npz"))
+    g = np.load(os.path.join(golden_dir, "runs_float_f32.npz"))
     d = dev()
     for tag, kw, slot_major in [
         ("V3_run71", dict(combine="add"), True),

@@ -136,7 +136,7 @@ def test_reference_golden_projection_through_cuda(golden_dir):
     (scaled-pre-train), generated by tests/golden/make_golden.py, reproduced by the CUDA path."""
     import mot_b200
     d = dev()
-    g = np.load(os.path.join(golden_dir, "runs_float.npz"))
+    g = np.load(os.path.join(golden_dir, "runs_float_bf16.npz"))
     for tag, variant in [("V1_run7_bf16", "V1"), ("V2_run72_bf16", "V2")]:
         m = mot_b200.MoTProjEmbedding(80, 458, 32, 8, 40, 16, variant=variant).to(d)
         with torch.no_grad():
@@ -252,8 +252,8 @@ def test_byte_fc_variant_matches_reference_golden_and_oracle(golden_dir):
     reference's own bf16 / fp32 outputs and gradients at toy size, then the shipped 1024 = 16 x 64 shape vs the oracle."""
     import mot_b200
     d = dev()
-    g = np.load(os.path.join(golden_dir, "runs_float.npz"))
     for tag, dtype, tol in (("V3f_run71051_bf16", torch.bfloat16, TOL_CHAIN), ("V3f_run71051_f32", torch.float32, TOL_TF32_CHAIN)):
+        g = np.load(os.path.join(golden_dir, f"runs_float_{tag.rsplit('_', 1)[1]}.npz"))
         V, Dm = g[f"{tag}_E_tok"].shape
         bd = g[f"{tag}_E_byte"].shape[1]
         m = mot_b200.MoTByteFcEmbedding(V, 458, Dm, bd, Dm // bd).to(d)

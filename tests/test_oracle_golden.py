@@ -147,7 +147,7 @@ def test_runs_variants_match_reference(golden_dir, tag, dt):
     """fp32: oracle == reference to fp32 round-off.  bf16: the reference rounds
     every intermediate to bf16 (eager), the oracle does fp32 math on the same
     bf16 parameters -> agreement to a few bf16 ulps of the largest element."""
-    g = load(golden_dir, "runs_float.npz")
+    g = load(golden_dir, f"runs_float_{dt}.npz")
     variant, slot_major, wkey = RUN_CASES[tag]
     spec, _ = O.VARIANTS[variant]
     k = f"{tag}_{dt}"

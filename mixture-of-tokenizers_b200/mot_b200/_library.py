@@ -24,7 +24,7 @@ from typing import List, Optional, Tuple
 import torch
 from torch import Tensor
 
-from . import _lib as L
+from . import ops as O   # ops imports this module at its end: the name resolves from sys.modules
 
 _FORCE: Optional[bool] = {"1": True, "0": False}.get(os.environ.get("MOT_CUSTOM_OPS", ""), None)
 
@@ -45,7 +45,7 @@ def custom_ops_wanted() -> bool:
 # ---------------------------------------------------------------------------------------------------------------
 # MixSpec <-> int (operator schemas carry ints, floats, bools and tensors)
 # ---------------------------------------------------------------------------------------------------------------
-_COMBINE_NAMES = ("add", "concat", "tok_only", "bytes_only", "mean")
+_COMBINE_NAMES = tuple(O._COMBINE)   # the combine mode is its index in this order (bits 0-3 of the code)
 
 
 def pack_spec(spec) -> int:
@@ -55,46 +55,36 @@ def pack_spec(spec) -> int:
 
 
 def unpack_spec(code: int, eps: float):
-    from .ops import MixSpec
-    return MixSpec(combine=_COMBINE_NAMES[code & 15], tok_norm=bool(code & 16), byte_norm=bool(code & 32),
-                   out_norm=bool(code & 64), bytes_first=bool(code & 128), slot_major=bool(code & 256),
-                   ttb_scramble=bool(code & 512), eps=eps)
+    return O.MixSpec(combine=_COMBINE_NAMES[code & 15], tok_norm=bool(code & 16), byte_norm=bool(code & 32),
+                     out_norm=bool(code & 64), bytes_first=bool(code & 128), slot_major=bool(code & 256),
+                     ttb_scramble=bool(code & 512), eps=eps)
 
 
-def _none_if_empty(t: Optional[Tensor]) -> Optional[Tensor]:
-    return None if t is None or t.numel() == 0 else t
-
-
-_EVENTS: dict = {}
-
-
-def _events(dev):
-    ev = _EVENTS.get(dev.index)
-    if ev is None:
-        ev = _EVENTS[dev.index] = (torch.cuda.Event(), torch.cuda.Event())
-        cur = torch.cuda.current_stream(dev)
-        ev[0].record(cur)
-        ev[1].record(cur)
-    return ev
+_PLANNERS: dict = {}
 
 
 def _plan_beside(desc, tok: Tensor, dev) -> Tensor:
     """A fresh workspace with the sort plan of `tok`, started on the side stream (fork after everything queued on the
     current stream; the library zeroes the head of the fresh buffer there first).  The caller launches its forward
     kernels and then calls _rejoin()."""
-    from . import ops as O
-    ws = torch.empty(O.embed_workspace_bytes(desc), dtype=torch.uint8, device=dev)
-    ev_fork, ev_join = _events(dev)
-    with O._on_device(dev):
-        rc = L.lib().mot_embed_plan_async(desc, tok.data_ptr(), ws.data_ptr(), ws.numel(), 0, O._stream(dev),
-                                          O.side_stream(dev).cuda_stream, ev_fork.cuda_event, ev_join.cuda_event)
-    L.check(rc, "mot_embed_plan_async")
-    return ws
+    ws = _PLANNERS.get(dev.index)
+    if ws is None:   # one per device; the operators share its fork / join events, never its buffer
+        ws = _PLANNERS[dev.index] = O.Workspace(None, dev)
+    ws.buf = torch.empty(O.embed_workspace_bytes(desc), dtype=torch.uint8, device=dev)
+    O.embed_plan_async(desc, tok, ws, dev)         # ws.clean stays False: the plan clears the fresh buffer
+    buf, ws.buf = ws.buf, None
+    return buf
 
 
 def _rejoin(dev) -> None:
-    from . import ops as O
-    L.check(L.lib().mot_stream_wait_event(O._stream(dev), _events(dev)[1].cuda_event), "mot_stream_wait_event")
+    O.embed_plan_join(_PLANNERS[dev.index], dev)
+
+
+def _bwd_workspace(ws: Tensor, desc, dev) -> Tuple[Tensor, bool]:
+    """-> (workspace, plan_ready): the forward's planned workspace (left clean by the plan), else a fresh one."""
+    if ws.numel() > 0:
+        return ws, True
+    return torch.empty(O.embed_workspace_bytes(desc), dtype=torch.uint8, device=dev), False
 
 
 def _empty(dev, dtype=torch.uint8) -> Tensor:
@@ -104,21 +94,13 @@ def _empty(dev, dtype=torch.uint8) -> Tensor:
 # ---------------------------------------------------------------------------------------------------------------
 # mot_b200::embed  (fused gather + pool + combine + norm; every variant without a dense projection)
 # ---------------------------------------------------------------------------------------------------------------
-def _embed_desc(tok, ids, ttb, E_tok, E_byte, lam, spec, bpt, seq_len, eps):
-    from . import ops as O
-    sp = unpack_spec(spec, eps)
-    n = tok.numel() if tok is not None else ids.numel() // bpt
-    desc = O.make_desc(sp, n, E_tok, E_byte, bpt, ids=ids, ttb=ttb, has_lam=lam is not None, seq_len=seq_len)
-    return desc, n, (E_tok if E_tok is not None else E_byte)
-
-
 @torch.library.custom_op("mot_b200::embed", mutates_args=(), device_types="cuda")
 def embed_op(tok: Optional[Tensor], ids: Optional[Tensor], ttb: Optional[Tensor], E_tok: Optional[Tensor],
              E_byte: Optional[Tensor], lam: Optional[Tensor], spec: int, bpt: int, seq_len: int, eps: float,
              plan: bool) -> Tuple[Tensor, Tensor, Tensor]:
     """-> (out [n, out_dim], rstd [n] fp32 or [0], workspace uint8 or [0])."""
-    from . import ops as O
-    desc, n, ref = _embed_desc(tok, ids, ttb, E_tok, E_byte, lam, spec, bpt, seq_len, eps)
+    desc = O._embed_desc(unpack_spec(spec, eps), bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None)
+    n, ref = desc.n_tokens, (E_tok if E_tok is not None else E_byte)
     dev = ref.device
     out = torch.empty((n, desc.out_dim), dtype=ref.dtype, device=dev)
     planned = plan and tok is not None and n > 0
@@ -133,8 +115,8 @@ def embed_op(tok: Optional[Tensor], ids: Optional[Tensor], ttb: Optional[Tensor]
 
 @embed_op.register_fake
 def _(tok, ids, ttb, E_tok, E_byte, lam, spec, bpt, seq_len, eps, plan):
-    from . import ops as O
-    desc, n, ref = _embed_desc(tok, ids, ttb, E_tok, E_byte, lam, spec, bpt, seq_len, eps)
+    desc = O._embed_desc(unpack_spec(spec, eps), bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None)
+    n, ref = desc.n_tokens, (E_tok if E_tok is not None else E_byte)
     planned = plan and tok is not None and n > 0
     keep = plan and n > 0 and O.embed_bwd_uses_saved(desc)
     return (ref.new_empty((n, desc.out_dim)), ref.new_empty((n if keep else 0,), dtype=torch.float32),
@@ -146,17 +128,15 @@ def embed_bwd_op(grad_out: Tensor, tok: Optional[Tensor], ids: Optional[Tensor],
                  E_tok: Optional[Tensor], E_byte: Optional[Tensor], lam: Optional[Tensor], out_saved: Optional[Tensor],
                  rstd: Tensor, ws: Tensor, spec: int, bpt: int, seq_len: int, eps: float) -> Tuple[Tensor, Tensor, Tensor]:
     """-> (gE_tok dense or [0], gE_byte dense or [0], g_lam fp32 [2] or [0])."""
-    from . import ops as O
-    desc, n, ref = _embed_desc(tok, ids, ttb, E_tok, E_byte, lam, spec, bpt, seq_len, eps)
+    desc = O._embed_desc(unpack_spec(spec, eps), bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None)
+    n, ref = desc.n_tokens, (E_tok if E_tok is not None else E_byte)
     dev = ref.device
     g = grad_out.reshape(n, desc.out_dim)
     g = (g if g.dtype == ref.dtype else g.to(ref.dtype)).contiguous()
     gE_tok = torch.empty_like(E_tok) if E_tok is not None else _empty(dev, ref.dtype)
     gE_byte = torch.empty_like(E_byte) if E_byte is not None else _empty(dev, ref.dtype)
     g_lam = torch.empty(2 if lam is not None else 0, dtype=torch.float32, device=dev)
-    planned = ws.numel() > 0
-    if not planned:
-        ws = torch.empty(O.embed_workspace_bytes(desc), dtype=torch.uint8, device=dev)
+    ws, planned = _bwd_workspace(ws, desc, dev)
     keep = rstd.numel() > 0 and out_saved is not None
     O.embed_backward_out(desc, tok, ids, ttb, E_tok, E_byte, lam, g, gE_tok if E_tok is not None else None,
                          gE_byte if E_byte is not None else None, g_lam if lam is not None else None, ws,
@@ -190,56 +170,17 @@ def _embed_backward(ctx, g_out, g_rstd, g_ws):
 embed_op.register_autograd(_embed_backward, setup_context=_embed_setup)
 
 
-def embed_via_custom_op(spec, bpt, seq_len, tokens, byte_ids, ttb, E_tok, E_byte, lam):
-    """mot_b200.ops.mot_embed through torch.ops.mot_b200.embed (same argument handling as _MotEmbedFn.forward)."""
-    from . import ops as O
-    O._require_cuda(tokens, byte_ids, ttb, E_tok, E_byte, lam)
-    tok = None
-    if tokens is not None:
-        tok = tokens.reshape(-1)
-        tok = (tok if tok.dtype == torch.int32 else tok.to(torch.int32)).contiguous()
-    ids = None
-    if byte_ids is not None:
-        if byte_ids.dtype not in (torch.int32, torch.int64):
-            raise NotImplementedError("mot_b200: byte ids must be int32 or int64")
-        ids = byte_ids.contiguous()
-    n = tok.numel() if tok is not None else ids.numel() // bpt
-    if ids is not None and ids.numel() != n * bpt:
-        raise RuntimeError(f"mot_b200: byte ids have {ids.numel()} entries, expected {n}*{bpt}")
-    E_tok_c = E_tok.contiguous() if E_tok is not None else None
-    E_byte_c = E_byte.contiguous() if E_byte is not None else None
-    if E_tok_c is not None and E_byte_c is not None and E_tok_c.dtype != E_byte_c.dtype:
-        raise NotImplementedError("mot_b200: token and byte tables must share one dtype")
-    lam32 = lam.to(torch.float32).contiguous() if lam is not None else None   # differentiable cast
-    need = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (E_tok, E_byte, lam))
-    out, _, _ = torch.ops.mot_b200.embed(tok, ids, ttb.contiguous() if ttb is not None else None, E_tok_c, E_byte_c, lam32,
-                                         pack_spec(spec), bpt, seq_len, float(spec.eps), need)
-    return out
-
-
 # ---------------------------------------------------------------------------------------------------------------
 # mot_b200::tok_gather  (several tables gathered with the same token ids: the value embeddings)
 # ---------------------------------------------------------------------------------------------------------------
-def _gather_desc(tok, table):
-    from . import ops as O
-    return O.make_desc(O.MixSpec(combine="tok_only", out_norm=False), tok.numel(), table, None, 0, ids=None, ttb=None,
-                       has_lam=False)
-
-
 @torch.library.custom_op("mot_b200::tok_gather", mutates_args=(), device_types="cuda")
 def tok_gather_op(tok: Tensor, tables: List[Tensor], plan: bool) -> List[Tensor]:
     """-> [tables[0][tok], ..., tables[k-1][tok], workspace]."""
-    from . import ops as O
     dev = tok.device
-    desc = _gather_desc(tok, tables[0])
-    n = tok.numel()
-    planned = plan and n > 0
+    desc = O._gather_desc(tok, tables[0])
+    planned = plan and tok.numel() > 0
     ws = _plan_beside(desc, tok, dev) if planned else _empty(dev)
-    outs = []
-    for E in tables:
-        out = torch.empty((n, E.shape[1]), dtype=E.dtype, device=dev)
-        O.embed_forward_out(desc, tok, None, None, E, None, None, out)
-        outs.append(out)
+    outs = O._gather_forward(desc, tok, tables, dev)
     if planned:
         _rejoin(dev)
     return outs + [ws]
@@ -247,9 +188,8 @@ def tok_gather_op(tok: Tensor, tables: List[Tensor], plan: bool) -> List[Tensor]
 
 @tok_gather_op.register_fake
 def _(tok, tables, plan):
-    from . import ops as O
     n = tok.numel()
-    desc = _gather_desc(tok, tables[0])
+    desc = O._gather_desc(tok, tables[0])
     outs = [E.new_empty((n, E.shape[1])) for E in tables]
     return outs + [tok.new_empty((O.embed_workspace_bytes(desc) if plan and n > 0 else 0,), dtype=torch.uint8)]
 
@@ -258,25 +198,12 @@ def _(tok, tables, plan):
 def tok_gather_bwd_op(tok: Tensor, tables: List[Tensor], grads: List[Tensor], ws: Tensor, want_mask: int) -> List[Tensor]:
     """Dense gradients of the tables whose bit is set in want_mask ([0]-sized placeholders for the others); one sort
     plan serves every scatter."""
-    from . import ops as O
     dev = tok.device
-    desc = _gather_desc(tok, tables[0])
-    planned = ws.numel() > 0
-    if not planned:
-        ws = torch.empty(O.embed_workspace_bytes(desc), dtype=torch.uint8, device=dev)
-    clean = planned
-    outs = []
-    for i, (E, g) in enumerate(zip(tables, grads)):
-        if not (want_mask >> i) & 1:
-            outs.append(_empty(dev, E.dtype))
-            continue
-        g = g.reshape(-1, E.shape[1])
-        g = (g if g.dtype == E.dtype else g.to(E.dtype)).contiguous()
-        gE = torch.empty_like(E)
-        O.embed_backward_out(desc, tok, None, None, E, None, None, g, gE, None, None, ws, plan_ready=planned, ws_clean=clean)
-        planned, clean = True, True
-        outs.append(gE)
-    return outs
+    desc = O._gather_desc(tok, tables[0])
+    ws, planned = _bwd_workspace(ws, desc, dev)
+    want = [(want_mask >> i) & 1 for i in range(len(tables))]
+    gEs = O._gather_backward(desc, tok, tables, grads, want, ws, planned, planned)
+    return [gE if gE is not None else _empty(dev, E.dtype) for gE, E in zip(gEs, tables)]
 
 
 @tok_gather_bwd_op.register_fake
@@ -305,84 +232,30 @@ def _tok_gather_backward(ctx, grads):
 tok_gather_op.register_autograd(_tok_gather_backward, setup_context=_tok_gather_setup)
 
 
-def tok_gather_via_custom_op(tokens, tables):
-    from . import ops as O
-    O._require_cuda(tokens, *tables)
-    if not tables:
-        raise RuntimeError("mot_b200.tok_gather: need at least one table")
-    shape, dtype = tables[0].shape, tables[0].dtype
-    for E in tables:
-        if E.shape != shape or E.dtype != dtype or E.dim() != 2:
-            raise NotImplementedError("mot_b200.tok_gather: tables must share one [V, D] shape and dtype")
-    tok = tokens.reshape(-1)
-    tok = (tok if tok.dtype == torch.int32 else tok.to(torch.int32)).contiguous()
-    need = torch.is_grad_enabled() and any(E.requires_grad for E in tables)
-    res = torch.ops.mot_b200.tok_gather(tok, [E.contiguous() for E in tables], need)
-    return tuple(res[:-1])
-
-
 # ---------------------------------------------------------------------------------------------------------------
 # mot_b200::embed_proj  (concat + dense projection variants, tcgen05)
 # ---------------------------------------------------------------------------------------------------------------
-def _proj_descs(spec_code, eps, bpt, tok, ids, E_tok, E_byte, pair: bool):
-    import dataclasses
-    from . import ops as O
-    spec = unpack_spec(spec_code, eps)
-    n = tok.numel()
-    if pair:
-        K = E_tok.shape[1] + bpt * E_byte.shape[1]
-        desc = O.make_desc(O.MixSpec(combine="tok_only", tok_norm=spec.tok_norm, out_norm=False, eps=spec.eps), n, E_tok,
-                           None, 0, ids=None, ttb=None, has_lam=False, row_stride=K, col_offset=0)
-    else:
-        desc = O.make_desc(dataclasses.replace(spec, combine="concat", out_norm=False), n, E_tok, E_byte, bpt, ids=ids,
-                           ttb=None, has_lam=False)
-        K = desc.out_dim
-    return spec, desc, K, n
-
-
-def _gather_operand(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, A) -> None:
-    from . import ops as O
-    if ids2 is None:
-        O.embed_forward_out(desc, tok, ids, None, E_tok, E_byte, None, A)
-    elif tok.numel() > 0:
-        O.embed_forward_out(desc, tok, None, None, E_tok, None, None, A)
-        O.byte_pair_forward_out(ids, ids2, bpt, E_byte, A, E_tok.shape[1], spec.eps)
-
-
 @torch.library.custom_op("mot_b200::embed_proj", mutates_args=(), device_types="cuda")
 def embed_proj_op(tok: Tensor, ids: Tensor, ids2: Optional[Tensor], E_tok: Tensor, E_byte: Tensor, W: Tensor,
                   bias: Optional[Tensor], spec: int, bpt: int, eps: float, plan: bool) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
     """-> (out [n, Do], Y = the product before the row norm or [0], W in the compute dtype or [0], workspace or [0])."""
-    from . import ops as O
-    dev = E_tok.device
-    cdt = E_tok.dtype
-    sp, desc, K, n = _proj_descs(spec, eps, bpt, tok, ids, E_tok, E_byte, ids2 is not None)
-    Do = W.shape[0]
+    dev, cdt = E_tok.device, E_tok.dtype
+    sp = unpack_spec(spec, eps)
+    desc = O._proj_desc(sp, bpt, tok, ids, E_tok, E_byte, ids2 is not None)
     w_c = W if W.dtype == cdt else O.cast_out(W, cdt)
-    planned = plan and n > 0
+    planned = plan and tok.numel() > 0
     ws = _plan_beside(desc, tok, dev) if planned else _empty(dev)
-    A = torch.empty((n, K), dtype=cdt, device=dev)
-    _gather_operand(sp, desc, bpt, tok, ids, ids2, E_tok, E_byte, A)
-    Y = torch.empty((n, Do), dtype=cdt, device=dev)
-    if bias is not None and bias.dtype != torch.float32:
-        raise NotImplementedError("mot_b200: the projection bias must be fp32 (mathblations/model.py:261)")
-    O.linear_forward_out(A, w_c, Y, bias.contiguous() if bias is not None else None)
-    del A
-    if sp.out_norm:
-        out = torch.empty_like(Y)
-        O.rmsnorm_forward_out(Y, out, sp.eps)
-    else:
-        out, Y = Y, _empty(dev, cdt)
+    out, Y, _ = O._proj_forward(sp, desc, bpt, tok, ids, ids2, E_tok, E_byte, w_c, bias, False)
     if planned:
         _rejoin(dev)
-    return out, Y, (w_c if w_c is not W else _empty(dev, cdt)), ws
+    return out, (Y if sp.out_norm else _empty(dev, cdt)), (w_c if w_c is not W else _empty(dev, cdt)), ws
 
 
 @embed_proj_op.register_fake
 def _(tok, ids, ids2, E_tok, E_byte, W, bias, spec, bpt, eps, plan):
-    from . import ops as O
-    sp, desc, K, n = _proj_descs(spec, eps, bpt, tok, ids, E_tok, E_byte, ids2 is not None)
-    cdt = E_tok.dtype
+    sp = unpack_spec(spec, eps)
+    desc = O._proj_desc(sp, bpt, tok, ids, E_tok, E_byte, ids2 is not None)
+    n, cdt = tok.numel(), E_tok.dtype
     out = E_tok.new_empty((n, W.shape[0]))
     Y = E_tok.new_empty((n, W.shape[0]) if sp.out_norm else (0,))
     w_c = E_tok.new_empty(tuple(W.shape) if W.dtype != cdt else (0,))
@@ -394,40 +267,14 @@ def embed_proj_bwd_op(grad_out: Tensor, tok: Tensor, ids: Tensor, ids2: Optional
                       W: Tensor, w_c: Tensor, Y: Tensor, ws: Tensor, spec: int, bpt: int, eps: float,
                       has_bias: bool) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
     """-> (gE_tok, gE_byte, gW in W's dtype, g_bias fp32 [Do] or [0])."""
-    from . import ops as O
     dev = E_tok.device
-    cdt = E_tok.dtype
-    sp, desc, K, n = _proj_descs(spec, eps, bpt, tok, ids, E_tok, E_byte, ids2 is not None)
-    Do = W.shape[0]
-    w_use = w_c if w_c.numel() > 0 else W
-    g = grad_out.reshape(n, Do)
-    g = (g if g.dtype == cdt else g.to(cdt)).contiguous()
-    if sp.out_norm:
-        dY = torch.empty_like(g)
-        O.rmsnorm_backward_out(Y, g, dY, sp.eps)
-    else:
-        dY = g
-    g_bias = O.colsum_out(dY) if has_bias else _empty(dev, torch.float32)
-    A = torch.empty((n, K), dtype=cdt, device=dev)
-    _gather_operand(sp, desc, bpt, tok, ids, ids2, E_tok, E_byte, A)      # gathered again, not kept
-    dW32 = torch.empty((Do, K), dtype=torch.float32, device=dev)
-    dW16 = torch.empty((Do, K), dtype=torch.bfloat16, device=dev) if W.dtype == torch.bfloat16 else None
-    O.linear_bwd_weight_out(dY, A, dW32, dW16)
-    dA = A
-    O.linear_bwd_input_out(dY, w_use, dA)
-    gE_tok, gE_byte = torch.empty_like(E_tok), torch.empty_like(E_byte)
-    planned = ws.numel() > 0
-    if not planned:
-        ws = torch.empty(O.embed_workspace_bytes(desc), dtype=torch.uint8, device=dev)
-    if ids2 is None:
-        O.embed_backward_out(desc, tok, ids, None, E_tok, E_byte, None, dA, gE_tok, gE_byte, None, ws,
-                             plan_ready=planned, ws_clean=planned)
-    else:
-        O.embed_backward_out(desc, tok, None, None, E_tok, None, None, dA, gE_tok, None, None, ws,
-                             plan_ready=planned, ws_clean=planned)
-        O.byte_pair_backward_out(ids, ids2, bpt, E_byte, dA, E_tok.shape[1], gE_byte, sp.eps)
-    gW = dW16 if dW16 is not None else dW32
-    return gE_tok, gE_byte, gW, g_bias
+    sp = unpack_spec(spec, eps)
+    desc = O._proj_desc(sp, bpt, tok, ids, E_tok, E_byte, ids2 is not None)
+    dA, gW, g_bias = O._proj_backward(sp, desc, bpt, tok, ids, ids2, E_tok, E_byte, w_c if w_c.numel() > 0 else W,
+                                      W.dtype, has_bias, Y, None, grad_out)    # the operand is gathered again, not kept
+    ws, planned = _bwd_workspace(ws, desc, dev)
+    gE_tok, gE_byte = O._scatter_operand(sp, desc, bpt, tok, ids, ids2, E_tok, E_byte, dA, ws, planned, planned)
+    return gE_tok, gE_byte, gW, (g_bias if has_bias else _empty(dev, torch.float32))
 
 
 @embed_proj_bwd_op.register_fake
@@ -453,69 +300,19 @@ def _proj_backward(ctx, g_out, g_Y, g_wc, g_ws):
 embed_proj_op.register_autograd(_proj_backward, setup_context=_proj_setup)
 
 
-def proj_via_custom_op(spec, bpt, tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2):
-    from . import ops as O
-    O._require_cuda(tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2)
-    cdt = E_tok.dtype
-    if cdt not in (torch.bfloat16, torch.float32) or E_byte.dtype != cdt:
-        raise NotImplementedError("mot_b200: token and byte tables must both be bf16 or both fp32")
-    tok = tokens.reshape(-1)
-    tok = (tok if tok.dtype == torch.int32 else tok.to(torch.int32)).contiguous()
-    if byte_ids.dtype not in (torch.int32, torch.int64):
-        raise NotImplementedError("mot_b200: byte ids must be int32 or int64")
-    ids = byte_ids.contiguous()
-    n = tok.numel()
-    if ids.numel() != n * bpt:
-        raise RuntimeError(f"mot_b200: byte ids have {ids.numel()} entries, expected {n}*{bpt}")
-    ids2 = None
-    if byte_ids2 is not None:
-        if not spec.byte_norm or spec.slot_major or spec.bytes_first:
-            raise NotImplementedError("mot_b200: the padded+pulled sum exists only with per-byte norms, token-major "
-                                      "ids and [tok | bytes] order (spt/train_gpt.py:371-379,442-443)")
-        ids2 = byte_ids2.contiguous()
-        if ids2.dtype != ids.dtype or ids2.numel() != ids.numel():
-            raise RuntimeError("mot_b200: the two byte-id tensors must share dtype and size")
-    K = E_tok.shape[1] + bpt * E_byte.shape[1]
-    if W.shape[1] != K:
-        raise RuntimeError(f"mot_b200: projection weight is {tuple(W.shape)}, expected [{W.shape[0]}, {K}]")
-    need = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (E_tok, E_byte, W, bias))
-    out, _, _, _ = torch.ops.mot_b200.embed_proj(tok, ids, ids2, E_tok.contiguous(), E_byte.contiguous(), W.contiguous(),
-                                                 bias, pack_spec(spec), bpt, float(spec.eps), need)
-    return out
-
-
 # ---------------------------------------------------------------------------------------------------------------
 # mot_b200::embed_byte_fc  (runs/71051: norm(tok + F.linear(cat(bytes), byte_fc)))
 # ---------------------------------------------------------------------------------------------------------------
-def _fc_descs(spec_b_code, eps, bpt, tok, ids, E_tok, E_byte):
-    from . import ops as O
-    n = tok.numel()
-    spec_b = unpack_spec(spec_b_code, eps)
-    desc_b = O.make_desc(spec_b, n, None, E_byte, bpt, ids=ids, ttb=None, has_lam=False)
-    desc_t = O.make_desc(O.MixSpec(combine="tok_only", out_norm=True, eps=eps), n, E_tok, None, 0, ids=None, ttb=None,
-                         has_lam=False)
-    return desc_b, desc_t, n
-
-
 @torch.library.custom_op("mot_b200::embed_byte_fc", mutates_args=(), device_types="cuda")
 def embed_byte_fc_op(tok: Tensor, ids: Tensor, E_tok: Tensor, E_byte: Tensor, W: Tensor, spec_b: int, bpt: int, eps: float,
                      plan: bool) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
     """-> (out [n, D], Y = the byte-FC product, W in the compute dtype or [0], workspace or [0])."""
-    from . import ops as O
     dev, cdt = E_tok.device, E_tok.dtype
-    desc_b, desc_t, n = _fc_descs(spec_b, eps, bpt, tok, ids, E_tok, E_byte)
-    D = E_tok.shape[1]
+    desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, tok, ids, E_tok, E_byte)
     w_c = W if W.dtype == cdt else O.cast_out(W, cdt)
-    planned = plan and n > 0
+    planned = plan and tok.numel() > 0
     ws = _plan_beside(desc_t, tok, dev) if planned else _empty(dev)
-    C = torch.empty((n, D), dtype=cdt, device=dev)
-    O.embed_forward_out(desc_b, None, ids, None, None, E_byte, None, C)
-    Y = torch.empty((n, D), dtype=cdt, device=dev)
-    O.linear_forward_out(C, w_c, Y)
-    del C
-    out = torch.empty((n, D), dtype=cdt, device=dev)
-    if n > 0:
-        O.embed_forward_out(desc_t, tok, None, None, E_tok, None, None, out, addend=Y)
+    out, Y = O._byte_fc_forward(desc_b, desc_t, tok, ids, E_tok, E_byte, w_c)
     if planned:
         _rejoin(dev)
     return out, Y, (w_c if w_c is not W else _empty(dev, cdt)), ws
@@ -523,9 +320,8 @@ def embed_byte_fc_op(tok: Tensor, ids: Tensor, E_tok: Tensor, E_byte: Tensor, W:
 
 @embed_byte_fc_op.register_fake
 def _(tok, ids, E_tok, E_byte, W, spec_b, bpt, eps, plan):
-    from . import ops as O
-    desc_b, desc_t, n = _fc_descs(spec_b, eps, bpt, tok, ids, E_tok, E_byte)
-    D = E_tok.shape[1]
+    desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, tok, ids, E_tok, E_byte)
+    n, D = tok.numel(), E_tok.shape[1]
     return (E_tok.new_empty((n, D)), E_tok.new_empty((n, D)), E_tok.new_empty(tuple(W.shape) if W.dtype != E_tok.dtype else (0,)),
             E_tok.new_empty((O.embed_workspace_bytes(desc_t) if plan and n > 0 else 0,), dtype=torch.uint8))
 
@@ -533,31 +329,12 @@ def _(tok, ids, E_tok, E_byte, W, spec_b, bpt, eps, plan):
 @torch.library.custom_op("mot_b200::embed_byte_fc_bwd", mutates_args=(), device_types="cuda")
 def embed_byte_fc_bwd_op(grad_out: Tensor, tok: Tensor, ids: Tensor, E_tok: Tensor, E_byte: Tensor, W: Tensor, w_c: Tensor,
                          Y: Tensor, ws: Tensor, spec_b: int, bpt: int, eps: float) -> Tuple[Tensor, Tensor, Tensor]:
-    from . import ops as O
-    dev, cdt = E_tok.device, E_tok.dtype
-    desc_b, desc_t, n = _fc_descs(spec_b, eps, bpt, tok, ids, E_tok, E_byte)
-    D = E_tok.shape[1]
-    w_use = w_c if w_c.numel() > 0 else W
-    g = grad_out.reshape(n, D)
-    g = (g if g.dtype == cdt else g.to(cdt)).contiguous()
-    gE_tok, gE_byte = torch.empty_like(E_tok), torch.empty_like(E_byte)
-    dY = torch.empty_like(Y)
-    planned = ws.numel() > 0
-    if not planned:
-        ws = torch.empty(O.embed_workspace_bytes(desc_t), dtype=torch.uint8, device=dev)
-    O.embed_backward_out(desc_t, tok, None, None, E_tok, None, None, g, gE_tok, None, None, ws, plan_ready=planned,
-                         ws_clean=planned, addend=Y, d_addend=dY)
-    C = torch.empty((n, D), dtype=cdt, device=dev)
-    O.embed_forward_out(desc_b, None, ids, None, None, E_byte, None, C)            # gathered again, not kept
-    dW32 = torch.empty((D, D), dtype=torch.float32, device=dev)
-    dW16 = torch.empty((D, D), dtype=torch.bfloat16, device=dev) if W.dtype == torch.bfloat16 else None
-    O.linear_bwd_weight_out(dY, C, dW32, dW16)
-    O.linear_bwd_input_out(dY, w_use, C)
+    dev = E_tok.device
+    desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, tok, ids, E_tok, E_byte)
+    ws, planned = _bwd_workspace(ws, desc_t, dev)
     wsb = torch.empty(O.embed_workspace_bytes(desc_b), dtype=torch.uint8, device=dev)
-    O.embed_backward_out(desc_b, None, ids, None, None, E_byte, None, C, None, gE_byte, None, wsb, plan_ready=False,
-                         ws_clean=False)
-    gW = dW16 if dW16 is not None else dW32
-    return gE_tok, gE_byte, gW
+    return O._byte_fc_backward(desc_b, desc_t, tok, ids, E_tok, E_byte, w_c if w_c.numel() > 0 else W, W.dtype, Y,
+                               grad_out, ws, planned, planned, wsb, False)
 
 
 @embed_byte_fc_bwd_op.register_fake
@@ -581,33 +358,12 @@ def _fc_backward(ctx, g_out, g_Y, g_wc, g_ws):
 embed_byte_fc_op.register_autograd(_fc_backward, setup_context=_fc_setup)
 
 
-def byte_fc_via_custom_op(spec_b, bpt, eps, tokens, byte_ids, E_tok, E_byte, W):
-    from . import ops as O
-    O._require_cuda(tokens, byte_ids, E_tok, E_byte, W)
-    cdt = E_tok.dtype
-    if cdt not in (torch.bfloat16, torch.float32) or E_byte.dtype != cdt:
-        raise NotImplementedError("mot_b200: token and byte tables must both be bf16 or both fp32")
-    tok = tokens.reshape(-1)
-    tok = (tok if tok.dtype == torch.int32 else tok.to(torch.int32)).contiguous()
-    if byte_ids.dtype not in (torch.int32, torch.int64):
-        raise NotImplementedError("mot_b200: byte ids must be int32 or int64")
-    ids = byte_ids.contiguous()
-    n, D = tok.numel(), E_tok.shape[1]
-    if ids.numel() != n * bpt or bpt * E_byte.shape[1] != D or tuple(W.shape) != (D, D):
-        raise RuntimeError("mot_b200: byte-FC mix needs bpt*byte_dim == token_dim and a square [D, D] weight")
-    need = torch.is_grad_enabled() and any(t.requires_grad for t in (E_tok, E_byte, W))
-    out, _, _, _ = torch.ops.mot_b200.embed_byte_fc(tok, ids, E_tok.contiguous(), E_byte.contiguous(), W.contiguous(),
-                                                    pack_spec(spec_b), bpt, float(eps), need)
-    return out
-
-
 # ---------------------------------------------------------------------------------------------------------------
 # integer half and the output-side expand
 # ---------------------------------------------------------------------------------------------------------------
 @torch.library.custom_op("mot_b200::ttb_expand", mutates_args=(), device_types="cuda")
 def ttb_expand_op(tok: Tensor, ttb: Tensor, out_i64: bool) -> Tensor:
     """-> [n, bpt] int64 / int32 (tokens_to_bytes, spt/data_creation.py:61-67)."""
-    from . import ops as O
     return O._ttb_expand_impl(tok, ttb, torch.int64 if out_i64 else torch.int32)
 
 
@@ -618,7 +374,6 @@ def _(tok, ttb, out_i64):
 
 @torch.library.custom_op("mot_b200::pull", mutates_args=(), device_types="cuda")
 def pull_op(byte_tensor: Tensor, bpt: int, pad_byte: int, eot_byte: int, from_right: bool) -> Tensor:
-    from . import ops as O
     return O._pull_impl(byte_tensor, bpt, pad_byte, eot_byte, from_right)
 
 
@@ -629,7 +384,6 @@ def _(byte_tensor, bpt, pad_byte, eot_byte, from_right):
 
 @torch.library.custom_op("mot_b200::tokens_to_digits", mutates_args=(), device_types="cuda")
 def tokens_to_digits_op(tok: Tensor, dpt: int, op_token: int, eq_token: int, pad_token: int, out_i64: bool) -> Tensor:
-    from . import ops as O
     return O._tokens_to_digits_impl(tok, dpt, op_token, eq_token, pad_token, torch.int64 if out_i64 else torch.int32)
 
 
@@ -641,7 +395,6 @@ def _(tok, dpt, op_token, eq_token, pad_token, out_i64):
 @torch.library.custom_op("mot_b200::mixout_copy", mutates_args=(), device_types="cuda")
 def mixout_copy_op(x: Tensor, bpt: int) -> Tensor:
     """[rows, D] -> [rows*bpt, D]: every row repeated bpt times (ByteMixoutCopy, spt/train_gpt.py:493)."""
-    from . import ops as O
     return O._mixout_copy_impl(x, bpt, backward=False)
 
 
@@ -652,7 +405,6 @@ def _(x, bpt):
 
 @torch.library.custom_op("mot_b200::mixout_copy_bwd", mutates_args=(), device_types="cuda")
 def mixout_copy_bwd_op(grad_y: Tensor, bpt: int) -> Tensor:
-    from . import ops as O
     return O._mixout_copy_impl(grad_y, bpt, backward=True)
 
 

@@ -325,6 +325,11 @@ class Workspace:
             self.clean = False
         return self.buf
 
+    def take_clean(self) -> bool:
+        """Whether the head of buf is zero; the buffer counts as dirty until a completed backward marks it clean."""
+        clean, self.clean = self.clean, False
+        return clean
+
     def __del__(self):   # dropped with a plan in flight (forward without backward): keep the allocator off the buffer
         try:
             if self.pending and self.buf is not None:
@@ -366,7 +371,7 @@ def side_stream(dev) -> torch.cuda.Stream:
 def embed_plan_async(desc: L.MotDesc, tok, ws: Workspace, dev, stream: Optional[int] = None) -> None:
     """mot_embed_plan_async: fork from the current stream, run the plan on the side stream, record ws.ev_join.  The
     backward waits for it with embed_plan_join()."""
-    clean, ws.clean = ws.clean, False
+    clean = ws.take_clean()
     with _on_device(dev):
         rc = L.lib().mot_embed_plan_async(desc, _ptr(tok), _ptr(ws.buf), ws.buf.numel(), L.WS_CLEAN if clean else 0,
                                           _stream(dev) if stream is None else stream, side_stream(dev).cuda_stream,
@@ -388,31 +393,84 @@ def embed_plan_join(ws: Workspace, dev, stream: Optional[int] = None) -> None:
     ws.pending = False
 
 
+def _planned_workspace(desc: L.MotDesc, tok, dev, stream: Optional[int] = None) -> Workspace:
+    """A pooled workspace with the backward's sort plan of `tok` started on the side stream, beside the forward."""
+    ws = acquire_workspace(desc, dev)
+    embed_plan_async(desc, tok, ws, dev, stream)
+    return ws
+
+
+def _take_workspace(ws: Optional[Workspace], desc: L.MotDesc, dev, stream: Optional[int] = None):
+    """The workspace of an eager backward -> (ws, plan_ready, ws_clean): the one its forward planned in (joined here
+    unless a captured forward joined at its own end), else one from the pool.  Hand it back with _return_workspace."""
+    if ws is None:
+        ws = acquire_workspace(desc, dev)
+        return ws, False, ws.take_clean()
+    if ws.pending:
+        embed_plan_join(ws, dev, stream)
+    return ws, True, True     # the plan ran on a clean (or freshly cleared) workspace and leaves it clean
+
+
+def _return_workspace(ws: Workspace) -> None:
+    ws.clean = True           # every completed backward leaves the head of the workspace zeroed
+    release_workspace(ws)
+
+
+# ------------------------------------------------------------------------------------------------------------
+# argument checks shared by both dispatch paths (autograd.Function and torch.ops.mot_b200)
+# ------------------------------------------------------------------------------------------------------------
+def _tok_i32(tokens: torch.Tensor) -> torch.Tensor:
+    """Token ids as the kernels read them: flat, contiguous int32."""
+    tok = tokens.reshape(-1)
+    return (tok if tok.dtype == torch.int32 else tok.to(torch.int32)).contiguous()
+
+
+def _byte_ids(byte_ids: torch.Tensor) -> torch.Tensor:
+    if byte_ids.dtype not in (torch.int32, torch.int64):
+        raise NotImplementedError("mot_b200: byte ids must be int32 or int64")
+    return byte_ids.contiguous()
+
+
+def _check_id_count(ids: torch.Tensor, n: int, bpt: int) -> None:
+    if ids.numel() != n * bpt:
+        raise RuntimeError(f"mot_b200: byte ids have {ids.numel()} entries, expected {n}*{bpt}")
+
+
+def _require_chain_dtype(E_tok: torch.Tensor, E_byte: torch.Tensor) -> None:
+    """The projection chains compute in the table dtype: bf16, or fp32 on the TF32 tensor-core path."""
+    if E_tok.dtype not in (torch.bfloat16, torch.float32) or E_byte.dtype != E_tok.dtype:
+        raise NotImplementedError("mot_b200: token and byte tables must both be bf16 or both fp32")
+
+
+def _embed_args(bpt: int, tokens, byte_ids, ttb, E_tok, E_byte, lam):
+    """mot_embed's arguments checked and normalised -> (dev, tok, ids, E_tok, E_byte)."""
+    dev = _require_cuda(tokens, byte_ids, ttb, E_tok, E_byte, lam)
+    tok = _tok_i32(tokens) if tokens is not None else None
+    ids = None
+    if byte_ids is not None:
+        ids = _byte_ids(byte_ids)
+        _check_id_count(ids, tok.numel() if tok is not None else ids.numel() // bpt, bpt)
+    E_tok = E_tok.contiguous() if E_tok is not None else None
+    E_byte = E_byte.contiguous() if E_byte is not None else None
+    if E_tok is not None and E_byte is not None and E_tok.dtype != E_byte.dtype:
+        raise NotImplementedError("mot_b200: token and byte tables must share one dtype")
+    return dev, tok, ids, E_tok, E_byte
+
+
+def _embed_desc(spec: MixSpec, bpt: int, seq_len: int, tok, ids, ttb, E_tok, E_byte, has_lam: bool,
+                dp_slabs: int = 0) -> L.MotDesc:
+    n = tok.numel() if tok is not None else ids.numel() // bpt
+    return make_desc(spec, n, E_tok, E_byte, bpt, ids=ids, ttb=ttb, has_lam=has_lam, seq_len=seq_len, dp_slabs=dp_slabs)
+
+
 class _MotEmbedFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, spec: MixSpec, bpt: int, seq_len: int, tokens, byte_ids, ttb, E_tok, E_byte, lam, grad_bufs=None):
-        dev = _require_cuda(tokens, byte_ids, ttb, E_tok, E_byte, lam)
+    def forward(ctx, spec: MixSpec, bpt: int, seq_len: int, dev, tok, ids, ttb, E_tok, E_byte, lam, grad_bufs=None):
         # optional ((param_tok, view_tok), (param_byte, view_byte)): views of a dp.GradBucket that become param.grad
         ctx.grad_bufs = grad_bufs
-        tok = None
-        if tokens is not None:
-            tok = tokens.reshape(-1)
-            tok = tok if tok.dtype == torch.int32 else tok.to(torch.int32)
-            tok = tok.contiguous()
-        ids = None
-        if byte_ids is not None:
-            if byte_ids.dtype not in (torch.int32, torch.int64):
-                raise NotImplementedError("mot_b200: byte ids must be int32 or int64")
-            ids = byte_ids.contiguous()
-        n = tok.numel() if tok is not None else ids.numel() // bpt
-        if ids is not None and ids.numel() != n * bpt:
-            raise RuntimeError(f"mot_b200: byte ids have {ids.numel()} entries, expected {n}*{bpt}")
-        E_tok_c = E_tok.contiguous() if E_tok is not None else None
-        E_byte_c = E_byte.contiguous() if E_byte is not None else None
-        if E_tok_c is not None and E_byte_c is not None and E_tok_c.dtype != E_byte_c.dtype:
-            raise NotImplementedError("mot_b200: token and byte tables must share one dtype")
         lam_c = lam.detach().to(torch.float32).contiguous() if lam is not None else None
-        desc = make_desc(spec, n, E_tok_c, E_byte_c, bpt, ids=ids, ttb=ttb, has_lam=lam is not None, seq_len=seq_len)
+        desc = _embed_desc(spec, bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None)
+        n = desc.n_tokens
         # data-parallel pipeline: a bucket that holds exactly [token table | byte table] in symmetric memory lets the
         # backward run as vocabulary slabs with the exchange of slab k beside the backward of slab k + 1
         ctx.dp_bucket = None
@@ -420,26 +478,22 @@ class _MotEmbedFn(torch.autograd.Function):
         if bucket is not None and bucket.pipelined and n > 0 and E_tok is not None and E_byte is not None \
                 and len(bucket.params) == 2 and bucket.params[0] is grad_bufs[0][0] and bucket.params[1] is grad_bufs[1][0] \
                 and bool(L.lib().mot_embed_bwd_uses_saved(desc)):
-            desc = make_desc(spec, n, E_tok_c, E_byte_c, bpt, ids=ids, ttb=ttb, has_lam=lam is not None, seq_len=seq_len,
-                             dp_slabs=bucket.n_slabs)
+            desc = _embed_desc(spec, bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None, dp_slabs=bucket.n_slabs)
             ctx.dp_bucket = bucket
-        ref = E_tok_c if E_tok_c is not None else E_byte_c
+        ref = E_tok if E_tok is not None else E_byte
         out = torch.empty((n, desc.out_dim), dtype=ref.dtype, device=dev)
         # the backward needs the positions grouped by token id: start that sort now, beside the forward kernel
-        ctx.ws = None
         st = _stream(dev)
-        needs_grad = any(ctx.needs_input_grad[6:9])   # E_tok, E_byte, lam
-        if needs_grad and tok is not None and n > 0:
-            ctx.ws = acquire_workspace(desc, dev)
-            embed_plan_async(desc, tok, ctx.ws, dev, st)
+        needs_grad = any(ctx.needs_input_grad[7:10])   # E_tok, E_byte, lam
+        ctx.ws = _planned_workspace(desc, tok, dev, st) if needs_grad and tok is not None and n > 0 else None
         # MoT-sum (runs/71): keep what rms_norm's autograd node keeps (its result and rstd); the backward then reads two
         # rows per occurrence instead of rebuilding the mixed row (mot_embed_bwd_ex)
         keep = needs_grad and n > 0 and bool(L.lib().mot_embed_bwd_uses_saved(desc))
         rstd = torch.empty(n, dtype=torch.float32, device=dev) if keep else None
-        embed_forward_out(desc, tok, ids, ttb, E_tok_c, E_byte_c, lam_c, out, st, rstd=rstd)
+        embed_forward_out(desc, tok, ids, ttb, E_tok, E_byte, lam_c, out, st, rstd=rstd)
         embed_plan_join_if_capturing(ctx.ws, dev, st)
         ctx.desc, ctx.dev = desc, dev
-        saved = (tok, ids, ttb, E_tok_c, E_byte_c, lam_c, out if keep else None, rstd)
+        saved = (tok, ids, ttb, E_tok, E_byte, lam_c, out if keep else None, rstd)
         ctx.save_for_backward(*[t if t is not None else _ABSENT for t in saved])
         ctx.present = [t is not None for t in saved]
         ctx.lam_dtype = lam.dtype if lam is not None else None
@@ -470,15 +524,7 @@ class _MotEmbedFn(torch.autograd.Function):
         gE_byte = direct[1][1] if direct[1] is not None else (torch.empty_like(E_byte) if E_byte is not None else None)
         g_lam = torch.empty(2, dtype=torch.float32, device=dev) if lam is not None else None
         st = _stream(dev)
-        ws, planned = ctx.ws, ctx.ws is not None
-        if ws is None:
-            ws = acquire_workspace(desc, dev)
-        if planned:
-            if ws.pending:        # not yet joined (a captured forward joins at its own end)
-                embed_plan_join(ws, dev, st)
-            clean = True          # the plan ran on a clean (or freshly cleared) workspace and leaves it clean
-        else:
-            clean, ws.clean = ws.clean, False
+        ws, planned, clean = _take_workspace(ctx.ws, desc, dev, st)
         bucket = ctx.dp_bucket
         if bucket is not None and direct[0] is not None and direct[1] is not None and out_saved is not None \
                 and not torch.cuda.is_current_stream_capturing():
@@ -495,20 +541,19 @@ class _MotEmbedFn(torch.autograd.Function):
             embed_backward_out(desc, tok, ids, ttb, E_tok, E_byte, lam, g, gE_tok, gE_byte, g_lam, ws.buf,
                                plan_ready=planned, ws_clean=clean, stream=st, out_saved=out_saved, rstd=rstd,
                                plan_joined=planned)
-        ws.clean = True           # every completed backward leaves the head of the workspace zeroed
         if ctx.grad_bufs is not None and len(ctx.grad_bufs) > 2 and direct[0] is not None and tok is not None:
             bk = ctx.grad_bufs[2]
             if bk is not None and bk.sparse_rows and bk.params[0] is direct[0][0] and not bk._pending:
                 bk.mark_rows(desc, ws.buf)      # the rows this batch gathered: the exchange moves only the union
         ctx.ws = None
-        release_workspace(ws)
+        _return_workspace(ws)
         if g_lam is not None:
             g_lam = g_lam.to(ctx.lam_dtype)
         if direct[0] is not None:
             direct[0][0].grad, gE_tok = gE_tok, None
         if direct[1] is not None:
             direct[1][0].grad, gE_byte = gE_byte, None
-        return None, None, None, None, None, None, gE_tok, gE_byte, g_lam, None
+        return None, None, None, None, None, None, None, gE_tok, gE_byte, g_lam, None
 
 
 def mot_embed(tokens: Optional[torch.Tensor], byte_ids: Optional[torch.Tensor], E_tok: Optional[torch.Tensor],
@@ -521,86 +566,100 @@ def mot_embed(tokens: Optional[torch.Tensor], byte_ids: Optional[torch.Tensor], 
     inside the kernel.  lam = float tensor [2] = (lam_tok, lam_byte) or None.  grad_bufs = optional
     ((param, view), (param, view)) pairs for the token / byte table: the backward writes the dense gradient into `view`
     (a slice of a dp.GradBucket) and installs it as `param.grad`."""
+    dev, tok, ids, E_tok_c, E_byte_c = _embed_args(bpt, tokens, byte_ids, ttb, E_tok, E_byte, lam)
     if grad_bufs is None and _custom_ops_wanted():
-        return _embed_via_custom_op(spec, bpt, seq_len, tokens, byte_ids, ttb, E_tok, E_byte, lam)
-    return _MotEmbedFn.apply(spec, bpt, seq_len, tokens, byte_ids, ttb, E_tok, E_byte, lam, grad_bufs)
+        lam32 = lam.to(torch.float32).contiguous() if lam is not None else None   # differentiable cast
+        need = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (E_tok, E_byte, lam))
+        return torch.ops.mot_b200.embed(tok, ids, ttb.contiguous() if ttb is not None else None, E_tok_c, E_byte_c, lam32,
+                                        pack_spec(spec), bpt, seq_len, float(spec.eps), need)[0]
+    return _MotEmbedFn.apply(spec, bpt, seq_len, dev, tok, ids, ttb, E_tok_c, E_byte_c, lam, grad_bufs)
 
 
 # ------------------------------------------------------------------------------------------------------------
 # several tables gathered with the same token ids (the value embeddings, runs/7:252,308; spt/train_gpt.py:566,600)
 # ------------------------------------------------------------------------------------------------------------
+_GATHER_SPEC = MixSpec(combine="tok_only", out_norm=False)
+
+
+def _gather_args(tokens, tables):
+    """tok_gather's arguments checked and normalised -> (dev, tok, tables)."""
+    dev = _require_cuda(tokens, *tables)
+    if not tables:
+        raise RuntimeError("mot_b200.tok_gather: need at least one table")
+    shape, dtype = tables[0].shape, tables[0].dtype
+    for E in tables:
+        if E.shape != shape or E.dtype != dtype or E.dim() != 2:
+            raise NotImplementedError("mot_b200.tok_gather: tables must share one [V, D] shape and dtype")
+    return dev, _tok_i32(tokens), [E.contiguous() for E in tables]
+
+
+def _gather_desc(tok, table) -> L.MotDesc:
+    return make_desc(_GATHER_SPEC, tok.numel(), table, None, 0, ids=None, ttb=None, has_lam=False)
+
+
+def _gather_forward(desc: L.MotDesc, tok, tables, dev, stream: Optional[int] = None):
+    outs = []
+    for E in tables:
+        out = torch.empty((tok.numel(), E.shape[1]), dtype=E.dtype, device=dev)
+        embed_forward_out(desc, tok, None, None, E, None, None, out, stream)
+        outs.append(out)
+    return outs
+
+
+def _gather_backward(desc: L.MotDesc, tok, tables, grads, want, ws_buf, plan_ready: bool, ws_clean: bool,
+                     stream: Optional[int] = None):
+    """Dense gradients of the tables whose `want` entry is true (None for the others), one scatter launch each; the
+    first one finds the plan in place or builds it, and every one leaves the accumulators zeroed."""
+    gEs = []
+    for E, g, w in zip(tables, grads, want):
+        if not w:
+            gEs.append(None)
+            continue
+        g = g.reshape(-1, E.shape[1]).to(E.dtype).contiguous()
+        gE = torch.empty_like(E)
+        embed_backward_out(desc, tok, None, None, E, None, None, g, gE, None, None, ws_buf,
+                           plan_ready=plan_ready, ws_clean=ws_clean, stream=stream)
+        plan_ready, ws_clean = True, True
+        gEs.append(gE)
+    return gEs
+
+
 class _TokGatherFn(torch.autograd.Function):
     """outs[i] = tables[i][tokens]: plain gathers (no norm) of same-shaped tables.  The backward needs the positions
     grouped by token id once for all tables: one sort plan (started beside the first forward gather), one scatter
     launch per table reusing it (MOT_WS_PLAN_READY); the dense gradients need no token rows (R = 0)."""
 
     @staticmethod
-    def forward(ctx, tokens, *tables):
-        dev = _require_cuda(tokens, *tables)
-        if not tables:
-            raise RuntimeError("mot_b200.tok_gather: need at least one table")
-        shape, dtype = tables[0].shape, tables[0].dtype
-        for E in tables:
-            if E.shape != shape or E.dtype != dtype or E.dim() != 2:
-                raise NotImplementedError("mot_b200.tok_gather: tables must share one [V, D] shape and dtype")
-        tok = tokens.reshape(-1)
-        tok = (tok if tok.dtype == torch.int32 else tok.to(torch.int32)).contiguous()
-        n = tok.numel()
-        spec = MixSpec(combine="tok_only", out_norm=False)
-        Es = [E.contiguous() for E in tables]
-        desc = make_desc(spec, n, Es[0], None, 0, ids=None, ttb=None, has_lam=False)
-        ctx.ws = None
+    def forward(ctx, dev, tok, *tables):
+        desc = _gather_desc(tok, tables[0])
         st = _stream(dev)
-        if any(ctx.needs_input_grad[1:]) and n > 0:
-            ctx.ws = acquire_workspace(desc, dev)
-            embed_plan_async(desc, tok, ctx.ws, dev, st)
-        outs = []
-        for E in Es:
-            out = torch.empty((n, shape[1]), dtype=dtype, device=dev)
-            embed_forward_out(desc, tok, None, None, E, None, None, out, st)
-            outs.append(out)
+        ctx.ws = _planned_workspace(desc, tok, dev, st) if any(ctx.needs_input_grad[2:]) and tok.numel() > 0 else None
+        outs = _gather_forward(desc, tok, tables, dev, st)
         embed_plan_join_if_capturing(ctx.ws, dev, st)
-        ctx.desc, ctx.dev, ctx.n_tables = desc, dev, len(Es)
-        ctx.save_for_backward(tok, *Es)
+        ctx.desc, ctx.dev = desc, dev
+        ctx.save_for_backward(tok, *tables)
         return tuple(outs)
 
     @staticmethod
     def backward(ctx, *grad_outs):
         tok, *Es = ctx.saved_tensors
-        desc, dev = ctx.desc, ctx.dev
-        st = _stream(dev)
-        ws, planned = ctx.ws, ctx.ws is not None
-        if ws is None:
-            ws = acquire_workspace(desc, dev)
-        if planned:
-            if ws.pending:
-                embed_plan_join(ws, dev, st)
-            clean = True
-        else:
-            clean, ws.clean = ws.clean, False
-        grads = []
-        for i, (E, g) in enumerate(zip(Es, grad_outs)):
-            if g is None or not ctx.needs_input_grad[1 + i]:
-                grads.append(None)
-                continue
-            g = g.reshape(-1, E.shape[1]).to(E.dtype).contiguous()
-            gE = torch.empty_like(E)
-            embed_backward_out(desc, tok, None, None, E, None, None, g, gE, None, None, ws.buf,
-                               plan_ready=planned, ws_clean=clean, stream=st)
-            planned, clean = True, True     # the first scatter leaves the plan in place and the accumulators zeroed
-            grads.append(gE)
-        ws.clean = True
+        st = _stream(ctx.dev)
+        ws, planned, clean = _take_workspace(ctx.ws, ctx.desc, ctx.dev, st)
+        want = [g is not None and ctx.needs_input_grad[2 + i] for i, g in enumerate(grad_outs)]
+        grads = _gather_backward(ctx.desc, tok, Es, grad_outs, want, ws.buf, planned, clean, st)
         ctx.ws = None
-        release_workspace(ws)
-        return (None, *grads)
+        _return_workspace(ws)
+        return (None, None, *grads)
 
 
 def tok_gather(tokens: torch.Tensor, *tables: torch.Tensor):
     """`[E(tokens) for E in tables]` (the value embeddings of runs/7:308 / spt/train_gpt.py:600): returns a tuple of
     [n_tokens, D] tensors; dense gradients, one token sort shared by every table."""
+    dev, tok, Es = _gather_args(tokens, tables)
     if _custom_ops_wanted():
-        return _tok_gather_via_custom_op(tokens, tables)
-    return _TokGatherFn.apply(tokens, *tables)
+        need = torch.is_grad_enabled() and any(E.requires_grad for E in tables)
+        return tuple(torch.ops.mot_b200.tok_gather(tok, Es, need)[:-1])
+    return _TokGatherFn.apply(dev, tok, *Es)
 
 
 # ------------------------------------------------------------------------------------------------------------
@@ -775,6 +834,109 @@ def mixout_split(x: torch.Tensor, bytes_per_token: int) -> torch.Tensor:
 _PROJ_KEEP_OPERAND = not __import__("os").environ.get("MOT_PROJ_REGATHER")
 
 
+def _proj_args(spec: MixSpec, bpt: int, tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2):
+    """mot_embed_proj's arguments checked and normalised -> (dev, tok, ids, ids2, E_tok, E_byte)."""
+    dev = _require_cuda(tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2)
+    _require_chain_dtype(E_tok, E_byte)
+    tok = _tok_i32(tokens)
+    ids = _byte_ids(byte_ids)
+    _check_id_count(ids, tok.numel(), bpt)
+    ids2 = None
+    if byte_ids2 is not None:
+        # `--add-padded-and-pulled` (spt/train_gpt.py:371-379): two gathers summed before the per-byte norm.  The
+        # token columns of the operand come from the fused kernel (tok-only, strided rows), the byte columns from
+        # the pair kernels.
+        if not spec.byte_norm or spec.slot_major or spec.bytes_first:
+            raise NotImplementedError("mot_b200: the padded+pulled sum exists only with per-byte norms, token-major "
+                                      "ids and [tok | bytes] order (spt/train_gpt.py:371-379,442-443)")
+        ids2 = byte_ids2.contiguous()
+        if ids2.dtype != ids.dtype or ids2.numel() != ids.numel():
+            raise RuntimeError("mot_b200: the two byte-id tensors must share dtype and size")
+    K = E_tok.shape[1] + bpt * E_byte.shape[1]
+    if W.shape[1] != K:
+        raise RuntimeError(f"mot_b200: projection weight is {tuple(W.shape)}, expected [{W.shape[0]}, {K}]")
+    if bias is not None and bias.dtype != torch.float32:
+        raise NotImplementedError("mot_b200: the projection bias must be fp32 (mathblations/model.py:261)")
+    return dev, tok, ids, ids2, E_tok.contiguous(), E_byte.contiguous()
+
+
+def _proj_desc(spec: MixSpec, bpt: int, tok, ids, E_tok, E_byte, pair: bool) -> L.MotDesc:
+    """Descriptor of the gather of the [n, K] operand: the concat of both tables, or with `pair` (two byte-id tensors)
+    only its token columns, written with row stride K (the pair kernels write the byte columns)."""
+    if pair:
+        return make_desc(MixSpec(combine="tok_only", tok_norm=spec.tok_norm, out_norm=False, eps=spec.eps), tok.numel(),
+                         E_tok, None, 0, ids=None, ttb=None, has_lam=False,
+                         row_stride=E_tok.shape[1] + bpt * E_byte.shape[1], col_offset=0)
+    return make_desc(dataclasses.replace(spec, combine="concat", out_norm=False), tok.numel(), E_tok, E_byte, bpt,
+                     ids=ids, ttb=None, has_lam=False)
+
+
+def _gather_operand(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_tok, E_byte, A) -> None:
+    if ids2 is None:
+        embed_forward_out(desc, tok, ids, None, E_tok, E_byte, None, A)
+    elif tok.numel() > 0:
+        embed_forward_out(desc, tok, None, None, E_tok, None, None, A)
+        byte_pair_forward_out(ids, ids2, bpt, E_byte, A, E_tok.shape[1], spec.eps)
+
+
+def _scatter_operand(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_tok, E_byte, dA, ws_buf,
+                     plan_ready: bool, ws_clean: bool):
+    """The backward of _gather_operand: dense (gE_tok, gE_byte) from the operand's gradient dA."""
+    gE_tok, gE_byte = torch.empty_like(E_tok), torch.empty_like(E_byte)
+    if ids2 is None:
+        embed_backward_out(desc, tok, ids, None, E_tok, E_byte, None, dA, gE_tok, gE_byte, None, ws_buf,
+                           plan_ready=plan_ready, ws_clean=ws_clean)
+    else:   # token columns through the sorted-stream scatter, byte columns through the pair kernel
+        embed_backward_out(desc, tok, None, None, E_tok, None, None, dA, gE_tok, None, None, ws_buf,
+                           plan_ready=plan_ready, ws_clean=ws_clean)
+        byte_pair_backward_out(ids, ids2, bpt, E_byte, dA, E_tok.shape[1], gE_byte, spec.eps)
+    return gE_tok, gE_byte
+
+
+def _proj_forward(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_tok, E_byte, w_c, bias,
+                  keep_operand: bool):
+    """-> (out, Y, A): Y = A . w_c^T (+ bias) with the gathered [n, K] operand A (None unless keep_operand), out = the
+    row norm of Y under spec.out_norm, else Y itself.  w_c: the weight in the table dtype."""
+    n, (Do, K), dev, cdt = tok.numel(), w_c.shape, E_tok.device, E_tok.dtype
+    A = torch.empty((n, K), dtype=cdt, device=dev)
+    _gather_operand(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, A)
+    Y = torch.empty((n, Do), dtype=cdt, device=dev)
+    linear_forward_out(A, w_c, Y, bias.contiguous() if bias is not None else None)
+    if not keep_operand:
+        A = None
+    if spec.out_norm:
+        out = torch.empty_like(Y)
+        rmsnorm_forward_out(Y, out, spec.eps)
+    else:
+        out = Y
+    return out, Y, A
+
+
+def _proj_backward(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_tok, E_byte, w_c, w_dtype, has_bias: bool,
+                   Y, A, grad_out):
+    """The backward of _proj_forward down to the operand -> (dA, gW in w_dtype, g_bias fp32 or None).  A: the forward's
+    operand if it was kept, else None (gathered again here)."""
+    n, (Do, K), dev, cdt = tok.numel(), w_c.shape, E_tok.device, E_tok.dtype
+    g = grad_out.reshape(n, Do).to(cdt).contiguous()
+    if spec.out_norm:
+        dY = torch.empty_like(Y)
+        rmsnorm_backward_out(Y, g, dY, spec.eps)
+    else:
+        dY = g
+    g_bias = colsum_out(dY) if has_bias else None
+    if A is not None:
+        dA = torch.empty((n, K), dtype=cdt, device=dev)                   # a saved tensor is never overwritten
+    else:
+        A = torch.empty((n, K), dtype=cdt, device=dev)
+        _gather_operand(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, A)
+        dA = A                                                            # dX may overwrite the private copy
+    dW32 = torch.empty((Do, K), dtype=torch.float32, device=dev)
+    dW16 = torch.empty((Do, K), dtype=torch.bfloat16, device=dev) if w_dtype == torch.bfloat16 else None
+    linear_bwd_weight_out(dY, A, dW32, dW16)
+    linear_bwd_input_out(dY, w_c, dA)
+    return dA, (dW16 if dW16 is not None else dW32), g_bias      # cast_out admits bf16 or fp32 weights only
+
+
 class _MotEmbedProjFn(torch.autograd.Function):
     """out = f_out( [tok | bytes] . W^T + bias ): the fused gather builds the [n, K] operand (mot_embed_fwd, CONCAT),
     the projection runs on the tensor cores (mot_linear_fwd), the row norm after it is a separate HBM-bound pass over
@@ -783,124 +945,87 @@ class _MotEmbedProjFn(torch.autograd.Function):
     step); MOT_PROJ_REGATHER=1 gathers it again instead (the round-1 behaviour, for memory-tight callers)."""
 
     @staticmethod
-    def forward(ctx, spec: MixSpec, bpt: int, tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2=None):
-        dev = _require_cuda(tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2)
-        cdt = E_tok.dtype                      # compute dtype of the chain: bf16, or fp32 on the TF32 tensor-core path
-        if cdt not in (torch.bfloat16, torch.float32) or E_byte.dtype != cdt:
-            raise NotImplementedError("mot_b200: token and byte tables must both be bf16 or both fp32")
-        tok = tokens.reshape(-1)
-        tok = (tok if tok.dtype == torch.int32 else tok.to(torch.int32)).contiguous()
-        if byte_ids.dtype not in (torch.int32, torch.int64):
-            raise NotImplementedError("mot_b200: byte ids must be int32 or int64")
-        ids = byte_ids.contiguous()
-        n = tok.numel()
-        if ids.numel() != n * bpt:
-            raise RuntimeError(f"mot_b200: byte ids have {ids.numel()} entries, expected {n}*{bpt}")
-        E_tok_c, E_byte_c = E_tok.contiguous(), E_byte.contiguous()
-        ids2 = None
-        if byte_ids2 is not None:
-            # `--add-padded-and-pulled` (spt/train_gpt.py:371-379): two gathers summed before the per-byte norm.  The
-            # token columns of the operand come from the fused kernel (tok-only, strided rows), the byte columns from
-            # the pair kernels.
-            if not spec.byte_norm or spec.slot_major or spec.bytes_first:
-                raise NotImplementedError("mot_b200: the padded+pulled sum exists only with per-byte norms, token-major "
-                                          "ids and [tok | bytes] order (spt/train_gpt.py:371-379,442-443)")
-            ids2 = byte_ids2.contiguous()
-            if ids2.dtype != ids.dtype or ids2.numel() != ids.numel():
-                raise RuntimeError("mot_b200: the two byte-id tensors must share dtype and size")
-            K = E_tok_c.shape[1] + bpt * E_byte_c.shape[1]
-            desc = make_desc(MixSpec(combine="tok_only", tok_norm=spec.tok_norm, out_norm=False, eps=spec.eps), n, E_tok_c,
-                             None, 0, ids=None, ttb=None, has_lam=False, row_stride=K, col_offset=0)
-        else:
-            a_spec = dataclasses.replace(spec, combine="concat", out_norm=False)
-            desc = make_desc(a_spec, n, E_tok_c, E_byte_c, bpt, ids=ids, ttb=None, has_lam=False)
-            K = desc.out_dim
-        Do = W.shape[0]
-        if W.shape[1] != K:
-            raise RuntimeError(f"mot_b200: projection weight is {tuple(W.shape)}, expected [{Do}, {K}]")
-        w16 = cast_out(W, cdt)                                 # CastedLinear: W.type_as(x) (spt/train_gpt.py:186)
-        ctx.ws = None
-        if any(ctx.needs_input_grad[4:6]) and n > 0:
-            ctx.ws = acquire_workspace(desc, dev)
-            embed_plan_async(desc, tok, ctx.ws, dev)
-        A = torch.empty((n, K), dtype=cdt, device=dev)
-        if ids2 is None:
-            embed_forward_out(desc, tok, ids, None, E_tok_c, E_byte_c, None, A)
-        elif n > 0:
-            embed_forward_out(desc, tok, None, None, E_tok_c, None, None, A)
-            byte_pair_forward_out(ids, ids2, bpt, E_byte_c, A, E_tok_c.shape[1], spec.eps)
-        Y = torch.empty((n, Do), dtype=cdt, device=dev)
-        if bias is not None and bias.dtype != torch.float32:
-            raise NotImplementedError("mot_b200: the projection bias must be fp32 (mathblations/model.py:261)")
-        b32 = bias.detach().contiguous() if bias is not None else None
-        linear_forward_out(A, w16, Y, b32)
-        keep_A = _PROJ_KEEP_OPERAND and any(ctx.needs_input_grad[4:8])
-        if not keep_A:
-            del A
-        if spec.out_norm:
-            out = torch.empty_like(Y)
-            rmsnorm_forward_out(Y, out, spec.eps)
-        else:
-            out = Y
+    def forward(ctx, spec: MixSpec, bpt: int, dev, tok, ids, ids2, E_tok, E_byte, W, bias):
+        desc = _proj_desc(spec, bpt, tok, ids, E_tok, E_byte, ids2 is not None)
+        w16 = cast_out(W, E_tok.dtype)                         # CastedLinear: W.type_as(x) (spt/train_gpt.py:186)
+        ctx.ws = _planned_workspace(desc, tok, dev) if any(ctx.needs_input_grad[6:8]) and tok.numel() > 0 else None
+        keep_A = _PROJ_KEEP_OPERAND and any(ctx.needs_input_grad[6:10])
+        out, Y, A = _proj_forward(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, w16, bias, keep_A)
         embed_plan_join_if_capturing(ctx.ws, dev)
-        ctx.desc, ctx.dev, ctx.spec = desc, dev, spec
+        ctx.desc, ctx.dev, ctx.spec, ctx.bpt = desc, dev, spec, bpt
         ctx.w_dtype, ctx.has_bias = W.dtype, bias is not None
-        ctx.pair, ctx.bpt, ctx.K = ids2 is not None, bpt, K
-        ctx.save_for_backward(tok, ids, E_tok_c, E_byte_c, w16, Y, ids2 if ids2 is not None else _ABSENT,
+        ctx.pair, ctx.kept_A = ids2 is not None, keep_A
+        ctx.save_for_backward(tok, ids, E_tok, E_byte, w16, Y, ids2 if ids2 is not None else _ABSENT,
                               A if keep_A else _ABSENT)
-        ctx.kept_A = keep_A
         return out
 
     @staticmethod
     def backward(ctx, grad_out):
-        tok, ids, E_tok, E_byte, w16, Y, ids2, A_kept = ctx.saved_tensors
-        desc, dev, spec = ctx.desc, ctx.dev, ctx.spec
-        n, K, Do = tok.numel(), ctx.K, w16.shape[0]
-        cdt = Y.dtype
-        g = grad_out.reshape(n, Do).to(cdt).contiguous()
-        if spec.out_norm:
-            dY = torch.empty_like(Y)
-            rmsnorm_backward_out(Y, g, dY, spec.eps)
-        else:
-            dY = g
-        g_bias = colsum_out(dY) if ctx.has_bias else None
-        if ctx.kept_A:
-            A = A_kept                                                        # the forward's operand (n*K elements held)
-            dA = torch.empty((n, K), dtype=cdt, device=dev)                   # a saved tensor is never overwritten
-        else:
-            A = torch.empty((n, K), dtype=cdt, device=dev)
-            if not ctx.pair:
-                embed_forward_out(desc, tok, ids, None, E_tok, E_byte, None, A)   # gathered again (MOT_PROJ_REGATHER=1)
-            elif n > 0:
-                embed_forward_out(desc, tok, None, None, E_tok, None, None, A)
-                byte_pair_forward_out(ids, ids2, ctx.bpt, E_byte, A, E_tok.shape[1], spec.eps)
-            dA = A                                                            # dX may overwrite the private copy
-        dW32 = torch.empty((Do, K), dtype=torch.float32, device=dev)
-        dW16 = torch.empty((Do, K), dtype=torch.bfloat16, device=dev) if ctx.w_dtype == torch.bfloat16 else None
-        linear_bwd_weight_out(dY, A, dW32, dW16)
-        linear_bwd_input_out(dY, w16, dA)
-        gE_tok, gE_byte = torch.empty_like(E_tok), torch.empty_like(E_byte)
-        ws, planned = ctx.ws, ctx.ws is not None
-        if ws is None:
-            ws = acquire_workspace(desc, dev)
-        if planned:
-            if ws.pending:
-                embed_plan_join(ws, dev)
-            clean = True
-        else:
-            clean, ws.clean = ws.clean, False
-        if not ctx.pair:
-            embed_backward_out(desc, tok, ids, None, E_tok, E_byte, None, dA, gE_tok, gE_byte, None, ws.buf,
-                               plan_ready=planned, ws_clean=clean)
-        else:   # token columns through the sorted-stream scatter, byte columns through the pair kernel
-            embed_backward_out(desc, tok, None, None, E_tok, None, None, dA, gE_tok, None, None, ws.buf,
-                               plan_ready=planned, ws_clean=clean)
-            byte_pair_backward_out(ids, ids2, ctx.bpt, E_byte, dA, E_tok.shape[1], gE_byte, spec.eps)
-        ws.clean = True
+        tok, ids, E_tok, E_byte, w16, Y, ids2, A = ctx.saved_tensors
+        desc, dev, spec, bpt = ctx.desc, ctx.dev, ctx.spec, ctx.bpt
+        ids2 = ids2 if ctx.pair else None
+        dA, gW, g_bias = _proj_backward(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, w16, ctx.w_dtype, ctx.has_bias,
+                                        Y, A if ctx.kept_A else None, grad_out)
+        ws, planned, clean = _take_workspace(ctx.ws, desc, dev)
+        gE_tok, gE_byte = _scatter_operand(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, dA, ws.buf, planned, clean)
         ctx.ws = None
-        release_workspace(ws)
-        gW = dW16 if dW16 is not None else dW32          # cast_out admits bf16 or fp32 weights only
-        return (None, None, None, None, gE_tok, gE_byte, gW, g_bias, None)
+        _return_workspace(ws)
+        return None, None, None, None, None, None, gE_tok, gE_byte, gW, g_bias
+
+
+def _byte_fc_args(bpt: int, tokens, byte_ids, E_tok, E_byte, W):
+    """mot_embed_byte_fc's arguments checked and normalised -> (dev, tok, ids, E_tok, E_byte)."""
+    dev = _require_cuda(tokens, byte_ids, E_tok, E_byte, W)
+    _require_chain_dtype(E_tok, E_byte)
+    tok = _tok_i32(tokens)
+    ids = _byte_ids(byte_ids)
+    D = E_tok.shape[1]
+    if ids.numel() != tok.numel() * bpt or bpt * E_byte.shape[1] != D or tuple(W.shape) != (D, D):
+        raise RuntimeError("mot_b200: byte-FC mix needs bpt*byte_dim == token_dim and a square [D, D] weight")
+    return dev, tok, ids, E_tok.contiguous(), E_byte.contiguous()
+
+
+def _fc_descs(spec_b: MixSpec, bpt: int, tok, ids, E_tok, E_byte):
+    """-> (desc_b, desc_t): the bytes-only gather of the product's operand; the token gather + addend + norm."""
+    n = tok.numel()
+    return (make_desc(spec_b, n, None, E_byte, bpt, ids=ids, ttb=None, has_lam=False),
+            make_desc(MixSpec(combine="tok_only", out_norm=True, eps=spec_b.eps), n, E_tok, None, 0, ids=None, ttb=None,
+                      has_lam=False))
+
+
+def _byte_fc_forward(desc_b: L.MotDesc, desc_t: L.MotDesc, tok, ids, E_tok, E_byte, w_c):
+    """-> (out, Y): Y = C . w_c^T with C the bytes-only gather (not kept), out = norm(E_tok[tok] + Y)."""
+    n, D, dev, cdt = tok.numel(), E_tok.shape[1], E_tok.device, E_tok.dtype
+    C = torch.empty((n, D), dtype=cdt, device=dev)
+    embed_forward_out(desc_b, None, ids, None, None, E_byte, None, C)
+    Y = torch.empty((n, D), dtype=cdt, device=dev)
+    linear_forward_out(C, w_c, Y)
+    del C
+    out = torch.empty((n, D), dtype=cdt, device=dev)
+    if n > 0:
+        embed_forward_out(desc_t, tok, None, None, E_tok, None, None, out, addend=Y)
+    return out, Y
+
+
+def _byte_fc_backward(desc_b: L.MotDesc, desc_t: L.MotDesc, tok, ids, E_tok, E_byte, w_c, w_dtype, Y, grad_out,
+                      ws_buf, plan_ready: bool, ws_clean: bool, wsb_buf, wsb_clean: bool):
+    """-> (gE_tok, gE_byte, gW in w_dtype).  ws_*: the workspace of the token scatter; wsb_*: the workspace of the
+    bytes-only scatter, which is never planned ahead."""
+    (n, D), dev, cdt = Y.shape, Y.device, Y.dtype
+    g = grad_out.reshape(n, D).to(cdt).contiguous()
+    gE_tok, gE_byte = torch.empty_like(E_tok), torch.empty_like(E_byte)
+    dY = torch.empty_like(Y)
+    embed_backward_out(desc_t, tok, None, None, E_tok, None, None, g, gE_tok, None, None, ws_buf,
+                       plan_ready=plan_ready, ws_clean=ws_clean, addend=Y, d_addend=dY)
+    C = torch.empty((n, D), dtype=cdt, device=dev)
+    embed_forward_out(desc_b, None, ids, None, None, E_byte, None, C)            # gathered again, not kept
+    dW32 = torch.empty((D, D), dtype=torch.float32, device=dev)
+    dW16 = torch.empty((D, D), dtype=torch.bfloat16, device=dev) if w_dtype == torch.bfloat16 else None
+    linear_bwd_weight_out(dY, C, dW32, dW16)
+    linear_bwd_input_out(dY, w_c, C)                                             # dC overwrites the operand buffer
+    embed_backward_out(desc_b, None, ids, None, None, E_byte, None, C, None, gE_byte, None, wsb_buf,
+                       plan_ready=False, ws_clean=wsb_clean)
+    return gE_tok, gE_byte, (dW16 if dW16 is not None else dW32)
 
 
 class _MotEmbedByteFcFn(torch.autograd.Function):
@@ -911,88 +1036,39 @@ class _MotEmbedByteFcFn(torch.autograd.Function):
     cores; bytes-only scatter.  The operand is gathered again in the backward, not kept."""
 
     @staticmethod
-    def forward(ctx, spec_b: MixSpec, bpt: int, eps: float, tokens, byte_ids, E_tok, E_byte, W):
-        dev = _require_cuda(tokens, byte_ids, E_tok, E_byte, W)
-        cdt = E_tok.dtype
-        if cdt not in (torch.bfloat16, torch.float32) or E_byte.dtype != cdt:
-            raise NotImplementedError("mot_b200: token and byte tables must both be bf16 or both fp32")
-        tok = tokens.reshape(-1)
-        tok = (tok if tok.dtype == torch.int32 else tok.to(torch.int32)).contiguous()
-        if byte_ids.dtype not in (torch.int32, torch.int64):
-            raise NotImplementedError("mot_b200: byte ids must be int32 or int64")
-        ids = byte_ids.contiguous()
-        n = tok.numel()
-        E_tok_c, E_byte_c = E_tok.contiguous(), E_byte.contiguous()
-        D = E_tok_c.shape[1]
-        if ids.numel() != n * bpt or bpt * E_byte_c.shape[1] != D or tuple(W.shape) != (D, D):
-            raise RuntimeError("mot_b200: byte-FC mix needs bpt*byte_dim == token_dim and a square [D, D] weight")
-        w16 = cast_out(W, cdt)
-        desc_b = make_desc(spec_b, n, None, E_byte_c, bpt, ids=ids, ttb=None, has_lam=False)
-        desc_t = make_desc(MixSpec(combine="tok_only", out_norm=True, eps=eps), n, E_tok_c, None, 0, ids=None, ttb=None,
-                           has_lam=False)
-        ctx.ws = None
-        if ctx.needs_input_grad[5] and n > 0:
-            ctx.ws = acquire_workspace(desc_t, dev)
-            embed_plan_async(desc_t, tok, ctx.ws, dev)
-        C = torch.empty((n, D), dtype=cdt, device=dev)
-        embed_forward_out(desc_b, None, ids, None, None, E_byte_c, None, C)
-        Y = torch.empty((n, D), dtype=cdt, device=dev)
-        linear_forward_out(C, w16, Y)
-        del C
-        out = torch.empty((n, D), dtype=cdt, device=dev)
-        if n > 0:
-            embed_forward_out(desc_t, tok, None, None, E_tok_c, None, None, out, addend=Y)
+    def forward(ctx, spec_b: MixSpec, bpt: int, dev, tok, ids, E_tok, E_byte, W):
+        w16 = cast_out(W, E_tok.dtype)
+        desc_b, desc_t = _fc_descs(spec_b, bpt, tok, ids, E_tok, E_byte)
+        ctx.ws = _planned_workspace(desc_t, tok, dev) if ctx.needs_input_grad[5] and tok.numel() > 0 else None
+        out, Y = _byte_fc_forward(desc_b, desc_t, tok, ids, E_tok, E_byte, w16)
         embed_plan_join_if_capturing(ctx.ws, dev)
         ctx.desc_b, ctx.desc_t, ctx.dev, ctx.w_dtype = desc_b, desc_t, dev, W.dtype
-        ctx.save_for_backward(tok, ids, E_tok_c, E_byte_c, w16, Y)
+        ctx.save_for_backward(tok, ids, E_tok, E_byte, w16, Y)
         return out
 
     @staticmethod
     def backward(ctx, grad_out):
         tok, ids, E_tok, E_byte, w16, Y = ctx.saved_tensors
-        desc_b, desc_t, dev = ctx.desc_b, ctx.desc_t, ctx.dev
-        n, D = Y.shape
-        cdt = Y.dtype
-        g = grad_out.reshape(n, D).to(cdt).contiguous()
-        gE_tok, gE_byte = torch.empty_like(E_tok), torch.empty_like(E_byte)
-        dY = torch.empty_like(Y)
-        ws, planned = ctx.ws, ctx.ws is not None
-        if ws is None:
-            ws = acquire_workspace(desc_t, dev)
-        if planned:
-            if ws.pending:
-                embed_plan_join(ws, dev)
-            clean = True
-        else:
-            clean, ws.clean = ws.clean, False
-        embed_backward_out(desc_t, tok, None, None, E_tok, None, None, g, gE_tok, None, None, ws.buf,
-                           plan_ready=planned, ws_clean=clean, addend=Y, d_addend=dY)
-        ws.clean = True
+        ws, planned, clean = _take_workspace(ctx.ws, ctx.desc_t, ctx.dev)
+        wsb, _, clean_b = _take_workspace(None, ctx.desc_b, ctx.dev)
+        gE_tok, gE_byte, gW = _byte_fc_backward(ctx.desc_b, ctx.desc_t, tok, ids, E_tok, E_byte, w16, ctx.w_dtype, Y,
+                                                grad_out, ws.buf, planned, clean, wsb.buf, clean_b)
         ctx.ws = None
-        release_workspace(ws)
-        C = torch.empty((n, D), dtype=cdt, device=dev)
-        embed_forward_out(desc_b, None, ids, None, None, E_byte, None, C)            # gathered again, not kept
-        dW32 = torch.empty((D, D), dtype=torch.float32, device=dev)
-        dW16 = torch.empty((D, D), dtype=torch.bfloat16, device=dev) if ctx.w_dtype == torch.bfloat16 else None
-        linear_bwd_weight_out(dY, C, dW32, dW16)
-        linear_bwd_input_out(dY, w16, C)                                             # dC overwrites the operand buffer
-        wsb = acquire_workspace(desc_b, dev)
-        clean_b, wsb.clean = wsb.clean, False
-        embed_backward_out(desc_b, None, ids, None, None, E_byte, None, C, None, gE_byte, None, wsb.buf,
-                           plan_ready=False, ws_clean=clean_b)
-        wsb.clean = True
-        release_workspace(wsb)
-        gW = dW16 if dW16 is not None else dW32
+        _return_workspace(ws)
+        _return_workspace(wsb)
         return None, None, None, None, None, gE_tok, gE_byte, gW
 
 
 def mot_embed_byte_fc(tokens: torch.Tensor, byte_ids: torch.Tensor, E_tok: torch.Tensor, E_byte: torch.Tensor,
                       W_fc: torch.Tensor, *, bpt: int = 16, slot_major: bool = True, eps: float = FP32_EPS) -> torch.Tensor:
     """`norm(token_embs + F.linear(cat(byte_embs), byte_fc))` (runs/71051:226-229,312-314): [n_tokens, D]."""
+    dev, tok, ids, E_tok_c, E_byte_c = _byte_fc_args(bpt, tokens, byte_ids, E_tok, E_byte, W_fc)
     spec_b = MixSpec(combine="bytes_only", out_norm=False, slot_major=slot_major, eps=eps)
     if _custom_ops_wanted():
-        return _byte_fc_via_custom_op(spec_b, bpt, eps, tokens, byte_ids, E_tok, E_byte, W_fc)
-    return _MotEmbedByteFcFn.apply(spec_b, bpt, eps, tokens, byte_ids, E_tok, E_byte, W_fc)
+        need = torch.is_grad_enabled() and any(t.requires_grad for t in (E_tok, E_byte, W_fc))
+        return torch.ops.mot_b200.embed_byte_fc(tok, ids, E_tok_c, E_byte_c, W_fc.contiguous(), pack_spec(spec_b), bpt,
+                                                float(eps), need)[0]
+    return _MotEmbedByteFcFn.apply(spec_b, bpt, dev, tok, ids, E_tok_c, E_byte_c, W_fc)
 
 
 def mot_embed_proj(tokens: torch.Tensor, byte_ids: torch.Tensor, E_tok: torch.Tensor, E_byte: torch.Tensor,
@@ -1004,9 +1080,12 @@ def mot_embed_proj(tokens: torch.Tensor, byte_ids: torch.Tensor, E_tok: torch.Te
     call, gradient returned in fp32); or everything fp32 (mathblations: TF32 tensor cores).  byte_ids2: the second id
     tensor of `--add-padded-and-pulled` (spt/train_gpt.py:371-379), rows summed before the per-byte norm.  Returns
     [n_tokens, W.shape[0]] in the table dtype."""
+    dev, tok, ids, ids2, E_tok_c, E_byte_c = _proj_args(spec, bpt, tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2)
     if _custom_ops_wanted():
-        return _proj_via_custom_op(spec, bpt, tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2)
-    return _MotEmbedProjFn.apply(spec, bpt, tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2)
+        need = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (E_tok, E_byte, W, bias))
+        return torch.ops.mot_b200.embed_proj(tok, ids, ids2, E_tok_c, E_byte_c, W.contiguous(), bias, pack_spec(spec), bpt,
+                                             float(spec.eps), need)[0]
+    return _MotEmbedProjFn.apply(spec, bpt, dev, tok, ids, ids2, E_tok_c, E_byte_c, W, bias)
 
 
 def launch_count() -> int:
@@ -1018,6 +1097,4 @@ def reset_launch_count() -> None:
 
 
 # torch.library registration of the same entry points (torch.compile / compiled autograd see opaque operators)
-from ._library import (custom_ops_wanted as _custom_ops_wanted, set_custom_ops,  # noqa: E402,F401
-                       embed_via_custom_op as _embed_via_custom_op, tok_gather_via_custom_op as _tok_gather_via_custom_op,
-                       proj_via_custom_op as _proj_via_custom_op, byte_fc_via_custom_op as _byte_fc_via_custom_op)
+from ._library import custom_ops_wanted as _custom_ops_wanted, pack_spec, set_custom_ops  # noqa: E402,F401

@@ -110,6 +110,32 @@ def test_custom_op_path_projection_and_others(addpp):
     for k in res[None][1]:
         assert nerr(res[True][1][k], res[None][1][k]) <= 2.0 ** -8, k
     assert res[True][1]["front.byte_mixin.mixin.mixin.weight"].dtype == torch.float32   # fp32 master-weight gradient
+    # mathblations' digit mixin (fp32 tables on the TF32 path, projection bias: colsum_out and the bias gradient) and
+    # value embeddings with one frozen table (the want_mask of tok_gather_bwd)
+    dm = mot_b200.DigitMixinEmbedding(1000, 64, 64, 4).to(d)
+    ve = mot_b200.TokenValueEmbeddings(1500, 128, n_tables=3).to(d).bfloat16()
+    ve.value_embeds[1].weight.requires_grad_(False)
+    idx = torch.randint(0, 1000, (8, 11), generator=g, device=d)
+    digits = torch.randint(0, 14, (8, 11 * 4), generator=g, device=d)
+    go_dm = torch.randn(8, 11, 64, generator=g, device=d)
+    go_ve = [torch.randn(4, 128, 128, generator=g, device=d).bfloat16() for _ in range(3)]
+    res = {}
+    for mode in (None, True):
+        mot_b200.set_custom_ops(mode)
+        try:
+            dm.zero_grad(set_to_none=True)
+            ve.zero_grad(set_to_none=True)
+            loss = (dm(idx, digits) * go_dm).sum()
+            loss = loss + sum((o.float() * go.float()).sum() for o, go in zip(ve(tok), go_ve))
+            loss.backward()
+            res[mode] = (float(loss), {**_grads(dm), **{"ve." + k: v for k, v in _grads(ve).items()}})
+        finally:
+            mot_b200.set_custom_ops(None)
+    assert abs(res[None][0] - res[True][0]) <= 1e-5 * abs(res[None][0])
+    assert res[None][1].keys() == res[True][1].keys()
+    assert "digit_mixin.fc.bias" in res[True][1] and "ve.value_embeds.1.weight" not in res[True][1]
+    for k in res[None][1]:
+        assert nerr(res[True][1][k], res[None][1][k]) <= 2.0 ** -8, k
     # byte-FC variant, digits, integer ops and the expand through the operators
     mot_b200.set_custom_ops(True)
     try:

@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define MOT_B200_ABI_VERSION 4
+#define MOT_B200_ABI_VERSION 5
 
 /* ---- error codes ------------------------------------------------------- */
 enum {
@@ -70,7 +70,11 @@ enum {
   MOT_F_TTB_SCRAMBLE = 1 << 6, /* with IDS_FROM_TTB: slot i of position s is flat byte i*seq_len + s of its
                                   row of seq_len tokens (the `.view(bpt,-1)` of runs/71:479)           */
   MOT_F_IDS_I64 = 1 << 7,      /* byte-id tensors hold int64 (spt), else int32 (runs)                  */
-  MOT_F_HAS_LAMBDAS = 1 << 8   /* lam[0] = lam_tok, lam[1] = lam_byte (runs/74:314-315)                */
+  MOT_F_HAS_LAMBDAS = 1 << 8,  /* lam[0] = lam_tok, lam[1] = lam_byte (runs/74:314-315)                */
+  MOT_F_TTB_PULL_LEFT = 1 << 9 /* with IDS_FROM_TTB: the ids are the PULLED ids of pull_from_left (mot_pull) over rows of
+                                  seq_len tokens (n_tokens % seq_len == 0, bpt <= 32, tok_vocab = the ttb table's rows
+                                  also for MOT_BYTES_ONLY), pad_id / eot_id as there;
+                                  with TTB_SCRAMBLE the scramble picks (token, slot) and the id comes from the pulled row */
 };
 
 typedef struct MotDesc {
@@ -94,6 +98,9 @@ typedef struct MotDesc {
   int32_t col_offset;  /* first column of this call's slice inside those rows (multiple of 8) */
   int32_t dp_slabs;    /* 0 / 1: the backward runs in one piece.  n > 1: the caller will run it as n vocabulary slabs
                           (mot_embed_bwd_slab); only sizes the workspace (one fp32 slot per finer stream chunk) */
+  int32_t pad_id;      /* with MOT_F_TTB_PULL_LEFT: the pad byte (456) and the end-of-text byte (457) of the ttb table,
+                          each in the int16 range */
+  int32_t eot_id;
 } MotDesc;
 
 const char* mot_strerror(int rc);
@@ -253,6 +260,19 @@ int mot_byte_pair_bwd(const void* ids_a, const void* ids_b, int32_t ids_i64, int
                       const void* E_byte, int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps,
                       const void* grad_out, int64_t row_stride, int32_t col_offset, void* gE_byte, void* workspace,
                       size_t ws_bytes, void* stream);
+
+/* The same pair with both id tensors derived from the token ids inside the kernels: ids_a = the padded ids (the ttb rows
+ * of `tok`, mot_ttb_expand), ids_b = the pulled ids of pull_from_left over rows of seq_len tokens (MOT_F_TTB_PULL_LEFT).
+ * tok: int32 [n_tokens], n_tokens % seq_len == 0; ttb [tok_vocab, bpt] of ttb_dtype.  Otherwise as above. */
+int mot_byte_pair_ttb_fwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
+                          int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt, const void* E_byte,
+                          int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps, void* out, int64_t row_stride,
+                          int32_t col_offset, void* stream);
+int mot_byte_pair_ttb_bwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
+                          int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt, const void* E_byte,
+                          int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps, const void* grad_out,
+                          int64_t row_stride, int32_t col_offset, void* gE_byte, void* workspace, size_t ws_bytes,
+                          void* stream);
 
 /* ---- data-parallel exchange: average the gradient bucket across ranks through NVLink / NVSwitch -----------------
  * Replaces the per-parameter dist.all_reduce(param.grad, AVG) of spt/train_gpt.py:1320-1321 and runs/7:697-700 (launched

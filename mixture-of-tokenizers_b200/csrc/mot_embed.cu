@@ -178,8 +178,12 @@ static int validate(const MotDesc* d) {
   if (d->dp_slabs < 0 || d->dp_slabs > 64) return MOT_ERR_BAD_ARG;
   if ((d->flags & MOT_F_IDS_FROM_TTB) && has_bytes) {
     if (d->ttb_dtype < MOT_TTB_I16 || d->ttb_dtype > MOT_TTB_BF16) return MOT_ERR_UNSUPPORTED;
-    if (d->flags & MOT_F_TTB_SCRAMBLE)
+    if (d->flags & (MOT_F_TTB_SCRAMBLE | MOT_F_TTB_PULL_LEFT))
       if (d->seq_len <= 0 || d->n_tokens % d->seq_len) return MOT_ERR_BAD_ARG;
+    if (d->flags & MOT_F_TTB_PULL_LEFT) {
+      if (d->tok_vocab <= 0) return MOT_ERR_BAD_ARG;  // rows of the ttb table, also without a token table
+      if (d->pad_id != (int16_t)d->pad_id || d->eot_id != (int16_t)d->eot_id) return MOT_ERR_BAD_ARG;  // int16, as in mot_pull
+    }
   }
   return MOT_OK;
 }
@@ -199,6 +203,7 @@ static void fill_params(const MotDesc* d, EmbedParams& p) {
   p.combine = d->combine;
   p.flags = d->flags;
   p.ttb_dtype = d->ttb_dtype;
+  p.pad_eot = (d->pad_id & 0xffff) | (d->eot_id << 16);
   p.n_chunks = d->out_dim / kChunk;
   p.io_ld = d->row_stride ? d->row_stride : d->out_dim;
   p.io_col = d->col_offset;

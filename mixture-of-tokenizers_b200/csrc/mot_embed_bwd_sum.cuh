@@ -81,7 +81,7 @@ struct SumBatch {
   int v_next;  // last batch: token id of the stream entry after the chunk (-1: none)
 };
 
-template <typename T, int CPL>
+template <typename T, int CPL, bool PULL>
 __global__ void __launch_bounds__(kSumThreads, 1) mot_bwd_sum_kernel(const EmbedParams p) {
   constexpr int CW = kBwdCW;
   using V = Vec<T, CW>;
@@ -265,7 +265,8 @@ __global__ void __launch_bounds__(kSumThreads, 1) mot_bwd_sum_kernel(const Embed
   int id_next = 0;  // raw byte id (lane = slot) of the next occurrence, fetched one occurrence ahead
   if (A.cnt > 0) {
     const int pos0 = __shfl_sync(kFull, A.pos, 0);
-    if (id_lane) id_next = load_raw_id(p, idsrc, pos0, lane);
+    if constexpr (PULL) id_next = pulled_lane_id(p, pos0, id_lane);
+    else if (id_lane) id_next = load_raw_id(p, idsrc, pos0, lane);
   }
   while (A.cnt > 0) {
     const int cnt = A.cnt;
@@ -281,7 +282,11 @@ __global__ void __launch_bounds__(kSumThreads, 1) mot_bwd_sum_kernel(const Embed
       {  // byte ids of the next occurrence (the first entry of the next batch after the last one of this batch)
         const bool more = k + 1 < cnt;  // warp-uniform
         const int pos_n = __shfl_sync(kFull, more ? A.pos : B.pos, more ? k + 1 : 0);
-        if (id_lane && (more || B.cnt > 0)) id_next = load_raw_id(p, idsrc, pos_n, lane);
+        if constexpr (PULL) {
+          if (more || B.cnt > 0) id_next = pulled_lane_id(p, pos_n, id_lane);
+        } else {
+          if (id_lane && (more || B.cnt > 0)) id_next = load_raw_id(p, idsrc, pos_n, lane);
+        }
       }
 
       mbar_wait_s(bars_s + (uint32_t)cs * 8u, cpar);
@@ -450,8 +455,11 @@ __global__ void __launch_bounds__(kSumThreads, 1) mot_bwd_sum_kernel(const Embed
 #endif
 }
 
-template <typename T, int CPL>
+template <typename T, int CPL, bool PULL = false>
 static int launch_bwd_sum(const EmbedParams& p_in, cudaStream_t s) {
+  if constexpr (!PULL) {
+    if (ids_pulled(p_in)) return launch_bwd_sum<T, CPL, true>(p_in, s);
+  }
   int sms = 0, optin = 0;
   if (int rc = device_props(&sms, &optin)) return rc;
   EmbedParams p = p_in;
@@ -469,7 +477,7 @@ static int launch_bwd_sum(const EmbedParams& p_in, cudaStream_t s) {
   }
   if (smem == 0) return MOT_ERR_UNSUPPORTED;
   p.trace = g_trace ? g_trace + 4096 * 64 : nullptr;
-  auto kern = mot_bwd_sum_kernel<T, CPL>;
+  auto kern = mot_bwd_sum_kernel<T, CPL, PULL>;
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return check_launch();
   if (g_prof_start) cudaEventRecord(g_prof_start, s);
   const int ctas = (p.grid_cap > 0 && p.grid_cap < sms) ? p.grid_cap : sms;

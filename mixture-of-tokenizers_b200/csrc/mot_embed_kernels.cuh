@@ -81,6 +81,7 @@ struct EmbedParams {
   long long* trace;  // MOT_TRACE builds: per-warp time stamps (nullptr: off)
   long long* chk;    // MOT_CHECK builds: violation record
   int n_slots;       // fp32 slots of `partial` (MOT_CHECK builds verify every slot index against it)
+  int pad_eot;      // MOT_F_TTB_PULL_LEFT: pad byte | end-of-text byte << 16 (int16 each; fits the struct's tail padding)
 };
 
 struct ChunkMap {
@@ -161,6 +162,98 @@ __device__ __forceinline__ int fetch_id(const EmbedParams& p, long long pos, int
 }
 __device__ __forceinline__ int clamp_id(const EmbedParams& p, int id) { return clampi(id, p.Vb - 1); }
 
+// ---- pulled ids derived from the token ids (MOT_F_TTB_PULL_LEFT) ----
+// Entry k of ttb row tv as mot_ttb_expand writes it (float rows truncated to int64) and mot_pull reads it back (int).
+__device__ __forceinline__ int ttb_raw(const void* ttb, int ttb_dtype, int tv, int bpt, int k) {
+  const size_t e = (size_t)tv * bpt + k;
+  if (ttb_dtype == MOT_TTB_I16) return ld_g(reinterpret_cast<const short*>(ttb) + e);
+  if (ttb_dtype == MOT_TTB_F32) return (int)(long long)ld_g(reinterpret_cast<const float*>(ttb) + e);
+  return (int)(long long)__bfloat162float(reinterpret_cast<const __nv_bfloat16*>(ttb)[e]);
+}
+
+struct PullSrc {
+  const int32_t* tok;
+  const void* ttb;
+  long long T;  // tokens per row
+  int V, bpt, ttb_dtype, pad, eot, scramble;
+};
+
+// The bpt pulled ids of token t (pull_from_left over its row of T tokens, mot_pull.cu), computed by one warp without
+// the pulled tensor: lane k < bpt returns slot k.  Raw values: pads and EOT are detected on them, the caller clamps.
+// Lanes take tokens t, t-1, ..., t-31 of the row, each its non-pad count and EOT flag from its ttb row; the segment
+// ends (going back) at an EOT token or the row start; an inclusive scan of the counts gives every token the range of
+// backward byte indices it holds, and slot k receives backward index bpt - k.  Tokens with no non-pad byte can leave
+// the 32-token window short of bpt bytes: the next window continues.  Integer work, bit-exact with mot_pull, whose
+// compacted stream keeps the bytes as int16 (hence the (short) below).
+__device__ __forceinline__ int pulled_ids_warp(const PullSrc q, int t) {
+  const int lane = lane_id();
+  const int row0 = (int)(t - t % q.T);
+  const int want = q.bpt - lane;  // backward index (1 = last byte of the segment) of this lane's slot
+  int res = q.pad, acc = 0;
+  for (int base = t;; base -= 32) {
+    const int j = base - lane;
+    const bool valid = j >= row0;
+    int cnt = 0, tv = 0;
+    bool eot = false;
+    if (valid) {
+      tv = clampi(ld_g(q.tok + j), q.V - 1);
+      int n_eot = 0;
+      for (int k = 0; k < q.bpt; ++k) {
+        const int id = ttb_raw(q.ttb, q.ttb_dtype, tv, q.bpt, k);
+        cnt += id != q.pad;
+        n_eot += id == q.eot;
+      }
+      eot = n_eot == q.bpt;
+    }
+    if (base == t && __shfl_sync(0xffffffffu, eot, 0)) return q.eot;  // EOT tokens pass through unchanged
+    const unsigned stop = __ballot_sync(0xffffffffu, !valid || eot);
+    const int f = stop ? __ffs(stop) - 1 : 32;  // lanes [0, f) belong to the segment
+    if (lane >= f) cnt = 0;
+    int incl = cnt;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int u = __shfl_up_sync(0xffffffffu, incl, o);
+      if (lane >= o) incl += u;
+    }
+    incl += acc;
+    const int total = __shfl_sync(0xffffffffu, incl, 31);
+    int l = 0;  // first lane whose inclusive count reaches `want`
+#pragma unroll
+    for (int step = 16; step > 0; step >>= 1)
+      if (__shfl_sync(0xffffffffu, incl, l + step - 1) < want) l += step;
+    const int o_tv = __shfl_sync(0xffffffffu, tv, l), o_incl = __shfl_sync(0xffffffffu, incl, l);
+    if (lane < q.bpt && want > acc && want <= total) {
+      int fi = o_incl - want;  // index of the byte among the owner's non-pad bytes, in row order
+      for (int k = 0; k < q.bpt; ++k) {
+        const int id = ttb_raw(q.ttb, q.ttb_dtype, o_tv, q.bpt, k);
+        if (id != q.pad && fi-- == 0) {
+          res = (int)(short)id;
+          break;
+        }
+      }
+    }
+    if (total >= q.bpt || f < 32) return res;
+    acc = total;
+  }
+}
+
+// Pulled id of this lane's slot at position pos (warp collective).  With the `.view(bpt,-1)` scramble every slot lane
+// reads another token: the warp derives the pulled row of each of them in turn.
+__device__ __forceinline__ int fetch_pulled_id(const PullSrc q, int pos) {
+  const int lane = lane_id();
+  if (!q.scramble) return pulled_ids_warp(q, pos);
+  const long long row = pos / q.T, s = pos - row * q.T;
+  const long long f = (long long)min(lane, q.bpt - 1) * q.T + s;
+  const int tokpos = (int)(row * q.T + f / q.bpt), k = (int)(f % q.bpt);
+  int id = 0;
+  for (int r = 0; r < q.bpt; ++r) {
+    const int v = pulled_ids_warp(q, __shfl_sync(0xffffffffu, tokpos, r));
+    const int got = __shfl_sync(0xffffffffu, v, __shfl_sync(0xffffffffu, k, r));
+    if (lane == r) id = got;
+  }
+  return id;
+}
+
 // Per-lane view of the byte-id source, set up once: one multiply-add + load per position.
 struct IdSrc {
   const char* base;      // address of (position 0, slot = lane) for id tensors
@@ -180,6 +273,17 @@ __device__ __forceinline__ int load_raw_id(const EmbedParams& p, const IdSrc& s,
   if (s.kind == 2) return fetch_id(p, pos, slot);
   const char* a = s.base + (unsigned long long)(unsigned)pos * s.pos_stride;  // one 32 x 32 -> 64 multiply-add
   return s.kind == 1 ? (int)ld_g(reinterpret_cast<const long long*>(a)) : ld_g(reinterpret_cast<const int*>(a));
+}
+// The descriptor asks for pulled ids derived in the kernel: the kernels run their PULL instantiation, in which every
+// id load is the warp collective fetch_pulled_id (the other instantiations carry none of its code).
+inline bool ids_pulled(const EmbedParams& p) {
+  return (p.flags & MOT_F_IDS_FROM_TTB) && (p.flags & MOT_F_TTB_PULL_LEFT) && p.bpt > 0;
+}
+// Raw pulled id of this lane's slot (0 on lanes that hold no slot).  Every lane of the warp must call it.
+__device__ __forceinline__ int pulled_lane_id(const EmbedParams& p, int pos, bool id_lane) {
+  const int id = fetch_pulled_id(PullSrc{p.tok, p.ttb, p.T, p.V, p.bpt, p.ttb_dtype, (short)(p.pad_eot & 0xffff),
+                                         p.pad_eot >> 16, (p.flags & MOT_F_TTB_SCRAMBLE) ? 1 : 0}, pos);
+  return id_lane ? id : 0;
 }
 
 // Compile-time specialisation of the variant flags.  MODE 0: everything decided at run time (all variants);
@@ -334,7 +438,7 @@ __device__ __forceinline__ void gmem_add4(float* a, const float (&v)[4]) {
 // ======================================================================================
 // Forward
 // ======================================================================================
-template <typename T, int CPL, int MODE, int NT>
+template <typename T, int CPL, int MODE, int NT, bool PULL>
 __global__ void __launch_bounds__(NT, 1) mot_fwd_kernel(const EmbedParams p) {
   using C = Cfg<MODE>;
   constexpr int CW = 8;
@@ -402,15 +506,25 @@ __global__ void __launch_bounds__(NT, 1) mot_fwd_kernel(const EmbedParams p) {
   const bool id_lane = has_bytes && lane < p.bpt;
   const IdSrc idsrc = make_id_src(p, lane);
   // raw byte ids are fetched two positions ahead and clamped where they are consumed
-  int id_n1 = (id_lane && n_i > 0) ? load_raw_id(p, idsrc, gw, lane) : 0;
-  int id_n2 = (id_lane && n_i > 1) ? load_raw_id(p, idsrc, gw + stride, lane) : 0;
+  int id_n1, id_n2;
+  if constexpr (PULL) {
+    id_n1 = n_i > 0 ? pulled_lane_id(p, gw, id_lane) : 0;
+    id_n2 = n_i > 1 ? pulled_lane_id(p, gw + stride, id_lane) : 0;
+  } else {
+    id_n1 = (id_lane && n_i > 0) ? load_raw_id(p, idsrc, gw, lane) : 0;
+    id_n2 = (id_lane && n_i > 1) ? load_raw_id(p, idsrc, gw + stride, lane) : 0;
+  }
   int s = 0;
   uint32_t parity = 0;
   int pos = gw;
   for (int i = 0; i < n_i; ++i, pos += stride) {
     const int idreg = clamp_id(p, id_n1);
     id_n1 = id_n2;
-    if (id_lane && i + 2 < n_i) id_n2 = load_raw_id(p, idsrc, pos + 2 * stride, lane);
+    if constexpr (PULL) {
+      if (i + 2 < n_i) id_n2 = pulled_lane_id(p, pos + 2 * stride, id_lane);
+    } else {
+      if (id_lane && i + 2 < n_i) id_n2 = load_raw_id(p, idsrc, pos + 2 * stride, lane);
+    }
 
     float x[CPL][8];
     float ss_t = 0.f;
@@ -599,7 +713,7 @@ struct Batch {
 template <int CPL, int MODE>
 constexpr int bwd_threads() { return (MOT_ADDFLAG(MODE, 4) && CPL >= 8) ? MOT_WIDE_STATIC_THREADS : kBwdThreads; }
 
-template <typename T, int CPL, int MODE>
+template <typename T, int CPL, int MODE, bool PULL>
 __global__ void __launch_bounds__((bwd_threads<CPL, MODE>()), 1) mot_bwd_kernel(const EmbedParams p) {
   using C = Cfg<MODE>;
   constexpr int CW = kBwdCW;
@@ -782,7 +896,9 @@ __global__ void __launch_bounds__((bwd_threads<CPL, MODE>()), 1) mot_bwd_kernel(
     int v_before = -1;
     if (has_tok && chunk_first && a > 0) v_before = ld_g(p.stok + a - 1);
     const int pos_first = __shfl_sync(0xffffffffu, A.pos, 0);  // warp collective: outside lane-dependent branches
-    int id_next = id_lane ? load_raw_id(p, idsrc, pos_first, lane) : 0;
+    int id_next;
+    if constexpr (PULL) id_next = pulled_lane_id(p, pos_first, id_lane);
+    else id_next = id_lane ? load_raw_id(p, idsrc, pos_first, lane) : 0;
     for (int k = 0; k < A.cnt; ++k) {
       const int v = __shfl_sync(0xffffffffu, A.v, k);
       const int pos_k = __shfl_sync(0xffffffffu, A.pos, k);  // position of this occurrence (dense addend rows)
@@ -795,7 +911,11 @@ __global__ void __launch_bounds__((bwd_threads<CPL, MODE>()), 1) mot_bwd_kernel(
       if (issued - consumed < D) try_issue();  // one stage was freed by the previous occurrence
       const int idreg = clamp_id(p, id_next);
       const int pos_ahead = __shfl_sync(0xffffffffu, A.pos, (k + 1) & 31);
-      if (id_lane && k + 1 < A.cnt) id_next = load_raw_id(p, idsrc, pos_ahead, lane);
+      if constexpr (PULL) {
+        if (k + 1 < A.cnt) id_next = pulled_lane_id(p, pos_ahead, id_lane);
+      } else {
+        if (id_lane && k + 1 < A.cnt) id_next = load_raw_id(p, idsrc, pos_ahead, lane);
+      }
 
       mbar_wait(bars + cs, cpar);
       ++consumed;
@@ -1183,8 +1303,11 @@ inline size_t plan_smem(EmbedParams& p, size_t esz, int warps, bool backward, in
   return 0;
 }
 
-template <typename T, int CPL, int MODE>
+template <typename T, int CPL, int MODE, bool PULL = false>
 static int launch_fwd(const EmbedParams& p_in, cudaStream_t s) {
+  if constexpr (!PULL && MODE != 2 && MODE != 5) {
+    if (ids_pulled(p_in)) return launch_fwd<T, CPL, MODE, true>(p_in, s);
+  }
   int sms = 0, optin = 0;
   if (int rc = device_props(&sms, &optin)) return rc;
   EmbedParams p = p_in;
@@ -1200,9 +1323,9 @@ static int launch_fwd(const EmbedParams& p_in, cudaStream_t s) {
     if (smem != 0 && (p.tab_smem || p.combine == MOT_TOK_ONLY || threads == 256)) break;
   }
   if (smem == 0) return MOT_ERR_UNSUPPORTED;
-  if ((MODE == 1 || MOT_ADDFAM(MODE)) && !p.tab_smem) return launch_fwd<T, CPL, 0>(p_in, s);  // fast paths assume the table in smem
+  if ((MODE == 1 || MOT_ADDFAM(MODE)) && !p.tab_smem) return launch_fwd<T, CPL, 0, PULL>(p_in, s);  // fast paths assume the table in smem
   p.trace = g_trace;
-  auto kern = mot_fwd_kernel<T, CPL, MODE, NT>;
+  auto kern = mot_fwd_kernel<T, CPL, MODE, NT, PULL>;
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return check_launch();
   const long long warps_needed = p.N;
   long long blocks = (warps_needed + (threads / 32) - 1) / (threads / 32);
@@ -1215,16 +1338,19 @@ static int launch_fwd(const EmbedParams& p_in, cudaStream_t s) {
   return check_launch();
 }
 
-template <typename T, int CPL, int MODE>
+template <typename T, int CPL, int MODE, bool PULL = false>
 static int launch_bwd(const EmbedParams& p_in, cudaStream_t s) {
+  if constexpr (!PULL && MODE != 2 && MODE != 5) {
+    if (ids_pulled(p_in)) return launch_bwd<T, CPL, MODE, true>(p_in, s);
+  }
   int sms = 0, optin = 0;
   if (int rc = device_props(&sms, &optin)) return rc;
   EmbedParams p = p_in;
   constexpr int NT = bwd_threads<CPL, MODE>();
   const size_t smem = plan_smem(p, sizeof(T), NT / 32, true, optin);
   if (smem == 0) return MOT_ERR_UNSUPPORTED;
-  if ((MODE == 1 || MODE == 3 || MODE == 6 || MOT_ADDFAM(MODE)) && !p.tab_smem) return launch_bwd<T, CPL, 0>(p_in, s);  // fast paths assume the table in smem
-  auto kern = mot_bwd_kernel<T, CPL, MODE>;
+  if ((MODE == 1 || MODE == 3 || MODE == 6 || MOT_ADDFAM(MODE)) && !p.tab_smem) return launch_bwd<T, CPL, 0, PULL>(p_in, s);  // fast paths assume the table in smem
+  auto kern = mot_bwd_kernel<T, CPL, MODE, PULL>;
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return check_launch();
   if (g_prof_start) cudaEventRecord(g_prof_start, s);
   launch_pdl(kern, dim3((unsigned)sms), dim3(NT), smem, s, p);

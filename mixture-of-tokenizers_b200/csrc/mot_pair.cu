@@ -10,6 +10,8 @@
 // sums of squares / dot products are G-lane butterfly reductions; adjacent lanes touch adjacent 16-byte chunks, so
 // every 32-byte sector of the output row is written whole.  HBM-bound: per position 2*bpt ids + bpt*bd*e output bytes
 // (forward) / the same read of the upstream gradient plus 2*bpt*bd fp32 REDs into L2-resident replicas (backward).
+#include <type_traits>
+
 #include "mot_embed_kernels.cuh"
 
 namespace mot {
@@ -24,6 +26,11 @@ struct PairParams {
   long long N, ld;
   int col, Vb, bpt, bd, ids_i64, n_rep, G;
   float eps;
+};
+// Both id sets derived from the token ids (a padded, b pulled).  A separate type, so that the kernels of explicit ids keep
+// their parameter block.
+struct PairTtbParams : PairParams {
+  PullSrc ttb;
 };
 
 constexpr int kPairThreads = 512;
@@ -52,6 +59,18 @@ __device__ __forceinline__ int pair_load_id(const void* ids, int i64, long long 
   return clampi(v, hi);
 }
 
+// Byte ids (ia, ib) of this lane's slot at position pos derived from the token ids: padded ids for a, pulled ids for b.
+// Warp collective; clamped; 0 on inactive lanes.
+__device__ __forceinline__ void pair_ttb_ids(const PairTtbParams& p, long long pos, int slot, bool active, int& ia, int& ib) {
+  const int lane = lane_id();
+  const int tv = clampi(ld_g(p.ttb.tok + pos), p.ttb.V - 1);
+  const int a = lane < p.bpt ? ttb_raw(p.ttb.ttb, p.ttb.ttb_dtype, tv, p.bpt, lane) : 0;
+  const int b = pulled_ids_warp(p.ttb, (int)pos);
+  ia = clampi(__shfl_sync(0xffffffffu, a, slot & 31), p.Vb - 1);
+  ib = clampi(__shfl_sync(0xffffffffu, b, slot & 31), p.Vb - 1);
+  if (!active) ia = ib = 0;
+}
+
 template <int G>
 __device__ __forceinline__ float group_sum(float v) {
 #pragma unroll
@@ -60,8 +79,8 @@ __device__ __forceinline__ float group_sum(float v) {
 }
 
 // MAXJ = 8-element chunks per lane (ceil(bd / 8 / G))
-template <typename T, int G, int MAXJ>
-__global__ void __launch_bounds__(kPairThreads, MAXJ <= 4 ? 2 : 1) mot_pair_fwd_kernel(const PairParams p) {
+template <typename T, int G, int MAXJ, typename P>
+__global__ void __launch_bounds__(kPairThreads, MAXJ <= 4 ? 2 : 1) mot_pair_fwd_kernel(const P p) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   __shared__ uint64_t tab_bar;
   T* tab = reinterpret_cast<T*>(smem_raw);
@@ -77,7 +96,9 @@ __global__ void __launch_bounds__(kPairThreads, MAXJ <= 4 ? 2 : 1) mot_pair_fwd_
   const long long W = (long long)gridDim.x * nw;
   for (long long pos = (long long)warp * gridDim.x + blockIdx.x; pos < p.N; pos += W) {
     int ia = 0, ib = 0;
-    if (active) {
+    if constexpr (std::is_same_v<P, PairTtbParams>) {
+      pair_ttb_ids(p, pos, slot, active, ia, ib);
+    } else if (active) {
       ia = pair_load_id(p.ids_a, p.ids_i64, pos * p.bpt + slot, p.Vb - 1);
       ib = pair_load_id(p.ids_b, p.ids_i64, pos * p.bpt + slot, p.Vb - 1);
     }
@@ -115,8 +136,8 @@ __global__ void __launch_bounds__(kPairThreads, MAXJ <= 4 ? 2 : 1) mot_pair_fwd_
 // Backward: with s = E[ia] + E[ib], r = rsqrt(mean(s^2) + eps): ds = r*g - s * r^3 * mean(g.s); both gathered rows
 // receive ds (fp32 RED.v4 into one of n_rep L2-resident replicas; mot_bwd_finalize_kernel sums and casts them).
 // Two passes over the slot (reduce, then scatter) so that nothing of the row is held across the reduction.
-template <typename T, int G, int MAXJ>
-__global__ void __launch_bounds__(kPairThreads, MAXJ <= 4 ? 2 : 1) mot_pair_bwd_kernel(const PairParams p) {
+template <typename T, int G, int MAXJ, typename P>
+__global__ void __launch_bounds__(kPairThreads, MAXJ <= 4 ? 2 : 1) mot_pair_bwd_kernel(const P p) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   __shared__ uint64_t tab_bar;
   T* tab = reinterpret_cast<T*>(smem_raw);
@@ -134,7 +155,9 @@ __global__ void __launch_bounds__(kPairThreads, MAXJ <= 4 ? 2 : 1) mot_pair_bwd_
   const long long W = (long long)gridDim.x * nw;
   for (long long pos = gw; pos < p.N; pos += W) {
     int ia = 0, ib = 0;
-    if (active) {
+    if constexpr (std::is_same_v<P, PairTtbParams>) {
+      pair_ttb_ids(p, pos, slot, active, ia, ib);
+    } else if (active) {
       ia = pair_load_id(p.ids_a, p.ids_i64, pos * p.bpt + slot, p.Vb - 1);
       ib = pair_load_id(p.ids_b, p.ids_i64, pos * p.bpt + slot, p.Vb - 1);
     }
@@ -185,8 +208,8 @@ __global__ void __launch_bounds__(kPairThreads, MAXJ <= 4 ? 2 : 1) mot_pair_bwd_
   }
 }
 
-template <typename T, int G, int MAXJ>
-static int launch_pair(const PairParams& p, bool backward, cudaStream_t s) {
+template <typename T, int G, int MAXJ, typename P>
+static int launch_pair(const P& p, bool backward, cudaStream_t s) {
   int sms = 0, optin = 0;
   if (int rc = device_props(&sms, &optin)) return rc;
   const size_t smem = align_up((size_t)p.Vb * p.bd * sizeof(T), 128);
@@ -196,11 +219,11 @@ static int launch_pair(const PairParams& p, bool backward, cudaStream_t s) {
   if (blocks > (long long)per_sm * sms) blocks = (long long)per_sm * sms;
   if (blocks < 1) blocks = 1;
   if (backward) {
-    auto kern = mot_pair_bwd_kernel<T, G, MAXJ>;
+    auto kern = mot_pair_bwd_kernel<T, G, MAXJ, P>;
     if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return check_launch();
     launch_pdl(kern, dim3((unsigned)blocks), dim3(kPairThreads), smem, s, p);
   } else {
-    auto kern = mot_pair_fwd_kernel<T, G, MAXJ>;
+    auto kern = mot_pair_fwd_kernel<T, G, MAXJ, P>;
     if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return check_launch();
     launch_pdl(kern, dim3((unsigned)blocks), dim3(kPairThreads), smem, s, p);
   }
@@ -208,8 +231,8 @@ static int launch_pair(const PairParams& p, bool backward, cudaStream_t s) {
   return check_launch();
 }
 
-template <typename T>
-static int dispatch_pair(const PairParams& p, bool backward, cudaStream_t s) {
+template <typename T, typename P>
+static int dispatch_pair(const P& p, bool backward, cudaStream_t s) {
   const int per_lane = (p.bd / kChunk + p.G - 1) / p.G;  // 8-element chunks per lane
   const int mj = per_lane <= 4 ? 4 : 8;
   if (per_lane > 8) return MOT_ERR_UNSUPPORTED;
@@ -224,6 +247,14 @@ static int dispatch_pair(const PairParams& p, bool backward, cudaStream_t s) {
   }
 #undef MOT_PAIR_CASE
   return MOT_ERR_UNSUPPORTED;
+}
+
+static int pair_ttb_validate(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
+                             int64_t n) {
+  if (ttb_dtype < MOT_TTB_I16 || ttb_dtype > MOT_TTB_BF16) return MOT_ERR_UNSUPPORTED;
+  if (tok_vocab <= 0 || seq_len <= 0 || n % seq_len) return MOT_ERR_BAD_ARG;
+  if (n > 0 && (!tok || !ttb)) return MOT_ERR_BAD_ARG;
+  return MOT_OK;
 }
 
 static int pair_validate(const void* ids_a, const void* ids_b, int64_t n, int32_t bpt, const void* E_byte, int32_t Vb,
@@ -253,6 +284,43 @@ static void pair_fill(PairParams& p, const void* ids_a, const void* ids_b, int32
 
 using namespace mot;
 
+template <typename P>
+static int pair_fwd(const P& p, int32_t dtype, void* stream) {
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  return dtype == MOT_BF16 ? dispatch_pair<__nv_bfloat16>(p, false, s) : dispatch_pair<float>(p, false, s);
+}
+
+template <typename P>
+static int pair_bwd(P& p, int32_t dtype, void* gE_byte, void* workspace, size_t ws_bytes, void* stream) {
+  if (!gE_byte) return MOT_ERR_BAD_ARG;
+  if (reinterpret_cast<uintptr_t>(gE_byte) & 15u) return MOT_ERR_MISALIGNED;
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  const size_t esz = dtype == MOT_BF16 ? 2 : 4;
+  if (p.N == 0) {  // nothing gathered: dense zero gradient
+    if (cudaMemsetAsync(gE_byte, 0, (size_t)p.Vb * p.bd * esz, s) != cudaSuccess) return check_launch();
+    return MOT_OK;
+  }
+  const size_t need = mot_byte_pair_workspace_bytes(p.Vb, p.bd);
+  if (!workspace || ws_bytes < need) return MOT_ERR_WORKSPACE;
+  if (reinterpret_cast<uintptr_t>(workspace) & 15u) return MOT_ERR_MISALIGNED;
+  if (cudaMemsetAsync(workspace, 0, need, s) != cudaSuccess) return check_launch();
+  p.acc = reinterpret_cast<float*>(workspace);
+  if (int rc = dtype == MOT_BF16 ? dispatch_pair<__nv_bfloat16>(p, true, s) : dispatch_pair<float>(p, true, s)) return rc;
+  // sum the replicas and cast (the norm backward already happened per occurrence: no MOT_F_BYTE_NORM here)
+  EmbedParams q{};
+  q.combine = MOT_BYTES_ONLY;
+  q.N = p.N; q.R = 32; q.Vb = p.Vb; q.bd = p.bd; q.bpt = p.bpt; q.Do = p.bpt * p.bd;
+  q.n_rep = kByteRep; q.byte_acc = p.acc; q.E_byte = p.E_byte; q.gE_byte = gE_byte; q.eps = p.eps;
+  q.last_slab = 1;  // the byte rows are this launch's only work
+  const int fb = (p.Vb + 7) / 8;
+  return dtype == MOT_BF16 ? launch_finalize_bf16(q, fb, s) : launch_finalize_f32(q, fb, s);
+}
+
+static PullSrc pair_pull_src(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
+                             int32_t pad_id, int32_t eot_id, int32_t bpt) {
+  return PullSrc{tok, ttb, seq_len, tok_vocab, bpt, ttb_dtype, pad_id, eot_id, 0};
+}
+
 extern "C" int mot_byte_pair_fwd(const void* ids_a, const void* ids_b, int32_t ids_i64, int64_t n_tokens, int32_t bpt,
                                  const void* E_byte, int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps,
                                  void* out, int64_t row_stride, int32_t col_offset, void* stream) {
@@ -261,8 +329,7 @@ extern "C" int mot_byte_pair_fwd(const void* ids_a, const void* ids_b, int32_t i
   PairParams p;
   pair_fill(p, ids_a, ids_b, ids_i64, n_tokens, bpt, E_byte, byte_vocab, byte_dim, eps, row_stride, col_offset);
   p.out = out;
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  return dtype == MOT_BF16 ? dispatch_pair<__nv_bfloat16>(p, false, s) : dispatch_pair<float>(p, false, s);
+  return pair_fwd(p, dtype, stream);
 }
 
 extern "C" size_t mot_byte_pair_workspace_bytes(int32_t byte_vocab, int32_t byte_dim) {
@@ -276,29 +343,38 @@ extern "C" int mot_byte_pair_bwd(const void* ids_a, const void* ids_b, int32_t i
                                  void* workspace, size_t ws_bytes, void* stream) {
   if (int rc = pair_validate(ids_a, ids_b, n_tokens, bpt, E_byte, byte_vocab, byte_dim, dtype, grad_out, row_stride, col_offset))
     return rc;
-  if (!gE_byte) return MOT_ERR_BAD_ARG;
-  if (reinterpret_cast<uintptr_t>(gE_byte) & 15u) return MOT_ERR_MISALIGNED;
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  const size_t esz = dtype == MOT_BF16 ? 2 : 4;
-  if (n_tokens == 0) {  // nothing gathered: dense zero gradient
-    if (cudaMemsetAsync(gE_byte, 0, (size_t)byte_vocab * byte_dim * esz, s) != cudaSuccess) return check_launch();
-    return MOT_OK;
-  }
-  const size_t need = mot_byte_pair_workspace_bytes(byte_vocab, byte_dim);
-  if (!workspace || ws_bytes < need) return MOT_ERR_WORKSPACE;
-  if (reinterpret_cast<uintptr_t>(workspace) & 15u) return MOT_ERR_MISALIGNED;
-  if (cudaMemsetAsync(workspace, 0, need, s) != cudaSuccess) return check_launch();
   PairParams p;
   pair_fill(p, ids_a, ids_b, ids_i64, n_tokens, bpt, E_byte, byte_vocab, byte_dim, eps, row_stride, col_offset);
   p.gout = grad_out;
-  p.acc = reinterpret_cast<float*>(workspace);
-  if (int rc = dtype == MOT_BF16 ? dispatch_pair<__nv_bfloat16>(p, true, s) : dispatch_pair<float>(p, true, s)) return rc;
-  // sum the replicas and cast (the norm backward already happened per occurrence: no MOT_F_BYTE_NORM here)
-  EmbedParams q{};
-  q.combine = MOT_BYTES_ONLY;
-  q.N = n_tokens; q.R = 32; q.Vb = byte_vocab; q.bd = byte_dim; q.bpt = bpt; q.Do = bpt * byte_dim;
-  q.n_rep = kByteRep; q.byte_acc = p.acc; q.E_byte = E_byte; q.gE_byte = gE_byte; q.eps = eps;
-  q.last_slab = 1;  // the byte rows are this launch's only work
-  const int fb = (byte_vocab + 7) / 8;
-  return dtype == MOT_BF16 ? launch_finalize_bf16(q, fb, s) : launch_finalize_f32(q, fb, s);
+  return pair_bwd(p, dtype, gE_byte, workspace, ws_bytes, stream);
+}
+
+// The id tensors' null checks of pair_validate do not apply here: a non-null placeholder stands in for them.
+extern "C" int mot_byte_pair_ttb_fwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
+                                     int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt, const void* E_byte,
+                                     int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps, void* out,
+                                     int64_t row_stride, int32_t col_offset, void* stream) {
+  if (int rc = pair_ttb_validate(tok, ttb, tok_vocab, ttb_dtype, seq_len, n_tokens)) return rc;
+  if (int rc = pair_validate(tok, tok, n_tokens, bpt, E_byte, byte_vocab, byte_dim, dtype, out, row_stride, col_offset)) return rc;
+  if (n_tokens == 0) return MOT_OK;
+  PairTtbParams p;
+  pair_fill(p, nullptr, nullptr, 0, n_tokens, bpt, E_byte, byte_vocab, byte_dim, eps, row_stride, col_offset);
+  p.ttb = pair_pull_src(tok, ttb, tok_vocab, ttb_dtype, seq_len, pad_id, eot_id, bpt);
+  p.out = out;
+  return pair_fwd(p, dtype, stream);
+}
+
+extern "C" int mot_byte_pair_ttb_bwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
+                                     int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt, const void* E_byte,
+                                     int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps, const void* grad_out,
+                                     int64_t row_stride, int32_t col_offset, void* gE_byte, void* workspace, size_t ws_bytes,
+                                     void* stream) {
+  if (int rc = pair_ttb_validate(tok, ttb, tok_vocab, ttb_dtype, seq_len, n_tokens)) return rc;
+  if (int rc = pair_validate(tok, tok, n_tokens, bpt, E_byte, byte_vocab, byte_dim, dtype, grad_out, row_stride, col_offset))
+    return rc;
+  PairTtbParams p;
+  pair_fill(p, nullptr, nullptr, 0, n_tokens, bpt, E_byte, byte_vocab, byte_dim, eps, row_stride, col_offset);
+  p.ttb = pair_pull_src(tok, ttb, tok_vocab, ttb_dtype, seq_len, pad_id, eot_id, bpt);
+  p.gout = grad_out;
+  return pair_bwd(p, dtype, gE_byte, workspace, ws_bytes, stream);
 }

@@ -13,7 +13,7 @@ import sys
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmot_b200" + os.environ.get("MOT_LIB_SUFFIX", "") + ".so")  # suffix: experiment builds
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 # enums of include/mot_b200.h
 OK, ERR_BAD_ARG, ERR_UNSUPPORTED, ERR_MISALIGNED, ERR_WORKSPACE, ERR_CUDA, ERR_NO_DEVICE = range(7)
 BF16, F32 = 0, 1
@@ -21,6 +21,7 @@ TTB_I16, TTB_F32, TTB_BF16 = 0, 1, 2
 ADD, CONCAT, TOK_ONLY, BYTES_ONLY, MEAN = range(5)
 F_TOK_NORM, F_BYTE_NORM, F_OUT_NORM, F_BYTES_FIRST = 1, 2, 4, 8
 F_SLOT_MAJOR, F_IDS_FROM_TTB, F_TTB_SCRAMBLE, F_IDS_I64, F_HAS_LAMBDAS = 16, 32, 64, 128, 256
+F_TTB_PULL_LEFT = 512
 WS_PLAN_READY, WS_CLEAN, WS_PLAN_JOINED = 1, 2, 4
 DP_NVLS, DP_P2P = 0, 1
 
@@ -34,6 +35,7 @@ class MotDesc(C.Structure):
         ("combine", C.c_int32), ("flags", C.c_int32), ("ttb_dtype", C.c_int32),
         ("eps", C.c_float),
         ("row_stride", C.c_int64), ("col_offset", C.c_int32), ("dp_slabs", C.c_int32),
+        ("pad_id", C.c_int32), ("eot_id", C.c_int32),
     ]
 
 
@@ -71,6 +73,11 @@ _SIGNATURES = {
     "mot_byte_pair_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32]),
     "mot_byte_pair_bwd": (C.c_int, [_P, _P, C.c_int32, C.c_int64, C.c_int32, _P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P,
                                     C.c_int64, C.c_int32, _P, _P, C.c_size_t, _P]),
+    "mot_byte_pair_ttb_fwd": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int32,
+                                        _P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, C.c_int64, C.c_int32, _P]),
+    "mot_byte_pair_ttb_bwd": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int32,
+                                        _P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, C.c_int64, C.c_int32, _P, _P,
+                                        C.c_size_t, _P]),
     "mot_dp_exchange": (C.c_int, [_P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int64, C.c_int64, C.c_int32, C.c_uint32, C.c_int32,
                                   C.c_int32, _P]),
     "mot_embed_touched_rows": (C.c_int, [C.POINTER(MotDesc), _P, C.c_size_t, _P, _P]),

@@ -51,13 +51,13 @@ _COMBINE_NAMES = tuple(O._COMBINE)   # the combine mode is its index in this ord
 def pack_spec(spec) -> int:
     return (_COMBINE_NAMES.index(spec.combine) | (16 if spec.tok_norm else 0) | (32 if spec.byte_norm else 0) |
             (64 if spec.out_norm else 0) | (128 if spec.bytes_first else 0) | (256 if spec.slot_major else 0) |
-            (512 if spec.ttb_scramble else 0))
+            (512 if spec.ttb_scramble else 0) | (1024 if spec.ttb_pull else 0))
 
 
 def unpack_spec(code: int, eps: float):
     return O.MixSpec(combine=_COMBINE_NAMES[code & 15], tok_norm=bool(code & 16), byte_norm=bool(code & 32),
                      out_norm=bool(code & 64), bytes_first=bool(code & 128), slot_major=bool(code & 256),
-                     ttb_scramble=bool(code & 512), eps=eps)
+                     ttb_scramble=bool(code & 512), ttb_pull=bool(code & 1024), eps=eps)
 
 
 _PLANNERS: dict = {}
@@ -237,24 +237,28 @@ tok_gather_op.register_autograd(_tok_gather_backward, setup_context=_tok_gather_
 # ---------------------------------------------------------------------------------------------------------------
 @torch.library.custom_op("mot_b200::embed_proj", mutates_args=(), device_types="cuda")
 def embed_proj_op(tok: Tensor, ids: Tensor, ids2: Optional[Tensor], E_tok: Tensor, E_byte: Tensor, W: Tensor,
-                  bias: Optional[Tensor], spec: int, bpt: int, eps: float, plan: bool) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
-    """-> (out [n, Do], Y = the product before the row norm or [0], W in the compute dtype or [0], workspace or [0])."""
+                  bias: Optional[Tensor], spec: int, bpt: int, eps: float, plan: bool, ttb: Optional[Tensor] = None,
+                  seq_len: int = 0, ttb_pair: bool = False) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """-> (out [n, Do], Y = the product before the row norm or [0], W in the compute dtype or [0], workspace or [0]).
+    With `ttb` the byte ids come from the table inside the kernels and `ids` is an unused placeholder."""
     dev, cdt = E_tok.device, E_tok.dtype
     sp = unpack_spec(spec, eps)
-    desc = O._proj_desc(sp, bpt, tok, ids, E_tok, E_byte, ids2 is not None)
+    ids = ids if ttb is None else None
+    pair = ids2 is not None or ttb_pair
+    desc = O._proj_desc(sp, bpt, tok, ids, E_tok, E_byte, pair, ttb, seq_len)
     w_c = W if W.dtype == cdt else O.cast_out(W, cdt)
     planned = plan and tok.numel() > 0
     ws = _plan_beside(desc, tok, dev) if planned else _empty(dev)
-    out, Y, _ = O._proj_forward(sp, desc, bpt, tok, ids, ids2, E_tok, E_byte, w_c, bias, False)
+    out, Y, _ = O._proj_forward(sp, desc, bpt, tok, ids, ids2, E_tok, E_byte, w_c, bias, False, ttb, seq_len, pair)
     if planned:
         _rejoin(dev)
     return out, (Y if sp.out_norm else _empty(dev, cdt)), (w_c if w_c is not W else _empty(dev, cdt)), ws
 
 
 @embed_proj_op.register_fake
-def _(tok, ids, ids2, E_tok, E_byte, W, bias, spec, bpt, eps, plan):
+def _(tok, ids, ids2, E_tok, E_byte, W, bias, spec, bpt, eps, plan, ttb=None, seq_len=0, ttb_pair=False):
     sp = unpack_spec(spec, eps)
-    desc = O._proj_desc(sp, bpt, tok, ids, E_tok, E_byte, ids2 is not None)
+    desc = O._proj_desc(sp, bpt, tok, ids if ttb is None else None, E_tok, E_byte, ids2 is not None or ttb_pair, ttb, seq_len)
     n, cdt = tok.numel(), E_tok.dtype
     out = E_tok.new_empty((n, W.shape[0]))
     Y = E_tok.new_empty((n, W.shape[0]) if sp.out_norm else (0,))
@@ -265,36 +269,44 @@ def _(tok, ids, ids2, E_tok, E_byte, W, bias, spec, bpt, eps, plan):
 @torch.library.custom_op("mot_b200::embed_proj_bwd", mutates_args=(), device_types="cuda")
 def embed_proj_bwd_op(grad_out: Tensor, tok: Tensor, ids: Tensor, ids2: Optional[Tensor], E_tok: Tensor, E_byte: Tensor,
                       W: Tensor, w_c: Tensor, Y: Tensor, ws: Tensor, spec: int, bpt: int, eps: float,
-                      has_bias: bool) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+                      has_bias: bool, ttb: Optional[Tensor] = None, seq_len: int = 0,
+                      ttb_pair: bool = False) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
     """-> (gE_tok, gE_byte, gW in W's dtype, g_bias fp32 [Do] or [0])."""
     dev = E_tok.device
     sp = unpack_spec(spec, eps)
-    desc = O._proj_desc(sp, bpt, tok, ids, E_tok, E_byte, ids2 is not None)
+    ids = ids if ttb is None else None
+    pair = ids2 is not None or ttb_pair
+    desc = O._proj_desc(sp, bpt, tok, ids, E_tok, E_byte, pair, ttb, seq_len)
     dA, gW, g_bias = O._proj_backward(sp, desc, bpt, tok, ids, ids2, E_tok, E_byte, w_c if w_c.numel() > 0 else W,
-                                      W.dtype, has_bias, Y, None, grad_out)    # the operand is gathered again, not kept
+                                      W.dtype, has_bias, Y, None, grad_out,    # the operand is gathered again, not kept
+                                      ttb, seq_len, pair)
     ws, planned = _bwd_workspace(ws, desc, dev)
-    gE_tok, gE_byte = O._scatter_operand(sp, desc, bpt, tok, ids, ids2, E_tok, E_byte, dA, ws, planned, planned)
+    gE_tok, gE_byte = O._scatter_operand(sp, desc, bpt, tok, ids, ids2, E_tok, E_byte, dA, ws, planned, planned,
+                                         ttb, seq_len, pair)
     return gE_tok, gE_byte, gW, (g_bias if has_bias else _empty(dev, torch.float32))
 
 
 @embed_proj_bwd_op.register_fake
-def _(grad_out, tok, ids, ids2, E_tok, E_byte, W, w_c, Y, ws, spec, bpt, eps, has_bias):
+def _(grad_out, tok, ids, ids2, E_tok, E_byte, W, w_c, Y, ws, spec, bpt, eps, has_bias, ttb=None, seq_len=0, ttb_pair=False):
     return (torch.empty_like(E_tok), torch.empty_like(E_byte), torch.empty_like(W),
             E_tok.new_empty((W.shape[0] if has_bias else 0,), dtype=torch.float32))
 
 
 def _proj_setup(ctx, inputs, output):
-    tok, ids, ids2, E_tok, E_byte, W, bias, spec, bpt, eps, plan = inputs
+    tok, ids, ids2, E_tok, E_byte, W, bias, spec, bpt, eps, plan, ttb, seq_len, ttb_pair = inputs
     out, Y, w_c, ws = output
-    ctx.save_for_backward(tok, ids, ids2, E_tok, E_byte, W, w_c, Y, ws)
+    ctx.save_for_backward(tok, ids, ids2, E_tok, E_byte, W, w_c, Y, ws, ttb)
     ctx.cfg = (spec, bpt, eps, bias is not None)
+    ctx.ttb_cfg = (seq_len, ttb_pair)
     ctx.bias_dtype = bias.dtype if bias is not None else None
 
 
 def _proj_backward(ctx, g_out, g_Y, g_wc, g_ws):
-    tok, ids, ids2, E_tok, E_byte, W, w_c, Y, ws = ctx.saved_tensors
-    gt, gb, gW, gbias = torch.ops.mot_b200.embed_proj_bwd(g_out, tok, ids, ids2, E_tok, E_byte, W, w_c, Y, ws, *ctx.cfg)
-    return (None, None, None, gt, gb, gW, gbias.to(ctx.bias_dtype) if ctx.cfg[3] else None, None, None, None, None)
+    tok, ids, ids2, E_tok, E_byte, W, w_c, Y, ws, ttb = ctx.saved_tensors
+    gt, gb, gW, gbias = torch.ops.mot_b200.embed_proj_bwd(g_out, tok, ids, ids2, E_tok, E_byte, W, w_c, Y, ws, *ctx.cfg,
+                                                          ttb, *ctx.ttb_cfg)
+    return (None, None, None, gt, gb, gW, gbias.to(ctx.bias_dtype) if ctx.cfg[3] else None, None, None, None, None,
+            None, None, None)
 
 
 embed_proj_op.register_autograd(_proj_backward, setup_context=_proj_setup)
@@ -305,22 +317,25 @@ embed_proj_op.register_autograd(_proj_backward, setup_context=_proj_setup)
 # ---------------------------------------------------------------------------------------------------------------
 @torch.library.custom_op("mot_b200::embed_byte_fc", mutates_args=(), device_types="cuda")
 def embed_byte_fc_op(tok: Tensor, ids: Tensor, E_tok: Tensor, E_byte: Tensor, W: Tensor, spec_b: int, bpt: int, eps: float,
-                     plan: bool) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
-    """-> (out [n, D], Y = the byte-FC product, W in the compute dtype or [0], workspace or [0])."""
+                     plan: bool, ttb: Optional[Tensor] = None, seq_len: int = 0) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """-> (out [n, D], Y = the byte-FC product, W in the compute dtype or [0], workspace or [0]).  With `ttb` the byte
+    ids come from the table inside the kernels and `ids` is an unused placeholder."""
     dev, cdt = E_tok.device, E_tok.dtype
-    desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, tok, ids, E_tok, E_byte)
+    ids = ids if ttb is None else None
+    desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, tok, ids, E_tok, E_byte, ttb, seq_len)
     w_c = W if W.dtype == cdt else O.cast_out(W, cdt)
     planned = plan and tok.numel() > 0
     ws = _plan_beside(desc_t, tok, dev) if planned else _empty(dev)
-    out, Y = O._byte_fc_forward(desc_b, desc_t, tok, ids, E_tok, E_byte, w_c)
+    out, Y = O._byte_fc_forward(desc_b, desc_t, tok, ids, E_tok, E_byte, w_c, ttb)
     if planned:
         _rejoin(dev)
     return out, Y, (w_c if w_c is not W else _empty(dev, cdt)), ws
 
 
 @embed_byte_fc_op.register_fake
-def _(tok, ids, E_tok, E_byte, W, spec_b, bpt, eps, plan):
-    desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, tok, ids, E_tok, E_byte)
+def _(tok, ids, E_tok, E_byte, W, spec_b, bpt, eps, plan, ttb=None, seq_len=0):
+    desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, tok, ids if ttb is None else None, E_tok, E_byte, ttb,
+                                 seq_len)
     n, D = tok.numel(), E_tok.shape[1]
     return (E_tok.new_empty((n, D)), E_tok.new_empty((n, D)), E_tok.new_empty(tuple(W.shape) if W.dtype != E_tok.dtype else (0,)),
             E_tok.new_empty((O.embed_workspace_bytes(desc_t) if plan and n > 0 else 0,), dtype=torch.uint8))
@@ -328,31 +343,35 @@ def _(tok, ids, E_tok, E_byte, W, spec_b, bpt, eps, plan):
 
 @torch.library.custom_op("mot_b200::embed_byte_fc_bwd", mutates_args=(), device_types="cuda")
 def embed_byte_fc_bwd_op(grad_out: Tensor, tok: Tensor, ids: Tensor, E_tok: Tensor, E_byte: Tensor, W: Tensor, w_c: Tensor,
-                         Y: Tensor, ws: Tensor, spec_b: int, bpt: int, eps: float) -> Tuple[Tensor, Tensor, Tensor]:
+                         Y: Tensor, ws: Tensor, spec_b: int, bpt: int, eps: float, ttb: Optional[Tensor] = None,
+                         seq_len: int = 0) -> Tuple[Tensor, Tensor, Tensor]:
     dev = E_tok.device
-    desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, tok, ids, E_tok, E_byte)
+    ids = ids if ttb is None else None
+    desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, tok, ids, E_tok, E_byte, ttb, seq_len)
     ws, planned = _bwd_workspace(ws, desc_t, dev)
     wsb = torch.empty(O.embed_workspace_bytes(desc_b), dtype=torch.uint8, device=dev)
     return O._byte_fc_backward(desc_b, desc_t, tok, ids, E_tok, E_byte, w_c if w_c.numel() > 0 else W, W.dtype, Y,
-                               grad_out, ws, planned, planned, wsb, False)
+                               grad_out, ws, planned, planned, wsb, False, ttb)
 
 
 @embed_byte_fc_bwd_op.register_fake
-def _(grad_out, tok, ids, E_tok, E_byte, W, w_c, Y, ws, spec_b, bpt, eps):
+def _(grad_out, tok, ids, E_tok, E_byte, W, w_c, Y, ws, spec_b, bpt, eps, ttb=None, seq_len=0):
     return torch.empty_like(E_tok), torch.empty_like(E_byte), torch.empty_like(W)
 
 
 def _fc_setup(ctx, inputs, output):
-    tok, ids, E_tok, E_byte, W, spec_b, bpt, eps, plan = inputs
+    tok, ids, E_tok, E_byte, W, spec_b, bpt, eps, plan, ttb, seq_len = inputs
     out, Y, w_c, ws = output
-    ctx.save_for_backward(tok, ids, E_tok, E_byte, W, w_c, Y, ws)
+    ctx.save_for_backward(tok, ids, E_tok, E_byte, W, w_c, Y, ws, ttb)
     ctx.cfg = (spec_b, bpt, eps)
+    ctx.seq_len = seq_len
 
 
 def _fc_backward(ctx, g_out, g_Y, g_wc, g_ws):
-    tok, ids, E_tok, E_byte, W, w_c, Y, ws = ctx.saved_tensors
-    gt, gb, gW = torch.ops.mot_b200.embed_byte_fc_bwd(g_out, tok, ids, E_tok, E_byte, W, w_c, Y, ws, *ctx.cfg)
-    return None, None, gt, gb, gW, None, None, None, None
+    tok, ids, E_tok, E_byte, W, w_c, Y, ws, ttb = ctx.saved_tensors
+    gt, gb, gW = torch.ops.mot_b200.embed_byte_fc_bwd(g_out, tok, ids, E_tok, E_byte, W, w_c, Y, ws, *ctx.cfg, ttb,
+                                                      ctx.seq_len)
+    return None, None, gt, gb, gW, None, None, None, None, None, None
 
 
 embed_byte_fc_op.register_autograd(_fc_backward, setup_context=_fc_setup)

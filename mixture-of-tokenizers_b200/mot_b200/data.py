@@ -72,11 +72,13 @@ def tokens_to_device(tokens: torch.Tensor, device) -> torch.Tensor:
 
 def create_batch(toks: torch.Tensor, ttb_in: Optional[torch.Tensor], ttb_out: Optional[torch.Tensor], bytes_per_token: int, *,
                  byte_in: bool = True, pull_in: bool = True, byte_out: bool = False, pull_out: bool = False,
-                 padding_in: str = "left", padding_out: str = "left", pad_byte: int = 456, eot_byte: int = 457):
+                 padding_in: str = "left", padding_out: str = "left", pad_byte: int = 456, eot_byte: int = 457,
+                 byte_ids: bool = True):
     """The `_create_data_from_toks_*` family (spt/train_gpt.py:686-764) for toks [B, S+1] on the device ->
     (toks_in [B,S], bytes_padded_in [B,S*bpt] | None, bytes_pulled_in | None, targets).  (byte_in, pull_in, byte_out,
     pull_out) = (byte_mixin_method != "noop", pull_in, byte_mixout_method != "noop", pull_out) as at :766-779; invalid
-    combinations raise KeyError like the reference's dict lookup."""
+    combinations raise KeyError like the reference's dict lookup.  byte_ids=False skips the input byte tensors (both
+    None): a loader then ships token ids only and the embedding derives the ids from its ttb table."""
     _require_cuda(toks, ttb_in, ttb_out)
     key = (bool(byte_in), bool(pull_in), bool(byte_out), bool(pull_out))
     valid = {(True, True, True, True), (True, False, True, True), (True, True, True, False), (True, True, False, False),
@@ -86,7 +88,7 @@ def create_batch(toks: torch.Tensor, ttb_in: Optional[torch.Tensor], ttb_out: Op
     bpt = bytes_per_token
     pull = {"left": pull_from_left, "right": pull_from_right}
     bytes_padded_in = bytes_pulled_in = None
-    if byte_in:
+    if byte_in and byte_ids:
         full = ttb_expand(toks, ttb_in)                                                # tokens_to_bytes(toks, ttb_in)
         if pull_in:
             bytes_pulled_in = pull[padding_in](full, bpt, pad_byte, eot_byte)[:, :-bpt].contiguous()
@@ -105,10 +107,12 @@ def distributed_data_generator(filename_patterns: Union[str, Sequence[str]], seq
                                world_size: int, *, bytes_per_token: int, ttb_in: Optional[torch.Tensor] = None,
                                ttb_out: Optional[torch.Tensor] = None, byte_in: bool = True, pull_in: bool = True,
                                byte_out: bool = False, pull_out: bool = False, padding_in: str = "left",
-                               padding_out: str = "left", device="cuda", seed: int = 12345) -> Iterator[Tuple]:
+                               padding_out: str = "left", device="cuda", seed: int = 12345,
+                               byte_ids: bool = True) -> Iterator[Tuple]:
     """`distributed_data_generator` (spt/train_gpt.py:651-806): same shard order (sorted glob, `random.seed(seed)`
     shuffle), same windows (rank r takes `data[pos + r*local : pos + (r+1)*local]` viewed as [-1, seq_len+1]), batches
-    built by create_batch on the device.  Raises StopIteration when the shards run out, like the reference."""
+    built by create_batch on the device (byte_ids=False: token ids only).  Raises StopIteration when the shards run out,
+    like the reference."""
     if isinstance(filename_patterns, str):
         filename_patterns = [filename_patterns]
     files: List[str] = []
@@ -142,4 +146,5 @@ def distributed_data_generator(filename_patterns: Union[str, Sequence[str]], seq
         window = data[pos + rank * local_batch_size:][:local_batch_size].view(-1, local_seq_len)
         pos += batch_size * local_seq_len
         yield create_batch(tokens_to_device(window, device), ttb_in, ttb_out, bytes_per_token, byte_in=byte_in, pull_in=pull_in,
-                           byte_out=byte_out, pull_out=pull_out, padding_in=padding_in, padding_out=padding_out)
+                           byte_out=byte_out, pull_out=pull_out, padding_in=padding_in, padding_out=padding_out,
+                           byte_ids=byte_ids)

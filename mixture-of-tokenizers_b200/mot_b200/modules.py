@@ -10,6 +10,7 @@ Reference call sites:
 """
 from __future__ import annotations
 
+import dataclasses
 from typing import Optional
 
 import torch
@@ -38,15 +39,16 @@ class MoTEmbedding(nn.Module):
     `embed_bytes.weight` (and `lambdas` = the two trailing entries of the reference's `scalars`,
     [byte, token] order as in runs/74:259,314-315); forward(token_inputs [T] int32,
     byte_inputs int32 [bpt, T] or [1, T*bpt]) -> [1, T, model_dim].  With byte_inputs=None and a ttb
-    table the byte ids are derived inside the kernel (no-pull path)."""
+    table the byte ids are derived inside the kernel: the padded ids, or with pull_in=True the pulled ids of
+    pull_from_left over the T tokens."""
 
     def __init__(self, token_vocab_size: int, byte_vocab_size: int, token_dim: int, byte_dim: int,
                  bytes_per_token: int = 16, variant: str = "V3", ttb: Optional[torch.Tensor] = None,
-                 lambda_init=(0.5, 0.5)):
+                 lambda_init=(0.5, 0.5), pull_in: bool = False):
         super().__init__()
         if variant not in RUN_VARIANTS:
             raise NotImplementedError(f"mot_b200: variant {variant!r} has no fused kernel")
-        self.variant, self.bpt = variant, bytes_per_token
+        self.variant, self.bpt, self.pull_in = variant, bytes_per_token, pull_in
         self.spec = MixSpec(**RUN_VARIANTS[variant])
         self.embed_tokens = nn.Embedding(token_vocab_size, token_dim) if variant != "V5" else None
         self.embed_bytes = nn.Embedding(byte_vocab_size, byte_dim) if variant != "V0" else None
@@ -74,8 +76,9 @@ class MoTEmbedding(nn.Module):
         spec = self.spec
         if byte_inputs is None and self.embed_bytes is not None:
             spec = MixSpec(**{**RUN_VARIANTS[self.variant], "slot_major": False,
-                              "ttb_scramble": RUN_VARIANTS[self.variant].get("slot_major", False)})
-        x = mot_embed(token_inputs if self.embed_tokens is not None else None, byte_inputs,
+                              "ttb_scramble": RUN_VARIANTS[self.variant].get("slot_major", False), "ttb_pull": self.pull_in})
+        derive = byte_inputs is None and self.embed_bytes is not None   # the ids come from the tokens and the ttb table
+        x = mot_embed(token_inputs if self.embed_tokens is not None or derive else None, byte_inputs,
                       self.embed_tokens.weight if self.embed_tokens is not None else None,
                       self.embed_bytes.weight if self.embed_bytes is not None else None,
                       spec, bpt=self.bpt, lam=lam, ttb=self.ttb if byte_inputs is None else None,
@@ -109,10 +112,11 @@ class MoTProjEmbedding(nn.Module):
     """The concat + projection front of the modded-nanogpt runs (runs/7, 72, 75-79): parameters `embed_tokens.weight`,
     `embed_bytes.weight`, `byte_mixin_weight` [model_dim, token_dim + bpt*byte_dim] (bf16 like runs/7:249).
     forward(token_inputs [T] int32, byte_inputs int32 [1, T*bpt] (V1) or [bpt, T] (V2)) -> [1, T, model_dim]:
-    fused gather of the [tok | bytes] operand, tcgen05 projection, rms_norm."""
+    fused gather of the [tok | bytes] operand, tcgen05 projection, rms_norm.  With a ttb table, byte_inputs=None derives
+    the ids inside the kernels (the pulled ids of pull_from_left over the T tokens with pull_in=True)."""
 
     def __init__(self, token_vocab_size: int, byte_vocab_size: int, token_dim: int, byte_dim: int, model_dim: int,
-                 bytes_per_token: int = 16, variant: str = "V1"):
+                 bytes_per_token: int = 16, variant: str = "V1", ttb: Optional[torch.Tensor] = None, pull_in: bool = False):
         super().__init__()
         if variant not in PROJ_VARIANTS:
             raise NotImplementedError(f"mot_b200: projection variant {variant!r} has no fused kernel")
@@ -122,11 +126,18 @@ class MoTProjEmbedding(nn.Module):
         self.embed_bytes = nn.Embedding(byte_vocab_size, byte_dim)
         self.byte_mixin_weight = nn.Parameter(
             _init_linear_(torch.empty(model_dim, token_dim + bytes_per_token * byte_dim)).bfloat16())
+        self.register_buffer("ttb", ttb, persistent=False)
+        self.pull_in = pull_in
 
-    def forward(self, token_inputs: torch.Tensor, byte_inputs: torch.Tensor) -> torch.Tensor:
+    def forward(self, token_inputs: torch.Tensor, byte_inputs: Optional[torch.Tensor] = None) -> torch.Tensor:
         assert token_inputs.ndim == 1  # runs/7:305
+        spec = self.spec
+        if byte_inputs is None:
+            spec = MixSpec(**{**PROJ_VARIANTS[self.variant], "slot_major": False,
+                              "ttb_scramble": PROJ_VARIANTS[self.variant].get("slot_major", False), "ttb_pull": self.pull_in})
         x = mot_embed_proj(token_inputs, byte_inputs, self.embed_tokens.weight, self.embed_bytes.weight,
-                           self.byte_mixin_weight, self.spec, bpt=self.bpt)
+                           self.byte_mixin_weight, spec, bpt=self.bpt, ttb=self.ttb if byte_inputs is None else None,
+                           seq_len=token_inputs.numel())
         return x[None]
 
 
@@ -236,11 +247,15 @@ class SptByteMixEmbedding(nn.Module):
     `embed.embed_bytes.weight`, `byte_mixin.mixin.mixin.weight` (fp32 master, cast to bf16 per call like
     CastedLinear, gradient returned in fp32).  byte_mixin_method "noop" gives norm(embed_tokens(tokens)).
     add_padded_and_pulled=True sums the padded and the pulled byte rows before the per-byte norm (:371-379).
-    Refused (no fallback): cross_attn, byte self-attention."""
+    With the input ttb table `ttb` ([V, bpt], left padded), forward(tokens) alone derives the byte ids inside the
+    kernels (both byte tensors None): the pulled ids of every row of S tokens with pull_in, else the padded ids.
+    Refused (no fallback): cross_attn, byte self-attention; right-padded pulls from token ids alone (a token's pulled
+    bytes come from the tokens after it, and the last input token needs the one after the row)."""
 
     def __init__(self, vocab_size: int, byte_vocab_size: int, token_dim: int, byte_dim: int, model_dim: int,
                  bytes_per_token: int = 16, byte_mixin_method: str = "concat", pull_in: bool = True,
-                 add_padded_and_pulled: bool = False, use_byte_self_attn: bool = False):
+                 add_padded_and_pulled: bool = False, use_byte_self_attn: bool = False,
+                 ttb: Optional[torch.Tensor] = None, padding_in: str = "left"):
         super().__init__()
         if byte_mixin_method not in ("concat", "noop"):
             raise NotImplementedError(f"mot_b200: byte_mixin_method={byte_mixin_method!r} is attention pooling, "
@@ -259,6 +274,10 @@ class SptByteMixEmbedding(nn.Module):
             self.byte_mixin.mixin.mixin.weight = nn.Parameter(
                 _init_linear_(torch.empty(model_dim, token_dim + bytes_per_token * byte_dim)))
         self.spec = MixSpec(combine="concat", tok_norm=True, byte_norm=True, out_norm=True)
+        if padding_in not in ("left", "right"):
+            raise ValueError(f"padding_in must be 'left' or 'right', got {padding_in!r}")
+        self.padding_in = padding_in
+        self.register_buffer("ttb", ttb, persistent=False)
 
     def forward(self, tokens: torch.Tensor, byte_tensor: Optional[torch.Tensor] = None,
                 byte_tensor_pulled: Optional[torch.Tensor] = None) -> torch.Tensor:
@@ -266,6 +285,8 @@ class SptByteMixEmbedding(nn.Module):
         if self.method == "noop":   # _forward_tokens, :342-348
             x = mot_embed(tokens, None, self.embed.embed_tokens.weight, None, MixSpec(combine="tok_only"))
             return x.view(B, S, -1)
+        if byte_tensor is None and byte_tensor_pulled is None and self.ttb is not None:
+            return self._forward_from_tokens(tokens)
         ids = byte_tensor_pulled if self.pull_in else byte_tensor   # _forward_bytes_pulled / _padded, :350-369
         if ids is None:
             raise RuntimeError("mot_b200: byte ids are required (byte_tensor_pulled with pull_in, else byte_tensor)")
@@ -276,6 +297,17 @@ class SptByteMixEmbedding(nn.Module):
             ids, ids2 = byte_tensor, byte_tensor_pulled
         x = mot_embed_proj(tokens, ids, self.embed.embed_tokens.weight, self.embed.embed_bytes.weight,
                            self.byte_mixin.mixin.mixin.weight, self.spec, bpt=self.bpt, byte_ids2=ids2)
+        return x.view(B, S, -1)
+
+    def _forward_from_tokens(self, tokens: torch.Tensor) -> torch.Tensor:
+        B, S = tokens.shape
+        if self.pull_in and self.padding_in == "right":
+            raise NotImplementedError("mot_b200: pulled ids of right-padded rows need the token after the last input; "
+                                      "pass byte_tensor_pulled instead")
+        spec = dataclasses.replace(self.spec, ttb_pull=self.pull_in and not self.add_padded_and_pulled)
+        x = mot_embed_proj(tokens, None, self.embed.embed_tokens.weight, self.embed.embed_bytes.weight,
+                           self.byte_mixin.mixin.mixin.weight, spec, bpt=self.bpt, ttb=self.ttb, seq_len=S,
+                           padded_and_pulled=self.add_padded_and_pulled)
         return x.view(B, S, -1)
 
 

@@ -27,6 +27,7 @@ class MixSpec:
     bytes_first: bool = False     # concat order [bytes | tok]      mathblations/model.py:267
     slot_major: bool = False      # byte ids are [bpt, T]           runs/71:479
     ttb_scramble: bool = False    # ids from ttb with the `.view(bpt,-1)` index map
+    ttb_pull: bool = False        # ids from ttb: the pulled ids of pull_from_left over rows of seq_len tokens
     eps: float = FP32_EPS
 
 
@@ -175,9 +176,12 @@ def pull_from_right(byte_tensor: torch.Tensor, bytes_per_token: int, pad_byte: i
     return _pull(byte_tensor, bytes_per_token, pad_byte, eot_byte, True)
 
 
+PAD_ID, EOT_ID = 456, 457   # pad and end-of-text byte of the ttb tables (spt/data_creation.py; pull_from_left's defaults)
+
+
 def make_desc(spec: MixSpec, n_tokens: int, E_tok, E_byte, bpt: int, *, ids: Optional[torch.Tensor],
               ttb: Optional[torch.Tensor], has_lam: bool, seq_len: int = 0, row_stride: int = 0,
-              col_offset: int = 0, dp_slabs: int = 0) -> L.MotDesc:
+              col_offset: int = 0, dp_slabs: int = 0, pad_id: int = PAD_ID, eot_id: int = EOT_ID) -> L.MotDesc:
     ref = E_tok if E_tok is not None else E_byte
     if ref.dtype not in _DTYPE:
         raise NotImplementedError(f"mot_b200: embedding dtype {ref.dtype} is not supported (bf16 / fp32 only)")
@@ -205,13 +209,17 @@ def make_desc(spec: MixSpec, n_tokens: int, E_tok, E_byte, bpt: int, *, ids: Opt
                 raise RuntimeError("mot_b200: need byte ids or a ttb table")
             flags |= L.F_IDS_FROM_TTB
             flags |= L.F_TTB_SCRAMBLE if spec.ttb_scramble else 0
+            flags |= L.F_TTB_PULL_LEFT if spec.ttb_pull else 0
             ttb_dtype = _TTB_DTYPE[ttb.dtype]
         else:
             flags |= L.F_SLOT_MAJOR if spec.slot_major else 0
             flags |= L.F_IDS_I64 if ids.dtype == torch.int64 else 0
+    # without a token table the token ids still index the ttb table when the kernels derive the byte ids from it
+    tok_vocab = E_tok.shape[0] if has_tok else (ttb.shape[0] if has_bytes and ids is None else 0)
     return L.MotDesc(L.ABI_VERSION, _DTYPE[ref.dtype], n_tokens, seq_len,
-                     E_tok.shape[0] if has_tok else 0, E_byte.shape[0] if has_bytes else 0, bpt if has_bytes else 0,
-                     Dt, bd, Do, _COMBINE[spec.combine], flags, ttb_dtype, spec.eps, row_stride, col_offset, dp_slabs)
+                     tok_vocab, E_byte.shape[0] if has_bytes else 0, bpt if has_bytes else 0,
+                     Dt, bd, Do, _COMBINE[spec.combine], flags, ttb_dtype, spec.eps, row_stride, col_offset, dp_slabs,
+                     pad_id, eot_id)
 
 
 def embed_forward_out(desc: L.MotDesc, tok, ids, ttb, E_tok, E_byte, lam, out, stream: Optional[int] = None,
@@ -755,6 +763,34 @@ def byte_pair_backward_out(ids_a, ids_b, bpt: int, E_byte, grad_rows, col_offset
     L.check(rc, "mot_byte_pair_bwd")
 
 
+def _ttb_pair_args(tok, ttb, seq_len: int):
+    return (_ptr(tok), _ptr(ttb), ttb.shape[0], _TTB_DTYPE[ttb.dtype], seq_len, PAD_ID, EOT_ID, tok.numel())
+
+
+def byte_pair_ttb_forward_out(tok, ttb, seq_len: int, bpt: int, E_byte, out, col_offset: int, eps: float = FP32_EPS) -> None:
+    """mot_byte_pair_ttb_fwd: byte_pair_forward_out with ids_a = the padded and ids_b = the pulled ids of `tok`, both
+    derived from the ttb table inside the kernel (rows of seq_len tokens)."""
+    dev = _require_cuda(tok, ttb, E_byte, out)
+    with _on_device(dev):
+        rc = L.lib().mot_byte_pair_ttb_fwd(*_ttb_pair_args(tok, ttb, seq_len), bpt, _ptr(E_byte), E_byte.shape[0],
+                                           E_byte.shape[1], _DTYPE[E_byte.dtype], eps, _ptr(out), out.stride(0), col_offset,
+                                           _stream(dev))
+    L.check(rc, "mot_byte_pair_ttb_fwd")
+
+
+def byte_pair_ttb_backward_out(tok, ttb, seq_len: int, bpt: int, E_byte, grad_rows, col_offset: int, gE_byte,
+                               eps: float = FP32_EPS) -> None:
+    """mot_byte_pair_ttb_bwd: byte_pair_backward_out with both id sets derived from `tok` and the ttb table."""
+    dev = _require_cuda(tok, ttb, E_byte, grad_rows, gE_byte)
+    need = int(L.lib().mot_byte_pair_workspace_bytes(E_byte.shape[0], E_byte.shape[1]))
+    ws = torch.empty(need, dtype=torch.uint8, device=dev)
+    with _on_device(dev):
+        rc = L.lib().mot_byte_pair_ttb_bwd(*_ttb_pair_args(tok, ttb, seq_len), bpt, _ptr(E_byte), E_byte.shape[0],
+                                           E_byte.shape[1], _DTYPE[E_byte.dtype], eps, _ptr(grad_rows), grad_rows.stride(0),
+                                           col_offset, _ptr(gE_byte), _ptr(ws), ws.numel(), _stream(dev))
+    L.check(rc, "mot_byte_pair_ttb_bwd")
+
+
 def cast_out(w: torch.Tensor, dtype: torch.dtype) -> torch.Tensor:
     """CastedLinear's per-call `self.weight.type_as(x)` (spt/train_gpt.py:185-186) inside the library: fp32 -> bf16
     (mot_cast_f32_bf16).  Same dtype: returned as is."""
@@ -834,15 +870,37 @@ def mixout_split(x: torch.Tensor, bytes_per_token: int) -> torch.Tensor:
 _PROJ_KEEP_OPERAND = not __import__("os").environ.get("MOT_PROJ_REGATHER")
 
 
-def _proj_args(spec: MixSpec, bpt: int, tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2):
-    """mot_embed_proj's arguments checked and normalised -> (dev, tok, ids, ids2, E_tok, E_byte)."""
-    dev = _require_cuda(tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2)
+def _ttb_ids_args(spec: MixSpec, tok, ttb, seq_len: int) -> torch.Tensor:
+    """Checks of the token-only call form (byte ids derived from `ttb` inside the kernels) -> the table, contiguous."""
+    if ttb.dtype not in _TTB_DTYPE or ttb.dim() != 2:
+        raise NotImplementedError(f"mot_b200: ttb must be a 2-D int16/float32/bfloat16 table, got {ttb.dtype}")
+    if spec.ttb_pull and (seq_len <= 0 or tok.numel() % seq_len):
+        raise RuntimeError(f"mot_b200: pulled ids need rows of seq_len tokens (seq_len={seq_len}, {tok.numel()} tokens)")
+    return ttb.contiguous()
+
+
+def _proj_args(spec: MixSpec, bpt: int, tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2, ttb=None, seq_len: int = 0,
+               ttb_pair: bool = False):
+    """mot_embed_proj's arguments checked and normalised -> (dev, tok, ids, ids2, E_tok, E_byte, ttb).  Without byte
+    ids the ids come from `ttb` (the pulled ones under spec.ttb_pull; with ttb_pair the padded and the pulled ones)."""
+    dev = _require_cuda(tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2, ttb)
     _require_chain_dtype(E_tok, E_byte)
     tok = _tok_i32(tokens)
-    ids = _byte_ids(byte_ids)
-    _check_id_count(ids, tok.numel(), bpt)
-    ids2 = None
-    if byte_ids2 is not None:
+    ids = ids2 = None
+    if byte_ids is None:
+        if ttb is None:
+            raise RuntimeError("mot_b200: need byte ids or a ttb table")
+        if ttb_pair:
+            if not spec.byte_norm or spec.slot_major or spec.bytes_first or spec.ttb_scramble:
+                raise NotImplementedError("mot_b200: the padded+pulled sum exists only with per-byte norms, token-major "
+                                          "ids and [tok | bytes] order (spt/train_gpt.py:371-379,442-443)")
+            spec = dataclasses.replace(spec, ttb_pull=True)
+        ttb = _ttb_ids_args(spec, tok, ttb, seq_len)
+    else:
+        ttb = None
+        ids = _byte_ids(byte_ids)
+        _check_id_count(ids, tok.numel(), bpt)
+    if byte_ids2 is not None and ids is not None:
         # `--add-padded-and-pulled` (spt/train_gpt.py:371-379): two gathers summed before the per-byte norm.  The
         # token columns of the operand come from the fused kernel (tok-only, strided rows), the byte columns from
         # the pair kernels.
@@ -857,49 +915,57 @@ def _proj_args(spec: MixSpec, bpt: int, tokens, byte_ids, E_tok, E_byte, W, bias
         raise RuntimeError(f"mot_b200: projection weight is {tuple(W.shape)}, expected [{W.shape[0]}, {K}]")
     if bias is not None and bias.dtype != torch.float32:
         raise NotImplementedError("mot_b200: the projection bias must be fp32 (mathblations/model.py:261)")
-    return dev, tok, ids, ids2, E_tok.contiguous(), E_byte.contiguous()
+    return dev, tok, ids, ids2, E_tok.contiguous(), E_byte.contiguous(), ttb
 
 
-def _proj_desc(spec: MixSpec, bpt: int, tok, ids, E_tok, E_byte, pair: bool) -> L.MotDesc:
+def _proj_desc(spec: MixSpec, bpt: int, tok, ids, E_tok, E_byte, pair: bool, ttb=None, seq_len: int = 0) -> L.MotDesc:
     """Descriptor of the gather of the [n, K] operand: the concat of both tables, or with `pair` (two byte-id tensors)
-    only its token columns, written with row stride K (the pair kernels write the byte columns)."""
+    only its token columns, written with row stride K (the pair kernels write the byte columns).  ids=None: the ids come
+    from `ttb` (rows of seq_len tokens)."""
     if pair:
         return make_desc(MixSpec(combine="tok_only", tok_norm=spec.tok_norm, out_norm=False, eps=spec.eps), tok.numel(),
                          E_tok, None, 0, ids=None, ttb=None, has_lam=False,
                          row_stride=E_tok.shape[1] + bpt * E_byte.shape[1], col_offset=0)
     return make_desc(dataclasses.replace(spec, combine="concat", out_norm=False), tok.numel(), E_tok, E_byte, bpt,
-                     ids=ids, ttb=None, has_lam=False)
+                     ids=ids, ttb=ttb, has_lam=False, seq_len=seq_len)
 
 
-def _gather_operand(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_tok, E_byte, A) -> None:
-    if ids2 is None:
-        embed_forward_out(desc, tok, ids, None, E_tok, E_byte, None, A)
+def _gather_operand(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_tok, E_byte, A, ttb=None,
+                    seq_len: int = 0, pair: bool = False) -> None:
+    if not pair:
+        embed_forward_out(desc, tok, ids, ttb, E_tok, E_byte, None, A)
     elif tok.numel() > 0:
         embed_forward_out(desc, tok, None, None, E_tok, None, None, A)
-        byte_pair_forward_out(ids, ids2, bpt, E_byte, A, E_tok.shape[1], spec.eps)
+        if ttb is not None:
+            byte_pair_ttb_forward_out(tok, ttb, seq_len, bpt, E_byte, A, E_tok.shape[1], spec.eps)
+        else:
+            byte_pair_forward_out(ids, ids2, bpt, E_byte, A, E_tok.shape[1], spec.eps)
 
 
 def _scatter_operand(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_tok, E_byte, dA, ws_buf,
-                     plan_ready: bool, ws_clean: bool):
+                     plan_ready: bool, ws_clean: bool, ttb=None, seq_len: int = 0, pair: bool = False):
     """The backward of _gather_operand: dense (gE_tok, gE_byte) from the operand's gradient dA."""
     gE_tok, gE_byte = torch.empty_like(E_tok), torch.empty_like(E_byte)
-    if ids2 is None:
-        embed_backward_out(desc, tok, ids, None, E_tok, E_byte, None, dA, gE_tok, gE_byte, None, ws_buf,
+    if not pair:
+        embed_backward_out(desc, tok, ids, ttb, E_tok, E_byte, None, dA, gE_tok, gE_byte, None, ws_buf,
                            plan_ready=plan_ready, ws_clean=ws_clean)
     else:   # token columns through the sorted-stream scatter, byte columns through the pair kernel
         embed_backward_out(desc, tok, None, None, E_tok, None, None, dA, gE_tok, None, None, ws_buf,
                            plan_ready=plan_ready, ws_clean=ws_clean)
-        byte_pair_backward_out(ids, ids2, bpt, E_byte, dA, E_tok.shape[1], gE_byte, spec.eps)
+        if ttb is not None:
+            byte_pair_ttb_backward_out(tok, ttb, seq_len, bpt, E_byte, dA, E_tok.shape[1], gE_byte, spec.eps)
+        else:
+            byte_pair_backward_out(ids, ids2, bpt, E_byte, dA, E_tok.shape[1], gE_byte, spec.eps)
     return gE_tok, gE_byte
 
 
 def _proj_forward(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_tok, E_byte, w_c, bias,
-                  keep_operand: bool):
+                  keep_operand: bool, ttb=None, seq_len: int = 0, pair: bool = False):
     """-> (out, Y, A): Y = A . w_c^T (+ bias) with the gathered [n, K] operand A (None unless keep_operand), out = the
     row norm of Y under spec.out_norm, else Y itself.  w_c: the weight in the table dtype."""
     n, (Do, K), dev, cdt = tok.numel(), w_c.shape, E_tok.device, E_tok.dtype
     A = torch.empty((n, K), dtype=cdt, device=dev)
-    _gather_operand(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, A)
+    _gather_operand(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, A, ttb, seq_len, pair)
     Y = torch.empty((n, Do), dtype=cdt, device=dev)
     linear_forward_out(A, w_c, Y, bias.contiguous() if bias is not None else None)
     if not keep_operand:
@@ -913,7 +979,7 @@ def _proj_forward(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_to
 
 
 def _proj_backward(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_tok, E_byte, w_c, w_dtype, has_bias: bool,
-                   Y, A, grad_out):
+                   Y, A, grad_out, ttb=None, seq_len: int = 0, pair: bool = False):
     """The backward of _proj_forward down to the operand -> (dA, gW in w_dtype, g_bias fp32 or None).  A: the forward's
     operand if it was kept, else None (gathered again here)."""
     n, (Do, K), dev, cdt = tok.numel(), w_c.shape, E_tok.device, E_tok.dtype
@@ -928,7 +994,7 @@ def _proj_backward(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_t
         dA = torch.empty((n, K), dtype=cdt, device=dev)                   # a saved tensor is never overwritten
     else:
         A = torch.empty((n, K), dtype=cdt, device=dev)
-        _gather_operand(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, A)
+        _gather_operand(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, A, ttb, seq_len, pair)
         dA = A                                                            # dX may overwrite the private copy
     dW32 = torch.empty((Do, K), dtype=torch.float32, device=dev)
     dW16 = torch.empty((Do, K), dtype=torch.bfloat16, device=dev) if w_dtype == torch.bfloat16 else None
@@ -945,59 +1011,72 @@ class _MotEmbedProjFn(torch.autograd.Function):
     step); MOT_PROJ_REGATHER=1 gathers it again instead (the round-1 behaviour, for memory-tight callers)."""
 
     @staticmethod
-    def forward(ctx, spec: MixSpec, bpt: int, dev, tok, ids, ids2, E_tok, E_byte, W, bias):
-        desc = _proj_desc(spec, bpt, tok, ids, E_tok, E_byte, ids2 is not None)
+    def forward(ctx, spec: MixSpec, bpt: int, dev, tok, ids, ids2, E_tok, E_byte, W, bias, ttb=None, seq_len: int = 0,
+                pair: bool = False):
+        pair = pair or ids2 is not None
+        desc = _proj_desc(spec, bpt, tok, ids, E_tok, E_byte, pair, ttb, seq_len)
         w16 = cast_out(W, E_tok.dtype)                         # CastedLinear: W.type_as(x) (spt/train_gpt.py:186)
         ctx.ws = _planned_workspace(desc, tok, dev) if any(ctx.needs_input_grad[6:8]) and tok.numel() > 0 else None
         keep_A = _PROJ_KEEP_OPERAND and any(ctx.needs_input_grad[6:10])
-        out, Y, A = _proj_forward(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, w16, bias, keep_A)
+        out, Y, A = _proj_forward(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, w16, bias, keep_A, ttb, seq_len, pair)
         embed_plan_join_if_capturing(ctx.ws, dev)
-        ctx.desc, ctx.dev, ctx.spec, ctx.bpt = desc, dev, spec, bpt
+        ctx.desc, ctx.dev, ctx.spec, ctx.bpt, ctx.seq_len = desc, dev, spec, bpt, seq_len
         ctx.w_dtype, ctx.has_bias = W.dtype, bias is not None
-        ctx.pair, ctx.kept_A = ids2 is not None, keep_A
-        ctx.save_for_backward(tok, ids, E_tok, E_byte, w16, Y, ids2 if ids2 is not None else _ABSENT,
-                              A if keep_A else _ABSENT)
+        ctx.pair, ctx.kept_A = pair, keep_A
+        ctx.present = (ids is not None, ids2 is not None, keep_A, ttb is not None)
+        ctx.save_for_backward(tok, *[t if t is not None else _ABSENT for t in (ids, ids2, A if keep_A else None, ttb)],
+                              E_tok, E_byte, w16, Y)
         return out
 
     @staticmethod
     def backward(ctx, grad_out):
-        tok, ids, E_tok, E_byte, w16, Y, ids2, A = ctx.saved_tensors
-        desc, dev, spec, bpt = ctx.desc, ctx.dev, ctx.spec, ctx.bpt
-        ids2 = ids2 if ctx.pair else None
+        tok, ids, ids2, A, ttb, E_tok, E_byte, w16, Y = ctx.saved_tensors
+        ids, ids2, A, ttb = [t if ok else None for t, ok in zip((ids, ids2, A, ttb), ctx.present)]
+        desc, dev, spec, bpt, seq_len, pair = ctx.desc, ctx.dev, ctx.spec, ctx.bpt, ctx.seq_len, ctx.pair
         dA, gW, g_bias = _proj_backward(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, w16, ctx.w_dtype, ctx.has_bias,
-                                        Y, A if ctx.kept_A else None, grad_out)
+                                        Y, A, grad_out, ttb, seq_len, pair)
         ws, planned, clean = _take_workspace(ctx.ws, desc, dev)
-        gE_tok, gE_byte = _scatter_operand(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, dA, ws.buf, planned, clean)
+        gE_tok, gE_byte = _scatter_operand(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, dA, ws.buf, planned, clean,
+                                           ttb, seq_len, pair)
         ctx.ws = None
         _return_workspace(ws)
-        return None, None, None, None, None, None, gE_tok, gE_byte, gW, g_bias
+        return None, None, None, None, None, None, gE_tok, gE_byte, gW, g_bias, None, None, None
 
 
-def _byte_fc_args(bpt: int, tokens, byte_ids, E_tok, E_byte, W):
-    """mot_embed_byte_fc's arguments checked and normalised -> (dev, tok, ids, E_tok, E_byte)."""
-    dev = _require_cuda(tokens, byte_ids, E_tok, E_byte, W)
+def _byte_fc_args(bpt: int, tokens, byte_ids, E_tok, E_byte, W, spec_b: Optional[MixSpec] = None, ttb=None,
+                  seq_len: int = 0):
+    """mot_embed_byte_fc's arguments checked and normalised -> (dev, tok, ids, E_tok, E_byte, ttb)."""
+    dev = _require_cuda(tokens, byte_ids, E_tok, E_byte, W, ttb)
     _require_chain_dtype(E_tok, E_byte)
     tok = _tok_i32(tokens)
-    ids = _byte_ids(byte_ids)
     D = E_tok.shape[1]
-    if ids.numel() != tok.numel() * bpt or bpt * E_byte.shape[1] != D or tuple(W.shape) != (D, D):
+    if byte_ids is None:
+        if ttb is None:
+            raise RuntimeError("mot_b200: need byte ids or a ttb table")
+        ids, ttb = None, _ttb_ids_args(spec_b, tok, ttb, seq_len)
+        n_ids = tok.numel() * bpt
+    else:
+        ids, ttb = _byte_ids(byte_ids), None
+        n_ids = ids.numel()
+    if n_ids != tok.numel() * bpt or bpt * E_byte.shape[1] != D or tuple(W.shape) != (D, D):
         raise RuntimeError("mot_b200: byte-FC mix needs bpt*byte_dim == token_dim and a square [D, D] weight")
-    return dev, tok, ids, E_tok.contiguous(), E_byte.contiguous()
+    return dev, tok, ids, E_tok.contiguous(), E_byte.contiguous(), ttb
 
 
-def _fc_descs(spec_b: MixSpec, bpt: int, tok, ids, E_tok, E_byte):
-    """-> (desc_b, desc_t): the bytes-only gather of the product's operand; the token gather + addend + norm."""
+def _fc_descs(spec_b: MixSpec, bpt: int, tok, ids, E_tok, E_byte, ttb=None, seq_len: int = 0):
+    """-> (desc_b, desc_t): the bytes-only gather of the product's operand; the token gather + addend + norm.  ids=None:
+    the operand's ids come from `ttb`."""
     n = tok.numel()
-    return (make_desc(spec_b, n, None, E_byte, bpt, ids=ids, ttb=None, has_lam=False),
+    return (make_desc(spec_b, n, None, E_byte, bpt, ids=ids, ttb=ttb, has_lam=False, seq_len=seq_len),
             make_desc(MixSpec(combine="tok_only", out_norm=True, eps=spec_b.eps), n, E_tok, None, 0, ids=None, ttb=None,
                       has_lam=False))
 
 
-def _byte_fc_forward(desc_b: L.MotDesc, desc_t: L.MotDesc, tok, ids, E_tok, E_byte, w_c):
+def _byte_fc_forward(desc_b: L.MotDesc, desc_t: L.MotDesc, tok, ids, E_tok, E_byte, w_c, ttb=None):
     """-> (out, Y): Y = C . w_c^T with C the bytes-only gather (not kept), out = norm(E_tok[tok] + Y)."""
     n, D, dev, cdt = tok.numel(), E_tok.shape[1], E_tok.device, E_tok.dtype
     C = torch.empty((n, D), dtype=cdt, device=dev)
-    embed_forward_out(desc_b, None, ids, None, None, E_byte, None, C)
+    embed_forward_out(desc_b, tok if ttb is not None else None, ids, ttb, None, E_byte, None, C)
     Y = torch.empty((n, D), dtype=cdt, device=dev)
     linear_forward_out(C, w_c, Y)
     del C
@@ -1008,7 +1087,7 @@ def _byte_fc_forward(desc_b: L.MotDesc, desc_t: L.MotDesc, tok, ids, E_tok, E_by
 
 
 def _byte_fc_backward(desc_b: L.MotDesc, desc_t: L.MotDesc, tok, ids, E_tok, E_byte, w_c, w_dtype, Y, grad_out,
-                      ws_buf, plan_ready: bool, ws_clean: bool, wsb_buf, wsb_clean: bool):
+                      ws_buf, plan_ready: bool, ws_clean: bool, wsb_buf, wsb_clean: bool, ttb=None):
     """-> (gE_tok, gE_byte, gW in w_dtype).  ws_*: the workspace of the token scatter; wsb_*: the workspace of the
     bytes-only scatter, which is never planned ahead."""
     (n, D), dev, cdt = Y.shape, Y.device, Y.dtype
@@ -1018,12 +1097,13 @@ def _byte_fc_backward(desc_b: L.MotDesc, desc_t: L.MotDesc, tok, ids, E_tok, E_b
     embed_backward_out(desc_t, tok, None, None, E_tok, None, None, g, gE_tok, None, None, ws_buf,
                        plan_ready=plan_ready, ws_clean=ws_clean, addend=Y, d_addend=dY)
     C = torch.empty((n, D), dtype=cdt, device=dev)
-    embed_forward_out(desc_b, None, ids, None, None, E_byte, None, C)            # gathered again, not kept
+    tok_b = tok if ttb is not None else None                                     # the bytes-only gather reads tokens only to derive ids
+    embed_forward_out(desc_b, tok_b, ids, ttb, None, E_byte, None, C)            # gathered again, not kept
     dW32 = torch.empty((D, D), dtype=torch.float32, device=dev)
     dW16 = torch.empty((D, D), dtype=torch.bfloat16, device=dev) if w_dtype == torch.bfloat16 else None
     linear_bwd_weight_out(dY, C, dW32, dW16)
     linear_bwd_input_out(dY, w_c, C)                                             # dC overwrites the operand buffer
-    embed_backward_out(desc_b, None, ids, None, None, E_byte, None, C, None, gE_byte, None, wsb_buf,
+    embed_backward_out(desc_b, tok_b, ids, ttb, None, E_byte, None, C, None, gE_byte, None, wsb_buf,
                        plan_ready=False, ws_clean=wsb_clean)
     return gE_tok, gE_byte, (dW16 if dW16 is not None else dW32)
 
@@ -1036,56 +1116,72 @@ class _MotEmbedByteFcFn(torch.autograd.Function):
     cores; bytes-only scatter.  The operand is gathered again in the backward, not kept."""
 
     @staticmethod
-    def forward(ctx, spec_b: MixSpec, bpt: int, dev, tok, ids, E_tok, E_byte, W):
+    def forward(ctx, spec_b: MixSpec, bpt: int, dev, tok, ids, E_tok, E_byte, W, ttb=None, seq_len: int = 0):
         w16 = cast_out(W, E_tok.dtype)
-        desc_b, desc_t = _fc_descs(spec_b, bpt, tok, ids, E_tok, E_byte)
+        desc_b, desc_t = _fc_descs(spec_b, bpt, tok, ids, E_tok, E_byte, ttb, seq_len)
         ctx.ws = _planned_workspace(desc_t, tok, dev) if ctx.needs_input_grad[5] and tok.numel() > 0 else None
-        out, Y = _byte_fc_forward(desc_b, desc_t, tok, ids, E_tok, E_byte, w16)
+        out, Y = _byte_fc_forward(desc_b, desc_t, tok, ids, E_tok, E_byte, w16, ttb)
         embed_plan_join_if_capturing(ctx.ws, dev)
         ctx.desc_b, ctx.desc_t, ctx.dev, ctx.w_dtype = desc_b, desc_t, dev, W.dtype
-        ctx.save_for_backward(tok, ids, E_tok, E_byte, w16, Y)
+        ctx.present = (ids is not None, ttb is not None)
+        ctx.save_for_backward(tok, ids if ids is not None else _ABSENT, ttb if ttb is not None else _ABSENT,
+                              E_tok, E_byte, w16, Y)
         return out
 
     @staticmethod
     def backward(ctx, grad_out):
-        tok, ids, E_tok, E_byte, w16, Y = ctx.saved_tensors
+        tok, ids, ttb, E_tok, E_byte, w16, Y = ctx.saved_tensors
+        ids, ttb = [t if ok else None for t, ok in zip((ids, ttb), ctx.present)]
         ws, planned, clean = _take_workspace(ctx.ws, ctx.desc_t, ctx.dev)
         wsb, _, clean_b = _take_workspace(None, ctx.desc_b, ctx.dev)
         gE_tok, gE_byte, gW = _byte_fc_backward(ctx.desc_b, ctx.desc_t, tok, ids, E_tok, E_byte, w16, ctx.w_dtype, Y,
-                                                grad_out, ws.buf, planned, clean, wsb.buf, clean_b)
+                                                grad_out, ws.buf, planned, clean, wsb.buf, clean_b, ttb)
         ctx.ws = None
         _return_workspace(ws)
         _return_workspace(wsb)
-        return None, None, None, None, None, gE_tok, gE_byte, gW
+        return None, None, None, None, None, gE_tok, gE_byte, gW, None, None
 
 
-def mot_embed_byte_fc(tokens: torch.Tensor, byte_ids: torch.Tensor, E_tok: torch.Tensor, E_byte: torch.Tensor,
-                      W_fc: torch.Tensor, *, bpt: int = 16, slot_major: bool = True, eps: float = FP32_EPS) -> torch.Tensor:
-    """`norm(token_embs + F.linear(cat(byte_embs), byte_fc))` (runs/71051:226-229,312-314): [n_tokens, D]."""
-    dev, tok, ids, E_tok_c, E_byte_c = _byte_fc_args(bpt, tokens, byte_ids, E_tok, E_byte, W_fc)
-    spec_b = MixSpec(combine="bytes_only", out_norm=False, slot_major=slot_major, eps=eps)
+def mot_embed_byte_fc(tokens: torch.Tensor, byte_ids: Optional[torch.Tensor], E_tok: torch.Tensor, E_byte: torch.Tensor,
+                      W_fc: torch.Tensor, *, bpt: int = 16, slot_major: bool = True, eps: float = FP32_EPS,
+                      ttb: Optional[torch.Tensor] = None, seq_len: int = 0, ttb_pull: bool = False) -> torch.Tensor:
+    """`norm(token_embs + F.linear(cat(byte_embs), byte_fc))` (runs/71051:226-229,312-314): [n_tokens, D].
+    byte_ids=None: the ids come from `ttb` inside the kernels (rows of seq_len tokens; the `.view(bpt,-1)` order under
+    slot_major), the pulled ids of pull_from_left with ttb_pull."""
+    spec_b = MixSpec(combine="bytes_only", out_norm=False, slot_major=slot_major and byte_ids is not None,
+                     ttb_scramble=slot_major and byte_ids is None, ttb_pull=ttb_pull and byte_ids is None, eps=eps)
+    dev, tok, ids, E_tok_c, E_byte_c, ttb_c = _byte_fc_args(bpt, tokens, byte_ids, E_tok, E_byte, W_fc, spec_b, ttb, seq_len)
     if _custom_ops_wanted():
         need = torch.is_grad_enabled() and any(t.requires_grad for t in (E_tok, E_byte, W_fc))
-        return torch.ops.mot_b200.embed_byte_fc(tok, ids, E_tok_c, E_byte_c, W_fc.contiguous(), pack_spec(spec_b), bpt,
-                                                float(eps), need)[0]
-    return _MotEmbedByteFcFn.apply(spec_b, bpt, dev, tok, ids, E_tok_c, E_byte_c, W_fc)
+        return torch.ops.mot_b200.embed_byte_fc(tok, ids if ids is not None else tok.new_empty(0), E_tok_c, E_byte_c,
+                                                W_fc.contiguous(), pack_spec(spec_b), bpt, float(eps), need, ttb_c,
+                                                seq_len)[0]
+    return _MotEmbedByteFcFn.apply(spec_b, bpt, dev, tok, ids, E_tok_c, E_byte_c, W_fc, ttb_c, seq_len)
 
 
-def mot_embed_proj(tokens: torch.Tensor, byte_ids: torch.Tensor, E_tok: torch.Tensor, E_byte: torch.Tensor,
+def mot_embed_proj(tokens: torch.Tensor, byte_ids: Optional[torch.Tensor], E_tok: torch.Tensor, E_byte: torch.Tensor,
                    W: torch.Tensor, spec: MixSpec, *, bpt: int = 16, bias: Optional[torch.Tensor] = None,
-                   byte_ids2: Optional[torch.Tensor] = None) -> torch.Tensor:
+                   byte_ids2: Optional[torch.Tensor] = None, ttb: Optional[torch.Tensor] = None, seq_len: int = 0,
+                   padded_and_pulled: bool = False) -> torch.Tensor:
     """Concat + dense projection variants: `norm(F.linear(cat([f(tok), f(bytes)]), W))` (runs/7:226-234, runs/72,
     spt/train_gpt.py:439-443).  spec.tok_norm / byte_norm are the per-input norms, spec.out_norm the norm after the
     projection, spec.bytes_first the operand order.  Tables bf16 with W bf16 (runs) or an fp32 master (spt: cast per
     call, gradient returned in fp32); or everything fp32 (mathblations: TF32 tensor cores).  byte_ids2: the second id
     tensor of `--add-padded-and-pulled` (spt/train_gpt.py:371-379), rows summed before the per-byte norm.  Returns
-    [n_tokens, W.shape[0]] in the table dtype."""
-    dev, tok, ids, ids2, E_tok_c, E_byte_c = _proj_args(spec, bpt, tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2)
+    [n_tokens, W.shape[0]] in the table dtype.
+
+    Token-only form: byte_ids=None with the [V, bpt] table `ttb` derives the ids inside the kernels -- the padded ids, or
+    with spec.ttb_pull the pulled ids of pull_from_left over rows of `seq_len` tokens; padded_and_pulled=True derives
+    both sets of `--add-padded-and-pulled`."""
+    pair = padded_and_pulled and byte_ids is None
+    dev, tok, ids, ids2, E_tok_c, E_byte_c, ttb_c = _proj_args(spec, bpt, tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2,
+                                                               ttb, seq_len, pair)
     if _custom_ops_wanted():
         need = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (E_tok, E_byte, W, bias))
-        return torch.ops.mot_b200.embed_proj(tok, ids, ids2, E_tok_c, E_byte_c, W.contiguous(), bias, pack_spec(spec), bpt,
-                                             float(spec.eps), need)[0]
-    return _MotEmbedProjFn.apply(spec, bpt, dev, tok, ids, ids2, E_tok_c, E_byte_c, W, bias)
+        return torch.ops.mot_b200.embed_proj(tok, ids if ids is not None else tok.new_empty(0), ids2, E_tok_c, E_byte_c,
+                                             W.contiguous(), bias, pack_spec(spec), bpt, float(spec.eps), need, ttb_c,
+                                             seq_len, pair)[0]
+    return _MotEmbedProjFn.apply(spec, bpt, dev, tok, ids, ids2, E_tok_c, E_byte_c, W, bias, ttb_c, seq_len, pair)
 
 
 def launch_count() -> int:

@@ -71,10 +71,17 @@ enum {
                                   row of seq_len tokens (the `.view(bpt,-1)` of runs/71:479)           */
   MOT_F_IDS_I64 = 1 << 7,      /* byte-id tensors hold int64 (spt), else int32 (runs)                  */
   MOT_F_HAS_LAMBDAS = 1 << 8,  /* lam[0] = lam_tok, lam[1] = lam_byte (runs/74:314-315)                */
-  MOT_F_TTB_PULL_LEFT = 1 << 9 /* with IDS_FROM_TTB: the ids are the PULLED ids of pull_from_left (mot_pull) over rows of
+  MOT_F_TTB_PULL_LEFT = 1 << 9, /* with IDS_FROM_TTB: the ids are the PULLED ids of pull_from_left (mot_pull) over rows of
                                   seq_len tokens (n_tokens % seq_len == 0, bpt <= 32, tok_vocab = the ttb table's rows
                                   also for MOT_BYTES_ONLY), pad_id / eot_id as there;
                                   with TTB_SCRAMBLE the scramble picks (token, slot) and the id comes from the pulled row */
+  MOT_F_TTB_PULL_RIGHT = 1 << 10, /* the same rules with the pulled ids of pull_from_right (rows right-padded); not
+                                     together with TTB_PULL_LEFT */
+  MOT_F_TTB_NEXT_TOK = 1 << 11    /* with TTB_PULL_RIGHT only: row r has one more token, the lookahead, at
+                                     tok[n_tokens + r] for r < n_tokens / seq_len (the loader's window of seq_len + 1
+                                     tokens, whose last token the right pull of the row's end reads).  Only the pull
+                                     reads this tail: the token gathers, the sort plan and the touched-rows bitmap see
+                                     tok[0, n_tokens) */
 };
 
 typedef struct MotDesc {
@@ -98,7 +105,7 @@ typedef struct MotDesc {
   int32_t col_offset;  /* first column of this call's slice inside those rows (multiple of 8) */
   int32_t dp_slabs;    /* 0 / 1: the backward runs in one piece.  n > 1: the caller will run it as n vocabulary slabs
                           (mot_embed_bwd_slab); only sizes the workspace (one fp32 slot per finer stream chunk) */
-  int32_t pad_id;      /* with MOT_F_TTB_PULL_LEFT: the pad byte (456) and the end-of-text byte (457) of the ttb table,
+  int32_t pad_id;      /* with MOT_F_TTB_PULL_LEFT / _RIGHT: the pad byte (456) and the end-of-text byte (457) of the ttb table,
                           each in the int16 range */
   int32_t eot_id;
 } MotDesc;
@@ -273,6 +280,18 @@ int mot_byte_pair_ttb_bwd(const int32_t* tok, const void* ttb, int32_t tok_vocab
                           int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps, const void* grad_out,
                           int64_t row_stride, int32_t col_offset, void* gE_byte, void* workspace, size_t ws_bytes,
                           void* stream);
+/* The same with the pull's direction in `flags`: MOT_F_TTB_PULL_LEFT (= mot_byte_pair_ttb_fwd/bwd), or
+ * MOT_F_TTB_PULL_RIGHT, optionally with MOT_F_TTB_NEXT_TOK (the lookahead tail tok[n_tokens + r] of every row r).  ids_a
+ * stay the ttb rows of `tok`: with a right-padded table these are the right-padded ids.  Other flags: MOT_ERR_BAD_ARG. */
+int mot_byte_pair_ttb_ex_fwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
+                             int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt, const void* E_byte,
+                             int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps, void* out,
+                             int64_t row_stride, int32_t col_offset, int32_t flags, void* stream);
+int mot_byte_pair_ttb_ex_bwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
+                             int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt, const void* E_byte,
+                             int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps, const void* grad_out,
+                             int64_t row_stride, int32_t col_offset, void* gE_byte, void* workspace, size_t ws_bytes,
+                             int32_t flags, void* stream);
 
 /* ---- data-parallel exchange: average the gradient bucket across ranks through NVLink / NVSwitch -----------------
  * Replaces the per-parameter dist.all_reduce(param.grad, AVG) of spt/train_gpt.py:1320-1321 and runs/7:697-700 (launched

@@ -176,11 +176,13 @@ static int validate(const MotDesc* d) {
     if (ld % 8 || d->col_offset % 8) return MOT_ERR_MISALIGNED;
   }
   if (d->dp_slabs < 0 || d->dp_slabs > 64) return MOT_ERR_BAD_ARG;
+  if ((d->flags & MOT_F_TTB_PULL_LEFT) && (d->flags & MOT_F_TTB_PULL_RIGHT)) return MOT_ERR_BAD_ARG;
+  if ((d->flags & MOT_F_TTB_NEXT_TOK) && !(d->flags & MOT_F_TTB_PULL_RIGHT)) return MOT_ERR_BAD_ARG;
   if ((d->flags & MOT_F_IDS_FROM_TTB) && has_bytes) {
     if (d->ttb_dtype < MOT_TTB_I16 || d->ttb_dtype > MOT_TTB_BF16) return MOT_ERR_UNSUPPORTED;
-    if (d->flags & (MOT_F_TTB_SCRAMBLE | MOT_F_TTB_PULL_LEFT))
+    if (d->flags & (MOT_F_TTB_SCRAMBLE | MOT_F_TTB_PULL_LEFT | MOT_F_TTB_PULL_RIGHT))
       if (d->seq_len <= 0 || d->n_tokens % d->seq_len) return MOT_ERR_BAD_ARG;
-    if (d->flags & MOT_F_TTB_PULL_LEFT) {
+    if (d->flags & (MOT_F_TTB_PULL_LEFT | MOT_F_TTB_PULL_RIGHT)) {
       if (d->tok_vocab <= 0) return MOT_ERR_BAD_ARG;  // rows of the ttb table, also without a token table
       if (d->pad_id != (int16_t)d->pad_id || d->eot_id != (int16_t)d->eot_id) return MOT_ERR_BAD_ARG;  // int16, as in mot_pull
     }

@@ -81,7 +81,7 @@ struct SumBatch {
   int v_next;  // last batch: token id of the stream entry after the chunk (-1: none)
 };
 
-template <typename T, int CPL, bool PULL>
+template <typename T, int CPL, int PULL>
 __global__ void __launch_bounds__(kSumThreads, 1) mot_bwd_sum_kernel(const EmbedParams p) {
   constexpr int CW = kBwdCW;
   using V = Vec<T, CW>;
@@ -265,7 +265,7 @@ __global__ void __launch_bounds__(kSumThreads, 1) mot_bwd_sum_kernel(const Embed
   int id_next = 0;  // raw byte id (lane = slot) of the next occurrence, fetched one occurrence ahead
   if (A.cnt > 0) {
     const int pos0 = __shfl_sync(kFull, A.pos, 0);
-    if constexpr (PULL) id_next = pulled_lane_id(p, pos0, id_lane);
+    if constexpr (PULL) id_next = pulled_lane_id<PULL>(p, pos0, id_lane);
     else if (id_lane) id_next = load_raw_id(p, idsrc, pos0, lane);
   }
   while (A.cnt > 0) {
@@ -283,7 +283,7 @@ __global__ void __launch_bounds__(kSumThreads, 1) mot_bwd_sum_kernel(const Embed
         const bool more = k + 1 < cnt;  // warp-uniform
         const int pos_n = __shfl_sync(kFull, more ? A.pos : B.pos, more ? k + 1 : 0);
         if constexpr (PULL) {
-          if (more || B.cnt > 0) id_next = pulled_lane_id(p, pos_n, id_lane);
+          if (more || B.cnt > 0) id_next = pulled_lane_id<PULL>(p, pos_n, id_lane);
         } else {
           if (id_lane && (more || B.cnt > 0)) id_next = load_raw_id(p, idsrc, pos_n, lane);
         }
@@ -455,10 +455,11 @@ __global__ void __launch_bounds__(kSumThreads, 1) mot_bwd_sum_kernel(const Embed
 #endif
 }
 
-template <typename T, int CPL, bool PULL = false>
+template <typename T, int CPL, int PULL = kNoPull>
 static int launch_bwd_sum(const EmbedParams& p_in, cudaStream_t s) {
-  if constexpr (!PULL) {
-    if (ids_pulled(p_in)) return launch_bwd_sum<T, CPL, true>(p_in, s);
+  if constexpr (PULL == kNoPull) {
+    if (const int k = ids_pulled(p_in))
+      return k == kPullLeft ? launch_bwd_sum<T, CPL, kPullLeft>(p_in, s) : launch_bwd_sum<T, CPL, kPullRight>(p_in, s);
   }
   int sms = 0, optin = 0;
   if (int rc = device_props(&sms, &optin)) return rc;

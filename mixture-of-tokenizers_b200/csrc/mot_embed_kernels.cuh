@@ -81,7 +81,7 @@ struct EmbedParams {
   long long* trace;  // MOT_TRACE builds: per-warp time stamps (nullptr: off)
   long long* chk;    // MOT_CHECK builds: violation record
   int n_slots;       // fp32 slots of `partial` (MOT_CHECK builds verify every slot index against it)
-  int pad_eot;      // MOT_F_TTB_PULL_LEFT: pad byte | end-of-text byte << 16 (int16 each; fits the struct's tail padding)
+  int pad_eot;      // MOT_F_TTB_PULL_LEFT / _RIGHT: pad byte | end-of-text byte << 16 (int16 each; fits the struct's tail padding)
 };
 
 struct ChunkMap {
@@ -176,7 +176,30 @@ struct PullSrc {
   const void* ttb;
   long long T;  // tokens per row
   int V, bpt, ttb_dtype, pad, eot, scramble;
+  const int32_t* next;  // right pulls with MOT_F_TTB_NEXT_TOK: next[r] = token T of row r (the lookahead); else nullptr
 };
+
+// Non-pad count of ttb row tv; eot = every entry is the EOT byte (mot_pull's pull_count_kernel).
+__device__ __forceinline__ int ttb_row_count(const PullSrc& q, int tv, bool& eot) {
+  int cnt = 0, n_eot = 0;
+  for (int k = 0; k < q.bpt; ++k) {
+    const int id = ttb_raw(q.ttb, q.ttb_dtype, tv, q.bpt, k);
+    cnt += id != q.pad;
+    n_eot += id == q.eot;
+  }
+  eot = n_eot == q.bpt;
+  return cnt;
+}
+// Non-pad byte fi of ttb row tv as mot_pull's compacted stream keeps it (int16, hence the (short)); res if none.
+__device__ __forceinline__ void ttb_nth_byte(const PullSrc& q, int tv, int fi, int& res) {
+  for (int k = 0; k < q.bpt; ++k) {
+    const int id = ttb_raw(q.ttb, q.ttb_dtype, tv, q.bpt, k);
+    if (id != q.pad && fi-- == 0) {
+      res = (int)(short)id;
+      break;
+    }
+  }
+}
 
 // The bpt pulled ids of token t (pull_from_left over its row of T tokens, mot_pull.cu), computed by one warp without
 // the pulled tensor: lane k < bpt returns slot k.  Raw values: pads and EOT are detected on them, the caller clamps.
@@ -184,7 +207,7 @@ struct PullSrc {
 // ends (going back) at an EOT token or the row start; an inclusive scan of the counts gives every token the range of
 // backward byte indices it holds, and slot k receives backward index bpt - k.  Tokens with no non-pad byte can leave
 // the 32-token window short of bpt bytes: the next window continues.  Integer work, bit-exact with mot_pull, whose
-// compacted stream keeps the bytes as int16 (hence the (short) below).
+// compacted stream keeps the bytes as int16 (ttb_nth_byte).
 __device__ __forceinline__ int pulled_ids_warp(const PullSrc q, int t) {
   const int lane = lane_id();
   const int row0 = (int)(t - t % q.T);
@@ -197,13 +220,7 @@ __device__ __forceinline__ int pulled_ids_warp(const PullSrc q, int t) {
     bool eot = false;
     if (valid) {
       tv = clampi(ld_g(q.tok + j), q.V - 1);
-      int n_eot = 0;
-      for (int k = 0; k < q.bpt; ++k) {
-        const int id = ttb_raw(q.ttb, q.ttb_dtype, tv, q.bpt, k);
-        cnt += id != q.pad;
-        n_eot += id == q.eot;
-      }
-      eot = n_eot == q.bpt;
+      cnt = ttb_row_count(q, tv, eot);
     }
     if (base == t && __shfl_sync(0xffffffffu, eot, 0)) return q.eot;  // EOT tokens pass through unchanged
     const unsigned stop = __ballot_sync(0xffffffffu, !valid || eot);
@@ -222,32 +239,78 @@ __device__ __forceinline__ int pulled_ids_warp(const PullSrc q, int t) {
     for (int step = 16; step > 0; step >>= 1)
       if (__shfl_sync(0xffffffffu, incl, l + step - 1) < want) l += step;
     const int o_tv = __shfl_sync(0xffffffffu, tv, l), o_incl = __shfl_sync(0xffffffffu, incl, l);
-    if (lane < q.bpt && want > acc && want <= total) {
-      int fi = o_incl - want;  // index of the byte among the owner's non-pad bytes, in row order
-      for (int k = 0; k < q.bpt; ++k) {
-        const int id = ttb_raw(q.ttb, q.ttb_dtype, o_tv, q.bpt, k);
-        if (id != q.pad && fi-- == 0) {
-          res = (int)(short)id;
-          break;
-        }
-      }
-    }
+    if (lane < q.bpt && want > acc && want <= total)  // index of the byte among the owner's non-pad bytes, in row order
+      ttb_nth_byte(q, o_tv, o_incl - want, res);
     if (total >= q.bpt || f < 32) return res;
     acc = total;
   }
 }
 
+// The mirror image for pull_from_right (mot_pull.cu reads the row backwards): token t receives the first min(bpt, n)
+// non-pad bytes of tokens t, t+1, ... before the next EOT token or the row end, left-aligned.  Lanes take tokens t,
+// t+1, ..., t+31; the row ends after token T-1, or after the lookahead q.next[row] (read as token T) when there is one;
+// the segment ends (going forward) before the first EOT token or the row end; the inclusive scan gives every token the
+// range of forward byte indices it holds, and slot k receives forward index k + 1.
+__device__ __forceinline__ int pulled_ids_right_warp(const PullSrc q, int t) {
+  const int lane = lane_id();
+  const int row = (int)(t / q.T);
+  const int row_end = (int)((row + 1) * q.T);        // first index past the row's own tokens
+  const int end = row_end + (q.next ? 1 : 0);        // index row_end reads the lookahead
+  const int want = lane + 1;                         // forward index (1 = first byte of the segment) of this slot
+  int res = q.pad, acc = 0;
+  for (int base = t;; base += 32) {
+    const int j = base + lane;
+    const bool valid = j < end;
+    int cnt = 0, tv = 0;
+    bool eot = false;
+    if (valid) {
+      tv = clampi(j < row_end ? ld_g(q.tok + j) : ld_g(q.next + row), q.V - 1);
+      cnt = ttb_row_count(q, tv, eot);
+    }
+    if (base == t && __shfl_sync(0xffffffffu, eot, 0)) return q.eot;  // EOT tokens pass through unchanged
+    const unsigned stop = __ballot_sync(0xffffffffu, !valid || eot);
+    const int f = stop ? __ffs(stop) - 1 : 32;  // lanes [0, f) belong to the segment
+    if (lane >= f) cnt = 0;
+    int incl = cnt;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int u = __shfl_up_sync(0xffffffffu, incl, o);
+      if (lane >= o) incl += u;
+    }
+    incl += acc;
+    const int total = __shfl_sync(0xffffffffu, incl, 31);
+    int l = 0;  // first lane whose inclusive count reaches `want`
+#pragma unroll
+    for (int step = 16; step > 0; step >>= 1)
+      if (__shfl_sync(0xffffffffu, incl, l + step - 1) < want) l += step;
+    const int o_tv = __shfl_sync(0xffffffffu, tv, l), o_incl = __shfl_sync(0xffffffffu, incl, l);
+    const int o_cnt = __shfl_sync(0xffffffffu, cnt, l);
+    if (lane < q.bpt && want > acc && want <= total)  // index of the byte among the owner's non-pad bytes, in row order
+      ttb_nth_byte(q, o_tv, want - (o_incl - o_cnt) - 1, res);
+    if (total >= q.bpt || f < 32) return res;
+    acc = total;
+  }
+}
+
+// The pulled row of token t; the direction is a compile-time value, so that each instantiation carries one routine.
+template <bool RIGHT>
+__device__ __forceinline__ int pulled_row_warp(const PullSrc q, int t) {
+  if constexpr (RIGHT) return pulled_ids_right_warp(q, t);
+  else return pulled_ids_warp(q, t);
+}
+
 // Pulled id of this lane's slot at position pos (warp collective).  With the `.view(bpt,-1)` scramble every slot lane
 // reads another token: the warp derives the pulled row of each of them in turn.
+template <bool RIGHT>
 __device__ __forceinline__ int fetch_pulled_id(const PullSrc q, int pos) {
   const int lane = lane_id();
-  if (!q.scramble) return pulled_ids_warp(q, pos);
+  if (!q.scramble) return pulled_row_warp<RIGHT>(q, pos);
   const long long row = pos / q.T, s = pos - row * q.T;
   const long long f = (long long)min(lane, q.bpt - 1) * q.T + s;
   const int tokpos = (int)(row * q.T + f / q.bpt), k = (int)(f % q.bpt);
   int id = 0;
   for (int r = 0; r < q.bpt; ++r) {
-    const int v = pulled_ids_warp(q, __shfl_sync(0xffffffffu, tokpos, r));
+    const int v = pulled_row_warp<RIGHT>(q, __shfl_sync(0xffffffffu, tokpos, r));
     const int got = __shfl_sync(0xffffffffu, v, __shfl_sync(0xffffffffu, k, r));
     if (lane == r) id = got;
   }
@@ -274,15 +337,23 @@ __device__ __forceinline__ int load_raw_id(const EmbedParams& p, const IdSrc& s,
   const char* a = s.base + (unsigned long long)(unsigned)pos * s.pos_stride;  // one 32 x 32 -> 64 multiply-add
   return s.kind == 1 ? (int)ld_g(reinterpret_cast<const long long*>(a)) : ld_g(reinterpret_cast<const int*>(a));
 }
-// The descriptor asks for pulled ids derived in the kernel: the kernels run their PULL instantiation, in which every
-// id load is the warp collective fetch_pulled_id (the other instantiations carry none of its code).
-inline bool ids_pulled(const EmbedParams& p) {
-  return (p.flags & MOT_F_IDS_FROM_TTB) && (p.flags & MOT_F_TTB_PULL_LEFT) && p.bpt > 0;
+// The kernels' PULL template value: kNoPull loads the byte ids (tensor or ttb rows); kPullLeft / kPullRight derive the
+// pulled ids in the kernel, every id load being the warp collective fetch_pulled_id (the kNoPull instantiations carry
+// none of its code, and each pulled instantiation one direction).
+constexpr int kNoPull = 0, kPullLeft = 1, kPullRight = 2;
+inline int ids_pulled(const EmbedParams& p) {
+  if (!(p.flags & MOT_F_IDS_FROM_TTB) || p.bpt <= 0) return kNoPull;
+  if (p.flags & MOT_F_TTB_PULL_LEFT) return kPullLeft;
+  return (p.flags & MOT_F_TTB_PULL_RIGHT) ? kPullRight : kNoPull;
 }
 // Raw pulled id of this lane's slot (0 on lanes that hold no slot).  Every lane of the warp must call it.
+// The lookahead tail of MOT_F_TTB_NEXT_TOK follows the N token ids.
+template <int PULL>
 __device__ __forceinline__ int pulled_lane_id(const EmbedParams& p, int pos, bool id_lane) {
-  const int id = fetch_pulled_id(PullSrc{p.tok, p.ttb, p.T, p.V, p.bpt, p.ttb_dtype, (short)(p.pad_eot & 0xffff),
-                                         p.pad_eot >> 16, (p.flags & MOT_F_TTB_SCRAMBLE) ? 1 : 0}, pos);
+  const int32_t* next = (PULL == kPullRight && (p.flags & MOT_F_TTB_NEXT_TOK)) ? p.tok + p.N : nullptr;
+  const int id = fetch_pulled_id<PULL == kPullRight>(
+      PullSrc{p.tok, p.ttb, p.T, p.V, p.bpt, p.ttb_dtype, (short)(p.pad_eot & 0xffff), p.pad_eot >> 16,
+              (p.flags & MOT_F_TTB_SCRAMBLE) ? 1 : 0, next}, pos);
   return id_lane ? id : 0;
 }
 
@@ -438,7 +509,7 @@ __device__ __forceinline__ void gmem_add4(float* a, const float (&v)[4]) {
 // ======================================================================================
 // Forward
 // ======================================================================================
-template <typename T, int CPL, int MODE, int NT, bool PULL>
+template <typename T, int CPL, int MODE, int NT, int PULL>
 __global__ void __launch_bounds__(NT, 1) mot_fwd_kernel(const EmbedParams p) {
   using C = Cfg<MODE>;
   constexpr int CW = 8;
@@ -508,8 +579,8 @@ __global__ void __launch_bounds__(NT, 1) mot_fwd_kernel(const EmbedParams p) {
   // raw byte ids are fetched two positions ahead and clamped where they are consumed
   int id_n1, id_n2;
   if constexpr (PULL) {
-    id_n1 = n_i > 0 ? pulled_lane_id(p, gw, id_lane) : 0;
-    id_n2 = n_i > 1 ? pulled_lane_id(p, gw + stride, id_lane) : 0;
+    id_n1 = n_i > 0 ? pulled_lane_id<PULL>(p, gw, id_lane) : 0;
+    id_n2 = n_i > 1 ? pulled_lane_id<PULL>(p, gw + stride, id_lane) : 0;
   } else {
     id_n1 = (id_lane && n_i > 0) ? load_raw_id(p, idsrc, gw, lane) : 0;
     id_n2 = (id_lane && n_i > 1) ? load_raw_id(p, idsrc, gw + stride, lane) : 0;
@@ -521,7 +592,7 @@ __global__ void __launch_bounds__(NT, 1) mot_fwd_kernel(const EmbedParams p) {
     const int idreg = clamp_id(p, id_n1);
     id_n1 = id_n2;
     if constexpr (PULL) {
-      if (i + 2 < n_i) id_n2 = pulled_lane_id(p, pos + 2 * stride, id_lane);
+      if (i + 2 < n_i) id_n2 = pulled_lane_id<PULL>(p, pos + 2 * stride, id_lane);
     } else {
       if (id_lane && i + 2 < n_i) id_n2 = load_raw_id(p, idsrc, pos + 2 * stride, lane);
     }
@@ -713,7 +784,7 @@ struct Batch {
 template <int CPL, int MODE>
 constexpr int bwd_threads() { return (MOT_ADDFLAG(MODE, 4) && CPL >= 8) ? MOT_WIDE_STATIC_THREADS : kBwdThreads; }
 
-template <typename T, int CPL, int MODE, bool PULL>
+template <typename T, int CPL, int MODE, int PULL>
 __global__ void __launch_bounds__((bwd_threads<CPL, MODE>()), 1) mot_bwd_kernel(const EmbedParams p) {
   using C = Cfg<MODE>;
   constexpr int CW = kBwdCW;
@@ -897,7 +968,7 @@ __global__ void __launch_bounds__((bwd_threads<CPL, MODE>()), 1) mot_bwd_kernel(
     if (has_tok && chunk_first && a > 0) v_before = ld_g(p.stok + a - 1);
     const int pos_first = __shfl_sync(0xffffffffu, A.pos, 0);  // warp collective: outside lane-dependent branches
     int id_next;
-    if constexpr (PULL) id_next = pulled_lane_id(p, pos_first, id_lane);
+    if constexpr (PULL) id_next = pulled_lane_id<PULL>(p, pos_first, id_lane);
     else id_next = id_lane ? load_raw_id(p, idsrc, pos_first, lane) : 0;
     for (int k = 0; k < A.cnt; ++k) {
       const int v = __shfl_sync(0xffffffffu, A.v, k);
@@ -912,7 +983,7 @@ __global__ void __launch_bounds__((bwd_threads<CPL, MODE>()), 1) mot_bwd_kernel(
       const int idreg = clamp_id(p, id_next);
       const int pos_ahead = __shfl_sync(0xffffffffu, A.pos, (k + 1) & 31);
       if constexpr (PULL) {
-        if (k + 1 < A.cnt) id_next = pulled_lane_id(p, pos_ahead, id_lane);
+        if (k + 1 < A.cnt) id_next = pulled_lane_id<PULL>(p, pos_ahead, id_lane);
       } else {
         if (id_lane && k + 1 < A.cnt) id_next = load_raw_id(p, idsrc, pos_ahead, lane);
       }
@@ -1303,10 +1374,11 @@ inline size_t plan_smem(EmbedParams& p, size_t esz, int warps, bool backward, in
   return 0;
 }
 
-template <typename T, int CPL, int MODE, bool PULL = false>
+template <typename T, int CPL, int MODE, int PULL = kNoPull>
 static int launch_fwd(const EmbedParams& p_in, cudaStream_t s) {
-  if constexpr (!PULL && MODE != 2 && MODE != 5) {
-    if (ids_pulled(p_in)) return launch_fwd<T, CPL, MODE, true>(p_in, s);
+  if constexpr (PULL == kNoPull && MODE != 2 && MODE != 5) {
+    if (const int k = ids_pulled(p_in))
+      return k == kPullLeft ? launch_fwd<T, CPL, MODE, kPullLeft>(p_in, s) : launch_fwd<T, CPL, MODE, kPullRight>(p_in, s);
   }
   int sms = 0, optin = 0;
   if (int rc = device_props(&sms, &optin)) return rc;
@@ -1338,10 +1410,11 @@ static int launch_fwd(const EmbedParams& p_in, cudaStream_t s) {
   return check_launch();
 }
 
-template <typename T, int CPL, int MODE, bool PULL = false>
+template <typename T, int CPL, int MODE, int PULL = kNoPull>
 static int launch_bwd(const EmbedParams& p_in, cudaStream_t s) {
-  if constexpr (!PULL && MODE != 2 && MODE != 5) {
-    if (ids_pulled(p_in)) return launch_bwd<T, CPL, MODE, true>(p_in, s);
+  if constexpr (PULL == kNoPull && MODE != 2 && MODE != 5) {
+    if (const int k = ids_pulled(p_in))
+      return k == kPullLeft ? launch_bwd<T, CPL, MODE, kPullLeft>(p_in, s) : launch_bwd<T, CPL, MODE, kPullRight>(p_in, s);
   }
   int sms = 0, optin = 0;
   if (int rc = device_props(&sms, &optin)) return rc;

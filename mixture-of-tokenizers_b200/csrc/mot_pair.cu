@@ -32,6 +32,10 @@ struct PairParams {
 struct PairTtbParams : PairParams {
   PullSrc ttb;
 };
+// The same with the pulled ids of pull_from_right (MOT_F_TTB_PULL_RIGHT): its own kernel instantiations.
+struct PairTtbRightParams : PairTtbParams {};
+template <typename P>
+constexpr bool kPairTtb = std::is_base_of_v<PairTtbParams, P>;
 
 constexpr int kPairThreads = 512;
 
@@ -61,11 +65,12 @@ __device__ __forceinline__ int pair_load_id(const void* ids, int i64, long long 
 
 // Byte ids (ia, ib) of this lane's slot at position pos derived from the token ids: padded ids for a, pulled ids for b.
 // Warp collective; clamped; 0 on inactive lanes.
-__device__ __forceinline__ void pair_ttb_ids(const PairTtbParams& p, long long pos, int slot, bool active, int& ia, int& ib) {
+template <typename P>
+__device__ __forceinline__ void pair_ttb_ids(const P& p, long long pos, int slot, bool active, int& ia, int& ib) {
   const int lane = lane_id();
   const int tv = clampi(ld_g(p.ttb.tok + pos), p.ttb.V - 1);
   const int a = lane < p.bpt ? ttb_raw(p.ttb.ttb, p.ttb.ttb_dtype, tv, p.bpt, lane) : 0;
-  const int b = pulled_ids_warp(p.ttb, (int)pos);
+  const int b = pulled_row_warp<std::is_same_v<P, PairTtbRightParams>>(p.ttb, (int)pos);
   ia = clampi(__shfl_sync(0xffffffffu, a, slot & 31), p.Vb - 1);
   ib = clampi(__shfl_sync(0xffffffffu, b, slot & 31), p.Vb - 1);
   if (!active) ia = ib = 0;
@@ -96,7 +101,7 @@ __global__ void __launch_bounds__(kPairThreads, MAXJ <= 4 ? 2 : 1) mot_pair_fwd_
   const long long W = (long long)gridDim.x * nw;
   for (long long pos = (long long)warp * gridDim.x + blockIdx.x; pos < p.N; pos += W) {
     int ia = 0, ib = 0;
-    if constexpr (std::is_same_v<P, PairTtbParams>) {
+    if constexpr (kPairTtb<P>) {
       pair_ttb_ids(p, pos, slot, active, ia, ib);
     } else if (active) {
       ia = pair_load_id(p.ids_a, p.ids_i64, pos * p.bpt + slot, p.Vb - 1);
@@ -155,7 +160,7 @@ __global__ void __launch_bounds__(kPairThreads, MAXJ <= 4 ? 2 : 1) mot_pair_bwd_
   const long long W = (long long)gridDim.x * nw;
   for (long long pos = gw; pos < p.N; pos += W) {
     int ia = 0, ib = 0;
-    if constexpr (std::is_same_v<P, PairTtbParams>) {
+    if constexpr (kPairTtb<P>) {
       pair_ttb_ids(p, pos, slot, active, ia, ib);
     } else if (active) {
       ia = pair_load_id(p.ids_a, p.ids_i64, pos * p.bpt + slot, p.Vb - 1);
@@ -316,9 +321,15 @@ static int pair_bwd(P& p, int32_t dtype, void* gE_byte, void* workspace, size_t 
   return dtype == MOT_BF16 ? launch_finalize_bf16(q, fb, s) : launch_finalize_f32(q, fb, s);
 }
 
+// flags: MOT_F_TTB_PULL_LEFT, or MOT_F_TTB_PULL_RIGHT with or without MOT_F_TTB_NEXT_TOK (the tail tok[n + r]).
 static PullSrc pair_pull_src(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
-                             int32_t pad_id, int32_t eot_id, int32_t bpt) {
-  return PullSrc{tok, ttb, seq_len, tok_vocab, bpt, ttb_dtype, pad_id, eot_id, 0};
+                             int32_t pad_id, int32_t eot_id, int64_t n, int32_t bpt, int32_t flags) {
+  return PullSrc{tok, ttb, seq_len, tok_vocab, bpt, ttb_dtype, pad_id, eot_id, 0,
+                 (flags & MOT_F_TTB_NEXT_TOK) ? tok + n : nullptr};
+}
+static bool pair_pull_flags_ok(int32_t flags) {
+  return flags == MOT_F_TTB_PULL_LEFT || flags == MOT_F_TTB_PULL_RIGHT ||
+         flags == (MOT_F_TTB_PULL_RIGHT | MOT_F_TTB_NEXT_TOK);
 }
 
 extern "C" int mot_byte_pair_fwd(const void* ids_a, const void* ids_b, int32_t ids_i64, int64_t n_tokens, int32_t bpt,
@@ -350,18 +361,47 @@ extern "C" int mot_byte_pair_bwd(const void* ids_a, const void* ids_b, int32_t i
 }
 
 // The id tensors' null checks of pair_validate do not apply here: a non-null placeholder stands in for them.
+extern "C" int mot_byte_pair_ttb_ex_fwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype,
+                                        int64_t seq_len, int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt,
+                                        const void* E_byte, int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps,
+                                        void* out, int64_t row_stride, int32_t col_offset, int32_t flags, void* stream) {
+  if (!pair_pull_flags_ok(flags)) return MOT_ERR_BAD_ARG;
+  if (int rc = pair_ttb_validate(tok, ttb, tok_vocab, ttb_dtype, seq_len, n_tokens)) return rc;
+  if (int rc = pair_validate(tok, tok, n_tokens, bpt, E_byte, byte_vocab, byte_dim, dtype, out, row_stride, col_offset)) return rc;
+  if (n_tokens == 0) return MOT_OK;
+  const auto run = [&](auto p) {
+    pair_fill(p, nullptr, nullptr, 0, n_tokens, bpt, E_byte, byte_vocab, byte_dim, eps, row_stride, col_offset);
+    p.ttb = pair_pull_src(tok, ttb, tok_vocab, ttb_dtype, seq_len, pad_id, eot_id, n_tokens, bpt, flags);
+    p.out = out;
+    return pair_fwd(p, dtype, stream);
+  };
+  return (flags & MOT_F_TTB_PULL_RIGHT) ? run(PairTtbRightParams{}) : run(PairTtbParams{});
+}
+
+extern "C" int mot_byte_pair_ttb_ex_bwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype,
+                                        int64_t seq_len, int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt,
+                                        const void* E_byte, int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps,
+                                        const void* grad_out, int64_t row_stride, int32_t col_offset, void* gE_byte,
+                                        void* workspace, size_t ws_bytes, int32_t flags, void* stream) {
+  if (!pair_pull_flags_ok(flags)) return MOT_ERR_BAD_ARG;
+  if (int rc = pair_ttb_validate(tok, ttb, tok_vocab, ttb_dtype, seq_len, n_tokens)) return rc;
+  if (int rc = pair_validate(tok, tok, n_tokens, bpt, E_byte, byte_vocab, byte_dim, dtype, grad_out, row_stride, col_offset))
+    return rc;
+  const auto run = [&](auto p) {
+    pair_fill(p, nullptr, nullptr, 0, n_tokens, bpt, E_byte, byte_vocab, byte_dim, eps, row_stride, col_offset);
+    p.ttb = pair_pull_src(tok, ttb, tok_vocab, ttb_dtype, seq_len, pad_id, eot_id, n_tokens, bpt, flags);
+    p.gout = grad_out;
+    return pair_bwd(p, dtype, gE_byte, workspace, ws_bytes, stream);
+  };
+  return (flags & MOT_F_TTB_PULL_RIGHT) ? run(PairTtbRightParams{}) : run(PairTtbParams{});
+}
+
 extern "C" int mot_byte_pair_ttb_fwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
                                      int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt, const void* E_byte,
                                      int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps, void* out,
                                      int64_t row_stride, int32_t col_offset, void* stream) {
-  if (int rc = pair_ttb_validate(tok, ttb, tok_vocab, ttb_dtype, seq_len, n_tokens)) return rc;
-  if (int rc = pair_validate(tok, tok, n_tokens, bpt, E_byte, byte_vocab, byte_dim, dtype, out, row_stride, col_offset)) return rc;
-  if (n_tokens == 0) return MOT_OK;
-  PairTtbParams p;
-  pair_fill(p, nullptr, nullptr, 0, n_tokens, bpt, E_byte, byte_vocab, byte_dim, eps, row_stride, col_offset);
-  p.ttb = pair_pull_src(tok, ttb, tok_vocab, ttb_dtype, seq_len, pad_id, eot_id, bpt);
-  p.out = out;
-  return pair_fwd(p, dtype, stream);
+  return mot_byte_pair_ttb_ex_fwd(tok, ttb, tok_vocab, ttb_dtype, seq_len, pad_id, eot_id, n_tokens, bpt, E_byte, byte_vocab,
+                                  byte_dim, dtype, eps, out, row_stride, col_offset, MOT_F_TTB_PULL_LEFT, stream);
 }
 
 extern "C" int mot_byte_pair_ttb_bwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
@@ -369,12 +409,7 @@ extern "C" int mot_byte_pair_ttb_bwd(const int32_t* tok, const void* ttb, int32_
                                      int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps, const void* grad_out,
                                      int64_t row_stride, int32_t col_offset, void* gE_byte, void* workspace, size_t ws_bytes,
                                      void* stream) {
-  if (int rc = pair_ttb_validate(tok, ttb, tok_vocab, ttb_dtype, seq_len, n_tokens)) return rc;
-  if (int rc = pair_validate(tok, tok, n_tokens, bpt, E_byte, byte_vocab, byte_dim, dtype, grad_out, row_stride, col_offset))
-    return rc;
-  PairTtbParams p;
-  pair_fill(p, nullptr, nullptr, 0, n_tokens, bpt, E_byte, byte_vocab, byte_dim, eps, row_stride, col_offset);
-  p.ttb = pair_pull_src(tok, ttb, tok_vocab, ttb_dtype, seq_len, pad_id, eot_id, bpt);
-  p.gout = grad_out;
-  return pair_bwd(p, dtype, gE_byte, workspace, ws_bytes, stream);
+  return mot_byte_pair_ttb_ex_bwd(tok, ttb, tok_vocab, ttb_dtype, seq_len, pad_id, eot_id, n_tokens, bpt, E_byte, byte_vocab,
+                                  byte_dim, dtype, eps, grad_out, row_stride, col_offset, gE_byte, workspace, ws_bytes,
+                                  MOT_F_TTB_PULL_LEFT, stream);
 }

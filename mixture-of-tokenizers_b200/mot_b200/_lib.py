@@ -21,7 +21,7 @@ TTB_I16, TTB_F32, TTB_BF16 = 0, 1, 2
 ADD, CONCAT, TOK_ONLY, BYTES_ONLY, MEAN = range(5)
 F_TOK_NORM, F_BYTE_NORM, F_OUT_NORM, F_BYTES_FIRST = 1, 2, 4, 8
 F_SLOT_MAJOR, F_IDS_FROM_TTB, F_TTB_SCRAMBLE, F_IDS_I64, F_HAS_LAMBDAS = 16, 32, 64, 128, 256
-F_TTB_PULL_LEFT = 512
+F_TTB_PULL_LEFT, F_TTB_PULL_RIGHT, F_TTB_NEXT_TOK = 512, 1024, 2048
 WS_PLAN_READY, WS_CLEAN, WS_PLAN_JOINED = 1, 2, 4
 DP_NVLS, DP_P2P = 0, 1
 
@@ -78,6 +78,12 @@ _SIGNATURES = {
     "mot_byte_pair_ttb_bwd": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int32,
                                         _P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, C.c_int64, C.c_int32, _P, _P,
                                         C.c_size_t, _P]),
+    "mot_byte_pair_ttb_ex_fwd": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int64,
+                                           C.c_int32, _P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, C.c_int64,
+                                           C.c_int32, C.c_int32, _P]),
+    "mot_byte_pair_ttb_ex_bwd": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int64,
+                                           C.c_int32, _P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, C.c_int64,
+                                           C.c_int32, _P, _P, C.c_size_t, C.c_int32, _P]),
     "mot_dp_exchange": (C.c_int, [_P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int64, C.c_int64, C.c_int32, C.c_uint32, C.c_int32,
                                   C.c_int32, _P]),
     "mot_embed_touched_rows": (C.c_int, [C.POINTER(MotDesc), _P, C.c_size_t, _P, _P]),

@@ -51,13 +51,15 @@ _COMBINE_NAMES = tuple(O._COMBINE)   # the combine mode is its index in this ord
 def pack_spec(spec) -> int:
     return (_COMBINE_NAMES.index(spec.combine) | (16 if spec.tok_norm else 0) | (32 if spec.byte_norm else 0) |
             (64 if spec.out_norm else 0) | (128 if spec.bytes_first else 0) | (256 if spec.slot_major else 0) |
-            (512 if spec.ttb_scramble else 0) | (1024 if spec.ttb_pull else 0))
+            (512 if spec.ttb_scramble else 0) | (1024 if spec.ttb_pull else 0) |
+            (2048 if spec.ttb_pull_side == "right" else 0))
 
 
 def unpack_spec(code: int, eps: float):
     return O.MixSpec(combine=_COMBINE_NAMES[code & 15], tok_norm=bool(code & 16), byte_norm=bool(code & 32),
                      out_norm=bool(code & 64), bytes_first=bool(code & 128), slot_major=bool(code & 256),
-                     ttb_scramble=bool(code & 512), ttb_pull=bool(code & 1024), eps=eps)
+                     ttb_scramble=bool(code & 512), ttb_pull=bool(code & 1024), eps=eps,
+                     ttb_pull_side="right" if code & 2048 else "left")
 
 
 _PLANNERS: dict = {}
@@ -97,9 +99,11 @@ def _empty(dev, dtype=torch.uint8) -> Tensor:
 @torch.library.custom_op("mot_b200::embed", mutates_args=(), device_types="cuda")
 def embed_op(tok: Optional[Tensor], ids: Optional[Tensor], ttb: Optional[Tensor], E_tok: Optional[Tensor],
              E_byte: Optional[Tensor], lam: Optional[Tensor], spec: int, bpt: int, seq_len: int, eps: float,
-             plan: bool) -> Tuple[Tensor, Tensor, Tensor]:
-    """-> (out [n, out_dim], rstd [n] fp32 or [0], workspace uint8 or [0])."""
-    desc = O._embed_desc(unpack_spec(spec, eps), bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None)
+             plan: bool, next_tok: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor]:
+    """-> (out [n, out_dim], rstd [n] fp32 or [0], workspace uint8 or [0]).  next_tok: the lookahead of a right pull."""
+    tok = O._tok_next(tok, next_tok)
+    desc = O._embed_desc(unpack_spec(spec, eps), bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None,
+                         next_tok=next_tok is not None)
     n, ref = desc.n_tokens, (E_tok if E_tok is not None else E_byte)
     dev = ref.device
     out = torch.empty((n, desc.out_dim), dtype=ref.dtype, device=dev)
@@ -114,8 +118,9 @@ def embed_op(tok: Optional[Tensor], ids: Optional[Tensor], ttb: Optional[Tensor]
 
 
 @embed_op.register_fake
-def _(tok, ids, ttb, E_tok, E_byte, lam, spec, bpt, seq_len, eps, plan):
-    desc = O._embed_desc(unpack_spec(spec, eps), bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None)
+def _(tok, ids, ttb, E_tok, E_byte, lam, spec, bpt, seq_len, eps, plan, next_tok=None):
+    desc = O._embed_desc(unpack_spec(spec, eps), bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None,
+                         next_tok=next_tok is not None)
     n, ref = desc.n_tokens, (E_tok if E_tok is not None else E_byte)
     planned = plan and tok is not None and n > 0
     keep = plan and n > 0 and O.embed_bwd_uses_saved(desc)
@@ -126,9 +131,12 @@ def _(tok, ids, ttb, E_tok, E_byte, lam, spec, bpt, seq_len, eps, plan):
 @torch.library.custom_op("mot_b200::embed_bwd", mutates_args=(), device_types="cuda")
 def embed_bwd_op(grad_out: Tensor, tok: Optional[Tensor], ids: Optional[Tensor], ttb: Optional[Tensor],
                  E_tok: Optional[Tensor], E_byte: Optional[Tensor], lam: Optional[Tensor], out_saved: Optional[Tensor],
-                 rstd: Tensor, ws: Tensor, spec: int, bpt: int, seq_len: int, eps: float) -> Tuple[Tensor, Tensor, Tensor]:
+                 rstd: Tensor, ws: Tensor, spec: int, bpt: int, seq_len: int, eps: float,
+                 next_tok: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor]:
     """-> (gE_tok dense or [0], gE_byte dense or [0], g_lam fp32 [2] or [0])."""
-    desc = O._embed_desc(unpack_spec(spec, eps), bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None)
+    tok = O._tok_next(tok, next_tok)
+    desc = O._embed_desc(unpack_spec(spec, eps), bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None,
+                         next_tok=next_tok is not None)
     n, ref = desc.n_tokens, (E_tok if E_tok is not None else E_byte)
     dev = ref.device
     g = grad_out.reshape(n, desc.out_dim)
@@ -146,7 +154,7 @@ def embed_bwd_op(grad_out: Tensor, tok: Optional[Tensor], ids: Optional[Tensor],
 
 
 @embed_bwd_op.register_fake
-def _(grad_out, tok, ids, ttb, E_tok, E_byte, lam, out_saved, rstd, ws, spec, bpt, seq_len, eps):
+def _(grad_out, tok, ids, ttb, E_tok, E_byte, lam, out_saved, rstd, ws, spec, bpt, seq_len, eps, next_tok=None):
     ref = E_tok if E_tok is not None else E_byte
     return (torch.empty_like(E_tok) if E_tok is not None else ref.new_empty((0,)),
             torch.empty_like(E_byte) if E_byte is not None else ref.new_empty((0,)),
@@ -154,17 +162,17 @@ def _(grad_out, tok, ids, ttb, E_tok, E_byte, lam, out_saved, rstd, ws, spec, bp
 
 
 def _embed_setup(ctx, inputs, output):
-    tok, ids, ttb, E_tok, E_byte, lam, spec, bpt, seq_len, eps, plan = inputs
+    tok, ids, ttb, E_tok, E_byte, lam, spec, bpt, seq_len, eps, plan, next_tok = inputs
     out, rstd, ws = output
-    ctx.save_for_backward(tok, ids, ttb, E_tok, E_byte, lam, out if rstd.numel() > 0 else None, rstd, ws)
+    ctx.save_for_backward(tok, ids, ttb, E_tok, E_byte, lam, out if rstd.numel() > 0 else None, rstd, ws, next_tok)
     ctx.cfg = (spec, bpt, seq_len, eps)
 
 
 def _embed_backward(ctx, g_out, g_rstd, g_ws):
-    tok, ids, ttb, E_tok, E_byte, lam, out, rstd, ws = ctx.saved_tensors
-    gt, gb, gl = torch.ops.mot_b200.embed_bwd(g_out, tok, ids, ttb, E_tok, E_byte, lam, out, rstd, ws, *ctx.cfg)
+    tok, ids, ttb, E_tok, E_byte, lam, out, rstd, ws, next_tok = ctx.saved_tensors
+    gt, gb, gl = torch.ops.mot_b200.embed_bwd(g_out, tok, ids, ttb, E_tok, E_byte, lam, out, rstd, ws, *ctx.cfg, next_tok)
     return (None, None, None, gt if E_tok is not None else None, gb if E_byte is not None else None,
-            gl if lam is not None else None, None, None, None, None, None)
+            gl if lam is not None else None, None, None, None, None, None, None)
 
 
 embed_op.register_autograd(_embed_backward, setup_context=_embed_setup)
@@ -238,27 +246,32 @@ tok_gather_op.register_autograd(_tok_gather_backward, setup_context=_tok_gather_
 @torch.library.custom_op("mot_b200::embed_proj", mutates_args=(), device_types="cuda")
 def embed_proj_op(tok: Tensor, ids: Tensor, ids2: Optional[Tensor], E_tok: Tensor, E_byte: Tensor, W: Tensor,
                   bias: Optional[Tensor], spec: int, bpt: int, eps: float, plan: bool, ttb: Optional[Tensor] = None,
-                  seq_len: int = 0, ttb_pair: bool = False) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+                  seq_len: int = 0, ttb_pair: bool = False,
+                  next_tok: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
     """-> (out [n, Do], Y = the product before the row norm or [0], W in the compute dtype or [0], workspace or [0]).
-    With `ttb` the byte ids come from the table inside the kernels and `ids` is an unused placeholder."""
+    With `ttb` the byte ids come from the table inside the kernels and `ids` is an unused placeholder; next_tok: the
+    lookahead of a right pull."""
     dev, cdt = E_tok.device, E_tok.dtype
     sp = unpack_spec(spec, eps)
     ids = ids if ttb is None else None
     pair = ids2 is not None or ttb_pair
-    desc = O._proj_desc(sp, bpt, tok, ids, E_tok, E_byte, pair, ttb, seq_len)
+    tok, has_next = O._tok_next(tok, next_tok), next_tok is not None
+    desc = O._proj_desc(sp, bpt, tok, ids, E_tok, E_byte, pair, ttb, seq_len, has_next)
     w_c = W if W.dtype == cdt else O.cast_out(W, cdt)
     planned = plan and tok.numel() > 0
     ws = _plan_beside(desc, tok, dev) if planned else _empty(dev)
-    out, Y, _ = O._proj_forward(sp, desc, bpt, tok, ids, ids2, E_tok, E_byte, w_c, bias, False, ttb, seq_len, pair)
+    out, Y, _ = O._proj_forward(sp, desc, bpt, tok, ids, ids2, E_tok, E_byte, w_c, bias, False, ttb, seq_len, pair,
+                                has_next)
     if planned:
         _rejoin(dev)
     return out, (Y if sp.out_norm else _empty(dev, cdt)), (w_c if w_c is not W else _empty(dev, cdt)), ws
 
 
 @embed_proj_op.register_fake
-def _(tok, ids, ids2, E_tok, E_byte, W, bias, spec, bpt, eps, plan, ttb=None, seq_len=0, ttb_pair=False):
+def _(tok, ids, ids2, E_tok, E_byte, W, bias, spec, bpt, eps, plan, ttb=None, seq_len=0, ttb_pair=False, next_tok=None):
     sp = unpack_spec(spec, eps)
-    desc = O._proj_desc(sp, bpt, tok, ids if ttb is None else None, E_tok, E_byte, ids2 is not None or ttb_pair, ttb, seq_len)
+    desc = O._proj_desc(sp, bpt, tok, ids if ttb is None else None, E_tok, E_byte, ids2 is not None or ttb_pair, ttb, seq_len,
+                        next_tok is not None)
     n, cdt = tok.numel(), E_tok.dtype
     out = E_tok.new_empty((n, W.shape[0]))
     Y = E_tok.new_empty((n, W.shape[0]) if sp.out_norm else (0,))
@@ -270,43 +283,45 @@ def _(tok, ids, ids2, E_tok, E_byte, W, bias, spec, bpt, eps, plan, ttb=None, se
 def embed_proj_bwd_op(grad_out: Tensor, tok: Tensor, ids: Tensor, ids2: Optional[Tensor], E_tok: Tensor, E_byte: Tensor,
                       W: Tensor, w_c: Tensor, Y: Tensor, ws: Tensor, spec: int, bpt: int, eps: float,
                       has_bias: bool, ttb: Optional[Tensor] = None, seq_len: int = 0,
-                      ttb_pair: bool = False) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+                      ttb_pair: bool = False, next_tok: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
     """-> (gE_tok, gE_byte, gW in W's dtype, g_bias fp32 [Do] or [0])."""
     dev = E_tok.device
     sp = unpack_spec(spec, eps)
     ids = ids if ttb is None else None
     pair = ids2 is not None or ttb_pair
-    desc = O._proj_desc(sp, bpt, tok, ids, E_tok, E_byte, pair, ttb, seq_len)
+    tok, has_next = O._tok_next(tok, next_tok), next_tok is not None
+    desc = O._proj_desc(sp, bpt, tok, ids, E_tok, E_byte, pair, ttb, seq_len, has_next)
     dA, gW, g_bias = O._proj_backward(sp, desc, bpt, tok, ids, ids2, E_tok, E_byte, w_c if w_c.numel() > 0 else W,
                                       W.dtype, has_bias, Y, None, grad_out,    # the operand is gathered again, not kept
-                                      ttb, seq_len, pair)
+                                      ttb, seq_len, pair, has_next)
     ws, planned = _bwd_workspace(ws, desc, dev)
     gE_tok, gE_byte = O._scatter_operand(sp, desc, bpt, tok, ids, ids2, E_tok, E_byte, dA, ws, planned, planned,
-                                         ttb, seq_len, pair)
+                                         ttb, seq_len, pair, has_next)
     return gE_tok, gE_byte, gW, (g_bias if has_bias else _empty(dev, torch.float32))
 
 
 @embed_proj_bwd_op.register_fake
-def _(grad_out, tok, ids, ids2, E_tok, E_byte, W, w_c, Y, ws, spec, bpt, eps, has_bias, ttb=None, seq_len=0, ttb_pair=False):
+def _(grad_out, tok, ids, ids2, E_tok, E_byte, W, w_c, Y, ws, spec, bpt, eps, has_bias, ttb=None, seq_len=0, ttb_pair=False,
+      next_tok=None):
     return (torch.empty_like(E_tok), torch.empty_like(E_byte), torch.empty_like(W),
             E_tok.new_empty((W.shape[0] if has_bias else 0,), dtype=torch.float32))
 
 
 def _proj_setup(ctx, inputs, output):
-    tok, ids, ids2, E_tok, E_byte, W, bias, spec, bpt, eps, plan, ttb, seq_len, ttb_pair = inputs
+    tok, ids, ids2, E_tok, E_byte, W, bias, spec, bpt, eps, plan, ttb, seq_len, ttb_pair, next_tok = inputs
     out, Y, w_c, ws = output
-    ctx.save_for_backward(tok, ids, ids2, E_tok, E_byte, W, w_c, Y, ws, ttb)
+    ctx.save_for_backward(tok, ids, ids2, E_tok, E_byte, W, w_c, Y, ws, ttb, next_tok)
     ctx.cfg = (spec, bpt, eps, bias is not None)
     ctx.ttb_cfg = (seq_len, ttb_pair)
     ctx.bias_dtype = bias.dtype if bias is not None else None
 
 
 def _proj_backward(ctx, g_out, g_Y, g_wc, g_ws):
-    tok, ids, ids2, E_tok, E_byte, W, w_c, Y, ws, ttb = ctx.saved_tensors
+    tok, ids, ids2, E_tok, E_byte, W, w_c, Y, ws, ttb, next_tok = ctx.saved_tensors
     gt, gb, gW, gbias = torch.ops.mot_b200.embed_proj_bwd(g_out, tok, ids, ids2, E_tok, E_byte, W, w_c, Y, ws, *ctx.cfg,
-                                                          ttb, *ctx.ttb_cfg)
+                                                          ttb, *ctx.ttb_cfg, next_tok)
     return (None, None, None, gt, gb, gW, gbias.to(ctx.bias_dtype) if ctx.cfg[3] else None, None, None, None, None,
-            None, None, None)
+            None, None, None, None)
 
 
 embed_proj_op.register_autograd(_proj_backward, setup_context=_proj_setup)
@@ -317,12 +332,15 @@ embed_proj_op.register_autograd(_proj_backward, setup_context=_proj_setup)
 # ---------------------------------------------------------------------------------------------------------------
 @torch.library.custom_op("mot_b200::embed_byte_fc", mutates_args=(), device_types="cuda")
 def embed_byte_fc_op(tok: Tensor, ids: Tensor, E_tok: Tensor, E_byte: Tensor, W: Tensor, spec_b: int, bpt: int, eps: float,
-                     plan: bool, ttb: Optional[Tensor] = None, seq_len: int = 0) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+                     plan: bool, ttb: Optional[Tensor] = None, seq_len: int = 0,
+                     next_tok: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
     """-> (out [n, D], Y = the byte-FC product, W in the compute dtype or [0], workspace or [0]).  With `ttb` the byte
-    ids come from the table inside the kernels and `ids` is an unused placeholder."""
+    ids come from the table inside the kernels and `ids` is an unused placeholder; next_tok: the lookahead of a right
+    pull."""
     dev, cdt = E_tok.device, E_tok.dtype
     ids = ids if ttb is None else None
-    desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, tok, ids, E_tok, E_byte, ttb, seq_len)
+    tok = O._tok_next(tok, next_tok)
+    desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, tok, ids, E_tok, E_byte, ttb, seq_len, next_tok is not None)
     w_c = W if W.dtype == cdt else O.cast_out(W, cdt)
     planned = plan and tok.numel() > 0
     ws = _plan_beside(desc_t, tok, dev) if planned else _empty(dev)
@@ -333,9 +351,9 @@ def embed_byte_fc_op(tok: Tensor, ids: Tensor, E_tok: Tensor, E_byte: Tensor, W:
 
 
 @embed_byte_fc_op.register_fake
-def _(tok, ids, E_tok, E_byte, W, spec_b, bpt, eps, plan, ttb=None, seq_len=0):
+def _(tok, ids, E_tok, E_byte, W, spec_b, bpt, eps, plan, ttb=None, seq_len=0, next_tok=None):
     desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, tok, ids if ttb is None else None, E_tok, E_byte, ttb,
-                                 seq_len)
+                                 seq_len, next_tok is not None)
     n, D = tok.numel(), E_tok.shape[1]
     return (E_tok.new_empty((n, D)), E_tok.new_empty((n, D)), E_tok.new_empty(tuple(W.shape) if W.dtype != E_tok.dtype else (0,)),
             E_tok.new_empty((O.embed_workspace_bytes(desc_t) if plan and n > 0 else 0,), dtype=torch.uint8))
@@ -344,10 +362,11 @@ def _(tok, ids, E_tok, E_byte, W, spec_b, bpt, eps, plan, ttb=None, seq_len=0):
 @torch.library.custom_op("mot_b200::embed_byte_fc_bwd", mutates_args=(), device_types="cuda")
 def embed_byte_fc_bwd_op(grad_out: Tensor, tok: Tensor, ids: Tensor, E_tok: Tensor, E_byte: Tensor, W: Tensor, w_c: Tensor,
                          Y: Tensor, ws: Tensor, spec_b: int, bpt: int, eps: float, ttb: Optional[Tensor] = None,
-                         seq_len: int = 0) -> Tuple[Tensor, Tensor, Tensor]:
+                         seq_len: int = 0, next_tok: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor]:
     dev = E_tok.device
     ids = ids if ttb is None else None
-    desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, tok, ids, E_tok, E_byte, ttb, seq_len)
+    tok = O._tok_next(tok, next_tok)
+    desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, tok, ids, E_tok, E_byte, ttb, seq_len, next_tok is not None)
     ws, planned = _bwd_workspace(ws, desc_t, dev)
     wsb = torch.empty(O.embed_workspace_bytes(desc_b), dtype=torch.uint8, device=dev)
     return O._byte_fc_backward(desc_b, desc_t, tok, ids, E_tok, E_byte, w_c if w_c.numel() > 0 else W, W.dtype, Y,
@@ -355,23 +374,23 @@ def embed_byte_fc_bwd_op(grad_out: Tensor, tok: Tensor, ids: Tensor, E_tok: Tens
 
 
 @embed_byte_fc_bwd_op.register_fake
-def _(grad_out, tok, ids, E_tok, E_byte, W, w_c, Y, ws, spec_b, bpt, eps, ttb=None, seq_len=0):
+def _(grad_out, tok, ids, E_tok, E_byte, W, w_c, Y, ws, spec_b, bpt, eps, ttb=None, seq_len=0, next_tok=None):
     return torch.empty_like(E_tok), torch.empty_like(E_byte), torch.empty_like(W)
 
 
 def _fc_setup(ctx, inputs, output):
-    tok, ids, E_tok, E_byte, W, spec_b, bpt, eps, plan, ttb, seq_len = inputs
+    tok, ids, E_tok, E_byte, W, spec_b, bpt, eps, plan, ttb, seq_len, next_tok = inputs
     out, Y, w_c, ws = output
-    ctx.save_for_backward(tok, ids, E_tok, E_byte, W, w_c, Y, ws, ttb)
+    ctx.save_for_backward(tok, ids, E_tok, E_byte, W, w_c, Y, ws, ttb, next_tok)
     ctx.cfg = (spec_b, bpt, eps)
     ctx.seq_len = seq_len
 
 
 def _fc_backward(ctx, g_out, g_Y, g_wc, g_ws):
-    tok, ids, E_tok, E_byte, W, w_c, Y, ws, ttb = ctx.saved_tensors
+    tok, ids, E_tok, E_byte, W, w_c, Y, ws, ttb, next_tok = ctx.saved_tensors
     gt, gb, gW = torch.ops.mot_b200.embed_byte_fc_bwd(g_out, tok, ids, E_tok, E_byte, W, w_c, Y, ws, *ctx.cfg, ttb,
-                                                      ctx.seq_len)
-    return None, None, gt, gb, gW, None, None, None, None, None, None
+                                                      ctx.seq_len, next_tok)
+    return None, None, gt, gb, gW, None, None, None, None, None, None, None
 
 
 embed_byte_fc_op.register_autograd(_fc_backward, setup_context=_fc_setup)

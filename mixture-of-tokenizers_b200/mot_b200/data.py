@@ -73,12 +73,14 @@ def tokens_to_device(tokens: torch.Tensor, device) -> torch.Tensor:
 def create_batch(toks: torch.Tensor, ttb_in: Optional[torch.Tensor], ttb_out: Optional[torch.Tensor], bytes_per_token: int, *,
                  byte_in: bool = True, pull_in: bool = True, byte_out: bool = False, pull_out: bool = False,
                  padding_in: str = "left", padding_out: str = "left", pad_byte: int = 456, eot_byte: int = 457,
-                 byte_ids: bool = True):
+                 byte_ids: bool = True, next_tokens: bool = False):
     """The `_create_data_from_toks_*` family (spt/train_gpt.py:686-764) for toks [B, S+1] on the device ->
     (toks_in [B,S], bytes_padded_in [B,S*bpt] | None, bytes_pulled_in | None, targets).  (byte_in, pull_in, byte_out,
     pull_out) = (byte_mixin_method != "noop", pull_in, byte_mixout_method != "noop", pull_out) as at :766-779; invalid
     combinations raise KeyError like the reference's dict lookup.  byte_ids=False skips the input byte tensors (both
-    None): a loader then ships token ids only and the embedding derives the ids from its ttb table."""
+    None): a loader then ships token ids only and the embedding derives the ids from its ttb table.  next_tokens=True
+    appends a fifth element, the window's last column toks[:, -1] as int32 [B]: the lookahead a right pull of token ids
+    alone needs (with byte_out the targets hold byte ids, so this is the only place the caller gets that token)."""
     _require_cuda(toks, ttb_in, ttb_out)
     key = (bool(byte_in), bool(pull_in), bool(byte_out), bool(pull_out))
     valid = {(True, True, True, True), (True, False, True, True), (True, True, True, False), (True, True, False, False),
@@ -100,6 +102,9 @@ def create_batch(toks: torch.Tensor, ttb_in: Optional[torch.Tensor], ttb_out: Op
         targets = out_full[:, bpt:].contiguous()
     else:
         targets = toks[:, 1:].contiguous()
+    if next_tokens:
+        return (toks[:, :-1].contiguous(), bytes_padded_in, bytes_pulled_in, targets,
+                toks[:, -1].to(torch.int32).contiguous())
     return toks[:, :-1].contiguous(), bytes_padded_in, bytes_pulled_in, targets
 
 
@@ -108,11 +113,11 @@ def distributed_data_generator(filename_patterns: Union[str, Sequence[str]], seq
                                ttb_out: Optional[torch.Tensor] = None, byte_in: bool = True, pull_in: bool = True,
                                byte_out: bool = False, pull_out: bool = False, padding_in: str = "left",
                                padding_out: str = "left", device="cuda", seed: int = 12345,
-                               byte_ids: bool = True) -> Iterator[Tuple]:
+                               byte_ids: bool = True, next_tokens: bool = False) -> Iterator[Tuple]:
     """`distributed_data_generator` (spt/train_gpt.py:651-806): same shard order (sorted glob, `random.seed(seed)`
     shuffle), same windows (rank r takes `data[pos + r*local : pos + (r+1)*local]` viewed as [-1, seq_len+1]), batches
-    built by create_batch on the device (byte_ids=False: token ids only).  Raises StopIteration when the shards run out,
-    like the reference."""
+    built by create_batch on the device (byte_ids=False: token ids only; next_tokens=True: the fifth element, the
+    lookahead of a right pull).  Raises StopIteration when the shards run out, like the reference."""
     if isinstance(filename_patterns, str):
         filename_patterns = [filename_patterns]
     files: List[str] = []
@@ -147,4 +152,4 @@ def distributed_data_generator(filename_patterns: Union[str, Sequence[str]], seq
         pos += batch_size * local_seq_len
         yield create_batch(tokens_to_device(window, device), ttb_in, ttb_out, bytes_per_token, byte_in=byte_in, pull_in=pull_in,
                            byte_out=byte_out, pull_out=pull_out, padding_in=padding_in, padding_out=padding_out,
-                           byte_ids=byte_ids)
+                           byte_ids=byte_ids, next_tokens=next_tokens)

@@ -247,10 +247,11 @@ class SptByteMixEmbedding(nn.Module):
     `embed.embed_bytes.weight`, `byte_mixin.mixin.mixin.weight` (fp32 master, cast to bf16 per call like
     CastedLinear, gradient returned in fp32).  byte_mixin_method "noop" gives norm(embed_tokens(tokens)).
     add_padded_and_pulled=True sums the padded and the pulled byte rows before the per-byte norm (:371-379).
-    With the input ttb table `ttb` ([V, bpt], left padded), forward(tokens) alone derives the byte ids inside the
-    kernels (both byte tensors None): the pulled ids of every row of S tokens with pull_in, else the padded ids.
-    Refused (no fallback): cross_attn, byte self-attention; right-padded pulls from token ids alone (a token's pulled
-    bytes come from the tokens after it, and the last input token needs the one after the row)."""
+    With the input ttb table `ttb` ([V, bpt], padded on the `padding_in` side), forward(tokens) alone derives the byte
+    ids inside the kernels (both byte tensors None): the pulled ids of every row of S tokens with pull_in, else the
+    padded ids.  A right pull (padding_in="right") reads a token's bytes from the tokens after it, so the last input
+    tokens of a row need token S of the loader's window: forward(tokens, next_tokens=window[:, -1]) ([B]).
+    Refused (no fallback): cross_attn, byte self-attention; a right pull from token ids without next_tokens."""
 
     def __init__(self, vocab_size: int, byte_vocab_size: int, token_dim: int, byte_dim: int, model_dim: int,
                  bytes_per_token: int = 16, byte_mixin_method: str = "concat", pull_in: bool = True,
@@ -280,13 +281,14 @@ class SptByteMixEmbedding(nn.Module):
         self.register_buffer("ttb", ttb, persistent=False)
 
     def forward(self, tokens: torch.Tensor, byte_tensor: Optional[torch.Tensor] = None,
-                byte_tensor_pulled: Optional[torch.Tensor] = None) -> torch.Tensor:
+                byte_tensor_pulled: Optional[torch.Tensor] = None, *,
+                next_tokens: Optional[torch.Tensor] = None) -> torch.Tensor:
         B, S = tokens.shape
         if self.method == "noop":   # _forward_tokens, :342-348
             x = mot_embed(tokens, None, self.embed.embed_tokens.weight, None, MixSpec(combine="tok_only"))
             return x.view(B, S, -1)
         if byte_tensor is None and byte_tensor_pulled is None and self.ttb is not None:
-            return self._forward_from_tokens(tokens)
+            return self._forward_from_tokens(tokens, next_tokens)
         ids = byte_tensor_pulled if self.pull_in else byte_tensor   # _forward_bytes_pulled / _padded, :350-369
         if ids is None:
             raise RuntimeError("mot_b200: byte ids are required (byte_tensor_pulled with pull_in, else byte_tensor)")
@@ -299,15 +301,16 @@ class SptByteMixEmbedding(nn.Module):
                            self.byte_mixin.mixin.mixin.weight, self.spec, bpt=self.bpt, byte_ids2=ids2)
         return x.view(B, S, -1)
 
-    def _forward_from_tokens(self, tokens: torch.Tensor) -> torch.Tensor:
+    def _forward_from_tokens(self, tokens: torch.Tensor, next_tokens: Optional[torch.Tensor]) -> torch.Tensor:
         B, S = tokens.shape
-        if self.pull_in and self.padding_in == "right":
+        if self.pull_in and self.padding_in == "right" and next_tokens is None:
             raise NotImplementedError("mot_b200: pulled ids of right-padded rows need the token after the last input; "
-                                      "pass byte_tensor_pulled instead")
-        spec = dataclasses.replace(self.spec, ttb_pull=self.pull_in and not self.add_padded_and_pulled)
+                                      "pass next_tokens= (the last column of the loader's window) or byte_tensor_pulled")
+        spec = dataclasses.replace(self.spec, ttb_pull=self.pull_in and not self.add_padded_and_pulled,
+                                   ttb_pull_side=self.padding_in)
         x = mot_embed_proj(tokens, None, self.embed.embed_tokens.weight, self.embed.embed_bytes.weight,
                            self.byte_mixin.mixin.mixin.weight, spec, bpt=self.bpt, ttb=self.ttb, seq_len=S,
-                           padded_and_pulled=self.add_padded_and_pulled)
+                           padded_and_pulled=self.add_padded_and_pulled, next_tokens=next_tokens)
         return x.view(B, S, -1)
 
 

@@ -29,6 +29,11 @@ class MixSpec:
     ttb_scramble: bool = False    # ids from ttb with the `.view(bpt,-1)` index map
     ttb_pull: bool = False        # ids from ttb: the pulled ids of pull_from_left over rows of seq_len tokens
     eps: float = FP32_EPS
+    ttb_pull_side: str = "left"   # with ttb_pull: "left" (pull_from_left) or "right" (pull_from_right)
+
+    def __post_init__(self):
+        if self.ttb_pull_side not in ("left", "right"):
+            raise ValueError(f"ttb_pull_side must be 'left' or 'right', got {self.ttb_pull_side!r}")
 
 
 def _require_cuda(*tensors) -> torch.device:
@@ -179,9 +184,19 @@ def pull_from_right(byte_tensor: torch.Tensor, bytes_per_token: int, pad_byte: i
 PAD_ID, EOT_ID = 456, 457   # pad and end-of-text byte of the ttb tables (spt/data_creation.py; pull_from_left's defaults)
 
 
+def _pull_flags(spec: MixSpec, next_tok: bool) -> int:
+    """MOT_F_TTB_PULL_LEFT / _RIGHT (+ MOT_F_TTB_NEXT_TOK: the lookahead tail after the token ids) of spec.ttb_pull."""
+    if not spec.ttb_pull:
+        return 0
+    if spec.ttb_pull_side == "left":
+        return L.F_TTB_PULL_LEFT
+    return L.F_TTB_PULL_RIGHT | (L.F_TTB_NEXT_TOK if next_tok else 0)
+
+
 def make_desc(spec: MixSpec, n_tokens: int, E_tok, E_byte, bpt: int, *, ids: Optional[torch.Tensor],
               ttb: Optional[torch.Tensor], has_lam: bool, seq_len: int = 0, row_stride: int = 0,
-              col_offset: int = 0, dp_slabs: int = 0, pad_id: int = PAD_ID, eot_id: int = EOT_ID) -> L.MotDesc:
+              col_offset: int = 0, dp_slabs: int = 0, pad_id: int = PAD_ID, eot_id: int = EOT_ID,
+              next_tok: bool = False) -> L.MotDesc:
     ref = E_tok if E_tok is not None else E_byte
     if ref.dtype not in _DTYPE:
         raise NotImplementedError(f"mot_b200: embedding dtype {ref.dtype} is not supported (bf16 / fp32 only)")
@@ -209,7 +224,7 @@ def make_desc(spec: MixSpec, n_tokens: int, E_tok, E_byte, bpt: int, *, ids: Opt
                 raise RuntimeError("mot_b200: need byte ids or a ttb table")
             flags |= L.F_IDS_FROM_TTB
             flags |= L.F_TTB_SCRAMBLE if spec.ttb_scramble else 0
-            flags |= L.F_TTB_PULL_LEFT if spec.ttb_pull else 0
+            flags |= _pull_flags(spec, next_tok)
             ttb_dtype = _TTB_DTYPE[ttb.dtype]
         else:
             flags |= L.F_SLOT_MAJOR if spec.slot_major else 0
@@ -444,15 +459,43 @@ def _check_id_count(ids: torch.Tensor, n: int, bpt: int) -> None:
         raise RuntimeError(f"mot_b200: byte ids have {ids.numel()} entries, expected {n}*{bpt}")
 
 
+def _with_next(spec: MixSpec, tok: torch.Tensor, next_tokens: Optional[torch.Tensor], seq_len: int):
+    """The lookahead of a right pull -> (tok, next): both views of ONE int32 buffer [tok | next], so that the kernels
+    find token seq_len of row r at tok[n + r] (MOT_F_TTB_NEXT_TOK) while the plan and the gathers see n tokens."""
+    if next_tokens is None:
+        return tok, None
+    if not (spec.ttb_pull and spec.ttb_pull_side == "right"):
+        raise RuntimeError("mot_b200: next_tokens= is the lookahead of a right pull (ttb ids with ttb_pull_side='right')")
+    if next_tokens.dtype not in (torch.int32, torch.int64):
+        raise NotImplementedError("mot_b200: next_tokens must be int32 or int64")
+    rows = tok.numel() // seq_len
+    if next_tokens.numel() != rows:
+        raise RuntimeError(f"mot_b200: next_tokens has {next_tokens.numel()} entries, expected one per row ({rows})")
+    n = tok.numel()
+    buf = torch.cat((tok, next_tokens.reshape(-1).to(torch.int32)))
+    return buf[:n], buf[n:]
+
+
+def _tok_next(tok: torch.Tensor, next_tok: Optional[torch.Tensor]) -> torch.Tensor:
+    """Token ids whose lookahead follows them in memory (the operators receive tok and next_tok as two tensors; the
+    argument helper made them views of one buffer, which a traced graph may not keep)."""
+    if next_tok is None or next_tok.numel() == 0:
+        return tok
+    if next_tok.data_ptr() == tok.data_ptr() + 4 * tok.numel():
+        return tok
+    return torch.cat((tok, next_tok))[:tok.numel()]
+
+
 def _require_chain_dtype(E_tok: torch.Tensor, E_byte: torch.Tensor) -> None:
     """The projection chains compute in the table dtype: bf16, or fp32 on the TF32 tensor-core path."""
     if E_tok.dtype not in (torch.bfloat16, torch.float32) or E_byte.dtype != E_tok.dtype:
         raise NotImplementedError("mot_b200: token and byte tables must both be bf16 or both fp32")
 
 
-def _embed_args(bpt: int, tokens, byte_ids, ttb, E_tok, E_byte, lam):
-    """mot_embed's arguments checked and normalised -> (dev, tok, ids, E_tok, E_byte)."""
-    dev = _require_cuda(tokens, byte_ids, ttb, E_tok, E_byte, lam)
+def _embed_args(bpt: int, tokens, byte_ids, ttb, E_tok, E_byte, lam, spec: Optional[MixSpec] = None, seq_len: int = 0,
+                next_tokens=None):
+    """mot_embed's arguments checked and normalised -> (dev, tok, ids, E_tok, E_byte, next_tok)."""
+    dev = _require_cuda(tokens, byte_ids, ttb, E_tok, E_byte, lam, next_tokens)
     tok = _tok_i32(tokens) if tokens is not None else None
     ids = None
     if byte_ids is not None:
@@ -462,22 +505,31 @@ def _embed_args(bpt: int, tokens, byte_ids, ttb, E_tok, E_byte, lam):
     E_byte = E_byte.contiguous() if E_byte is not None else None
     if E_tok is not None and E_byte is not None and E_tok.dtype != E_byte.dtype:
         raise NotImplementedError("mot_b200: token and byte tables must share one dtype")
-    return dev, tok, ids, E_tok, E_byte
+    nxt = None
+    if next_tokens is not None:
+        if tok is None or ids is not None or ttb is None:
+            raise RuntimeError("mot_b200: next_tokens= is the lookahead of a right pull (ttb ids with ttb_pull_side='right')")
+        _ttb_ids_args(spec, tok, ttb, seq_len)
+        tok, nxt = _with_next(spec, tok, next_tokens, seq_len)
+    return dev, tok, ids, E_tok, E_byte, nxt
 
 
 def _embed_desc(spec: MixSpec, bpt: int, seq_len: int, tok, ids, ttb, E_tok, E_byte, has_lam: bool,
-                dp_slabs: int = 0) -> L.MotDesc:
+                dp_slabs: int = 0, next_tok: bool = False) -> L.MotDesc:
     n = tok.numel() if tok is not None else ids.numel() // bpt
-    return make_desc(spec, n, E_tok, E_byte, bpt, ids=ids, ttb=ttb, has_lam=has_lam, seq_len=seq_len, dp_slabs=dp_slabs)
+    return make_desc(spec, n, E_tok, E_byte, bpt, ids=ids, ttb=ttb, has_lam=has_lam, seq_len=seq_len, dp_slabs=dp_slabs,
+                     next_tok=next_tok)
 
 
 class _MotEmbedFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, spec: MixSpec, bpt: int, seq_len: int, dev, tok, ids, ttb, E_tok, E_byte, lam, grad_bufs=None):
+    def forward(ctx, spec: MixSpec, bpt: int, seq_len: int, dev, tok, ids, ttb, E_tok, E_byte, lam, grad_bufs=None,
+                next_tok=None):
         # optional ((param_tok, view_tok), (param_byte, view_byte)): views of a dp.GradBucket that become param.grad
         ctx.grad_bufs = grad_bufs
         lam_c = lam.detach().to(torch.float32).contiguous() if lam is not None else None
-        desc = _embed_desc(spec, bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None)
+        has_next = next_tok is not None   # tok is the head of [tok | next_tok] (_with_next)
+        desc = _embed_desc(spec, bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None, next_tok=has_next)
         n = desc.n_tokens
         # data-parallel pipeline: a bucket that holds exactly [token table | byte table] in symmetric memory lets the
         # backward run as vocabulary slabs with the exchange of slab k beside the backward of slab k + 1
@@ -486,7 +538,8 @@ class _MotEmbedFn(torch.autograd.Function):
         if bucket is not None and bucket.pipelined and n > 0 and E_tok is not None and E_byte is not None \
                 and len(bucket.params) == 2 and bucket.params[0] is grad_bufs[0][0] and bucket.params[1] is grad_bufs[1][0] \
                 and bool(L.lib().mot_embed_bwd_uses_saved(desc)):
-            desc = _embed_desc(spec, bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None, dp_slabs=bucket.n_slabs)
+            desc = _embed_desc(spec, bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None, dp_slabs=bucket.n_slabs,
+                               next_tok=has_next)
             ctx.dp_bucket = bucket
         ref = E_tok if E_tok is not None else E_byte
         out = torch.empty((n, desc.out_dim), dtype=ref.dtype, device=dev)
@@ -561,26 +614,30 @@ class _MotEmbedFn(torch.autograd.Function):
             direct[0][0].grad, gE_tok = gE_tok, None
         if direct[1] is not None:
             direct[1][0].grad, gE_byte = gE_byte, None
-        return None, None, None, None, None, None, None, gE_tok, gE_byte, g_lam, None
+        return None, None, None, None, None, None, None, gE_tok, gE_byte, g_lam, None, None
 
 
 def mot_embed(tokens: Optional[torch.Tensor], byte_ids: Optional[torch.Tensor], E_tok: Optional[torch.Tensor],
               E_byte: Optional[torch.Tensor], spec: MixSpec, *, bpt: int = 16, lam: Optional[torch.Tensor] = None,
-              ttb: Optional[torch.Tensor] = None, seq_len: int = 0, grad_bufs=None) -> torch.Tensor:
+              ttb: Optional[torch.Tensor] = None, seq_len: int = 0, grad_bufs=None,
+              next_tokens: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Fused gather + pool + combine + norm.  Returns [n_tokens, out_dim] in the table dtype.
 
     tokens   int32/int64 [..] (flattened); byte_ids int32/int64 with n_tokens*bpt entries, token-major
     ([.., T*bpt]) or slot-major ([bpt, T], spec.slot_major); byte_ids=None derives the ids from `ttb`
     inside the kernel.  lam = float tensor [2] = (lam_tok, lam_byte) or None.  grad_bufs = optional
     ((param, view), (param, view)) pairs for the token / byte table: the backward writes the dense gradient into `view`
-    (a slice of a dp.GradBucket) and installs it as `param.grad`."""
-    dev, tok, ids, E_tok_c, E_byte_c = _embed_args(bpt, tokens, byte_ids, ttb, E_tok, E_byte, lam)
+    (a slice of a dp.GradBucket) and installs it as `param.grad`.  next_tokens: with spec.ttb_pull and
+    ttb_pull_side="right", token seq_len of every row ([n_tokens / seq_len], the last column of the loader's window of
+    seq_len + 1 tokens), which the right pull of the row's last tokens reads; without it the row ends at its last input."""
+    dev, tok, ids, E_tok_c, E_byte_c, nxt = _embed_args(bpt, tokens, byte_ids, ttb, E_tok, E_byte, lam, spec, seq_len,
+                                                        next_tokens)
     if grad_bufs is None and _custom_ops_wanted():
         lam32 = lam.to(torch.float32).contiguous() if lam is not None else None   # differentiable cast
         need = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (E_tok, E_byte, lam))
         return torch.ops.mot_b200.embed(tok, ids, ttb.contiguous() if ttb is not None else None, E_tok_c, E_byte_c, lam32,
-                                        pack_spec(spec), bpt, seq_len, float(spec.eps), need)[0]
-    return _MotEmbedFn.apply(spec, bpt, seq_len, dev, tok, ids, ttb, E_tok_c, E_byte_c, lam, grad_bufs)
+                                        pack_spec(spec), bpt, seq_len, float(spec.eps), need, nxt)[0]
+    return _MotEmbedFn.apply(spec, bpt, seq_len, dev, tok, ids, ttb, E_tok_c, E_byte_c, lam, grad_bufs, nxt)
 
 
 # ------------------------------------------------------------------------------------------------------------
@@ -767,27 +824,29 @@ def _ttb_pair_args(tok, ttb, seq_len: int):
     return (_ptr(tok), _ptr(ttb), ttb.shape[0], _TTB_DTYPE[ttb.dtype], seq_len, PAD_ID, EOT_ID, tok.numel())
 
 
-def byte_pair_ttb_forward_out(tok, ttb, seq_len: int, bpt: int, E_byte, out, col_offset: int, eps: float = FP32_EPS) -> None:
-    """mot_byte_pair_ttb_fwd: byte_pair_forward_out with ids_a = the padded and ids_b = the pulled ids of `tok`, both
-    derived from the ttb table inside the kernel (rows of seq_len tokens)."""
+def byte_pair_ttb_forward_out(tok, ttb, seq_len: int, bpt: int, E_byte, out, col_offset: int, eps: float = FP32_EPS,
+                              pull_flags: int = L.F_TTB_PULL_LEFT) -> None:
+    """mot_byte_pair_ttb_ex_fwd: byte_pair_forward_out with ids_a = the padded and ids_b = the pulled ids of `tok`, both
+    derived from the ttb table inside the kernel (rows of seq_len tokens).  pull_flags: the direction (_pull_flags)."""
     dev = _require_cuda(tok, ttb, E_byte, out)
     with _on_device(dev):
-        rc = L.lib().mot_byte_pair_ttb_fwd(*_ttb_pair_args(tok, ttb, seq_len), bpt, _ptr(E_byte), E_byte.shape[0],
-                                           E_byte.shape[1], _DTYPE[E_byte.dtype], eps, _ptr(out), out.stride(0), col_offset,
-                                           _stream(dev))
+        rc = L.lib().mot_byte_pair_ttb_ex_fwd(*_ttb_pair_args(tok, ttb, seq_len), bpt, _ptr(E_byte), E_byte.shape[0],
+                                              E_byte.shape[1], _DTYPE[E_byte.dtype], eps, _ptr(out), out.stride(0),
+                                              col_offset, pull_flags, _stream(dev))
     L.check(rc, "mot_byte_pair_ttb_fwd")
 
 
 def byte_pair_ttb_backward_out(tok, ttb, seq_len: int, bpt: int, E_byte, grad_rows, col_offset: int, gE_byte,
-                               eps: float = FP32_EPS) -> None:
-    """mot_byte_pair_ttb_bwd: byte_pair_backward_out with both id sets derived from `tok` and the ttb table."""
+                               eps: float = FP32_EPS, pull_flags: int = L.F_TTB_PULL_LEFT) -> None:
+    """mot_byte_pair_ttb_ex_bwd: byte_pair_backward_out with both id sets derived from `tok` and the ttb table."""
     dev = _require_cuda(tok, ttb, E_byte, grad_rows, gE_byte)
     need = int(L.lib().mot_byte_pair_workspace_bytes(E_byte.shape[0], E_byte.shape[1]))
     ws = torch.empty(need, dtype=torch.uint8, device=dev)
     with _on_device(dev):
-        rc = L.lib().mot_byte_pair_ttb_bwd(*_ttb_pair_args(tok, ttb, seq_len), bpt, _ptr(E_byte), E_byte.shape[0],
-                                           E_byte.shape[1], _DTYPE[E_byte.dtype], eps, _ptr(grad_rows), grad_rows.stride(0),
-                                           col_offset, _ptr(gE_byte), _ptr(ws), ws.numel(), _stream(dev))
+        rc = L.lib().mot_byte_pair_ttb_ex_bwd(*_ttb_pair_args(tok, ttb, seq_len), bpt, _ptr(E_byte), E_byte.shape[0],
+                                              E_byte.shape[1], _DTYPE[E_byte.dtype], eps, _ptr(grad_rows),
+                                              grad_rows.stride(0), col_offset, _ptr(gE_byte), _ptr(ws), ws.numel(),
+                                              pull_flags, _stream(dev))
     L.check(rc, "mot_byte_pair_ttb_bwd")
 
 
@@ -880,13 +939,14 @@ def _ttb_ids_args(spec: MixSpec, tok, ttb, seq_len: int) -> torch.Tensor:
 
 
 def _proj_args(spec: MixSpec, bpt: int, tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2, ttb=None, seq_len: int = 0,
-               ttb_pair: bool = False):
-    """mot_embed_proj's arguments checked and normalised -> (dev, tok, ids, ids2, E_tok, E_byte, ttb).  Without byte
-    ids the ids come from `ttb` (the pulled ones under spec.ttb_pull; with ttb_pair the padded and the pulled ones)."""
-    dev = _require_cuda(tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2, ttb)
+               ttb_pair: bool = False, next_tokens=None):
+    """mot_embed_proj's arguments checked and normalised -> (dev, tok, ids, ids2, E_tok, E_byte, ttb, next_tok).  Without
+    byte ids the ids come from `ttb` (the pulled ones under spec.ttb_pull; with ttb_pair the padded and the pulled ones);
+    next_tokens: the lookahead of a right pull (_with_next)."""
+    dev = _require_cuda(tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2, ttb, next_tokens)
     _require_chain_dtype(E_tok, E_byte)
     tok = _tok_i32(tokens)
-    ids = ids2 = None
+    ids = ids2 = nxt = None
     if byte_ids is None:
         if ttb is None:
             raise RuntimeError("mot_b200: need byte ids or a ttb table")
@@ -896,7 +956,10 @@ def _proj_args(spec: MixSpec, bpt: int, tokens, byte_ids, E_tok, E_byte, W, bias
                                           "ids and [tok | bytes] order (spt/train_gpt.py:371-379,442-443)")
             spec = dataclasses.replace(spec, ttb_pull=True)
         ttb = _ttb_ids_args(spec, tok, ttb, seq_len)
+        tok, nxt = _with_next(spec, tok, next_tokens, seq_len)
     else:
+        if next_tokens is not None:
+            raise RuntimeError("mot_b200: next_tokens= is the lookahead of a right pull (ttb ids with ttb_pull_side='right')")
         ttb = None
         ids = _byte_ids(byte_ids)
         _check_id_count(ids, tok.numel(), bpt)
@@ -915,10 +978,11 @@ def _proj_args(spec: MixSpec, bpt: int, tokens, byte_ids, E_tok, E_byte, W, bias
         raise RuntimeError(f"mot_b200: projection weight is {tuple(W.shape)}, expected [{W.shape[0]}, {K}]")
     if bias is not None and bias.dtype != torch.float32:
         raise NotImplementedError("mot_b200: the projection bias must be fp32 (mathblations/model.py:261)")
-    return dev, tok, ids, ids2, E_tok.contiguous(), E_byte.contiguous(), ttb
+    return dev, tok, ids, ids2, E_tok.contiguous(), E_byte.contiguous(), ttb, nxt
 
 
-def _proj_desc(spec: MixSpec, bpt: int, tok, ids, E_tok, E_byte, pair: bool, ttb=None, seq_len: int = 0) -> L.MotDesc:
+def _proj_desc(spec: MixSpec, bpt: int, tok, ids, E_tok, E_byte, pair: bool, ttb=None, seq_len: int = 0,
+               next_tok: bool = False) -> L.MotDesc:
     """Descriptor of the gather of the [n, K] operand: the concat of both tables, or with `pair` (two byte-id tensors)
     only its token columns, written with row stride K (the pair kernels write the byte columns).  ids=None: the ids come
     from `ttb` (rows of seq_len tokens)."""
@@ -927,23 +991,30 @@ def _proj_desc(spec: MixSpec, bpt: int, tok, ids, E_tok, E_byte, pair: bool, ttb
                          E_tok, None, 0, ids=None, ttb=None, has_lam=False,
                          row_stride=E_tok.shape[1] + bpt * E_byte.shape[1], col_offset=0)
     return make_desc(dataclasses.replace(spec, combine="concat", out_norm=False), tok.numel(), E_tok, E_byte, bpt,
-                     ids=ids, ttb=ttb, has_lam=False, seq_len=seq_len)
+                     ids=ids, ttb=ttb, has_lam=False, seq_len=seq_len, next_tok=next_tok)
+
+
+def _pair_pull_flags(spec: MixSpec, next_tok: bool) -> int:
+    """Direction of the pulled half of the token-only padded+pulled pair."""
+    return _pull_flags(dataclasses.replace(spec, ttb_pull=True), next_tok)
 
 
 def _gather_operand(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_tok, E_byte, A, ttb=None,
-                    seq_len: int = 0, pair: bool = False) -> None:
+                    seq_len: int = 0, pair: bool = False, next_tok: bool = False) -> None:
     if not pair:
         embed_forward_out(desc, tok, ids, ttb, E_tok, E_byte, None, A)
     elif tok.numel() > 0:
         embed_forward_out(desc, tok, None, None, E_tok, None, None, A)
         if ttb is not None:
-            byte_pair_ttb_forward_out(tok, ttb, seq_len, bpt, E_byte, A, E_tok.shape[1], spec.eps)
+            byte_pair_ttb_forward_out(tok, ttb, seq_len, bpt, E_byte, A, E_tok.shape[1], spec.eps,
+                                      _pair_pull_flags(spec, next_tok))
         else:
             byte_pair_forward_out(ids, ids2, bpt, E_byte, A, E_tok.shape[1], spec.eps)
 
 
 def _scatter_operand(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_tok, E_byte, dA, ws_buf,
-                     plan_ready: bool, ws_clean: bool, ttb=None, seq_len: int = 0, pair: bool = False):
+                     plan_ready: bool, ws_clean: bool, ttb=None, seq_len: int = 0, pair: bool = False,
+                     next_tok: bool = False):
     """The backward of _gather_operand: dense (gE_tok, gE_byte) from the operand's gradient dA."""
     gE_tok, gE_byte = torch.empty_like(E_tok), torch.empty_like(E_byte)
     if not pair:
@@ -953,19 +1024,20 @@ def _scatter_operand(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E
         embed_backward_out(desc, tok, None, None, E_tok, None, None, dA, gE_tok, None, None, ws_buf,
                            plan_ready=plan_ready, ws_clean=ws_clean)
         if ttb is not None:
-            byte_pair_ttb_backward_out(tok, ttb, seq_len, bpt, E_byte, dA, E_tok.shape[1], gE_byte, spec.eps)
+            byte_pair_ttb_backward_out(tok, ttb, seq_len, bpt, E_byte, dA, E_tok.shape[1], gE_byte, spec.eps,
+                                       _pair_pull_flags(spec, next_tok))
         else:
             byte_pair_backward_out(ids, ids2, bpt, E_byte, dA, E_tok.shape[1], gE_byte, spec.eps)
     return gE_tok, gE_byte
 
 
 def _proj_forward(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_tok, E_byte, w_c, bias,
-                  keep_operand: bool, ttb=None, seq_len: int = 0, pair: bool = False):
+                  keep_operand: bool, ttb=None, seq_len: int = 0, pair: bool = False, next_tok: bool = False):
     """-> (out, Y, A): Y = A . w_c^T (+ bias) with the gathered [n, K] operand A (None unless keep_operand), out = the
     row norm of Y under spec.out_norm, else Y itself.  w_c: the weight in the table dtype."""
     n, (Do, K), dev, cdt = tok.numel(), w_c.shape, E_tok.device, E_tok.dtype
     A = torch.empty((n, K), dtype=cdt, device=dev)
-    _gather_operand(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, A, ttb, seq_len, pair)
+    _gather_operand(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, A, ttb, seq_len, pair, next_tok)
     Y = torch.empty((n, Do), dtype=cdt, device=dev)
     linear_forward_out(A, w_c, Y, bias.contiguous() if bias is not None else None)
     if not keep_operand:
@@ -979,7 +1051,7 @@ def _proj_forward(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_to
 
 
 def _proj_backward(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_tok, E_byte, w_c, w_dtype, has_bias: bool,
-                   Y, A, grad_out, ttb=None, seq_len: int = 0, pair: bool = False):
+                   Y, A, grad_out, ttb=None, seq_len: int = 0, pair: bool = False, next_tok: bool = False):
     """The backward of _proj_forward down to the operand -> (dA, gW in w_dtype, g_bias fp32 or None).  A: the forward's
     operand if it was kept, else None (gathered again here)."""
     n, (Do, K), dev, cdt = tok.numel(), w_c.shape, E_tok.device, E_tok.dtype
@@ -994,7 +1066,7 @@ def _proj_backward(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_t
         dA = torch.empty((n, K), dtype=cdt, device=dev)                   # a saved tensor is never overwritten
     else:
         A = torch.empty((n, K), dtype=cdt, device=dev)
-        _gather_operand(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, A, ttb, seq_len, pair)
+        _gather_operand(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, A, ttb, seq_len, pair, next_tok)
         dA = A                                                            # dX may overwrite the private copy
     dW32 = torch.empty((Do, K), dtype=torch.float32, device=dev)
     dW16 = torch.empty((Do, K), dtype=torch.bfloat16, device=dev) if w_dtype == torch.bfloat16 else None
@@ -1012,15 +1084,17 @@ class _MotEmbedProjFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, spec: MixSpec, bpt: int, dev, tok, ids, ids2, E_tok, E_byte, W, bias, ttb=None, seq_len: int = 0,
-                pair: bool = False):
+                pair: bool = False, next_tok=None):
         pair = pair or ids2 is not None
-        desc = _proj_desc(spec, bpt, tok, ids, E_tok, E_byte, pair, ttb, seq_len)
+        has_next = next_tok is not None   # tok is the head of [tok | next_tok] (_with_next)
+        desc = _proj_desc(spec, bpt, tok, ids, E_tok, E_byte, pair, ttb, seq_len, has_next)
         w16 = cast_out(W, E_tok.dtype)                         # CastedLinear: W.type_as(x) (spt/train_gpt.py:186)
         ctx.ws = _planned_workspace(desc, tok, dev) if any(ctx.needs_input_grad[6:8]) and tok.numel() > 0 else None
         keep_A = _PROJ_KEEP_OPERAND and any(ctx.needs_input_grad[6:10])
-        out, Y, A = _proj_forward(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, w16, bias, keep_A, ttb, seq_len, pair)
+        out, Y, A = _proj_forward(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, w16, bias, keep_A, ttb, seq_len, pair,
+                                  has_next)
         embed_plan_join_if_capturing(ctx.ws, dev)
-        ctx.desc, ctx.dev, ctx.spec, ctx.bpt, ctx.seq_len = desc, dev, spec, bpt, seq_len
+        ctx.desc, ctx.dev, ctx.spec, ctx.bpt, ctx.seq_len, ctx.has_next = desc, dev, spec, bpt, seq_len, has_next
         ctx.w_dtype, ctx.has_bias = W.dtype, bias is not None
         ctx.pair, ctx.kept_A = pair, keep_A
         ctx.present = (ids is not None, ids2 is not None, keep_A, ttb is not None)
@@ -1034,40 +1108,44 @@ class _MotEmbedProjFn(torch.autograd.Function):
         ids, ids2, A, ttb = [t if ok else None for t, ok in zip((ids, ids2, A, ttb), ctx.present)]
         desc, dev, spec, bpt, seq_len, pair = ctx.desc, ctx.dev, ctx.spec, ctx.bpt, ctx.seq_len, ctx.pair
         dA, gW, g_bias = _proj_backward(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, w16, ctx.w_dtype, ctx.has_bias,
-                                        Y, A, grad_out, ttb, seq_len, pair)
+                                        Y, A, grad_out, ttb, seq_len, pair, ctx.has_next)
         ws, planned, clean = _take_workspace(ctx.ws, desc, dev)
         gE_tok, gE_byte = _scatter_operand(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, dA, ws.buf, planned, clean,
-                                           ttb, seq_len, pair)
+                                           ttb, seq_len, pair, ctx.has_next)
         ctx.ws = None
         _return_workspace(ws)
-        return None, None, None, None, None, None, gE_tok, gE_byte, gW, g_bias, None, None, None
+        return None, None, None, None, None, None, gE_tok, gE_byte, gW, g_bias, None, None, None, None
 
 
 def _byte_fc_args(bpt: int, tokens, byte_ids, E_tok, E_byte, W, spec_b: Optional[MixSpec] = None, ttb=None,
-                  seq_len: int = 0):
-    """mot_embed_byte_fc's arguments checked and normalised -> (dev, tok, ids, E_tok, E_byte, ttb)."""
-    dev = _require_cuda(tokens, byte_ids, E_tok, E_byte, W, ttb)
+                  seq_len: int = 0, next_tokens=None):
+    """mot_embed_byte_fc's arguments checked and normalised -> (dev, tok, ids, E_tok, E_byte, ttb, next_tok)."""
+    dev = _require_cuda(tokens, byte_ids, E_tok, E_byte, W, ttb, next_tokens)
     _require_chain_dtype(E_tok, E_byte)
     tok = _tok_i32(tokens)
     D = E_tok.shape[1]
+    nxt = None
     if byte_ids is None:
         if ttb is None:
             raise RuntimeError("mot_b200: need byte ids or a ttb table")
         ids, ttb = None, _ttb_ids_args(spec_b, tok, ttb, seq_len)
+        tok, nxt = _with_next(spec_b, tok, next_tokens, seq_len)
         n_ids = tok.numel() * bpt
     else:
+        if next_tokens is not None:
+            raise RuntimeError("mot_b200: next_tokens= is the lookahead of a right pull (ttb ids with ttb_pull_side='right')")
         ids, ttb = _byte_ids(byte_ids), None
         n_ids = ids.numel()
     if n_ids != tok.numel() * bpt or bpt * E_byte.shape[1] != D or tuple(W.shape) != (D, D):
         raise RuntimeError("mot_b200: byte-FC mix needs bpt*byte_dim == token_dim and a square [D, D] weight")
-    return dev, tok, ids, E_tok.contiguous(), E_byte.contiguous(), ttb
+    return dev, tok, ids, E_tok.contiguous(), E_byte.contiguous(), ttb, nxt
 
 
-def _fc_descs(spec_b: MixSpec, bpt: int, tok, ids, E_tok, E_byte, ttb=None, seq_len: int = 0):
+def _fc_descs(spec_b: MixSpec, bpt: int, tok, ids, E_tok, E_byte, ttb=None, seq_len: int = 0, next_tok: bool = False):
     """-> (desc_b, desc_t): the bytes-only gather of the product's operand; the token gather + addend + norm.  ids=None:
     the operand's ids come from `ttb`."""
     n = tok.numel()
-    return (make_desc(spec_b, n, None, E_byte, bpt, ids=ids, ttb=ttb, has_lam=False, seq_len=seq_len),
+    return (make_desc(spec_b, n, None, E_byte, bpt, ids=ids, ttb=ttb, has_lam=False, seq_len=seq_len, next_tok=next_tok),
             make_desc(MixSpec(combine="tok_only", out_norm=True, eps=spec_b.eps), n, E_tok, None, 0, ids=None, ttb=None,
                       has_lam=False))
 
@@ -1116,9 +1194,10 @@ class _MotEmbedByteFcFn(torch.autograd.Function):
     cores; bytes-only scatter.  The operand is gathered again in the backward, not kept."""
 
     @staticmethod
-    def forward(ctx, spec_b: MixSpec, bpt: int, dev, tok, ids, E_tok, E_byte, W, ttb=None, seq_len: int = 0):
+    def forward(ctx, spec_b: MixSpec, bpt: int, dev, tok, ids, E_tok, E_byte, W, ttb=None, seq_len: int = 0,
+                next_tok=None):
         w16 = cast_out(W, E_tok.dtype)
-        desc_b, desc_t = _fc_descs(spec_b, bpt, tok, ids, E_tok, E_byte, ttb, seq_len)
+        desc_b, desc_t = _fc_descs(spec_b, bpt, tok, ids, E_tok, E_byte, ttb, seq_len, next_tok is not None)
         ctx.ws = _planned_workspace(desc_t, tok, dev) if ctx.needs_input_grad[5] and tok.numel() > 0 else None
         out, Y = _byte_fc_forward(desc_b, desc_t, tok, ids, E_tok, E_byte, w16, ttb)
         embed_plan_join_if_capturing(ctx.ws, dev)
@@ -1139,30 +1218,34 @@ class _MotEmbedByteFcFn(torch.autograd.Function):
         ctx.ws = None
         _return_workspace(ws)
         _return_workspace(wsb)
-        return None, None, None, None, None, gE_tok, gE_byte, gW, None, None
+        return None, None, None, None, None, gE_tok, gE_byte, gW, None, None, None
 
 
 def mot_embed_byte_fc(tokens: torch.Tensor, byte_ids: Optional[torch.Tensor], E_tok: torch.Tensor, E_byte: torch.Tensor,
                       W_fc: torch.Tensor, *, bpt: int = 16, slot_major: bool = True, eps: float = FP32_EPS,
-                      ttb: Optional[torch.Tensor] = None, seq_len: int = 0, ttb_pull: bool = False) -> torch.Tensor:
+                      ttb: Optional[torch.Tensor] = None, seq_len: int = 0, ttb_pull: bool = False,
+                      ttb_pull_side: str = "left", next_tokens: Optional[torch.Tensor] = None) -> torch.Tensor:
     """`norm(token_embs + F.linear(cat(byte_embs), byte_fc))` (runs/71051:226-229,312-314): [n_tokens, D].
     byte_ids=None: the ids come from `ttb` inside the kernels (rows of seq_len tokens; the `.view(bpt,-1)` order under
-    slot_major), the pulled ids of pull_from_left with ttb_pull."""
+    slot_major), the pulled ids of pull_from_left with ttb_pull (pull_from_right with ttb_pull_side="right", whose
+    lookahead `next_tokens` holds token seq_len of every row, as in mot_embed)."""
     spec_b = MixSpec(combine="bytes_only", out_norm=False, slot_major=slot_major and byte_ids is not None,
-                     ttb_scramble=slot_major and byte_ids is None, ttb_pull=ttb_pull and byte_ids is None, eps=eps)
-    dev, tok, ids, E_tok_c, E_byte_c, ttb_c = _byte_fc_args(bpt, tokens, byte_ids, E_tok, E_byte, W_fc, spec_b, ttb, seq_len)
+                     ttb_scramble=slot_major and byte_ids is None, ttb_pull=ttb_pull and byte_ids is None, eps=eps,
+                     ttb_pull_side=ttb_pull_side)
+    dev, tok, ids, E_tok_c, E_byte_c, ttb_c, nxt = _byte_fc_args(bpt, tokens, byte_ids, E_tok, E_byte, W_fc, spec_b, ttb,
+                                                                 seq_len, next_tokens)
     if _custom_ops_wanted():
         need = torch.is_grad_enabled() and any(t.requires_grad for t in (E_tok, E_byte, W_fc))
         return torch.ops.mot_b200.embed_byte_fc(tok, ids if ids is not None else tok.new_empty(0), E_tok_c, E_byte_c,
                                                 W_fc.contiguous(), pack_spec(spec_b), bpt, float(eps), need, ttb_c,
-                                                seq_len)[0]
-    return _MotEmbedByteFcFn.apply(spec_b, bpt, dev, tok, ids, E_tok_c, E_byte_c, W_fc, ttb_c, seq_len)
+                                                seq_len, nxt)[0]
+    return _MotEmbedByteFcFn.apply(spec_b, bpt, dev, tok, ids, E_tok_c, E_byte_c, W_fc, ttb_c, seq_len, nxt)
 
 
 def mot_embed_proj(tokens: torch.Tensor, byte_ids: Optional[torch.Tensor], E_tok: torch.Tensor, E_byte: torch.Tensor,
                    W: torch.Tensor, spec: MixSpec, *, bpt: int = 16, bias: Optional[torch.Tensor] = None,
                    byte_ids2: Optional[torch.Tensor] = None, ttb: Optional[torch.Tensor] = None, seq_len: int = 0,
-                   padded_and_pulled: bool = False) -> torch.Tensor:
+                   padded_and_pulled: bool = False, next_tokens: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Concat + dense projection variants: `norm(F.linear(cat([f(tok), f(bytes)]), W))` (runs/7:226-234, runs/72,
     spt/train_gpt.py:439-443).  spec.tok_norm / byte_norm are the per-input norms, spec.out_norm the norm after the
     projection, spec.bytes_first the operand order.  Tables bf16 with W bf16 (runs) or an fp32 master (spt: cast per
@@ -1172,16 +1255,17 @@ def mot_embed_proj(tokens: torch.Tensor, byte_ids: Optional[torch.Tensor], E_tok
 
     Token-only form: byte_ids=None with the [V, bpt] table `ttb` derives the ids inside the kernels -- the padded ids, or
     with spec.ttb_pull the pulled ids of pull_from_left over rows of `seq_len` tokens; padded_and_pulled=True derives
-    both sets of `--add-padded-and-pulled`."""
+    both sets of `--add-padded-and-pulled`.  spec.ttb_pull_side="right": pull_from_right, with the lookahead
+    `next_tokens` (token seq_len of every row, as in mot_embed)."""
     pair = padded_and_pulled and byte_ids is None
-    dev, tok, ids, ids2, E_tok_c, E_byte_c, ttb_c = _proj_args(spec, bpt, tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2,
-                                                               ttb, seq_len, pair)
+    dev, tok, ids, ids2, E_tok_c, E_byte_c, ttb_c, nxt = _proj_args(spec, bpt, tokens, byte_ids, E_tok, E_byte, W, bias,
+                                                                    byte_ids2, ttb, seq_len, pair, next_tokens)
     if _custom_ops_wanted():
         need = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (E_tok, E_byte, W, bias))
         return torch.ops.mot_b200.embed_proj(tok, ids if ids is not None else tok.new_empty(0), ids2, E_tok_c, E_byte_c,
                                              W.contiguous(), bias, pack_spec(spec), bpt, float(spec.eps), need, ttb_c,
-                                             seq_len, pair)[0]
-    return _MotEmbedProjFn.apply(spec, bpt, dev, tok, ids, ids2, E_tok_c, E_byte_c, W, bias, ttb_c, seq_len, pair)
+                                             seq_len, pair, nxt)[0]
+    return _MotEmbedProjFn.apply(spec, bpt, dev, tok, ids, ids2, E_tok_c, E_byte_c, W, bias, ttb_c, seq_len, pair, nxt)
 
 
 def launch_count() -> int:

@@ -1,0 +1,201 @@
+"""Right pulls from token ids alone (MOT_F_TTB_PULL_RIGHT, with the lookahead tail of MOT_F_TTB_NEXT_TOK), checked
+without a GPU: the flag values, the library's verdict on the new flag combinations, the spec code, the fake shapes of
+the operators with `next_tok`, and the refusals of a bad `next_tokens` on both dispatch paths."""
+import dataclasses
+
+import pytest
+import torch
+from torch._subclasses.fake_tensor import FakeTensorMode
+
+import mot_b200
+from mot_b200 import _lib as L
+from mot_b200 import ops
+from mot_b200._library import pack_spec, unpack_spec
+
+
+def _desc(**kw):
+    base = dict(abi_version=L.ABI_VERSION, dtype=L.BF16, n_tokens=4096, seq_len=1024, tok_vocab=50257, byte_vocab=458,
+                bpt=16, tok_dim=768, byte_dim=48, out_dim=768, combine=L.ADD,
+                flags=L.F_OUT_NORM | L.F_IDS_FROM_TTB | L.F_TTB_PULL_RIGHT, ttb_dtype=L.TTB_I16, eps=1e-7,
+                pad_id=456, eot_id=457)
+    base.update(kw)
+    return L.MotDesc(**base)
+
+
+def test_flag_values_and_symbols():
+    assert L.F_TTB_PULL_RIGHT == 1 << 10 and L.F_TTB_NEXT_TOK == 1 << 11
+    assert L.ABI_VERSION == 5 and L.lib().mot_abi_version() == 5
+    for fn in ("mot_byte_pair_ttb_ex_fwd", "mot_byte_pair_ttb_ex_bwd"):
+        assert hasattr(L.lib(), fn)
+
+
+def test_validation_of_the_right_pull_flags():
+    ws = L.lib().mot_embed_workspace_bytes
+    right, nxt = _desc().flags, _desc().flags | L.F_TTB_NEXT_TOK
+    assert ws(_desc()) > 0 and ws(_desc(flags=nxt)) > 0
+    assert ws(_desc(flags=nxt | L.F_TTB_SCRAMBLE)) > 0
+    assert ws(_desc(flags=right | L.F_TTB_PULL_LEFT)) == 0                           # both directions
+    assert ws(_desc(flags=L.F_OUT_NORM | L.F_IDS_FROM_TTB | L.F_TTB_PULL_LEFT | L.F_TTB_NEXT_TOK)) == 0
+    assert ws(_desc(flags=L.F_OUT_NORM | L.F_IDS_FROM_TTB | L.F_TTB_NEXT_TOK)) == 0  # a lookahead without a right pull
+    assert ws(_desc(seq_len=0)) == 0 and ws(_desc(seq_len=1000)) == 0                # rows as for the left pull
+    assert ws(_desc(pad_id=70000)) == 0 and ws(_desc(eot_id=-40000)) == 0
+    assert ws(_desc(combine=L.BYTES_ONLY, tok_vocab=0, tok_dim=0, flags=nxt)) == 0
+    assert ws(_desc(bpt=33, tok_dim=33 * 8, byte_dim=8, out_dim=33 * 8)) == 0
+
+
+def test_pair_ex_refuses_bad_flags():
+    # checked before anything else: no pointer is dereferenced, no device is needed
+    args = (None, None, 100, L.TTB_I16, 16, 456, 457, 64, 4, None, 458, 16, L.BF16, 1e-7)
+    fwd, bwd = L.lib().mot_byte_pair_ttb_ex_fwd, L.lib().mot_byte_pair_ttb_ex_bwd
+    for flags in (0, L.F_TTB_PULL_LEFT | L.F_TTB_PULL_RIGHT, L.F_TTB_PULL_LEFT | L.F_TTB_NEXT_TOK, L.F_TTB_NEXT_TOK,
+                  L.F_TTB_PULL_RIGHT | L.F_TTB_SCRAMBLE):
+        assert fwd(*args, None, 64, 0, flags, None) == L.ERR_BAD_ARG
+        assert bwd(*args, None, 64, 0, None, None, 0, flags, None) == L.ERR_BAD_ARG
+
+
+def test_make_desc_sets_the_right_flags():
+    E_tok, E_byte = torch.empty(100, 64), torch.empty(458, 16)
+    ttb = torch.empty(100, 4, dtype=torch.int16)
+    spec = mot_b200.MixSpec(combine="add", ttb_pull=True, ttb_pull_side="right")
+    d = ops.make_desc(spec, 64, E_tok, E_byte, 4, ids=None, ttb=ttb, has_lam=False, seq_len=32)
+    assert d.flags & L.F_TTB_PULL_RIGHT and not d.flags & (L.F_TTB_PULL_LEFT | L.F_TTB_NEXT_TOK)
+    d = ops.make_desc(spec, 64, E_tok, E_byte, 4, ids=None, ttb=ttb, has_lam=False, seq_len=32, next_tok=True)
+    assert d.flags & L.F_TTB_PULL_RIGHT and d.flags & L.F_TTB_NEXT_TOK
+    d = ops.make_desc(spec, 64, E_tok, E_byte, 4, ids=torch.empty(256, dtype=torch.int64), ttb=None, has_lam=False)
+    assert not d.flags & (L.F_TTB_PULL_LEFT | L.F_TTB_PULL_RIGHT | L.F_TTB_NEXT_TOK)
+
+
+@pytest.mark.parametrize("side", ["left", "right"])
+@pytest.mark.parametrize("pull", [False, True])
+def test_spec_round_trip(pull, side):
+    spec = mot_b200.MixSpec(combine="concat", tok_norm=True, byte_norm=True, ttb_scramble=True, ttb_pull=pull,
+                            ttb_pull_side=side)
+    code = pack_spec(spec)
+    assert bool(code & 2048) == (side == "right")
+    assert unpack_spec(code, spec.eps) == spec
+
+
+def test_invalid_pull_side():
+    with pytest.raises(ValueError, match="ttb_pull_side"):
+        mot_b200.MixSpec(ttb_pull=True, ttb_pull_side="up")
+    with pytest.raises(ValueError, match="ttb_pull_side"):
+        mot_b200.mot_embed_byte_fc(torch.zeros(8, dtype=torch.int32), None, torch.empty(10, 64), torch.empty(458, 16),
+                                   torch.empty(64, 64), bpt=4, ttb_pull=True, ttb_pull_side="middle")
+
+
+def test_right_pull_without_lookahead_still_refused():
+    ttb = torch.full((100, 16), 456, dtype=torch.int16)
+    m = mot_b200.SptByteMixEmbedding(100, 458, 64, 16, 64, ttb=ttb, padding_in="right")
+    with pytest.raises(NotImplementedError, match="next_tokens="):
+        m(torch.zeros(2, 8, dtype=torch.int32))
+
+
+N, V, VB, BPT, BD, S = 64, 100, 458, 4, 16, 16
+R = N // S
+
+
+def _t(*shape, dtype=torch.bfloat16, grad=False):
+    return torch.empty(*shape, dtype=dtype, device="cuda", requires_grad=grad)
+
+
+def test_fake_shapes_with_next_tok():
+    with FakeTensorMode():
+        tok, nxt = _t(N, dtype=torch.int32), _t(R, dtype=torch.int32)
+        ph = _t(0, dtype=torch.int32)
+        ttb = _t(V, BPT, dtype=torch.int16)
+        Et, Eb = _t(V, 64), _t(VB, BD)
+        W = _t(32, 64 + BPT * BD, dtype=torch.float32)
+        spec = pack_spec(mot_b200.MixSpec(combine="concat", tok_norm=True, byte_norm=True, ttb_pull=True,
+                                          ttb_pull_side="right"))
+        for pair in (False, True):
+            out, Y, w_c, ws = torch.ops.mot_b200.embed_proj(tok, ph, None, Et, Eb, W, None, spec, BPT, 1e-7, True, ttb, S,
+                                                            pair, nxt)
+            assert out.shape == (N, 32) and Y.shape == (N, 32) and w_c.shape == W.shape and ws.numel() > 0
+            gt, gb, gW, gbias = torch.ops.mot_b200.embed_proj_bwd(out, tok, ph, None, Et, Eb, W, w_c, Y, ws, spec, BPT,
+                                                                  1e-7, False, ttb, S, pair, nxt)
+            assert gt.shape == Et.shape and gb.shape == Eb.shape and gW.shape == W.shape and gbias.numel() == 0
+        spec_b = pack_spec(mot_b200.MixSpec(combine="bytes_only", out_norm=False, ttb_scramble=True, ttb_pull=True,
+                                            ttb_pull_side="right"))
+        Wf = _t(64, 64)
+        out, Y, w_c, ws = torch.ops.mot_b200.embed_byte_fc(tok, ph, Et, Eb, Wf, spec_b, BPT, 1e-7, True, ttb, S, nxt)
+        assert out.shape == (N, 64) and Y.shape == (N, 64) and w_c.numel() == 0
+        gt, gb, gW = torch.ops.mot_b200.embed_byte_fc_bwd(out, tok, ph, Et, Eb, Wf, w_c, Y, ws, spec_b, BPT, 1e-7, ttb, S,
+                                                          nxt)
+        assert gt.shape == Et.shape and gb.shape == Eb.shape and gW.shape == Wf.shape
+        Ea = _t(V, BPT * BD)
+        spec_e = pack_spec(mot_b200.MixSpec(combine="add", ttb_pull=True, ttb_pull_side="right"))
+        out, rstd, ws = torch.ops.mot_b200.embed(tok, None, ttb, Ea, Eb, None, spec_e, BPT, S, 1e-7, True, nxt)
+        assert out.shape == (N, BPT * BD) and ws.numel() > 0
+        gt, gb, gl = torch.ops.mot_b200.embed_bwd(out, tok, None, ttb, Ea, Eb, None, out, rstd, ws, spec_e, BPT, S, 1e-7,
+                                                  nxt)
+        assert gt.shape == Ea.shape and gb.shape == Eb.shape and gl.numel() == 0
+
+
+_RIGHT = mot_b200.MixSpec(combine="concat", tok_norm=True, byte_norm=True, ttb_pull=True, ttb_pull_side="right")
+_LEFT = mot_b200.MixSpec(combine="concat", tok_norm=True, byte_norm=True, ttb_pull=True)
+
+
+def _proj(nxt, spec=_RIGHT, pair=False):
+    Et, Eb = _t(V, 64, grad=True), _t(VB, BD, grad=True)
+    return mot_b200.mot_embed_proj(_t(N, dtype=torch.int64), None, Et, Eb, _t(32, 64 + BPT * BD, grad=True), spec,
+                                   bpt=BPT, ttb=_t(V, BPT, dtype=torch.int16), seq_len=S, padded_and_pulled=pair,
+                                   next_tokens=nxt)
+
+
+def _embed(nxt, spec=mot_b200.MixSpec(combine="add", ttb_pull=True, ttb_pull_side="right")):
+    return mot_b200.mot_embed(_t(N, dtype=torch.int32), None, _t(V, BPT * BD, grad=True), _t(VB, BD, grad=True), spec,
+                              bpt=BPT, ttb=_t(V, BPT, dtype=torch.int16), seq_len=S, next_tokens=nxt)
+
+
+def _byte_fc(nxt, side="right"):
+    return mot_b200.mot_embed_byte_fc(_t(N, dtype=torch.int32), None, _t(V, 64, grad=True), _t(VB, BD, grad=True),
+                                      _t(64, 64, grad=True), bpt=BPT, ttb=_t(V, BPT, dtype=torch.int16), seq_len=S,
+                                      ttb_pull=True, ttb_pull_side=side, next_tokens=nxt)
+
+
+def _nxt(count=R, dtype=torch.int32, device="cuda"):
+    return torch.empty(count, dtype=dtype, device=device)
+
+
+# case -> (call, exception type, a piece of its message)
+CASES = {
+    "embed_count": (lambda: _embed(_nxt(R + 1)), RuntimeError, "one per row"),
+    "embed_dtype": (lambda: _embed(_nxt(dtype=torch.float32)), NotImplementedError, "next_tokens must be int32"),
+    "embed_device": (lambda: _embed(_nxt(device="cpu")), RuntimeError, "CUDA device"),
+    "embed_left": (lambda: _embed(_nxt(), mot_b200.MixSpec(combine="add", ttb_pull=True)), RuntimeError,
+                   "lookahead of a right pull"),
+    "embed_no_pull": (lambda: _embed(_nxt(), mot_b200.MixSpec(combine="add")), RuntimeError, "lookahead of a right pull"),
+    "proj_count": (lambda: _proj(_nxt(R - 1)), RuntimeError, "one per row"),
+    "proj_dtype": (lambda: _proj(_nxt(dtype=torch.int16)), NotImplementedError, "next_tokens must be int32"),
+    "proj_left": (lambda: _proj(_nxt(), _LEFT), RuntimeError, "lookahead of a right pull"),
+    "proj_pair_left": (lambda: _proj(_nxt(), dataclasses.replace(_LEFT, ttb_pull=False), pair=True), RuntimeError,
+                       "lookahead of a right pull"),
+    "proj_pair_count": (lambda: _proj(_nxt(2 * R), dataclasses.replace(_RIGHT, ttb_pull=False), pair=True),
+                        RuntimeError, "one per row"),
+    "byte_fc_count": (lambda: _byte_fc(_nxt(1)), RuntimeError, "one per row"),
+    "byte_fc_device": (lambda: _byte_fc(_nxt(device="cpu")), RuntimeError, "CUDA device"),
+    "byte_fc_left": (lambda: _byte_fc(_nxt(), side="left"), RuntimeError, "lookahead of a right pull"),
+}
+
+
+def _raised(call):
+    try:
+        call()
+    except Exception as e:   # noqa: BLE001 -- the exception itself is the result
+        return type(e), str(e)
+    return None
+
+
+@pytest.mark.parametrize("case", sorted(CASES))
+def test_both_paths_refuse_bad_next_tokens_alike(case):
+    call, exc, text = CASES[case]
+    got = {}
+    for custom_ops in (False, True):
+        mot_b200.set_custom_ops(custom_ops)
+        try:
+            with FakeTensorMode():
+                got[custom_ops] = _raised(call)
+        finally:
+            mot_b200.set_custom_ops(None)
+    assert got[False] is not None and got[False][0] is exc and text in got[False][1], got[False]
+    assert got[True] == got[False]

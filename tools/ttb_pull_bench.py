@@ -3,11 +3,14 @@
     python tools/ttb_pull_bench.py [--steps 20] [--rounds 5] [--out DIR]
 
 For each workload two arms run the same training step (forward + backward of the embedding front):
-  explicit   : create_batch's byte part (ttb_expand -> pull_from_left -> slices) feeding the explicit-id kernels;
-  token-only : the same call with token ids alone; the kernels derive the pulled ids from the ttb table.
+  explicit   : create_batch's byte part (ttb_expand -> pull_from_left / pull_from_right -> slices) feeding the
+               explicit-id kernels;
+  token-only : the same call with token ids alone (and, for right pulls, the window's last column as the lookahead);
+               the kernels derive the pulled ids from the ttb table.
 The arms alternate inside one process (rounds x steps each, CUDA events, median round reported).  A separate
-torch.profiler pass sums the device time per kernel group.  Workloads: mot-proj-spt-64k (pull_in), mot-proj-spt-addpp-64k
-and the MoT-sum front (V3) at 48K tokens with pulled ids.  Needs a CUDA device; there is no CPU path.
+torch.profiler pass sums the device time per kernel group.  Workloads: mot-proj-spt-64k (pull_in), mot-proj-spt-addpp-64k,
+both again with padding_in="right" (-right), and the MoT-sum front (V3) at 48K tokens with pulled ids.  Needs a CUDA
+device; there is no CPU path.
 """
 from __future__ import annotations
 
@@ -29,13 +32,16 @@ from mot_b200 import data as D  # noqa: E402
 V_TOK, V_BYTE, PAD, EOT = 50257, 458, 456, 457
 
 
-def make_ttb(bpt: int, dev) -> torch.Tensor:
-    """int16 left-padded table: 1..8 bytes per token (GPT-2 tokens are short), the end-of-text row all EOT."""
+def make_ttb(bpt: int, dev, side: str = "left") -> torch.Tensor:
+    """int16 table padded on `side`: 1..8 bytes per token (GPT-2 tokens are short), the end-of-text row all EOT."""
     g = torch.Generator().manual_seed(0)
     t = torch.full((V_TOK, bpt), PAD, dtype=torch.int16)
     lens = torch.randint(1, 9, (V_TOK,), generator=g)
     vals = torch.randint(0, 256, (V_TOK, bpt), generator=g).to(torch.int16)
-    mask = torch.arange(bpt)[None, :] >= (bpt - lens)[:, None]
+    if side == "left":
+        mask = torch.arange(bpt)[None, :] >= (bpt - lens)[:, None]
+    else:
+        mask = torch.arange(bpt)[None, :] < lens[:, None]
     t[mask] = vals[mask]
     t[V_TOK - 1] = EOT
     return t.to(dev)
@@ -52,21 +58,24 @@ def workloads(dev):
     bpt = 16
     ttb = make_ttb(bpt, dev)
     out = {}
-    for name, pair in (("mot-proj-spt-64k", False), ("mot-proj-spt-addpp-64k", True)):
+    for name, pair, side in (("mot-proj-spt-64k", False, "left"), ("mot-proj-spt-addpp-64k", True, "left"),
+                             ("mot-proj-spt-64k-right", False, "right"), ("mot-proj-spt-addpp-64k-right", True, "right")):
         torch.manual_seed(0)
+        tab = ttb if side == "left" else make_ttb(bpt, dev, "right")
         mod = mot_b200.SptByteMixEmbedding(V_TOK, V_BYTE, 256, 48, 1024, bpt, pull_in=True, add_padded_and_pulled=pair,
-                                           ttb=ttb).to(dev)
+                                           ttb=tab, padding_in=side).to(dev)
         mod.embed.bfloat16()
         toks = make_tokens(64, 1025, dev)                     # [B, S+1] as the loader yields them
         gout = torch.randn(64, 1024, 1024, device=dev, dtype=torch.bfloat16)
 
-        def explicit(mod=mod, toks=toks, gout=gout):
-            ti, bp, bl, _ = D.create_batch(toks, ttb, None, bpt, pull_in=True)
+        def explicit(mod=mod, toks=toks, gout=gout, tab=tab, side=side):
+            ti, bp, bl, _ = D.create_batch(toks, tab, None, bpt, pull_in=True, padding_in=side)
             mod(ti, bp, bl).backward(gout)
 
-        def token_only(mod=mod, toks=toks, gout=gout):
-            ti, _, _, _ = D.create_batch(toks, ttb, None, bpt, pull_in=True, byte_ids=False)
-            mod(ti).backward(gout)
+        def token_only(mod=mod, toks=toks, gout=gout, tab=tab, side=side):
+            ti, _, _, _, nxt = D.create_batch(toks, tab, None, bpt, pull_in=True, padding_in=side, byte_ids=False,
+                                              next_tokens=True)
+            mod(ti, next_tokens=nxt if side == "right" else None).backward(gout)
         out[name] = (mod, explicit, token_only)
 
     torch.manual_seed(0)

@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define MOT_B200_ABI_VERSION 5
+#define MOT_B200_ABI_VERSION 6
 
 /* ---- error codes ------------------------------------------------------- */
 enum {
@@ -269,29 +269,20 @@ int mot_byte_pair_bwd(const void* ids_a, const void* ids_b, int32_t ids_i64, int
                       size_t ws_bytes, void* stream);
 
 /* The same pair with both id tensors derived from the token ids inside the kernels: ids_a = the padded ids (the ttb rows
- * of `tok`, mot_ttb_expand), ids_b = the pulled ids of pull_from_left over rows of seq_len tokens (MOT_F_TTB_PULL_LEFT).
- * tok: int32 [n_tokens], n_tokens % seq_len == 0; ttb [tok_vocab, bpt] of ttb_dtype.  Otherwise as above. */
+ * of `tok`, mot_ttb_expand; with a right-padded table the right-padded ids), ids_b = the pulled ids over rows of seq_len
+ * tokens in the direction `flags` names: MOT_F_TTB_PULL_LEFT (pull_from_left), or MOT_F_TTB_PULL_RIGHT
+ * (pull_from_right), optionally with MOT_F_TTB_NEXT_TOK (the lookahead tail tok[n_tokens + r] of every row r).  Other
+ * flags: MOT_ERR_BAD_ARG.  tok: int32 [n_tokens], n_tokens % seq_len == 0; ttb [tok_vocab, bpt] of ttb_dtype.
+ * Otherwise as above. */
 int mot_byte_pair_ttb_fwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
                           int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt, const void* E_byte,
                           int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps, void* out, int64_t row_stride,
-                          int32_t col_offset, void* stream);
+                          int32_t col_offset, int32_t flags, void* stream);
 int mot_byte_pair_ttb_bwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
                           int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt, const void* E_byte,
                           int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps, const void* grad_out,
                           int64_t row_stride, int32_t col_offset, void* gE_byte, void* workspace, size_t ws_bytes,
-                          void* stream);
-/* The same with the pull's direction in `flags`: MOT_F_TTB_PULL_LEFT (= mot_byte_pair_ttb_fwd/bwd), or
- * MOT_F_TTB_PULL_RIGHT, optionally with MOT_F_TTB_NEXT_TOK (the lookahead tail tok[n_tokens + r] of every row r).  ids_a
- * stay the ttb rows of `tok`: with a right-padded table these are the right-padded ids.  Other flags: MOT_ERR_BAD_ARG. */
-int mot_byte_pair_ttb_ex_fwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
-                             int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt, const void* E_byte,
-                             int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps, void* out,
-                             int64_t row_stride, int32_t col_offset, int32_t flags, void* stream);
-int mot_byte_pair_ttb_ex_bwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
-                             int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt, const void* E_byte,
-                             int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps, const void* grad_out,
-                             int64_t row_stride, int32_t col_offset, void* gE_byte, void* workspace, size_t ws_bytes,
-                             int32_t flags, void* stream);
+                          int32_t flags, void* stream);
 
 /* ---- data-parallel exchange: average the gradient bucket across ranks through NVLink / NVSwitch -----------------
  * Replaces the per-parameter dist.all_reduce(param.grad, AVG) of spt/train_gpt.py:1320-1321 and runs/7:697-700 (launched

@@ -361,10 +361,10 @@ extern "C" int mot_byte_pair_bwd(const void* ids_a, const void* ids_b, int32_t i
 }
 
 // The id tensors' null checks of pair_validate do not apply here: a non-null placeholder stands in for them.
-extern "C" int mot_byte_pair_ttb_ex_fwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype,
-                                        int64_t seq_len, int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt,
-                                        const void* E_byte, int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps,
-                                        void* out, int64_t row_stride, int32_t col_offset, int32_t flags, void* stream) {
+extern "C" int mot_byte_pair_ttb_fwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype,
+                                     int64_t seq_len, int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt,
+                                     const void* E_byte, int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps,
+                                     void* out, int64_t row_stride, int32_t col_offset, int32_t flags, void* stream) {
   if (!pair_pull_flags_ok(flags)) return MOT_ERR_BAD_ARG;
   if (int rc = pair_ttb_validate(tok, ttb, tok_vocab, ttb_dtype, seq_len, n_tokens)) return rc;
   if (int rc = pair_validate(tok, tok, n_tokens, bpt, E_byte, byte_vocab, byte_dim, dtype, out, row_stride, col_offset)) return rc;
@@ -378,11 +378,11 @@ extern "C" int mot_byte_pair_ttb_ex_fwd(const int32_t* tok, const void* ttb, int
   return (flags & MOT_F_TTB_PULL_RIGHT) ? run(PairTtbRightParams{}) : run(PairTtbParams{});
 }
 
-extern "C" int mot_byte_pair_ttb_ex_bwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype,
-                                        int64_t seq_len, int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt,
-                                        const void* E_byte, int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps,
-                                        const void* grad_out, int64_t row_stride, int32_t col_offset, void* gE_byte,
-                                        void* workspace, size_t ws_bytes, int32_t flags, void* stream) {
+extern "C" int mot_byte_pair_ttb_bwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype,
+                                     int64_t seq_len, int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt,
+                                     const void* E_byte, int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps,
+                                     const void* grad_out, int64_t row_stride, int32_t col_offset, void* gE_byte,
+                                     void* workspace, size_t ws_bytes, int32_t flags, void* stream) {
   if (!pair_pull_flags_ok(flags)) return MOT_ERR_BAD_ARG;
   if (int rc = pair_ttb_validate(tok, ttb, tok_vocab, ttb_dtype, seq_len, n_tokens)) return rc;
   if (int rc = pair_validate(tok, tok, n_tokens, bpt, E_byte, byte_vocab, byte_dim, dtype, grad_out, row_stride, col_offset))
@@ -394,22 +394,4 @@ extern "C" int mot_byte_pair_ttb_ex_bwd(const int32_t* tok, const void* ttb, int
     return pair_bwd(p, dtype, gE_byte, workspace, ws_bytes, stream);
   };
   return (flags & MOT_F_TTB_PULL_RIGHT) ? run(PairTtbRightParams{}) : run(PairTtbParams{});
-}
-
-extern "C" int mot_byte_pair_ttb_fwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
-                                     int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt, const void* E_byte,
-                                     int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps, void* out,
-                                     int64_t row_stride, int32_t col_offset, void* stream) {
-  return mot_byte_pair_ttb_ex_fwd(tok, ttb, tok_vocab, ttb_dtype, seq_len, pad_id, eot_id, n_tokens, bpt, E_byte, byte_vocab,
-                                  byte_dim, dtype, eps, out, row_stride, col_offset, MOT_F_TTB_PULL_LEFT, stream);
-}
-
-extern "C" int mot_byte_pair_ttb_bwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
-                                     int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt, const void* E_byte,
-                                     int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps, const void* grad_out,
-                                     int64_t row_stride, int32_t col_offset, void* gE_byte, void* workspace, size_t ws_bytes,
-                                     void* stream) {
-  return mot_byte_pair_ttb_ex_bwd(tok, ttb, tok_vocab, ttb_dtype, seq_len, pad_id, eot_id, n_tokens, bpt, E_byte, byte_vocab,
-                                  byte_dim, dtype, eps, grad_out, row_stride, col_offset, gE_byte, workspace, ws_bytes,
-                                  MOT_F_TTB_PULL_LEFT, stream);
 }

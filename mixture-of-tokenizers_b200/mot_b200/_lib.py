@@ -13,7 +13,7 @@ import sys
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmot_b200" + os.environ.get("MOT_LIB_SUFFIX", "") + ".so")  # suffix: experiment builds
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 # enums of include/mot_b200.h
 OK, ERR_BAD_ARG, ERR_UNSUPPORTED, ERR_MISALIGNED, ERR_WORKSPACE, ERR_CUDA, ERR_NO_DEVICE = range(7)
 BF16, F32 = 0, 1
@@ -74,16 +74,11 @@ _SIGNATURES = {
     "mot_byte_pair_bwd": (C.c_int, [_P, _P, C.c_int32, C.c_int64, C.c_int32, _P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P,
                                     C.c_int64, C.c_int32, _P, _P, C.c_size_t, _P]),
     "mot_byte_pair_ttb_fwd": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int32,
-                                        _P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, C.c_int64, C.c_int32, _P]),
+                                        _P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, C.c_int64, C.c_int32, C.c_int32,
+                                        _P]),
     "mot_byte_pair_ttb_bwd": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int32,
                                         _P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, C.c_int64, C.c_int32, _P, _P,
-                                        C.c_size_t, _P]),
-    "mot_byte_pair_ttb_ex_fwd": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int64,
-                                           C.c_int32, _P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, C.c_int64,
-                                           C.c_int32, C.c_int32, _P]),
-    "mot_byte_pair_ttb_ex_bwd": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int64,
-                                           C.c_int32, _P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, C.c_int64,
-                                           C.c_int32, _P, _P, C.c_size_t, C.c_int32, _P]),
+                                        C.c_size_t, C.c_int32, _P]),
     "mot_dp_exchange": (C.c_int, [_P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int64, C.c_int64, C.c_int32, C.c_uint32, C.c_int32,
                                   C.c_int32, _P]),
     "mot_embed_touched_rows": (C.c_int, [C.POINTER(MotDesc), _P, C.c_size_t, _P, _P]),

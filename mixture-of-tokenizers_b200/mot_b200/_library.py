@@ -101,9 +101,7 @@ def embed_op(tok: Optional[Tensor], ids: Optional[Tensor], ttb: Optional[Tensor]
              E_byte: Optional[Tensor], lam: Optional[Tensor], spec: int, bpt: int, seq_len: int, eps: float,
              plan: bool, next_tok: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor]:
     """-> (out [n, out_dim], rstd [n] fp32 or [0], workspace uint8 or [0]).  next_tok: the lookahead of a right pull."""
-    tok = O._tok_next(tok, next_tok)
-    desc = O._embed_desc(unpack_spec(spec, eps), bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None,
-                         next_tok=next_tok is not None)
+    tok, desc = O._ids_desc(unpack_spec(spec, eps), bpt, seq_len, tok, next_tok, ids, ttb, E_tok, E_byte, lam is not None)
     n, ref = desc.n_tokens, (E_tok if E_tok is not None else E_byte)
     dev = ref.device
     out = torch.empty((n, desc.out_dim), dtype=ref.dtype, device=dev)
@@ -119,8 +117,7 @@ def embed_op(tok: Optional[Tensor], ids: Optional[Tensor], ttb: Optional[Tensor]
 
 @embed_op.register_fake
 def _(tok, ids, ttb, E_tok, E_byte, lam, spec, bpt, seq_len, eps, plan, next_tok=None):
-    desc = O._embed_desc(unpack_spec(spec, eps), bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None,
-                         next_tok=next_tok is not None)
+    tok, desc = O._ids_desc(unpack_spec(spec, eps), bpt, seq_len, tok, next_tok, ids, ttb, E_tok, E_byte, lam is not None)
     n, ref = desc.n_tokens, (E_tok if E_tok is not None else E_byte)
     planned = plan and tok is not None and n > 0
     keep = plan and n > 0 and O.embed_bwd_uses_saved(desc)
@@ -134,9 +131,7 @@ def embed_bwd_op(grad_out: Tensor, tok: Optional[Tensor], ids: Optional[Tensor],
                  rstd: Tensor, ws: Tensor, spec: int, bpt: int, seq_len: int, eps: float,
                  next_tok: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor]:
     """-> (gE_tok dense or [0], gE_byte dense or [0], g_lam fp32 [2] or [0])."""
-    tok = O._tok_next(tok, next_tok)
-    desc = O._embed_desc(unpack_spec(spec, eps), bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None,
-                         next_tok=next_tok is not None)
+    tok, desc = O._ids_desc(unpack_spec(spec, eps), bpt, seq_len, tok, next_tok, ids, ttb, E_tok, E_byte, lam is not None)
     n, ref = desc.n_tokens, (E_tok if E_tok is not None else E_byte)
     dev = ref.device
     g = grad_out.reshape(n, desc.out_dim)
@@ -244,24 +239,19 @@ tok_gather_op.register_autograd(_tok_gather_backward, setup_context=_tok_gather_
 # mot_b200::embed_proj  (concat + dense projection variants, tcgen05)
 # ---------------------------------------------------------------------------------------------------------------
 @torch.library.custom_op("mot_b200::embed_proj", mutates_args=(), device_types="cuda")
-def embed_proj_op(tok: Tensor, ids: Tensor, ids2: Optional[Tensor], E_tok: Tensor, E_byte: Tensor, W: Tensor,
+def embed_proj_op(tok: Tensor, ids: Optional[Tensor], ids2: Optional[Tensor], E_tok: Tensor, E_byte: Tensor, W: Tensor,
                   bias: Optional[Tensor], spec: int, bpt: int, eps: float, plan: bool, ttb: Optional[Tensor] = None,
                   seq_len: int = 0, ttb_pair: bool = False,
                   next_tok: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
     """-> (out [n, Do], Y = the product before the row norm or [0], W in the compute dtype or [0], workspace or [0]).
-    With `ttb` the byte ids come from the table inside the kernels and `ids` is an unused placeholder; next_tok: the
-    lookahead of a right pull."""
+    ids=None with `ttb`: the byte ids come from the table inside the kernels; next_tok: the lookahead of a right pull."""
     dev, cdt = E_tok.device, E_tok.dtype
     sp = unpack_spec(spec, eps)
-    ids = ids if ttb is None else None
-    pair = ids2 is not None or ttb_pair
-    tok, has_next = O._tok_next(tok, next_tok), next_tok is not None
-    desc = O._proj_desc(sp, bpt, tok, ids, E_tok, E_byte, pair, ttb, seq_len, has_next)
+    tok, desc, desc_pair = O._proj_descs(sp, bpt, seq_len, tok, next_tok, ids, ids2, ttb, ttb_pair, E_tok, E_byte)
     w_c = W if W.dtype == cdt else O.cast_out(W, cdt)
     planned = plan and tok.numel() > 0
     ws = _plan_beside(desc, tok, dev) if planned else _empty(dev)
-    out, Y, _ = O._proj_forward(sp, desc, bpt, tok, ids, ids2, E_tok, E_byte, w_c, bias, False, ttb, seq_len, pair,
-                                has_next)
+    out, Y, _ = O._proj_forward(sp, desc, desc_pair, tok, ids, ids2, ttb, E_tok, E_byte, w_c, bias, False)
     if planned:
         _rejoin(dev)
     return out, (Y if sp.out_norm else _empty(dev, cdt)), (w_c if w_c is not W else _empty(dev, cdt)), ws
@@ -270,8 +260,7 @@ def embed_proj_op(tok: Tensor, ids: Tensor, ids2: Optional[Tensor], E_tok: Tenso
 @embed_proj_op.register_fake
 def _(tok, ids, ids2, E_tok, E_byte, W, bias, spec, bpt, eps, plan, ttb=None, seq_len=0, ttb_pair=False, next_tok=None):
     sp = unpack_spec(spec, eps)
-    desc = O._proj_desc(sp, bpt, tok, ids if ttb is None else None, E_tok, E_byte, ids2 is not None or ttb_pair, ttb, seq_len,
-                        next_tok is not None)
+    tok, desc, _ = O._proj_descs(sp, bpt, seq_len, tok, next_tok, ids, ids2, ttb, ttb_pair, E_tok, E_byte)
     n, cdt = tok.numel(), E_tok.dtype
     out = E_tok.new_empty((n, W.shape[0]))
     Y = E_tok.new_empty((n, W.shape[0]) if sp.out_norm else (0,))
@@ -280,23 +269,19 @@ def _(tok, ids, ids2, E_tok, E_byte, W, bias, spec, bpt, eps, plan, ttb=None, se
 
 
 @torch.library.custom_op("mot_b200::embed_proj_bwd", mutates_args=(), device_types="cuda")
-def embed_proj_bwd_op(grad_out: Tensor, tok: Tensor, ids: Tensor, ids2: Optional[Tensor], E_tok: Tensor, E_byte: Tensor,
-                      W: Tensor, w_c: Tensor, Y: Tensor, ws: Tensor, spec: int, bpt: int, eps: float,
+def embed_proj_bwd_op(grad_out: Tensor, tok: Tensor, ids: Optional[Tensor], ids2: Optional[Tensor], E_tok: Tensor,
+                      E_byte: Tensor, W: Tensor, w_c: Tensor, Y: Tensor, ws: Tensor, spec: int, bpt: int, eps: float,
                       has_bias: bool, ttb: Optional[Tensor] = None, seq_len: int = 0,
                       ttb_pair: bool = False, next_tok: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
     """-> (gE_tok, gE_byte, gW in W's dtype, g_bias fp32 [Do] or [0])."""
     dev = E_tok.device
     sp = unpack_spec(spec, eps)
-    ids = ids if ttb is None else None
-    pair = ids2 is not None or ttb_pair
-    tok, has_next = O._tok_next(tok, next_tok), next_tok is not None
-    desc = O._proj_desc(sp, bpt, tok, ids, E_tok, E_byte, pair, ttb, seq_len, has_next)
-    dA, gW, g_bias = O._proj_backward(sp, desc, bpt, tok, ids, ids2, E_tok, E_byte, w_c if w_c.numel() > 0 else W,
-                                      W.dtype, has_bias, Y, None, grad_out,    # the operand is gathered again, not kept
-                                      ttb, seq_len, pair, has_next)
+    tok, desc, desc_pair = O._proj_descs(sp, bpt, seq_len, tok, next_tok, ids, ids2, ttb, ttb_pair, E_tok, E_byte)
+    dA, gW, g_bias = O._proj_backward(sp, desc, desc_pair, tok, ids, ids2, ttb, E_tok, E_byte,
+                                      w_c if w_c.numel() > 0 else W, W.dtype, has_bias, Y, None,   # operand gathered again
+                                      grad_out)
     ws, planned = _bwd_workspace(ws, desc, dev)
-    gE_tok, gE_byte = O._scatter_operand(sp, desc, bpt, tok, ids, ids2, E_tok, E_byte, dA, ws, planned, planned,
-                                         ttb, seq_len, pair, has_next)
+    gE_tok, gE_byte = O._scatter_operand(desc, desc_pair, tok, ids, ids2, ttb, E_tok, E_byte, dA, ws, planned, planned)
     return gE_tok, gE_byte, gW, (g_bias if has_bias else _empty(dev, torch.float32))
 
 
@@ -331,16 +316,13 @@ embed_proj_op.register_autograd(_proj_backward, setup_context=_proj_setup)
 # mot_b200::embed_byte_fc  (runs/71051: norm(tok + F.linear(cat(bytes), byte_fc)))
 # ---------------------------------------------------------------------------------------------------------------
 @torch.library.custom_op("mot_b200::embed_byte_fc", mutates_args=(), device_types="cuda")
-def embed_byte_fc_op(tok: Tensor, ids: Tensor, E_tok: Tensor, E_byte: Tensor, W: Tensor, spec_b: int, bpt: int, eps: float,
-                     plan: bool, ttb: Optional[Tensor] = None, seq_len: int = 0,
+def embed_byte_fc_op(tok: Tensor, ids: Optional[Tensor], E_tok: Tensor, E_byte: Tensor, W: Tensor, spec_b: int, bpt: int,
+                     eps: float, plan: bool, ttb: Optional[Tensor] = None, seq_len: int = 0,
                      next_tok: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
-    """-> (out [n, D], Y = the byte-FC product, W in the compute dtype or [0], workspace or [0]).  With `ttb` the byte
-    ids come from the table inside the kernels and `ids` is an unused placeholder; next_tok: the lookahead of a right
-    pull."""
+    """-> (out [n, D], Y = the byte-FC product, W in the compute dtype or [0], workspace or [0]).  ids=None with `ttb`:
+    the byte ids come from the table inside the kernels; next_tok: the lookahead of a right pull."""
     dev, cdt = E_tok.device, E_tok.dtype
-    ids = ids if ttb is None else None
-    tok = O._tok_next(tok, next_tok)
-    desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, tok, ids, E_tok, E_byte, ttb, seq_len, next_tok is not None)
+    tok, desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, seq_len, tok, next_tok, ids, ttb, E_tok, E_byte)
     w_c = W if W.dtype == cdt else O.cast_out(W, cdt)
     planned = plan and tok.numel() > 0
     ws = _plan_beside(desc_t, tok, dev) if planned else _empty(dev)
@@ -352,21 +334,19 @@ def embed_byte_fc_op(tok: Tensor, ids: Tensor, E_tok: Tensor, E_byte: Tensor, W:
 
 @embed_byte_fc_op.register_fake
 def _(tok, ids, E_tok, E_byte, W, spec_b, bpt, eps, plan, ttb=None, seq_len=0, next_tok=None):
-    desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, tok, ids if ttb is None else None, E_tok, E_byte, ttb,
-                                 seq_len, next_tok is not None)
+    tok, _, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, seq_len, tok, next_tok, ids, ttb, E_tok, E_byte)
     n, D = tok.numel(), E_tok.shape[1]
     return (E_tok.new_empty((n, D)), E_tok.new_empty((n, D)), E_tok.new_empty(tuple(W.shape) if W.dtype != E_tok.dtype else (0,)),
             E_tok.new_empty((O.embed_workspace_bytes(desc_t) if plan and n > 0 else 0,), dtype=torch.uint8))
 
 
 @torch.library.custom_op("mot_b200::embed_byte_fc_bwd", mutates_args=(), device_types="cuda")
-def embed_byte_fc_bwd_op(grad_out: Tensor, tok: Tensor, ids: Tensor, E_tok: Tensor, E_byte: Tensor, W: Tensor, w_c: Tensor,
-                         Y: Tensor, ws: Tensor, spec_b: int, bpt: int, eps: float, ttb: Optional[Tensor] = None,
-                         seq_len: int = 0, next_tok: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor]:
+def embed_byte_fc_bwd_op(grad_out: Tensor, tok: Tensor, ids: Optional[Tensor], E_tok: Tensor, E_byte: Tensor, W: Tensor,
+                         w_c: Tensor, Y: Tensor, ws: Tensor, spec_b: int, bpt: int, eps: float,
+                         ttb: Optional[Tensor] = None, seq_len: int = 0,
+                         next_tok: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor]:
     dev = E_tok.device
-    ids = ids if ttb is None else None
-    tok = O._tok_next(tok, next_tok)
-    desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, tok, ids, E_tok, E_byte, ttb, seq_len, next_tok is not None)
+    tok, desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, seq_len, tok, next_tok, ids, ttb, E_tok, E_byte)
     ws, planned = _bwd_workspace(ws, desc_t, dev)
     wsb = torch.empty(O.embed_workspace_bytes(desc_b), dtype=torch.uint8, device=dev)
     return O._byte_fc_backward(desc_b, desc_t, tok, ids, E_tok, E_byte, w_c if w_c.numel() > 0 else W, W.dtype, Y,

@@ -8,6 +8,8 @@ from typing import Optional
 
 import torch
 
+from torch._subclasses.fake_tensor import FakeTensor
+
 from . import _lib as L
 
 FP32_EPS = float(torch.finfo(torch.float32).eps)  # F.rms_norm's default eps (train_gpt.py:172-173)
@@ -220,8 +222,6 @@ def make_desc(spec: MixSpec, n_tokens: int, E_tok, E_byte, bpt: int, *, ids: Opt
     ttb_dtype = 0
     if has_bytes:
         if ids is None:
-            if ttb is None:
-                raise RuntimeError("mot_b200: need byte ids or a ttb table")
             flags |= L.F_IDS_FROM_TTB
             flags |= L.F_TTB_SCRAMBLE if spec.ttb_scramble else 0
             flags |= _pull_flags(spec, next_tok)
@@ -448,42 +448,71 @@ def _tok_i32(tokens: torch.Tensor) -> torch.Tensor:
     return (tok if tok.dtype == torch.int32 else tok.to(torch.int32)).contiguous()
 
 
-def _byte_ids(byte_ids: torch.Tensor) -> torch.Tensor:
-    if byte_ids.dtype not in (torch.int32, torch.int64):
-        raise NotImplementedError("mot_b200: byte ids must be int32 or int64")
-    return byte_ids.contiguous()
+def _id_args(spec: MixSpec, bpt: int, tokens, byte_ids, ttb, seq_len: int, next_tokens, byte_ids2=None,
+             ttb_pair: bool = False):
+    """Where the byte ids of a front come from, checked once for every front -> (tok, ids, ids2, ttb, next_tok).
 
-
-def _check_id_count(ids: torch.Tensor, n: int, bpt: int) -> None:
-    if ids.numel() != n * bpt:
-        raise RuntimeError(f"mot_b200: byte ids have {ids.numel()} entries, expected {n}*{bpt}")
-
-
-def _with_next(spec: MixSpec, tok: torch.Tensor, next_tokens: Optional[torch.Tensor], seq_len: int):
-    """The lookahead of a right pull -> (tok, next): both views of ONE int32 buffer [tok | next], so that the kernels
-    find token seq_len of row r at tok[n + r] (MOT_F_TTB_NEXT_TOK) while the plan and the gathers see n tokens."""
-    if next_tokens is None:
-        return tok, None
-    if not (spec.ttb_pull and spec.ttb_pull_side == "right"):
+    Explicit `byte_ids` (with `byte_ids2`: the second id tensor of `--add-padded-and-pulled`), or byte_ids=None with the
+    [V, bpt] table `ttb`: the kernels derive the padded ids, the pulled ones under spec.ttb_pull, both sets with ttb_pair.
+    next_tokens (a right pull's lookahead) comes back with tok as views of ONE int32 buffer [tok | next], so that the
+    kernels find token seq_len of row r at tok[n + r] (MOT_F_TTB_NEXT_TOK) while the plan and the gathers see n tokens."""
+    tok = _tok_i32(tokens) if tokens is not None else None
+    if byte_ids is None and ttb is None and spec.combine != "tok_only":
+        raise RuntimeError("mot_b200: need byte ids or a ttb table")
+    pull = spec.ttb_pull or ttb_pair
+    if next_tokens is not None and (tok is None or byte_ids is not None or ttb is None or not pull
+                                    or spec.ttb_pull_side != "right"):
         raise RuntimeError("mot_b200: next_tokens= is the lookahead of a right pull (ttb ids with ttb_pull_side='right')")
+    pair = ttb_pair if byte_ids is None else byte_ids2 is not None
+    if pair and (not spec.byte_norm or spec.slot_major or spec.bytes_first or (ttb_pair and spec.ttb_scramble)):
+        raise NotImplementedError("mot_b200: the padded+pulled sum exists only with per-byte norms, token-major "
+                                  "ids and [tok | bytes] order (spt/train_gpt.py:371-379,442-443)")
+    if byte_ids is not None:
+        if byte_ids.dtype not in (torch.int32, torch.int64):
+            raise NotImplementedError("mot_b200: byte ids must be int32 or int64")
+        ids = byte_ids.contiguous()
+        n = tok.numel() if tok is not None else ids.numel() // bpt
+        if ids.numel() != n * bpt:
+            raise RuntimeError(f"mot_b200: byte ids have {ids.numel()} entries, expected {n}*{bpt}")
+        ids2 = byte_ids2.contiguous() if pair else None
+        if pair and (ids2.dtype != ids.dtype or ids2.numel() != ids.numel()):
+            raise RuntimeError("mot_b200: the two byte-id tensors must share dtype and size")
+        return tok, ids, ids2, None, None
+    if ttb is None:
+        return tok, None, None, None, None
+    if ttb.dtype not in _TTB_DTYPE or ttb.dim() != 2:
+        raise NotImplementedError(f"mot_b200: ttb must be a 2-D int16/float32/bfloat16 table, got {ttb.dtype}")
+    if pull and (seq_len <= 0 or tok.numel() % seq_len):
+        raise RuntimeError(f"mot_b200: pulled ids need rows of seq_len tokens (seq_len={seq_len}, {tok.numel()} tokens)")
+    if next_tokens is None:
+        return tok, None, None, ttb.contiguous(), None
     if next_tokens.dtype not in (torch.int32, torch.int64):
         raise NotImplementedError("mot_b200: next_tokens must be int32 or int64")
-    rows = tok.numel() // seq_len
+    n, rows = tok.numel(), tok.numel() // seq_len
     if next_tokens.numel() != rows:
         raise RuntimeError(f"mot_b200: next_tokens has {next_tokens.numel()} entries, expected one per row ({rows})")
-    n = tok.numel()
     buf = torch.cat((tok, next_tokens.reshape(-1).to(torch.int32)))
-    return buf[:n], buf[n:]
+    return buf[:n], None, None, ttb.contiguous(), buf[n:]
 
 
 def _tok_next(tok: torch.Tensor, next_tok: Optional[torch.Tensor]) -> torch.Tensor:
-    """Token ids whose lookahead follows them in memory (the operators receive tok and next_tok as two tensors; the
-    argument helper made them views of one buffer, which a traced graph may not keep)."""
-    if next_tok is None or next_tok.numel() == 0:
+    """Token ids whose lookahead follows them in memory (the operators receive tok and next_tok as two tensors; _id_args
+    made them views of one buffer, which a traced graph may not keep).  A fake tensor only carries its shape."""
+    if next_tok is None or next_tok.numel() == 0 or isinstance(tok, FakeTensor):
         return tok
     if next_tok.data_ptr() == tok.data_ptr() + 4 * tok.numel():
         return tok
     return torch.cat((tok, next_tok))[:tok.numel()]
+
+
+def _ids_desc(spec: MixSpec, bpt: int, seq_len: int, tok, next_tok, ids, ttb, E_tok, E_byte, has_lam: bool = False,
+              row_stride: int = 0, col_offset: int = 0):
+    """-> (tok, desc): the descriptor of the gather that reads the byte ids (explicit `ids`, else derived from `ttb` over
+    rows of seq_len tokens, with the lookahead next_tok behind tok); tok with next_tok behind it in memory."""
+    tok = _tok_next(tok, next_tok)
+    n = tok.numel() if tok is not None else ids.numel() // bpt
+    return tok, make_desc(spec, n, E_tok, E_byte, bpt, ids=ids, ttb=ttb, has_lam=has_lam, seq_len=seq_len,
+                          row_stride=row_stride, col_offset=col_offset, next_tok=next_tok is not None)
 
 
 def _require_chain_dtype(E_tok: torch.Tensor, E_byte: torch.Tensor) -> None:
@@ -492,44 +521,23 @@ def _require_chain_dtype(E_tok: torch.Tensor, E_byte: torch.Tensor) -> None:
         raise NotImplementedError("mot_b200: token and byte tables must both be bf16 or both fp32")
 
 
-def _embed_args(bpt: int, tokens, byte_ids, ttb, E_tok, E_byte, lam, spec: Optional[MixSpec] = None, seq_len: int = 0,
-                next_tokens=None):
-    """mot_embed's arguments checked and normalised -> (dev, tok, ids, E_tok, E_byte, next_tok)."""
+def _embed_args(spec: MixSpec, bpt: int, tokens, byte_ids, ttb, E_tok, E_byte, lam, seq_len: int, next_tokens):
+    """mot_embed's arguments checked and normalised -> (dev, tok, ids, ttb, E_tok, E_byte, next_tok)."""
     dev = _require_cuda(tokens, byte_ids, ttb, E_tok, E_byte, lam, next_tokens)
-    tok = _tok_i32(tokens) if tokens is not None else None
-    ids = None
-    if byte_ids is not None:
-        ids = _byte_ids(byte_ids)
-        _check_id_count(ids, tok.numel() if tok is not None else ids.numel() // bpt, bpt)
+    tok, ids, _, ttb, nxt = _id_args(spec, bpt, tokens, byte_ids, ttb, seq_len, next_tokens)
     E_tok = E_tok.contiguous() if E_tok is not None else None
     E_byte = E_byte.contiguous() if E_byte is not None else None
     if E_tok is not None and E_byte is not None and E_tok.dtype != E_byte.dtype:
         raise NotImplementedError("mot_b200: token and byte tables must share one dtype")
-    nxt = None
-    if next_tokens is not None:
-        if tok is None or ids is not None or ttb is None:
-            raise RuntimeError("mot_b200: next_tokens= is the lookahead of a right pull (ttb ids with ttb_pull_side='right')")
-        _ttb_ids_args(spec, tok, ttb, seq_len)
-        tok, nxt = _with_next(spec, tok, next_tokens, seq_len)
-    return dev, tok, ids, E_tok, E_byte, nxt
-
-
-def _embed_desc(spec: MixSpec, bpt: int, seq_len: int, tok, ids, ttb, E_tok, E_byte, has_lam: bool,
-                dp_slabs: int = 0, next_tok: bool = False) -> L.MotDesc:
-    n = tok.numel() if tok is not None else ids.numel() // bpt
-    return make_desc(spec, n, E_tok, E_byte, bpt, ids=ids, ttb=ttb, has_lam=has_lam, seq_len=seq_len, dp_slabs=dp_slabs,
-                     next_tok=next_tok)
+    return dev, tok, ids, ttb, E_tok, E_byte, nxt
 
 
 class _MotEmbedFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, spec: MixSpec, bpt: int, seq_len: int, dev, tok, ids, ttb, E_tok, E_byte, lam, grad_bufs=None,
-                next_tok=None):
+    def forward(ctx, desc: L.MotDesc, dev, tok, ids, ttb, E_tok, E_byte, lam, grad_bufs=None):
         # optional ((param_tok, view_tok), (param_byte, view_byte)): views of a dp.GradBucket that become param.grad
         ctx.grad_bufs = grad_bufs
         lam_c = lam.detach().to(torch.float32).contiguous() if lam is not None else None
-        has_next = next_tok is not None   # tok is the head of [tok | next_tok] (_with_next)
-        desc = _embed_desc(spec, bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None, next_tok=has_next)
         n = desc.n_tokens
         # data-parallel pipeline: a bucket that holds exactly [token table | byte table] in symmetric memory lets the
         # backward run as vocabulary slabs with the exchange of slab k beside the backward of slab k + 1
@@ -538,14 +546,14 @@ class _MotEmbedFn(torch.autograd.Function):
         if bucket is not None and bucket.pipelined and n > 0 and E_tok is not None and E_byte is not None \
                 and len(bucket.params) == 2 and bucket.params[0] is grad_bufs[0][0] and bucket.params[1] is grad_bufs[1][0] \
                 and bool(L.lib().mot_embed_bwd_uses_saved(desc)):
-            desc = _embed_desc(spec, bpt, seq_len, tok, ids, ttb, E_tok, E_byte, lam is not None, dp_slabs=bucket.n_slabs,
-                               next_tok=has_next)
+            desc = L.MotDesc.from_buffer_copy(desc)
+            desc.dp_slabs = bucket.n_slabs
             ctx.dp_bucket = bucket
         ref = E_tok if E_tok is not None else E_byte
         out = torch.empty((n, desc.out_dim), dtype=ref.dtype, device=dev)
         # the backward needs the positions grouped by token id: start that sort now, beside the forward kernel
         st = _stream(dev)
-        needs_grad = any(ctx.needs_input_grad[7:10])   # E_tok, E_byte, lam
+        needs_grad = any(ctx.needs_input_grad[5:8])   # E_tok, E_byte, lam
         ctx.ws = _planned_workspace(desc, tok, dev, st) if needs_grad and tok is not None and n > 0 else None
         # MoT-sum (runs/71): keep what rms_norm's autograd node keeps (its result and rstd); the backward then reads two
         # rows per occurrence instead of rebuilding the mixed row (mot_embed_bwd_ex)
@@ -614,7 +622,7 @@ class _MotEmbedFn(torch.autograd.Function):
             direct[0][0].grad, gE_tok = gE_tok, None
         if direct[1] is not None:
             direct[1][0].grad, gE_byte = gE_byte, None
-        return None, None, None, None, None, None, None, gE_tok, gE_byte, g_lam, None, None
+        return None, None, None, None, None, gE_tok, gE_byte, g_lam, None
 
 
 def mot_embed(tokens: Optional[torch.Tensor], byte_ids: Optional[torch.Tensor], E_tok: Optional[torch.Tensor],
@@ -630,14 +638,15 @@ def mot_embed(tokens: Optional[torch.Tensor], byte_ids: Optional[torch.Tensor], 
     (a slice of a dp.GradBucket) and installs it as `param.grad`.  next_tokens: with spec.ttb_pull and
     ttb_pull_side="right", token seq_len of every row ([n_tokens / seq_len], the last column of the loader's window of
     seq_len + 1 tokens), which the right pull of the row's last tokens reads; without it the row ends at its last input."""
-    dev, tok, ids, E_tok_c, E_byte_c, nxt = _embed_args(bpt, tokens, byte_ids, ttb, E_tok, E_byte, lam, spec, seq_len,
-                                                        next_tokens)
+    dev, tok, ids, ttb_c, E_tok_c, E_byte_c, nxt = _embed_args(spec, bpt, tokens, byte_ids, ttb, E_tok, E_byte, lam,
+                                                               seq_len, next_tokens)
     if grad_bufs is None and _custom_ops_wanted():
         lam32 = lam.to(torch.float32).contiguous() if lam is not None else None   # differentiable cast
         need = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (E_tok, E_byte, lam))
-        return torch.ops.mot_b200.embed(tok, ids, ttb.contiguous() if ttb is not None else None, E_tok_c, E_byte_c, lam32,
-                                        pack_spec(spec), bpt, seq_len, float(spec.eps), need, nxt)[0]
-    return _MotEmbedFn.apply(spec, bpt, seq_len, dev, tok, ids, ttb, E_tok_c, E_byte_c, lam, grad_bufs, nxt)
+        return torch.ops.mot_b200.embed(tok, ids, ttb_c, E_tok_c, E_byte_c, lam32, pack_spec(spec), bpt, seq_len,
+                                        float(spec.eps), need, nxt)[0]
+    tok, desc = _ids_desc(spec, bpt, seq_len, tok, nxt, ids, ttb_c, E_tok_c, E_byte_c, has_lam=lam is not None)
+    return _MotEmbedFn.apply(desc, dev, tok, ids, ttb_c, E_tok_c, E_byte_c, lam, grad_bufs)
 
 
 # ------------------------------------------------------------------------------------------------------------
@@ -820,33 +829,33 @@ def byte_pair_backward_out(ids_a, ids_b, bpt: int, E_byte, grad_rows, col_offset
     L.check(rc, "mot_byte_pair_bwd")
 
 
-def _ttb_pair_args(tok, ttb, seq_len: int):
-    return (_ptr(tok), _ptr(ttb), ttb.shape[0], _TTB_DTYPE[ttb.dtype], seq_len, PAD_ID, EOT_ID, tok.numel())
+_PAIR_PULL = L.F_TTB_PULL_LEFT | L.F_TTB_PULL_RIGHT | L.F_TTB_NEXT_TOK
 
 
-def byte_pair_ttb_forward_out(tok, ttb, seq_len: int, bpt: int, E_byte, out, col_offset: int, eps: float = FP32_EPS,
-                              pull_flags: int = L.F_TTB_PULL_LEFT) -> None:
-    """mot_byte_pair_ttb_ex_fwd: byte_pair_forward_out with ids_a = the padded and ids_b = the pulled ids of `tok`, both
-    derived from the ttb table inside the kernel (rows of seq_len tokens).  pull_flags: the direction (_pull_flags)."""
+def byte_pair_ttb_forward_out(desc: L.MotDesc, tok, ttb, E_byte, out) -> None:
+    """mot_byte_pair_ttb_fwd: byte_pair_forward_out with ids_a = the padded and ids_b = the pulled ids of `tok`, both
+    derived from the ttb table inside the kernel.  desc: the bytes-only descriptor of the pair (_proj_descs), which holds
+    the rows of seq_len tokens, the pull flags and the byte columns of `out` (row_stride, col_offset)."""
     dev = _require_cuda(tok, ttb, E_byte, out)
     with _on_device(dev):
-        rc = L.lib().mot_byte_pair_ttb_ex_fwd(*_ttb_pair_args(tok, ttb, seq_len), bpt, _ptr(E_byte), E_byte.shape[0],
-                                              E_byte.shape[1], _DTYPE[E_byte.dtype], eps, _ptr(out), out.stride(0),
-                                              col_offset, pull_flags, _stream(dev))
+        rc = L.lib().mot_byte_pair_ttb_fwd(_ptr(tok), _ptr(ttb), desc.tok_vocab, desc.ttb_dtype, desc.seq_len, desc.pad_id,
+                                           desc.eot_id, desc.n_tokens, desc.bpt, _ptr(E_byte), desc.byte_vocab,
+                                           desc.byte_dim, desc.dtype, desc.eps, _ptr(out), desc.row_stride,
+                                           desc.col_offset, desc.flags & _PAIR_PULL, _stream(dev))
     L.check(rc, "mot_byte_pair_ttb_fwd")
 
 
-def byte_pair_ttb_backward_out(tok, ttb, seq_len: int, bpt: int, E_byte, grad_rows, col_offset: int, gE_byte,
-                               eps: float = FP32_EPS, pull_flags: int = L.F_TTB_PULL_LEFT) -> None:
-    """mot_byte_pair_ttb_ex_bwd: byte_pair_backward_out with both id sets derived from `tok` and the ttb table."""
+def byte_pair_ttb_backward_out(desc: L.MotDesc, tok, ttb, E_byte, grad_rows, gE_byte) -> None:
+    """mot_byte_pair_ttb_bwd: byte_pair_backward_out with both id sets derived from `tok` and the ttb table."""
     dev = _require_cuda(tok, ttb, E_byte, grad_rows, gE_byte)
-    need = int(L.lib().mot_byte_pair_workspace_bytes(E_byte.shape[0], E_byte.shape[1]))
+    need = int(L.lib().mot_byte_pair_workspace_bytes(desc.byte_vocab, desc.byte_dim))
     ws = torch.empty(need, dtype=torch.uint8, device=dev)
     with _on_device(dev):
-        rc = L.lib().mot_byte_pair_ttb_ex_bwd(*_ttb_pair_args(tok, ttb, seq_len), bpt, _ptr(E_byte), E_byte.shape[0],
-                                              E_byte.shape[1], _DTYPE[E_byte.dtype], eps, _ptr(grad_rows),
-                                              grad_rows.stride(0), col_offset, _ptr(gE_byte), _ptr(ws), ws.numel(),
-                                              pull_flags, _stream(dev))
+        rc = L.lib().mot_byte_pair_ttb_bwd(_ptr(tok), _ptr(ttb), desc.tok_vocab, desc.ttb_dtype, desc.seq_len, desc.pad_id,
+                                           desc.eot_id, desc.n_tokens, desc.bpt, _ptr(E_byte), desc.byte_vocab,
+                                           desc.byte_dim, desc.dtype, desc.eps, _ptr(grad_rows), desc.row_stride,
+                                           desc.col_offset, _ptr(gE_byte), _ptr(ws), ws.numel(), desc.flags & _PAIR_PULL,
+                                           _stream(dev))
     L.check(rc, "mot_byte_pair_ttb_bwd")
 
 
@@ -929,50 +938,12 @@ def mixout_split(x: torch.Tensor, bytes_per_token: int) -> torch.Tensor:
 _PROJ_KEEP_OPERAND = not __import__("os").environ.get("MOT_PROJ_REGATHER")
 
 
-def _ttb_ids_args(spec: MixSpec, tok, ttb, seq_len: int) -> torch.Tensor:
-    """Checks of the token-only call form (byte ids derived from `ttb` inside the kernels) -> the table, contiguous."""
-    if ttb.dtype not in _TTB_DTYPE or ttb.dim() != 2:
-        raise NotImplementedError(f"mot_b200: ttb must be a 2-D int16/float32/bfloat16 table, got {ttb.dtype}")
-    if spec.ttb_pull and (seq_len <= 0 or tok.numel() % seq_len):
-        raise RuntimeError(f"mot_b200: pulled ids need rows of seq_len tokens (seq_len={seq_len}, {tok.numel()} tokens)")
-    return ttb.contiguous()
-
-
-def _proj_args(spec: MixSpec, bpt: int, tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2, ttb=None, seq_len: int = 0,
-               ttb_pair: bool = False, next_tokens=None):
-    """mot_embed_proj's arguments checked and normalised -> (dev, tok, ids, ids2, E_tok, E_byte, ttb, next_tok).  Without
-    byte ids the ids come from `ttb` (the pulled ones under spec.ttb_pull; with ttb_pair the padded and the pulled ones);
-    next_tokens: the lookahead of a right pull (_with_next)."""
+def _proj_args(spec: MixSpec, bpt: int, tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2, ttb, seq_len: int,
+               ttb_pair: bool, next_tokens):
+    """mot_embed_proj's arguments checked and normalised -> (dev, tok, ids, ids2, E_tok, E_byte, ttb, next_tok)."""
     dev = _require_cuda(tokens, byte_ids, E_tok, E_byte, W, bias, byte_ids2, ttb, next_tokens)
     _require_chain_dtype(E_tok, E_byte)
-    tok = _tok_i32(tokens)
-    ids = ids2 = nxt = None
-    if byte_ids is None:
-        if ttb is None:
-            raise RuntimeError("mot_b200: need byte ids or a ttb table")
-        if ttb_pair:
-            if not spec.byte_norm or spec.slot_major or spec.bytes_first or spec.ttb_scramble:
-                raise NotImplementedError("mot_b200: the padded+pulled sum exists only with per-byte norms, token-major "
-                                          "ids and [tok | bytes] order (spt/train_gpt.py:371-379,442-443)")
-            spec = dataclasses.replace(spec, ttb_pull=True)
-        ttb = _ttb_ids_args(spec, tok, ttb, seq_len)
-        tok, nxt = _with_next(spec, tok, next_tokens, seq_len)
-    else:
-        if next_tokens is not None:
-            raise RuntimeError("mot_b200: next_tokens= is the lookahead of a right pull (ttb ids with ttb_pull_side='right')")
-        ttb = None
-        ids = _byte_ids(byte_ids)
-        _check_id_count(ids, tok.numel(), bpt)
-    if byte_ids2 is not None and ids is not None:
-        # `--add-padded-and-pulled` (spt/train_gpt.py:371-379): two gathers summed before the per-byte norm.  The
-        # token columns of the operand come from the fused kernel (tok-only, strided rows), the byte columns from
-        # the pair kernels.
-        if not spec.byte_norm or spec.slot_major or spec.bytes_first:
-            raise NotImplementedError("mot_b200: the padded+pulled sum exists only with per-byte norms, token-major "
-                                      "ids and [tok | bytes] order (spt/train_gpt.py:371-379,442-443)")
-        ids2 = byte_ids2.contiguous()
-        if ids2.dtype != ids.dtype or ids2.numel() != ids.numel():
-            raise RuntimeError("mot_b200: the two byte-id tensors must share dtype and size")
+    tok, ids, ids2, ttb, nxt = _id_args(spec, bpt, tokens, byte_ids, ttb, seq_len, next_tokens, byte_ids2, ttb_pair)
     K = E_tok.shape[1] + bpt * E_byte.shape[1]
     if W.shape[1] != K:
         raise RuntimeError(f"mot_b200: projection weight is {tuple(W.shape)}, expected [{W.shape[0]}, {K}]")
@@ -981,63 +952,59 @@ def _proj_args(spec: MixSpec, bpt: int, tokens, byte_ids, E_tok, E_byte, W, bias
     return dev, tok, ids, ids2, E_tok.contiguous(), E_byte.contiguous(), ttb, nxt
 
 
-def _proj_desc(spec: MixSpec, bpt: int, tok, ids, E_tok, E_byte, pair: bool, ttb=None, seq_len: int = 0,
-               next_tok: bool = False) -> L.MotDesc:
-    """Descriptor of the gather of the [n, K] operand: the concat of both tables, or with `pair` (two byte-id tensors)
-    only its token columns, written with row stride K (the pair kernels write the byte columns).  ids=None: the ids come
-    from `ttb` (rows of seq_len tokens)."""
-    if pair:
-        return make_desc(MixSpec(combine="tok_only", tok_norm=spec.tok_norm, out_norm=False, eps=spec.eps), tok.numel(),
-                         E_tok, None, 0, ids=None, ttb=None, has_lam=False,
-                         row_stride=E_tok.shape[1] + bpt * E_byte.shape[1], col_offset=0)
-    return make_desc(dataclasses.replace(spec, combine="concat", out_norm=False), tok.numel(), E_tok, E_byte, bpt,
-                     ids=ids, ttb=ttb, has_lam=False, seq_len=seq_len, next_tok=next_tok)
+def _proj_descs(spec: MixSpec, bpt: int, seq_len: int, tok, next_tok, ids, ids2, ttb, ttb_pair: bool, E_tok, E_byte):
+    """-> (tok, desc, desc_pair): desc gathers the [n, K] operand, the concat of both tables.  With a pair (`ids2`, or
+    ttb_pair: the padded and the pulled ids from `ttb`) desc gathers only the operand's token columns, with row stride K,
+    and desc_pair (bytes-only, per-byte norm) describes the byte columns that the pair kernels write.  Without a pair
+    desc_pair is None."""
+    if ids2 is None and not ttb_pair:
+        tok, desc = _ids_desc(dataclasses.replace(spec, combine="concat", out_norm=False), bpt, seq_len, tok, next_tok,
+                              ids, ttb, E_tok, E_byte)
+        return tok, desc, None
+    K = E_tok.shape[1] + bpt * E_byte.shape[1]
+    tok, desc_pair = _ids_desc(MixSpec(combine="bytes_only", byte_norm=True, out_norm=False, ttb_pull=True,
+                                       ttb_pull_side=spec.ttb_pull_side, eps=spec.eps),
+                               bpt, seq_len, tok, next_tok, ids, ttb, None, E_byte, row_stride=K, col_offset=E_tok.shape[1])
+    desc = make_desc(MixSpec(combine="tok_only", tok_norm=spec.tok_norm, out_norm=False, eps=spec.eps), tok.numel(),
+                     E_tok, None, 0, ids=None, ttb=None, has_lam=False, row_stride=K, col_offset=0)
+    return tok, desc, desc_pair
 
 
-def _pair_pull_flags(spec: MixSpec, next_tok: bool) -> int:
-    """Direction of the pulled half of the token-only padded+pulled pair."""
-    return _pull_flags(dataclasses.replace(spec, ttb_pull=True), next_tok)
-
-
-def _gather_operand(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_tok, E_byte, A, ttb=None,
-                    seq_len: int = 0, pair: bool = False, next_tok: bool = False) -> None:
-    if not pair:
+def _gather_operand(desc: L.MotDesc, desc_pair: Optional[L.MotDesc], tok, ids, ids2, ttb, E_tok, E_byte, A) -> None:
+    if desc_pair is None:
         embed_forward_out(desc, tok, ids, ttb, E_tok, E_byte, None, A)
     elif tok.numel() > 0:
         embed_forward_out(desc, tok, None, None, E_tok, None, None, A)
         if ttb is not None:
-            byte_pair_ttb_forward_out(tok, ttb, seq_len, bpt, E_byte, A, E_tok.shape[1], spec.eps,
-                                      _pair_pull_flags(spec, next_tok))
+            byte_pair_ttb_forward_out(desc_pair, tok, ttb, E_byte, A)
         else:
-            byte_pair_forward_out(ids, ids2, bpt, E_byte, A, E_tok.shape[1], spec.eps)
+            byte_pair_forward_out(ids, ids2, desc_pair.bpt, E_byte, A, desc_pair.col_offset, desc_pair.eps)
 
 
-def _scatter_operand(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_tok, E_byte, dA, ws_buf,
-                     plan_ready: bool, ws_clean: bool, ttb=None, seq_len: int = 0, pair: bool = False,
-                     next_tok: bool = False):
+def _scatter_operand(desc: L.MotDesc, desc_pair: Optional[L.MotDesc], tok, ids, ids2, ttb, E_tok, E_byte, dA, ws_buf,
+                     plan_ready: bool, ws_clean: bool):
     """The backward of _gather_operand: dense (gE_tok, gE_byte) from the operand's gradient dA."""
     gE_tok, gE_byte = torch.empty_like(E_tok), torch.empty_like(E_byte)
-    if not pair:
+    if desc_pair is None:
         embed_backward_out(desc, tok, ids, ttb, E_tok, E_byte, None, dA, gE_tok, gE_byte, None, ws_buf,
                            plan_ready=plan_ready, ws_clean=ws_clean)
     else:   # token columns through the sorted-stream scatter, byte columns through the pair kernel
         embed_backward_out(desc, tok, None, None, E_tok, None, None, dA, gE_tok, None, None, ws_buf,
                            plan_ready=plan_ready, ws_clean=ws_clean)
         if ttb is not None:
-            byte_pair_ttb_backward_out(tok, ttb, seq_len, bpt, E_byte, dA, E_tok.shape[1], gE_byte, spec.eps,
-                                       _pair_pull_flags(spec, next_tok))
+            byte_pair_ttb_backward_out(desc_pair, tok, ttb, E_byte, dA, gE_byte)
         else:
-            byte_pair_backward_out(ids, ids2, bpt, E_byte, dA, E_tok.shape[1], gE_byte, spec.eps)
+            byte_pair_backward_out(ids, ids2, desc_pair.bpt, E_byte, dA, desc_pair.col_offset, gE_byte, desc_pair.eps)
     return gE_tok, gE_byte
 
 
-def _proj_forward(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_tok, E_byte, w_c, bias,
-                  keep_operand: bool, ttb=None, seq_len: int = 0, pair: bool = False, next_tok: bool = False):
+def _proj_forward(spec: MixSpec, desc: L.MotDesc, desc_pair: Optional[L.MotDesc], tok, ids, ids2, ttb, E_tok, E_byte, w_c,
+                  bias, keep_operand: bool):
     """-> (out, Y, A): Y = A . w_c^T (+ bias) with the gathered [n, K] operand A (None unless keep_operand), out = the
     row norm of Y under spec.out_norm, else Y itself.  w_c: the weight in the table dtype."""
     n, (Do, K), dev, cdt = tok.numel(), w_c.shape, E_tok.device, E_tok.dtype
     A = torch.empty((n, K), dtype=cdt, device=dev)
-    _gather_operand(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, A, ttb, seq_len, pair, next_tok)
+    _gather_operand(desc, desc_pair, tok, ids, ids2, ttb, E_tok, E_byte, A)
     Y = torch.empty((n, Do), dtype=cdt, device=dev)
     linear_forward_out(A, w_c, Y, bias.contiguous() if bias is not None else None)
     if not keep_operand:
@@ -1050,8 +1017,8 @@ def _proj_forward(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_to
     return out, Y, A
 
 
-def _proj_backward(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_tok, E_byte, w_c, w_dtype, has_bias: bool,
-                   Y, A, grad_out, ttb=None, seq_len: int = 0, pair: bool = False, next_tok: bool = False):
+def _proj_backward(spec: MixSpec, desc: L.MotDesc, desc_pair: Optional[L.MotDesc], tok, ids, ids2, ttb, E_tok, E_byte, w_c,
+                   w_dtype, has_bias: bool, Y, A, grad_out):
     """The backward of _proj_forward down to the operand -> (dA, gW in w_dtype, g_bias fp32 or None).  A: the forward's
     operand if it was kept, else None (gathered again here)."""
     n, (Do, K), dev, cdt = tok.numel(), w_c.shape, E_tok.device, E_tok.dtype
@@ -1066,7 +1033,7 @@ def _proj_backward(spec: MixSpec, desc: L.MotDesc, bpt: int, tok, ids, ids2, E_t
         dA = torch.empty((n, K), dtype=cdt, device=dev)                   # a saved tensor is never overwritten
     else:
         A = torch.empty((n, K), dtype=cdt, device=dev)
-        _gather_operand(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, A, ttb, seq_len, pair, next_tok)
+        _gather_operand(desc, desc_pair, tok, ids, ids2, ttb, E_tok, E_byte, A)
         dA = A                                                            # dX may overwrite the private copy
     dW32 = torch.empty((Do, K), dtype=torch.float32, device=dev)
     dW16 = torch.empty((Do, K), dtype=torch.bfloat16, device=dev) if w_dtype == torch.bfloat16 else None
@@ -1083,20 +1050,15 @@ class _MotEmbedProjFn(torch.autograd.Function):
     step); MOT_PROJ_REGATHER=1 gathers it again instead (the round-1 behaviour, for memory-tight callers)."""
 
     @staticmethod
-    def forward(ctx, spec: MixSpec, bpt: int, dev, tok, ids, ids2, E_tok, E_byte, W, bias, ttb=None, seq_len: int = 0,
-                pair: bool = False, next_tok=None):
-        pair = pair or ids2 is not None
-        has_next = next_tok is not None   # tok is the head of [tok | next_tok] (_with_next)
-        desc = _proj_desc(spec, bpt, tok, ids, E_tok, E_byte, pair, ttb, seq_len, has_next)
+    def forward(ctx, spec: MixSpec, desc: L.MotDesc, desc_pair: Optional[L.MotDesc], dev, tok, ids, ids2, E_tok, E_byte, W,
+                bias, ttb=None):
         w16 = cast_out(W, E_tok.dtype)                         # CastedLinear: W.type_as(x) (spt/train_gpt.py:186)
-        ctx.ws = _planned_workspace(desc, tok, dev) if any(ctx.needs_input_grad[6:8]) and tok.numel() > 0 else None
-        keep_A = _PROJ_KEEP_OPERAND and any(ctx.needs_input_grad[6:10])
-        out, Y, A = _proj_forward(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, w16, bias, keep_A, ttb, seq_len, pair,
-                                  has_next)
+        ctx.ws = _planned_workspace(desc, tok, dev) if any(ctx.needs_input_grad[7:9]) and tok.numel() > 0 else None
+        keep_A = _PROJ_KEEP_OPERAND and any(ctx.needs_input_grad[7:11])
+        out, Y, A = _proj_forward(spec, desc, desc_pair, tok, ids, ids2, ttb, E_tok, E_byte, w16, bias, keep_A)
         embed_plan_join_if_capturing(ctx.ws, dev)
-        ctx.desc, ctx.dev, ctx.spec, ctx.bpt, ctx.seq_len, ctx.has_next = desc, dev, spec, bpt, seq_len, has_next
+        ctx.desc, ctx.desc_pair, ctx.dev, ctx.spec = desc, desc_pair, dev, spec
         ctx.w_dtype, ctx.has_bias = W.dtype, bias is not None
-        ctx.pair, ctx.kept_A = pair, keep_A
         ctx.present = (ids is not None, ids2 is not None, keep_A, ttb is not None)
         ctx.save_for_backward(tok, *[t if t is not None else _ABSENT for t in (ids, ids2, A if keep_A else None, ttb)],
                               E_tok, E_byte, w16, Y)
@@ -1106,48 +1068,33 @@ class _MotEmbedProjFn(torch.autograd.Function):
     def backward(ctx, grad_out):
         tok, ids, ids2, A, ttb, E_tok, E_byte, w16, Y = ctx.saved_tensors
         ids, ids2, A, ttb = [t if ok else None for t, ok in zip((ids, ids2, A, ttb), ctx.present)]
-        desc, dev, spec, bpt, seq_len, pair = ctx.desc, ctx.dev, ctx.spec, ctx.bpt, ctx.seq_len, ctx.pair
-        dA, gW, g_bias = _proj_backward(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, w16, ctx.w_dtype, ctx.has_bias,
-                                        Y, A, grad_out, ttb, seq_len, pair, ctx.has_next)
+        desc, desc_pair, dev = ctx.desc, ctx.desc_pair, ctx.dev
+        dA, gW, g_bias = _proj_backward(ctx.spec, desc, desc_pair, tok, ids, ids2, ttb, E_tok, E_byte, w16, ctx.w_dtype,
+                                        ctx.has_bias, Y, A, grad_out)
         ws, planned, clean = _take_workspace(ctx.ws, desc, dev)
-        gE_tok, gE_byte = _scatter_operand(spec, desc, bpt, tok, ids, ids2, E_tok, E_byte, dA, ws.buf, planned, clean,
-                                           ttb, seq_len, pair, ctx.has_next)
+        gE_tok, gE_byte = _scatter_operand(desc, desc_pair, tok, ids, ids2, ttb, E_tok, E_byte, dA, ws.buf, planned, clean)
         ctx.ws = None
         _return_workspace(ws)
-        return None, None, None, None, None, None, gE_tok, gE_byte, gW, g_bias, None, None, None, None
+        return None, None, None, None, None, None, None, gE_tok, gE_byte, gW, g_bias, None
 
 
-def _byte_fc_args(bpt: int, tokens, byte_ids, E_tok, E_byte, W, spec_b: Optional[MixSpec] = None, ttb=None,
-                  seq_len: int = 0, next_tokens=None):
+def _byte_fc_args(spec_b: MixSpec, bpt: int, tokens, byte_ids, E_tok, E_byte, W, ttb, seq_len: int, next_tokens):
     """mot_embed_byte_fc's arguments checked and normalised -> (dev, tok, ids, E_tok, E_byte, ttb, next_tok)."""
     dev = _require_cuda(tokens, byte_ids, E_tok, E_byte, W, ttb, next_tokens)
     _require_chain_dtype(E_tok, E_byte)
-    tok = _tok_i32(tokens)
     D = E_tok.shape[1]
-    nxt = None
-    if byte_ids is None:
-        if ttb is None:
-            raise RuntimeError("mot_b200: need byte ids or a ttb table")
-        ids, ttb = None, _ttb_ids_args(spec_b, tok, ttb, seq_len)
-        tok, nxt = _with_next(spec_b, tok, next_tokens, seq_len)
-        n_ids = tok.numel() * bpt
-    else:
-        if next_tokens is not None:
-            raise RuntimeError("mot_b200: next_tokens= is the lookahead of a right pull (ttb ids with ttb_pull_side='right')")
-        ids, ttb = _byte_ids(byte_ids), None
-        n_ids = ids.numel()
-    if n_ids != tok.numel() * bpt or bpt * E_byte.shape[1] != D or tuple(W.shape) != (D, D):
+    if (byte_ids is not None and byte_ids.numel() != tokens.numel() * bpt) or bpt * E_byte.shape[1] != D \
+            or tuple(W.shape) != (D, D):
         raise RuntimeError("mot_b200: byte-FC mix needs bpt*byte_dim == token_dim and a square [D, D] weight")
+    tok, ids, _, ttb, nxt = _id_args(spec_b, bpt, tokens, byte_ids, ttb, seq_len, next_tokens)
     return dev, tok, ids, E_tok.contiguous(), E_byte.contiguous(), ttb, nxt
 
 
-def _fc_descs(spec_b: MixSpec, bpt: int, tok, ids, E_tok, E_byte, ttb=None, seq_len: int = 0, next_tok: bool = False):
-    """-> (desc_b, desc_t): the bytes-only gather of the product's operand; the token gather + addend + norm.  ids=None:
-    the operand's ids come from `ttb`."""
-    n = tok.numel()
-    return (make_desc(spec_b, n, None, E_byte, bpt, ids=ids, ttb=ttb, has_lam=False, seq_len=seq_len, next_tok=next_tok),
-            make_desc(MixSpec(combine="tok_only", out_norm=True, eps=spec_b.eps), n, E_tok, None, 0, ids=None, ttb=None,
-                      has_lam=False))
+def _fc_descs(spec_b: MixSpec, bpt: int, seq_len: int, tok, next_tok, ids, ttb, E_tok, E_byte):
+    """-> (tok, desc_b, desc_t): the bytes-only gather of the product's operand; the token gather + addend + norm."""
+    tok, desc_b = _ids_desc(spec_b, bpt, seq_len, tok, next_tok, ids, ttb, None, E_byte)
+    return tok, desc_b, make_desc(MixSpec(combine="tok_only", out_norm=True, eps=spec_b.eps), tok.numel(), E_tok, None, 0,
+                                  ids=None, ttb=None, has_lam=False)
 
 
 def _byte_fc_forward(desc_b: L.MotDesc, desc_t: L.MotDesc, tok, ids, E_tok, E_byte, w_c, ttb=None):
@@ -1194,10 +1141,8 @@ class _MotEmbedByteFcFn(torch.autograd.Function):
     cores; bytes-only scatter.  The operand is gathered again in the backward, not kept."""
 
     @staticmethod
-    def forward(ctx, spec_b: MixSpec, bpt: int, dev, tok, ids, E_tok, E_byte, W, ttb=None, seq_len: int = 0,
-                next_tok=None):
+    def forward(ctx, desc_b: L.MotDesc, desc_t: L.MotDesc, dev, tok, ids, E_tok, E_byte, W, ttb=None):
         w16 = cast_out(W, E_tok.dtype)
-        desc_b, desc_t = _fc_descs(spec_b, bpt, tok, ids, E_tok, E_byte, ttb, seq_len, next_tok is not None)
         ctx.ws = _planned_workspace(desc_t, tok, dev) if ctx.needs_input_grad[5] and tok.numel() > 0 else None
         out, Y = _byte_fc_forward(desc_b, desc_t, tok, ids, E_tok, E_byte, w16, ttb)
         embed_plan_join_if_capturing(ctx.ws, dev)
@@ -1218,7 +1163,7 @@ class _MotEmbedByteFcFn(torch.autograd.Function):
         ctx.ws = None
         _return_workspace(ws)
         _return_workspace(wsb)
-        return None, None, None, None, None, gE_tok, gE_byte, gW, None, None, None
+        return None, None, None, None, None, gE_tok, gE_byte, gW, None
 
 
 def mot_embed_byte_fc(tokens: torch.Tensor, byte_ids: Optional[torch.Tensor], E_tok: torch.Tensor, E_byte: torch.Tensor,
@@ -1232,14 +1177,14 @@ def mot_embed_byte_fc(tokens: torch.Tensor, byte_ids: Optional[torch.Tensor], E_
     spec_b = MixSpec(combine="bytes_only", out_norm=False, slot_major=slot_major and byte_ids is not None,
                      ttb_scramble=slot_major and byte_ids is None, ttb_pull=ttb_pull and byte_ids is None, eps=eps,
                      ttb_pull_side=ttb_pull_side)
-    dev, tok, ids, E_tok_c, E_byte_c, ttb_c, nxt = _byte_fc_args(bpt, tokens, byte_ids, E_tok, E_byte, W_fc, spec_b, ttb,
+    dev, tok, ids, E_tok_c, E_byte_c, ttb_c, nxt = _byte_fc_args(spec_b, bpt, tokens, byte_ids, E_tok, E_byte, W_fc, ttb,
                                                                  seq_len, next_tokens)
     if _custom_ops_wanted():
         need = torch.is_grad_enabled() and any(t.requires_grad for t in (E_tok, E_byte, W_fc))
-        return torch.ops.mot_b200.embed_byte_fc(tok, ids if ids is not None else tok.new_empty(0), E_tok_c, E_byte_c,
-                                                W_fc.contiguous(), pack_spec(spec_b), bpt, float(eps), need, ttb_c,
-                                                seq_len, nxt)[0]
-    return _MotEmbedByteFcFn.apply(spec_b, bpt, dev, tok, ids, E_tok_c, E_byte_c, W_fc, ttb_c, seq_len, nxt)
+        return torch.ops.mot_b200.embed_byte_fc(tok, ids, E_tok_c, E_byte_c, W_fc.contiguous(), pack_spec(spec_b), bpt,
+                                                float(eps), need, ttb_c, seq_len, nxt)[0]
+    tok, desc_b, desc_t = _fc_descs(spec_b, bpt, seq_len, tok, nxt, ids, ttb_c, E_tok_c, E_byte_c)
+    return _MotEmbedByteFcFn.apply(desc_b, desc_t, dev, tok, ids, E_tok_c, E_byte_c, W_fc, ttb_c)
 
 
 def mot_embed_proj(tokens: torch.Tensor, byte_ids: Optional[torch.Tensor], E_tok: torch.Tensor, E_byte: torch.Tensor,
@@ -1257,15 +1202,15 @@ def mot_embed_proj(tokens: torch.Tensor, byte_ids: Optional[torch.Tensor], E_tok
     with spec.ttb_pull the pulled ids of pull_from_left over rows of `seq_len` tokens; padded_and_pulled=True derives
     both sets of `--add-padded-and-pulled`.  spec.ttb_pull_side="right": pull_from_right, with the lookahead
     `next_tokens` (token seq_len of every row, as in mot_embed)."""
-    pair = padded_and_pulled and byte_ids is None
+    ttb_pair = padded_and_pulled and byte_ids is None
     dev, tok, ids, ids2, E_tok_c, E_byte_c, ttb_c, nxt = _proj_args(spec, bpt, tokens, byte_ids, E_tok, E_byte, W, bias,
-                                                                    byte_ids2, ttb, seq_len, pair, next_tokens)
+                                                                    byte_ids2, ttb, seq_len, ttb_pair, next_tokens)
     if _custom_ops_wanted():
         need = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (E_tok, E_byte, W, bias))
-        return torch.ops.mot_b200.embed_proj(tok, ids if ids is not None else tok.new_empty(0), ids2, E_tok_c, E_byte_c,
-                                             W.contiguous(), bias, pack_spec(spec), bpt, float(spec.eps), need, ttb_c,
-                                             seq_len, pair, nxt)[0]
-    return _MotEmbedProjFn.apply(spec, bpt, dev, tok, ids, ids2, E_tok_c, E_byte_c, W, bias, ttb_c, seq_len, pair, nxt)
+        return torch.ops.mot_b200.embed_proj(tok, ids, ids2, E_tok_c, E_byte_c, W.contiguous(), bias, pack_spec(spec), bpt,
+                                             float(spec.eps), need, ttb_c, seq_len, ttb_pair, nxt)[0]
+    tok, desc, desc_pair = _proj_descs(spec, bpt, seq_len, tok, nxt, ids, ids2, ttb_c, ttb_pair, E_tok_c, E_byte_c)
+    return _MotEmbedProjFn.apply(spec, desc, desc_pair, dev, tok, ids, ids2, E_tok_c, E_byte_c, W, bias, ttb_c)
 
 
 def launch_count() -> int:

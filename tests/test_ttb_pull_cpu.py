@@ -1,6 +1,7 @@
 """The token-only call form (pulled byte ids derived from the ttb table inside the kernels), checked without a GPU: the
 C ABI flag and descriptor fields, the spec code of the operators, the refusals, and the fake shapes the operators report
-to torch.compile."""
+to torch.compile.  The right pull (test_ttb_pull_right_cpu.py) shares this file's descriptor, tensor and fake-shape
+helpers."""
 import pytest
 import torch
 from torch._subclasses.fake_tensor import FakeTensorMode
@@ -11,17 +12,18 @@ from mot_b200 import ops
 from mot_b200._library import pack_spec, unpack_spec
 
 
-def _desc(**kw):
+def _desc(side="left", **kw):
+    """A valid token-only descriptor with a pull from `side`; fields overridden by kw."""
     base = dict(abi_version=L.ABI_VERSION, dtype=L.BF16, n_tokens=4096, seq_len=1024, tok_vocab=50257, byte_vocab=458,
                 bpt=16, tok_dim=768, byte_dim=48, out_dim=768, combine=L.ADD,
-                flags=L.F_OUT_NORM | L.F_IDS_FROM_TTB | L.F_TTB_PULL_LEFT, ttb_dtype=L.TTB_I16, eps=1e-7,
-                pad_id=456, eot_id=457)
+                flags=L.F_OUT_NORM | L.F_IDS_FROM_TTB | (L.F_TTB_PULL_LEFT if side == "left" else L.F_TTB_PULL_RIGHT),
+                ttb_dtype=L.TTB_I16, eps=1e-7, pad_id=456, eot_id=457)
     base.update(kw)
     return L.MotDesc(**base)
 
 
 def test_flag_and_abi():
-    assert L.ABI_VERSION == 5 and L.lib().mot_abi_version() == 5
+    assert L.ABI_VERSION == 6 and L.lib().mot_abi_version() == 6
     assert L.F_TTB_PULL_LEFT == 1 << 9
     names = [f[0] for f in L.MotDesc._fields_]
     assert names[-2:] == ["pad_id", "eot_id"]
@@ -75,7 +77,8 @@ def test_right_pull_refused():
         mot_b200.SptByteMixEmbedding(100, 458, 64, 16, 64, padding_in="middle")
 
 
-N, V, VB, BPT, BD = 64, 100, 458, 4, 16
+N, V, VB, BPT, BD, S = 64, 100, 458, 4, 16, 16
+R = N // S
 
 
 def _t(*shape, dtype=torch.bfloat16, grad=False):
@@ -95,24 +98,40 @@ def test_bad_seq_len_refused_before_launch():
                                        seq_len=0, ttb_pull=True)
 
 
-def test_fake_shapes_with_ttb():
+def check_fake_shapes(side: str) -> None:
+    """The operators with `ttb` (ids=None) report the shapes of their outputs; a right pull also passes its lookahead
+    next_tok, one token per row of S."""
     with FakeTensorMode():
         tok = _t(N, dtype=torch.int32)
-        ph = _t(0, dtype=torch.int32)
+        nxt = (_t(R, dtype=torch.int32),) if side == "right" else ()
         ttb = _t(V, BPT, dtype=torch.int16)
         Et, Eb = _t(V, 64), _t(VB, BD)
         W = _t(32, 64 + BPT * BD, dtype=torch.float32)
-        spec = pack_spec(mot_b200.MixSpec(combine="concat", tok_norm=True, byte_norm=True, ttb_pull=True))
+        spec = pack_spec(mot_b200.MixSpec(combine="concat", tok_norm=True, byte_norm=True, ttb_pull=True,
+                                          ttb_pull_side=side))
         for pair in (False, True):
-            out, Y, w_c, ws = torch.ops.mot_b200.embed_proj(tok, ph, None, Et, Eb, W, None, spec, BPT, 1e-7, True, ttb, 16,
-                                                            pair)
+            out, Y, w_c, ws = torch.ops.mot_b200.embed_proj(tok, None, None, Et, Eb, W, None, spec, BPT, 1e-7, True, ttb, S,
+                                                            pair, *nxt)
             assert out.shape == (N, 32) and Y.shape == (N, 32) and w_c.shape == W.shape and ws.numel() > 0
-            gt, gb, gW, gbias = torch.ops.mot_b200.embed_proj_bwd(out, tok, ph, None, Et, Eb, W, w_c, Y, ws, spec, BPT,
-                                                                  1e-7, False, ttb, 16, pair)
+            gt, gb, gW, gbias = torch.ops.mot_b200.embed_proj_bwd(out, tok, None, None, Et, Eb, W, w_c, Y, ws, spec, BPT,
+                                                                  1e-7, False, ttb, S, pair, *nxt)
             assert gt.shape == Et.shape and gb.shape == Eb.shape and gW.shape == W.shape and gbias.numel() == 0
-        spec_b = pack_spec(mot_b200.MixSpec(combine="bytes_only", out_norm=False, ttb_scramble=True, ttb_pull=True))
+        spec_b = pack_spec(mot_b200.MixSpec(combine="bytes_only", out_norm=False, ttb_scramble=True, ttb_pull=True,
+                                            ttb_pull_side=side))
         Wf = _t(64, 64)
-        out, Y, w_c, ws = torch.ops.mot_b200.embed_byte_fc(tok, ph, Et, Eb, Wf, spec_b, BPT, 1e-7, True, ttb, 16)
+        out, Y, w_c, ws = torch.ops.mot_b200.embed_byte_fc(tok, None, Et, Eb, Wf, spec_b, BPT, 1e-7, True, ttb, S, *nxt)
         assert out.shape == (N, 64) and Y.shape == (N, 64) and w_c.numel() == 0
-        gt, gb, gW = torch.ops.mot_b200.embed_byte_fc_bwd(out, tok, ph, Et, Eb, Wf, w_c, Y, ws, spec_b, BPT, 1e-7, ttb, 16)
+        gt, gb, gW = torch.ops.mot_b200.embed_byte_fc_bwd(out, tok, None, Et, Eb, Wf, w_c, Y, ws, spec_b, BPT, 1e-7, ttb, S,
+                                                          *nxt)
         assert gt.shape == Et.shape and gb.shape == Eb.shape and gW.shape == Wf.shape
+        Ea = _t(V, BPT * BD)
+        spec_e = pack_spec(mot_b200.MixSpec(combine="add", ttb_pull=True, ttb_pull_side=side))
+        out, rstd, ws = torch.ops.mot_b200.embed(tok, None, ttb, Ea, Eb, None, spec_e, BPT, S, 1e-7, True, *nxt)
+        assert out.shape == (N, BPT * BD) and ws.numel() > 0
+        gt, gb, gl = torch.ops.mot_b200.embed_bwd(out, tok, None, ttb, Ea, Eb, None, out, rstd, ws, spec_e, BPT, S, 1e-7,
+                                                  *nxt)
+        assert gt.shape == Ea.shape and gb.shape == Eb.shape and gl.numel() == 0
+
+
+def test_fake_shapes_with_ttb():
+    check_fake_shapes("left")

@@ -11,42 +11,34 @@ import mot_b200
 from mot_b200 import _lib as L
 from mot_b200 import ops
 from mot_b200._library import pack_spec, unpack_spec
-
-
-def _desc(**kw):
-    base = dict(abi_version=L.ABI_VERSION, dtype=L.BF16, n_tokens=4096, seq_len=1024, tok_vocab=50257, byte_vocab=458,
-                bpt=16, tok_dim=768, byte_dim=48, out_dim=768, combine=L.ADD,
-                flags=L.F_OUT_NORM | L.F_IDS_FROM_TTB | L.F_TTB_PULL_RIGHT, ttb_dtype=L.TTB_I16, eps=1e-7,
-                pad_id=456, eot_id=457)
-    base.update(kw)
-    return L.MotDesc(**base)
+from test_ttb_pull_cpu import BD, BPT, N, R, S, V, VB, _desc, _t, check_fake_shapes
 
 
 def test_flag_values_and_symbols():
     assert L.F_TTB_PULL_RIGHT == 1 << 10 and L.F_TTB_NEXT_TOK == 1 << 11
-    assert L.ABI_VERSION == 5 and L.lib().mot_abi_version() == 5
-    for fn in ("mot_byte_pair_ttb_ex_fwd", "mot_byte_pair_ttb_ex_bwd"):
-        assert hasattr(L.lib(), fn)
+    assert L.ABI_VERSION == 6 and L.lib().mot_abi_version() == 6
+    for fn in ("mot_byte_pair_ttb_fwd", "mot_byte_pair_ttb_bwd"):   # the direction is their `flags` argument
+        assert hasattr(L.lib(), fn) and L._SIGNATURES[fn][1][-2] is L.C.c_int32
 
 
 def test_validation_of_the_right_pull_flags():
     ws = L.lib().mot_embed_workspace_bytes
-    right, nxt = _desc().flags, _desc().flags | L.F_TTB_NEXT_TOK
-    assert ws(_desc()) > 0 and ws(_desc(flags=nxt)) > 0
-    assert ws(_desc(flags=nxt | L.F_TTB_SCRAMBLE)) > 0
-    assert ws(_desc(flags=right | L.F_TTB_PULL_LEFT)) == 0                           # both directions
+    right, nxt = _desc("right").flags, _desc("right").flags | L.F_TTB_NEXT_TOK
+    assert ws(_desc("right")) > 0 and ws(_desc("right", flags=nxt)) > 0
+    assert ws(_desc("right", flags=nxt | L.F_TTB_SCRAMBLE)) > 0
+    assert ws(_desc("right", flags=right | L.F_TTB_PULL_LEFT)) == 0                  # both directions
     assert ws(_desc(flags=L.F_OUT_NORM | L.F_IDS_FROM_TTB | L.F_TTB_PULL_LEFT | L.F_TTB_NEXT_TOK)) == 0
     assert ws(_desc(flags=L.F_OUT_NORM | L.F_IDS_FROM_TTB | L.F_TTB_NEXT_TOK)) == 0  # a lookahead without a right pull
-    assert ws(_desc(seq_len=0)) == 0 and ws(_desc(seq_len=1000)) == 0                # rows as for the left pull
-    assert ws(_desc(pad_id=70000)) == 0 and ws(_desc(eot_id=-40000)) == 0
-    assert ws(_desc(combine=L.BYTES_ONLY, tok_vocab=0, tok_dim=0, flags=nxt)) == 0
-    assert ws(_desc(bpt=33, tok_dim=33 * 8, byte_dim=8, out_dim=33 * 8)) == 0
+    assert ws(_desc("right", seq_len=0)) == 0 and ws(_desc("right", seq_len=1000)) == 0   # rows as for the left pull
+    assert ws(_desc("right", pad_id=70000)) == 0 and ws(_desc("right", eot_id=-40000)) == 0
+    assert ws(_desc("right", combine=L.BYTES_ONLY, tok_vocab=0, tok_dim=0, flags=nxt)) == 0
+    assert ws(_desc("right", bpt=33, tok_dim=33 * 8, byte_dim=8, out_dim=33 * 8)) == 0
 
 
 def test_pair_ex_refuses_bad_flags():
     # checked before anything else: no pointer is dereferenced, no device is needed
     args = (None, None, 100, L.TTB_I16, 16, 456, 457, 64, 4, None, 458, 16, L.BF16, 1e-7)
-    fwd, bwd = L.lib().mot_byte_pair_ttb_ex_fwd, L.lib().mot_byte_pair_ttb_ex_bwd
+    fwd, bwd = L.lib().mot_byte_pair_ttb_fwd, L.lib().mot_byte_pair_ttb_bwd
     for flags in (0, L.F_TTB_PULL_LEFT | L.F_TTB_PULL_RIGHT, L.F_TTB_PULL_LEFT | L.F_TTB_NEXT_TOK, L.F_TTB_NEXT_TOK,
                   L.F_TTB_PULL_RIGHT | L.F_TTB_SCRAMBLE):
         assert fwd(*args, None, 64, 0, flags, None) == L.ERR_BAD_ARG
@@ -90,45 +82,8 @@ def test_right_pull_without_lookahead_still_refused():
         m(torch.zeros(2, 8, dtype=torch.int32))
 
 
-N, V, VB, BPT, BD, S = 64, 100, 458, 4, 16, 16
-R = N // S
-
-
-def _t(*shape, dtype=torch.bfloat16, grad=False):
-    return torch.empty(*shape, dtype=dtype, device="cuda", requires_grad=grad)
-
-
 def test_fake_shapes_with_next_tok():
-    with FakeTensorMode():
-        tok, nxt = _t(N, dtype=torch.int32), _t(R, dtype=torch.int32)
-        ph = _t(0, dtype=torch.int32)
-        ttb = _t(V, BPT, dtype=torch.int16)
-        Et, Eb = _t(V, 64), _t(VB, BD)
-        W = _t(32, 64 + BPT * BD, dtype=torch.float32)
-        spec = pack_spec(mot_b200.MixSpec(combine="concat", tok_norm=True, byte_norm=True, ttb_pull=True,
-                                          ttb_pull_side="right"))
-        for pair in (False, True):
-            out, Y, w_c, ws = torch.ops.mot_b200.embed_proj(tok, ph, None, Et, Eb, W, None, spec, BPT, 1e-7, True, ttb, S,
-                                                            pair, nxt)
-            assert out.shape == (N, 32) and Y.shape == (N, 32) and w_c.shape == W.shape and ws.numel() > 0
-            gt, gb, gW, gbias = torch.ops.mot_b200.embed_proj_bwd(out, tok, ph, None, Et, Eb, W, w_c, Y, ws, spec, BPT,
-                                                                  1e-7, False, ttb, S, pair, nxt)
-            assert gt.shape == Et.shape and gb.shape == Eb.shape and gW.shape == W.shape and gbias.numel() == 0
-        spec_b = pack_spec(mot_b200.MixSpec(combine="bytes_only", out_norm=False, ttb_scramble=True, ttb_pull=True,
-                                            ttb_pull_side="right"))
-        Wf = _t(64, 64)
-        out, Y, w_c, ws = torch.ops.mot_b200.embed_byte_fc(tok, ph, Et, Eb, Wf, spec_b, BPT, 1e-7, True, ttb, S, nxt)
-        assert out.shape == (N, 64) and Y.shape == (N, 64) and w_c.numel() == 0
-        gt, gb, gW = torch.ops.mot_b200.embed_byte_fc_bwd(out, tok, ph, Et, Eb, Wf, w_c, Y, ws, spec_b, BPT, 1e-7, ttb, S,
-                                                          nxt)
-        assert gt.shape == Et.shape and gb.shape == Eb.shape and gW.shape == Wf.shape
-        Ea = _t(V, BPT * BD)
-        spec_e = pack_spec(mot_b200.MixSpec(combine="add", ttb_pull=True, ttb_pull_side="right"))
-        out, rstd, ws = torch.ops.mot_b200.embed(tok, None, ttb, Ea, Eb, None, spec_e, BPT, S, 1e-7, True, nxt)
-        assert out.shape == (N, BPT * BD) and ws.numel() > 0
-        gt, gb, gl = torch.ops.mot_b200.embed_bwd(out, tok, None, ttb, Ea, Eb, None, out, rstd, ws, spec_e, BPT, S, 1e-7,
-                                                  nxt)
-        assert gt.shape == Ea.shape and gb.shape == Eb.shape and gl.numel() == 0
+    check_fake_shapes("right")
 
 
 _RIGHT = mot_b200.MixSpec(combine="concat", tok_norm=True, byte_norm=True, ttb_pull=True, ttb_pull_side="right")

@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define MOT_B200_ABI_VERSION 6
+#define MOT_B200_ABI_VERSION 7
 
 /* ---- error codes ------------------------------------------------------- */
 enum {
@@ -253,36 +253,23 @@ int mot_embed_bwd_uses_saved(const MotDesc* d);
 /* ---- byte half of `--add-padded-and-pulled` (spt/train_gpt.py:371-379) ----------------------------------------
  * rows[pos, col_offset + k*byte_dim : +byte_dim] = rms_norm(E_byte[ids_a[pos,k]] + E_byte[ids_b[pos,k]]) for k < bpt:
  * two gathers summed BEFORE the per-byte norm (`norm(self.embed_bytes(byte_tensor) + self.embed_bytes(byte_tensor_pulled))`).
- * ids_a / ids_b: token-major [n_tokens, bpt] int32 or int64 (ids_i64).  Rows have `row_stride` elements: the byte
- * columns of the [tok | bytes] projection operand, whose token columns mot_embed_fwd writes with MOT_TOK_ONLY and the
- * same row_stride (MotDesc.row_stride / col_offset).  bpt <= 32, byte_dim a multiple of 8 with byte_dim <= 64 * G,
- * G = the largest power of two <= 32 / bpt. */
-int mot_byte_pair_fwd(const void* ids_a, const void* ids_b, int32_t ids_i64, int64_t n_tokens, int32_t bpt,
-                      const void* E_byte, int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps, void* out,
-                      int64_t row_stride, int32_t col_offset, void* stream);
+ * d: MOT_BYTES_ONLY with MOT_F_BYTE_NORM, out_dim = bpt*byte_dim; row_stride / col_offset locate the byte columns of the
+ * [tok | bytes] projection operand, whose token columns mot_embed_fwd writes with MOT_TOK_ONLY and the same row_stride.
+ * bpt <= 32, byte_dim a multiple of 8 with byte_dim <= 64 * G, G = the largest power of two <= 32 / bpt.  The ids:
+ *   explicit : ids_a / ids_b token-major [n_tokens, bpt], int32 or int64 (MOT_F_IDS_I64); tok and ttb may be NULL;
+ *   derived  : MOT_F_IDS_FROM_TTB with MOT_F_TTB_PULL_LEFT, or MOT_F_TTB_PULL_RIGHT optionally with MOT_F_TTB_NEXT_TOK:
+ *              ids_a = the padded ids (the ttb rows of `tok`, mot_ttb_expand), ids_b = the pulled ids over rows of seq_len
+ *              tokens, both derived inside the kernels; tok int32 [n_tokens] (+ the lookahead tail), ttb [tok_vocab, bpt]
+ *              of ttb_dtype, pad_id / eot_id; ids_a and ids_b are NULL.
+ * Any other combine or flag: MOT_ERR_BAD_ARG. */
+int mot_byte_pair_fwd(const MotDesc* d, const int32_t* tok, const void* ids_a, const void* ids_b, const void* ttb,
+                      const void* E_byte, void* out, void* stream);
 /* Backward: gE_byte [byte_vocab, byte_dim] dense, fully overwritten, = the norm backward of every (position, slot)
  * added to BOTH gathered rows.  workspace: mot_byte_pair_workspace_bytes() bytes (cleared by the call). */
 size_t mot_byte_pair_workspace_bytes(int32_t byte_vocab, int32_t byte_dim);
-int mot_byte_pair_bwd(const void* ids_a, const void* ids_b, int32_t ids_i64, int64_t n_tokens, int32_t bpt,
-                      const void* E_byte, int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps,
-                      const void* grad_out, int64_t row_stride, int32_t col_offset, void* gE_byte, void* workspace,
-                      size_t ws_bytes, void* stream);
-
-/* The same pair with both id tensors derived from the token ids inside the kernels: ids_a = the padded ids (the ttb rows
- * of `tok`, mot_ttb_expand; with a right-padded table the right-padded ids), ids_b = the pulled ids over rows of seq_len
- * tokens in the direction `flags` names: MOT_F_TTB_PULL_LEFT (pull_from_left), or MOT_F_TTB_PULL_RIGHT
- * (pull_from_right), optionally with MOT_F_TTB_NEXT_TOK (the lookahead tail tok[n_tokens + r] of every row r).  Other
- * flags: MOT_ERR_BAD_ARG.  tok: int32 [n_tokens], n_tokens % seq_len == 0; ttb [tok_vocab, bpt] of ttb_dtype.
- * Otherwise as above. */
-int mot_byte_pair_ttb_fwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
-                          int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt, const void* E_byte,
-                          int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps, void* out, int64_t row_stride,
-                          int32_t col_offset, int32_t flags, void* stream);
-int mot_byte_pair_ttb_bwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
-                          int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt, const void* E_byte,
-                          int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps, const void* grad_out,
-                          int64_t row_stride, int32_t col_offset, void* gE_byte, void* workspace, size_t ws_bytes,
-                          int32_t flags, void* stream);
+int mot_byte_pair_bwd(const MotDesc* d, const int32_t* tok, const void* ids_a, const void* ids_b, const void* ttb,
+                      const void* E_byte, const void* grad_out, void* gE_byte, void* workspace, size_t ws_bytes,
+                      void* stream);
 
 /* ---- data-parallel exchange: average the gradient bucket across ranks through NVLink / NVSwitch -----------------
  * Replaces the per-parameter dist.all_reduce(param.grad, AVG) of spt/train_gpt.py:1320-1321 and runs/7:697-700 (launched

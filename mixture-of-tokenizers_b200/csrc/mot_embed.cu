@@ -138,21 +138,21 @@ static int stream_chunk_slab(long long n_tokens, int n_slabs, int warps_per_cta)
   return (int)R;
 }
 
-static int validate(const MotDesc* d) {
+// The rules every descriptor obeys, the byte pair's too (mot_pair.cu).
+int validate_desc(const MotDesc* d) {
   if (!d) return MOT_ERR_BAD_ARG;
   if (d->abi_version != MOT_B200_ABI_VERSION) return MOT_ERR_BAD_ARG;
   if (d->dtype != MOT_BF16 && d->dtype != MOT_F32) return MOT_ERR_UNSUPPORTED;
   if (d->n_tokens < 0 || d->n_tokens > 0x7fffffffLL) return MOT_ERR_BAD_ARG;
   if (d->combine < MOT_ADD || d->combine > MOT_MEAN) return MOT_ERR_UNSUPPORTED;
   const bool has_tok = d->combine != MOT_BYTES_ONLY, has_bytes = d->combine != MOT_TOK_ONLY;
-  if (d->out_dim <= 0 || d->out_dim % 8) return MOT_ERR_MISALIGNED;
   if (has_tok && (d->tok_vocab <= 0 || d->tok_dim <= 0)) return MOT_ERR_BAD_ARG;
   if (has_tok && d->tok_dim % 8) return MOT_ERR_MISALIGNED;
   if (has_bytes) {
     if (d->byte_vocab <= 0 || d->byte_dim <= 0 || d->bpt <= 0 || d->bpt > 32) return MOT_ERR_BAD_ARG;
     if (d->byte_dim % 8) return MOT_ERR_MISALIGNED;
-    if ((d->flags & MOT_F_BYTE_NORM) && d->byte_dim > 256) return MOT_ERR_UNSUPPORTED;
   }
+  if (d->out_dim <= 0 || d->out_dim % 8) return MOT_ERR_MISALIGNED;
   const long long db = (long long)d->bpt * d->byte_dim;
   switch (d->combine) {
     case MOT_ADD: if (d->tok_dim != db || d->out_dim != d->tok_dim) return MOT_ERR_BAD_ARG; break;
@@ -160,15 +160,6 @@ static int validate(const MotDesc* d) {
     case MOT_TOK_ONLY: if (d->out_dim != d->tok_dim) return MOT_ERR_BAD_ARG; break;
     case MOT_BYTES_ONLY: if (d->out_dim != db) return MOT_ERR_BAD_ARG; break;
     case MOT_MEAN: if (d->byte_dim != d->tok_dim || d->out_dim != d->tok_dim) return MOT_ERR_BAD_ARG; break;
-  }
-  // a lane holds at most 8 chunks of 8 elements per launch: 2048 columns.  A concat without a norm over the whole row
-  // runs as two launches (concat_splits), so the cap applies to each half: the widest reference operand
-  // (spt/experiments100_000steps.sh: 1024 + 16 x 128 = 3072 columns) fits.
-  constexpr int kMaxCols = 8 * 32 * 8;
-  if (d->combine == MOT_CONCAT && !(d->flags & (MOT_F_OUT_NORM | MOT_F_HAS_LAMBDAS))) {
-    if (d->tok_dim > kMaxCols || db > kMaxCols) return MOT_ERR_UNSUPPORTED;
-  } else if (d->out_dim > kMaxCols) {
-    return MOT_ERR_UNSUPPORTED;
   }
   if (d->row_stride != 0 || d->col_offset != 0) {  // a column slice of wider rows
     const long long ld = d->row_stride ? d->row_stride : d->out_dim;
@@ -186,6 +177,22 @@ static int validate(const MotDesc* d) {
       if (d->tok_vocab <= 0) return MOT_ERR_BAD_ARG;  // rows of the ttb table, also without a token table
       if (d->pad_id != (int16_t)d->pad_id || d->eot_id != (int16_t)d->eot_id) return MOT_ERR_BAD_ARG;  // int16, as in mot_pull
     }
+  }
+  return MOT_OK;
+}
+
+// validate_desc plus the capacity of the fused kernels.
+static int validate(const MotDesc* d) {
+  if (int rc = validate_desc(d)) return rc;
+  if ((d->flags & MOT_F_BYTE_NORM) && d->combine != MOT_TOK_ONLY && d->byte_dim > 256) return MOT_ERR_UNSUPPORTED;
+  // a lane holds at most 8 chunks of 8 elements per launch: 2048 columns.  A concat without a norm over the whole row
+  // runs as two launches (concat_splits), so the cap applies to each half: the widest reference operand
+  // (spt/experiments100_000steps.sh: 1024 + 16 x 128 = 3072 columns) fits.
+  constexpr int kMaxCols = 8 * 32 * 8;
+  if (d->combine == MOT_CONCAT && !(d->flags & (MOT_F_OUT_NORM | MOT_F_HAS_LAMBDAS))) {
+    if (d->tok_dim > kMaxCols || (long long)d->bpt * d->byte_dim > kMaxCols) return MOT_ERR_UNSUPPORTED;
+  } else if (d->out_dim > kMaxCols) {
+    return MOT_ERR_UNSUPPORTED;
   }
   return MOT_OK;
 }

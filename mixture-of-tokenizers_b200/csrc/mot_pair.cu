@@ -28,14 +28,12 @@ struct PairParams {
   float eps;
 };
 // Both id sets derived from the token ids (a padded, b pulled).  A separate type, so that the kernels of explicit ids keep
-// their parameter block.
+// their parameter block (and with it their register counts).
 struct PairTtbParams : PairParams {
   PullSrc ttb;
 };
-// The same with the pulled ids of pull_from_right (MOT_F_TTB_PULL_RIGHT): its own kernel instantiations.
-struct PairTtbRightParams : PairTtbParams {};
-template <typename P>
-constexpr bool kPairTtb = std::is_base_of_v<PairTtbParams, P>;
+template <int PULL>
+using PairArgs = std::conditional_t<PULL == kNoPull, PairParams, PairTtbParams>;
 
 constexpr int kPairThreads = 512;
 
@@ -65,12 +63,12 @@ __device__ __forceinline__ int pair_load_id(const void* ids, int i64, long long 
 
 // Byte ids (ia, ib) of this lane's slot at position pos derived from the token ids: padded ids for a, pulled ids for b.
 // Warp collective; clamped; 0 on inactive lanes.
-template <typename P>
-__device__ __forceinline__ void pair_ttb_ids(const P& p, long long pos, int slot, bool active, int& ia, int& ib) {
+template <int PULL>
+__device__ __forceinline__ void pair_ttb_ids(const PairTtbParams& p, long long pos, int slot, bool active, int& ia, int& ib) {
   const int lane = lane_id();
   const int tv = clampi(ld_g(p.ttb.tok + pos), p.ttb.V - 1);
   const int a = lane < p.bpt ? ttb_raw(p.ttb.ttb, p.ttb.ttb_dtype, tv, p.bpt, lane) : 0;
-  const int b = pulled_row_warp<std::is_same_v<P, PairTtbRightParams>>(p.ttb, (int)pos);
+  const int b = pulled_row_warp<PULL == kPullRight>(p.ttb, (int)pos);
   ia = clampi(__shfl_sync(0xffffffffu, a, slot & 31), p.Vb - 1);
   ib = clampi(__shfl_sync(0xffffffffu, b, slot & 31), p.Vb - 1);
   if (!active) ia = ib = 0;
@@ -83,9 +81,9 @@ __device__ __forceinline__ float group_sum(float v) {
   return v;
 }
 
-// MAXJ = 8-element chunks per lane (ceil(bd / 8 / G))
-template <typename T, int G, int MAXJ, typename P>
-__global__ void __launch_bounds__(kPairThreads, MAXJ <= 4 ? 2 : 1) mot_pair_fwd_kernel(const P p) {
+// MAXJ = 8-element chunks per lane (ceil(bd / 8 / G)); PULL: kNoPull loads the ids, kPullLeft / kPullRight derive them
+template <typename T, int G, int MAXJ, int PULL>
+__global__ void __launch_bounds__(kPairThreads, MAXJ <= 4 ? 2 : 1) mot_pair_fwd_kernel(const PairArgs<PULL> p) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   __shared__ uint64_t tab_bar;
   T* tab = reinterpret_cast<T*>(smem_raw);
@@ -101,8 +99,8 @@ __global__ void __launch_bounds__(kPairThreads, MAXJ <= 4 ? 2 : 1) mot_pair_fwd_
   const long long W = (long long)gridDim.x * nw;
   for (long long pos = (long long)warp * gridDim.x + blockIdx.x; pos < p.N; pos += W) {
     int ia = 0, ib = 0;
-    if constexpr (kPairTtb<P>) {
-      pair_ttb_ids(p, pos, slot, active, ia, ib);
+    if constexpr (PULL != kNoPull) {
+      pair_ttb_ids<PULL>(p, pos, slot, active, ia, ib);
     } else if (active) {
       ia = pair_load_id(p.ids_a, p.ids_i64, pos * p.bpt + slot, p.Vb - 1);
       ib = pair_load_id(p.ids_b, p.ids_i64, pos * p.bpt + slot, p.Vb - 1);
@@ -141,8 +139,8 @@ __global__ void __launch_bounds__(kPairThreads, MAXJ <= 4 ? 2 : 1) mot_pair_fwd_
 // Backward: with s = E[ia] + E[ib], r = rsqrt(mean(s^2) + eps): ds = r*g - s * r^3 * mean(g.s); both gathered rows
 // receive ds (fp32 RED.v4 into one of n_rep L2-resident replicas; mot_bwd_finalize_kernel sums and casts them).
 // Two passes over the slot (reduce, then scatter) so that nothing of the row is held across the reduction.
-template <typename T, int G, int MAXJ, typename P>
-__global__ void __launch_bounds__(kPairThreads, MAXJ <= 4 ? 2 : 1) mot_pair_bwd_kernel(const P p) {
+template <typename T, int G, int MAXJ, int PULL>
+__global__ void __launch_bounds__(kPairThreads, MAXJ <= 4 ? 2 : 1) mot_pair_bwd_kernel(const PairArgs<PULL> p) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   __shared__ uint64_t tab_bar;
   T* tab = reinterpret_cast<T*>(smem_raw);
@@ -160,8 +158,8 @@ __global__ void __launch_bounds__(kPairThreads, MAXJ <= 4 ? 2 : 1) mot_pair_bwd_
   const long long W = (long long)gridDim.x * nw;
   for (long long pos = gw; pos < p.N; pos += W) {
     int ia = 0, ib = 0;
-    if constexpr (kPairTtb<P>) {
-      pair_ttb_ids(p, pos, slot, active, ia, ib);
+    if constexpr (PULL != kNoPull) {
+      pair_ttb_ids<PULL>(p, pos, slot, active, ia, ib);
     } else if (active) {
       ia = pair_load_id(p.ids_a, p.ids_i64, pos * p.bpt + slot, p.Vb - 1);
       ib = pair_load_id(p.ids_b, p.ids_i64, pos * p.bpt + slot, p.Vb - 1);
@@ -213,8 +211,8 @@ __global__ void __launch_bounds__(kPairThreads, MAXJ <= 4 ? 2 : 1) mot_pair_bwd_
   }
 }
 
-template <typename T, int G, int MAXJ, typename P>
-static int launch_pair(const P& p, bool backward, cudaStream_t s) {
+template <typename T, int G, int MAXJ, int PULL>
+static int launch_pair(const PairTtbParams& p, bool backward, cudaStream_t s) {
   int sms = 0, optin = 0;
   if (int rc = device_props(&sms, &optin)) return rc;
   const size_t smem = align_up((size_t)p.Vb * p.bd * sizeof(T), 128);
@@ -224,11 +222,11 @@ static int launch_pair(const P& p, bool backward, cudaStream_t s) {
   if (blocks > (long long)per_sm * sms) blocks = (long long)per_sm * sms;
   if (blocks < 1) blocks = 1;
   if (backward) {
-    auto kern = mot_pair_bwd_kernel<T, G, MAXJ, P>;
+    auto kern = mot_pair_bwd_kernel<T, G, MAXJ, PULL>;
     if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return check_launch();
     launch_pdl(kern, dim3((unsigned)blocks), dim3(kPairThreads), smem, s, p);
   } else {
-    auto kern = mot_pair_fwd_kernel<T, G, MAXJ, P>;
+    auto kern = mot_pair_fwd_kernel<T, G, MAXJ, PULL>;
     if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return check_launch();
     launch_pdl(kern, dim3((unsigned)blocks), dim3(kPairThreads), smem, s, p);
   }
@@ -236,14 +234,14 @@ static int launch_pair(const P& p, bool backward, cudaStream_t s) {
   return check_launch();
 }
 
-template <typename T, typename P>
-static int dispatch_pair(const P& p, bool backward, cudaStream_t s) {
+template <typename T, int PULL>
+static int dispatch_pair(const PairTtbParams& p, bool backward, cudaStream_t s) {
   const int per_lane = (p.bd / kChunk + p.G - 1) / p.G;  // 8-element chunks per lane
   const int mj = per_lane <= 4 ? 4 : 8;
   if (per_lane > 8) return MOT_ERR_UNSUPPORTED;
 #define MOT_PAIR_CASE(GG)                                                     \
   case GG:                                                                    \
-    return mj == 4 ? launch_pair<T, GG, 4>(p, backward, s) : launch_pair<T, GG, 8>(p, backward, s);
+    return mj == 4 ? launch_pair<T, GG, 4, PULL>(p, backward, s) : launch_pair<T, GG, 8, PULL>(p, backward, s);
   switch (p.G) {
     MOT_PAIR_CASE(1)
     MOT_PAIR_CASE(2)
@@ -254,93 +252,68 @@ static int dispatch_pair(const P& p, bool backward, cudaStream_t s) {
   return MOT_ERR_UNSUPPORTED;
 }
 
-static int pair_ttb_validate(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
-                             int64_t n) {
-  if (ttb_dtype < MOT_TTB_I16 || ttb_dtype > MOT_TTB_BF16) return MOT_ERR_UNSUPPORTED;
-  if (tok_vocab <= 0 || seq_len <= 0 || n % seq_len) return MOT_ERR_BAD_ARG;
-  if (n > 0 && (!tok || !ttb)) return MOT_ERR_BAD_ARG;
-  return MOT_OK;
+// The instantiation of the descriptor's dtype and id source.
+static int run_pair(const MotDesc* d, const PairTtbParams& p, bool backward, cudaStream_t s) {
+  const bool bf16 = d->dtype == MOT_BF16;
+  if (d->flags & MOT_F_TTB_PULL_LEFT)
+    return bf16 ? dispatch_pair<__nv_bfloat16, kPullLeft>(p, backward, s) : dispatch_pair<float, kPullLeft>(p, backward, s);
+  if (d->flags & MOT_F_TTB_PULL_RIGHT)
+    return bf16 ? dispatch_pair<__nv_bfloat16, kPullRight>(p, backward, s) : dispatch_pair<float, kPullRight>(p, backward, s);
+  return bf16 ? dispatch_pair<__nv_bfloat16, kNoPull>(p, backward, s) : dispatch_pair<float, kNoPull>(p, backward, s);
 }
 
-static int pair_validate(const void* ids_a, const void* ids_b, int64_t n, int32_t bpt, const void* E_byte, int32_t Vb,
-                         int32_t bd, int32_t dtype, const void* rows, int64_t row_stride, int32_t col_offset) {
-  if (dtype != MOT_BF16 && dtype != MOT_F32) return MOT_ERR_UNSUPPORTED;
-  if (n < 0 || n > 0x7fffffffLL || bpt <= 0 || bpt > 32 || Vb <= 0 || bd <= 0) return MOT_ERR_BAD_ARG;
-  if (bd % 8 || row_stride % 8 || col_offset % 8) return MOT_ERR_MISALIGNED;
-  if (col_offset < 0 || row_stride < (int64_t)col_offset + (int64_t)bpt * bd) return MOT_ERR_BAD_ARG;
-  if (n == 0) return MOT_OK;
-  if (!ids_a || !ids_b || !E_byte || !rows) return MOT_ERR_BAD_ARG;
+int validate_desc(const MotDesc* d);  // mot_embed.cu: the rules every descriptor obeys
+
+// A pair descriptor (mot_b200.h): bytes-only with the per-byte norm; explicit ids (MOT_F_IDS_I64 gives their width), or
+// ids derived from the ttb table with exactly one pull, the right one optionally with its lookahead.
+static int pair_check(const MotDesc* d) {
+  constexpr int32_t kPull = MOT_F_TTB_PULL_LEFT | MOT_F_TTB_PULL_RIGHT;
+  if (d->combine != MOT_BYTES_ONLY || !(d->flags & MOT_F_BYTE_NORM)) return MOT_ERR_BAD_ARG;
+  const int32_t ids = d->flags & ~MOT_F_BYTE_NORM;
+  const bool ok = (ids & MOT_F_IDS_FROM_TTB) ? (ids & kPull) && !(ids & ~(MOT_F_IDS_FROM_TTB | kPull | MOT_F_TTB_NEXT_TOK))
+                                             : !(ids & ~MOT_F_IDS_I64);
+  return ok ? MOT_OK : MOT_ERR_BAD_ARG;
+}
+
+// Everything both entry points check before they touch the device; `rows` is out (forward) or grad_out (backward).
+static int pair_args(const MotDesc* d, const int32_t* tok, const void* ids_a, const void* ids_b, const void* ttb,
+                     const void* E_byte, const void* rows) {
+  if (int rc = validate_desc(d)) return rc;
+  if (int rc = pair_check(d)) return rc;
+  if (d->n_tokens == 0) return MOT_OK;
+  const bool derived = (d->flags & MOT_F_IDS_FROM_TTB) != 0;
+  if ((derived ? !tok || !ttb : !ids_a || !ids_b) || !E_byte || !rows) return MOT_ERR_BAD_ARG;
   if ((reinterpret_cast<uintptr_t>(E_byte) | reinterpret_cast<uintptr_t>(rows)) & 15u) return MOT_ERR_MISALIGNED;
   return MOT_OK;
 }
 
-static void pair_fill(PairParams& p, const void* ids_a, const void* ids_b, int32_t ids_i64, int64_t n, int32_t bpt,
-                      const void* E_byte, int32_t Vb, int32_t bd, float eps, int64_t row_stride, int32_t col_offset) {
-  p = PairParams{};
+static PairTtbParams pair_params(const MotDesc* d, const int32_t* tok, const void* ids_a, const void* ids_b,
+                                 const void* ttb, const void* E_byte) {
+  PairTtbParams p{};
   p.ids_a = ids_a; p.ids_b = ids_b; p.E_byte = E_byte;
-  p.N = n; p.ld = row_stride; p.col = col_offset;
-  p.Vb = Vb; p.bpt = bpt; p.bd = bd; p.ids_i64 = ids_i64 != 0; p.n_rep = kByteRep; p.eps = eps;
+  p.N = d->n_tokens; p.ld = d->row_stride ? d->row_stride : d->out_dim; p.col = d->col_offset;
+  p.Vb = d->byte_vocab; p.bpt = d->bpt; p.bd = d->byte_dim; p.ids_i64 = (d->flags & MOT_F_IDS_I64) != 0;
+  p.n_rep = kByteRep; p.eps = d->eps;
   int G = 1;
-  while (G * 2 * bpt <= 32 && G * 2 <= bd / kChunk) G *= 2;  // lanes per slot: power of two, at most one lane per chunk
+  while (G * 2 * p.bpt <= 32 && G * 2 <= p.bd / kChunk) G *= 2;  // lanes per slot: power of two, at most one lane per chunk
   p.G = G;
+  if (d->flags & MOT_F_IDS_FROM_TTB)
+    p.ttb = PullSrc{tok, ttb, d->seq_len, d->tok_vocab, d->bpt, d->ttb_dtype, d->pad_id, d->eot_id, 0,
+                    (d->flags & MOT_F_TTB_NEXT_TOK) ? tok + d->n_tokens : nullptr};
+  return p;
 }
 
 }  // namespace mot
 
 using namespace mot;
 
-template <typename P>
-static int pair_fwd(const P& p, int32_t dtype, void* stream) {
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  return dtype == MOT_BF16 ? dispatch_pair<__nv_bfloat16>(p, false, s) : dispatch_pair<float>(p, false, s);
-}
-
-template <typename P>
-static int pair_bwd(P& p, int32_t dtype, void* gE_byte, void* workspace, size_t ws_bytes, void* stream) {
-  if (!gE_byte) return MOT_ERR_BAD_ARG;
-  if (reinterpret_cast<uintptr_t>(gE_byte) & 15u) return MOT_ERR_MISALIGNED;
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  const size_t esz = dtype == MOT_BF16 ? 2 : 4;
-  if (p.N == 0) {  // nothing gathered: dense zero gradient
-    if (cudaMemsetAsync(gE_byte, 0, (size_t)p.Vb * p.bd * esz, s) != cudaSuccess) return check_launch();
-    return MOT_OK;
-  }
-  const size_t need = mot_byte_pair_workspace_bytes(p.Vb, p.bd);
-  if (!workspace || ws_bytes < need) return MOT_ERR_WORKSPACE;
-  if (reinterpret_cast<uintptr_t>(workspace) & 15u) return MOT_ERR_MISALIGNED;
-  if (cudaMemsetAsync(workspace, 0, need, s) != cudaSuccess) return check_launch();
-  p.acc = reinterpret_cast<float*>(workspace);
-  if (int rc = dtype == MOT_BF16 ? dispatch_pair<__nv_bfloat16>(p, true, s) : dispatch_pair<float>(p, true, s)) return rc;
-  // sum the replicas and cast (the norm backward already happened per occurrence: no MOT_F_BYTE_NORM here)
-  EmbedParams q{};
-  q.combine = MOT_BYTES_ONLY;
-  q.N = p.N; q.R = 32; q.Vb = p.Vb; q.bd = p.bd; q.bpt = p.bpt; q.Do = p.bpt * p.bd;
-  q.n_rep = kByteRep; q.byte_acc = p.acc; q.E_byte = p.E_byte; q.gE_byte = gE_byte; q.eps = p.eps;
-  q.last_slab = 1;  // the byte rows are this launch's only work
-  const int fb = (p.Vb + 7) / 8;
-  return dtype == MOT_BF16 ? launch_finalize_bf16(q, fb, s) : launch_finalize_f32(q, fb, s);
-}
-
-// flags: MOT_F_TTB_PULL_LEFT, or MOT_F_TTB_PULL_RIGHT with or without MOT_F_TTB_NEXT_TOK (the tail tok[n + r]).
-static PullSrc pair_pull_src(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype, int64_t seq_len,
-                             int32_t pad_id, int32_t eot_id, int64_t n, int32_t bpt, int32_t flags) {
-  return PullSrc{tok, ttb, seq_len, tok_vocab, bpt, ttb_dtype, pad_id, eot_id, 0,
-                 (flags & MOT_F_TTB_NEXT_TOK) ? tok + n : nullptr};
-}
-static bool pair_pull_flags_ok(int32_t flags) {
-  return flags == MOT_F_TTB_PULL_LEFT || flags == MOT_F_TTB_PULL_RIGHT ||
-         flags == (MOT_F_TTB_PULL_RIGHT | MOT_F_TTB_NEXT_TOK);
-}
-
-extern "C" int mot_byte_pair_fwd(const void* ids_a, const void* ids_b, int32_t ids_i64, int64_t n_tokens, int32_t bpt,
-                                 const void* E_byte, int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps,
-                                 void* out, int64_t row_stride, int32_t col_offset, void* stream) {
-  if (int rc = pair_validate(ids_a, ids_b, n_tokens, bpt, E_byte, byte_vocab, byte_dim, dtype, out, row_stride, col_offset)) return rc;
-  if (n_tokens == 0) return MOT_OK;
-  PairParams p;
-  pair_fill(p, ids_a, ids_b, ids_i64, n_tokens, bpt, E_byte, byte_vocab, byte_dim, eps, row_stride, col_offset);
+extern "C" int mot_byte_pair_fwd(const MotDesc* d, const int32_t* tok, const void* ids_a, const void* ids_b, const void* ttb,
+                                 const void* E_byte, void* out, void* stream) {
+  if (int rc = pair_args(d, tok, ids_a, ids_b, ttb, E_byte, out)) return rc;
+  if (d->n_tokens == 0) return MOT_OK;
+  PairTtbParams p = pair_params(d, tok, ids_a, ids_b, ttb, E_byte);
   p.out = out;
-  return pair_fwd(p, dtype, stream);
+  return run_pair(d, p, false, reinterpret_cast<cudaStream_t>(stream));
 }
 
 extern "C" size_t mot_byte_pair_workspace_bytes(int32_t byte_vocab, int32_t byte_dim) {
@@ -348,50 +321,32 @@ extern "C" size_t mot_byte_pair_workspace_bytes(int32_t byte_vocab, int32_t byte
   return align_up((size_t)kByteRep * byte_vocab * byte_dim * 4, 256);
 }
 
-extern "C" int mot_byte_pair_bwd(const void* ids_a, const void* ids_b, int32_t ids_i64, int64_t n_tokens, int32_t bpt,
-                                 const void* E_byte, int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps,
-                                 const void* grad_out, int64_t row_stride, int32_t col_offset, void* gE_byte,
-                                 void* workspace, size_t ws_bytes, void* stream) {
-  if (int rc = pair_validate(ids_a, ids_b, n_tokens, bpt, E_byte, byte_vocab, byte_dim, dtype, grad_out, row_stride, col_offset))
-    return rc;
-  PairParams p;
-  pair_fill(p, ids_a, ids_b, ids_i64, n_tokens, bpt, E_byte, byte_vocab, byte_dim, eps, row_stride, col_offset);
+extern "C" int mot_byte_pair_bwd(const MotDesc* d, const int32_t* tok, const void* ids_a, const void* ids_b, const void* ttb,
+                                 const void* E_byte, const void* grad_out, void* gE_byte, void* workspace, size_t ws_bytes,
+                                 void* stream) {
+  if (int rc = pair_args(d, tok, ids_a, ids_b, ttb, E_byte, grad_out)) return rc;
+  if (!gE_byte) return MOT_ERR_BAD_ARG;
+  if (reinterpret_cast<uintptr_t>(gE_byte) & 15u) return MOT_ERR_MISALIGNED;
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  const size_t esz = d->dtype == MOT_BF16 ? 2 : 4;
+  if (d->n_tokens == 0) {  // nothing gathered: dense zero gradient
+    if (cudaMemsetAsync(gE_byte, 0, (size_t)d->byte_vocab * d->byte_dim * esz, s) != cudaSuccess) return check_launch();
+    return MOT_OK;
+  }
+  const size_t need = mot_byte_pair_workspace_bytes(d->byte_vocab, d->byte_dim);
+  if (!workspace || ws_bytes < need) return MOT_ERR_WORKSPACE;
+  if (reinterpret_cast<uintptr_t>(workspace) & 15u) return MOT_ERR_MISALIGNED;
+  if (cudaMemsetAsync(workspace, 0, need, s) != cudaSuccess) return check_launch();
+  PairTtbParams p = pair_params(d, tok, ids_a, ids_b, ttb, E_byte);
   p.gout = grad_out;
-  return pair_bwd(p, dtype, gE_byte, workspace, ws_bytes, stream);
-}
-
-// The id tensors' null checks of pair_validate do not apply here: a non-null placeholder stands in for them.
-extern "C" int mot_byte_pair_ttb_fwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype,
-                                     int64_t seq_len, int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt,
-                                     const void* E_byte, int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps,
-                                     void* out, int64_t row_stride, int32_t col_offset, int32_t flags, void* stream) {
-  if (!pair_pull_flags_ok(flags)) return MOT_ERR_BAD_ARG;
-  if (int rc = pair_ttb_validate(tok, ttb, tok_vocab, ttb_dtype, seq_len, n_tokens)) return rc;
-  if (int rc = pair_validate(tok, tok, n_tokens, bpt, E_byte, byte_vocab, byte_dim, dtype, out, row_stride, col_offset)) return rc;
-  if (n_tokens == 0) return MOT_OK;
-  const auto run = [&](auto p) {
-    pair_fill(p, nullptr, nullptr, 0, n_tokens, bpt, E_byte, byte_vocab, byte_dim, eps, row_stride, col_offset);
-    p.ttb = pair_pull_src(tok, ttb, tok_vocab, ttb_dtype, seq_len, pad_id, eot_id, n_tokens, bpt, flags);
-    p.out = out;
-    return pair_fwd(p, dtype, stream);
-  };
-  return (flags & MOT_F_TTB_PULL_RIGHT) ? run(PairTtbRightParams{}) : run(PairTtbParams{});
-}
-
-extern "C" int mot_byte_pair_ttb_bwd(const int32_t* tok, const void* ttb, int32_t tok_vocab, int32_t ttb_dtype,
-                                     int64_t seq_len, int32_t pad_id, int32_t eot_id, int64_t n_tokens, int32_t bpt,
-                                     const void* E_byte, int32_t byte_vocab, int32_t byte_dim, int32_t dtype, float eps,
-                                     const void* grad_out, int64_t row_stride, int32_t col_offset, void* gE_byte,
-                                     void* workspace, size_t ws_bytes, int32_t flags, void* stream) {
-  if (!pair_pull_flags_ok(flags)) return MOT_ERR_BAD_ARG;
-  if (int rc = pair_ttb_validate(tok, ttb, tok_vocab, ttb_dtype, seq_len, n_tokens)) return rc;
-  if (int rc = pair_validate(tok, tok, n_tokens, bpt, E_byte, byte_vocab, byte_dim, dtype, grad_out, row_stride, col_offset))
-    return rc;
-  const auto run = [&](auto p) {
-    pair_fill(p, nullptr, nullptr, 0, n_tokens, bpt, E_byte, byte_vocab, byte_dim, eps, row_stride, col_offset);
-    p.ttb = pair_pull_src(tok, ttb, tok_vocab, ttb_dtype, seq_len, pad_id, eot_id, n_tokens, bpt, flags);
-    p.gout = grad_out;
-    return pair_bwd(p, dtype, gE_byte, workspace, ws_bytes, stream);
-  };
-  return (flags & MOT_F_TTB_PULL_RIGHT) ? run(PairTtbRightParams{}) : run(PairTtbParams{});
+  p.acc = reinterpret_cast<float*>(workspace);
+  if (int rc = run_pair(d, p, true, s)) return rc;
+  // sum the replicas and cast (the norm backward already happened per occurrence: no MOT_F_BYTE_NORM here)
+  EmbedParams q{};
+  q.combine = MOT_BYTES_ONLY;
+  q.N = p.N; q.R = 32; q.Vb = p.Vb; q.bd = p.bd; q.bpt = p.bpt; q.Do = p.bpt * p.bd;
+  q.n_rep = kByteRep; q.byte_acc = p.acc; q.E_byte = p.E_byte; q.gE_byte = gE_byte; q.eps = p.eps;
+  q.last_slab = 1;  // the byte rows are this launch's only work
+  const int fb = (p.Vb + 7) / 8;
+  return d->dtype == MOT_BF16 ? launch_finalize_bf16(q, fb, s) : launch_finalize_f32(q, fb, s);
 }

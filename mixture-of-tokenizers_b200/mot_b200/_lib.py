@@ -13,7 +13,7 @@ import sys
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmot_b200" + os.environ.get("MOT_LIB_SUFFIX", "") + ".so")  # suffix: experiment builds
 
-ABI_VERSION = 6
+ABI_VERSION = 7
 # enums of include/mot_b200.h
 OK, ERR_BAD_ARG, ERR_UNSUPPORTED, ERR_MISALIGNED, ERR_WORKSPACE, ERR_CUDA, ERR_NO_DEVICE = range(7)
 BF16, F32 = 0, 1
@@ -68,17 +68,9 @@ _SIGNATURES = {
     "mot_embed_slab_rows": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "mot_tokens_widen_u16": (C.c_int, [_P, C.c_int64, _P, _P]),
     "mot_embed_bwd_uses_saved": (C.c_int, [C.POINTER(MotDesc)]),
-    "mot_byte_pair_fwd": (C.c_int, [_P, _P, C.c_int32, C.c_int64, C.c_int32, _P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P,
-                                    C.c_int64, C.c_int32, _P]),
+    "mot_byte_pair_fwd": (C.c_int, [C.POINTER(MotDesc), _P, _P, _P, _P, _P, _P, _P]),
     "mot_byte_pair_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32]),
-    "mot_byte_pair_bwd": (C.c_int, [_P, _P, C.c_int32, C.c_int64, C.c_int32, _P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P,
-                                    C.c_int64, C.c_int32, _P, _P, C.c_size_t, _P]),
-    "mot_byte_pair_ttb_fwd": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int32,
-                                        _P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, C.c_int64, C.c_int32, C.c_int32,
-                                        _P]),
-    "mot_byte_pair_ttb_bwd": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int32,
-                                        _P, C.c_int32, C.c_int32, C.c_int32, C.c_float, _P, C.c_int64, C.c_int32, _P, _P,
-                                        C.c_size_t, C.c_int32, _P]),
+    "mot_byte_pair_bwd": (C.c_int, [C.POINTER(MotDesc), _P, _P, _P, _P, _P, _P, _P, _P, C.c_size_t, _P]),
     "mot_dp_exchange": (C.c_int, [_P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int64, C.c_int64, C.c_int32, C.c_uint32, C.c_int32,
                                   C.c_int32, _P]),
     "mot_embed_touched_rows": (C.c_int, [C.POINTER(MotDesc), _P, C.c_size_t, _P, _P]),

@@ -186,11 +186,9 @@ def pull_from_right(byte_tensor: torch.Tensor, bytes_per_token: int, pad_byte: i
 PAD_ID, EOT_ID = 456, 457   # pad and end-of-text byte of the ttb tables (spt/data_creation.py; pull_from_left's defaults)
 
 
-def _pull_flags(spec: MixSpec, next_tok: bool) -> int:
-    """MOT_F_TTB_PULL_LEFT / _RIGHT (+ MOT_F_TTB_NEXT_TOK: the lookahead tail after the token ids) of spec.ttb_pull."""
-    if not spec.ttb_pull:
-        return 0
-    if spec.ttb_pull_side == "left":
+def _pull_flags(side: str, next_tok: bool) -> int:
+    """MOT_F_TTB_PULL_LEFT / _RIGHT (+ MOT_F_TTB_NEXT_TOK: the lookahead tail after the token ids) of a pull from `side`."""
+    if side == "left":
         return L.F_TTB_PULL_LEFT
     return L.F_TTB_PULL_RIGHT | (L.F_TTB_NEXT_TOK if next_tok else 0)
 
@@ -224,7 +222,7 @@ def make_desc(spec: MixSpec, n_tokens: int, E_tok, E_byte, bpt: int, *, ids: Opt
         if ids is None:
             flags |= L.F_IDS_FROM_TTB
             flags |= L.F_TTB_SCRAMBLE if spec.ttb_scramble else 0
-            flags |= _pull_flags(spec, next_tok)
+            flags |= _pull_flags(spec.ttb_pull_side, next_tok) if spec.ttb_pull else 0
             ttb_dtype = _TTB_DTYPE[ttb.dtype]
         else:
             flags |= L.F_SLOT_MAJOR if spec.slot_major else 0
@@ -805,58 +803,56 @@ def rmsnorm_backward_out(y, grad_out, dy, eps: float = FP32_EPS) -> None:
     L.check(rc, "mot_rmsnorm_bwd")
 
 
-def byte_pair_forward_out(ids_a, ids_b, bpt: int, E_byte, out, col_offset: int, eps: float = FP32_EPS) -> None:
-    """mot_byte_pair_fwd: out[:, col_offset + k*bd : +bd] = rms_norm(E_byte[ids_a[:, k]] + E_byte[ids_b[:, k]])
-    (spt/train_gpt.py:371-379), written into the byte columns of the [n, K] operand `out`."""
-    dev = _require_cuda(ids_a, ids_b, E_byte, out)
+def _pair_desc(n: int, bpt: int, E_byte, row_stride: int, col_offset: int, eps: float, *, ids=None, ttb=None,
+               seq_len: int = 0, pull_side: str = "left", next_tok: bool = False) -> L.MotDesc:
+    """The descriptor of the padded+pulled byte pair (mot_byte_pair_fwd/bwd): bytes-only with the per-byte norm, written
+    into the columns [col_offset, col_offset + bpt*bd) of rows of row_stride elements.  Explicit `ids` (their dtype gives
+    the width), else both id sets derived from `ttb` over rows of seq_len tokens with a pull from pull_side.  Built
+    directly rather than through make_desc: the eager step calls it twice, and its host time adds to the step."""
+    flags, tok_vocab, ttb_dtype = L.F_BYTE_NORM, 0, 0
+    if ids is not None:
+        flags |= L.F_IDS_I64 if ids.dtype == torch.int64 else 0
+    else:
+        flags |= L.F_IDS_FROM_TTB | _pull_flags(pull_side, next_tok)
+        tok_vocab, ttb_dtype = ttb.shape[0], _TTB_DTYPE[ttb.dtype]
+    Vb, bd = E_byte.shape
+    return L.MotDesc(L.ABI_VERSION, _DTYPE[E_byte.dtype], n, seq_len, tok_vocab, Vb, bpt, 0, bd, bpt * bd, L.BYTES_ONLY, flags,
+                     ttb_dtype, eps, row_stride, col_offset, 0, PAD_ID, EOT_ID)
+
+
+def pair_forward_out(desc: L.MotDesc, tok, ids_a, ids_b, ttb, E_byte, out) -> None:
+    """mot_byte_pair_fwd: out[:, col + k*bd : +bd] = rms_norm(E_byte[a[:, k]] + E_byte[b[:, k]]) (spt/train_gpt.py:371-379)
+    in the byte columns that desc (_pair_desc) locates; (a, b) = (ids_a, ids_b), or the padded and the pulled ids of
+    `tok` derived from `ttb` inside the kernel."""
+    dev = _require_cuda(tok, ids_a, ids_b, ttb, E_byte, out)
     with _on_device(dev):
-        rc = L.lib().mot_byte_pair_fwd(_ptr(ids_a), _ptr(ids_b), 1 if ids_a.dtype == torch.int64 else 0, out.shape[0], bpt,
-                                       _ptr(E_byte), E_byte.shape[0], E_byte.shape[1], _DTYPE[E_byte.dtype], eps,
-                                       _ptr(out), out.stride(0), col_offset, _stream(dev))
+        rc = L.lib().mot_byte_pair_fwd(desc, _ptr(tok), _ptr(ids_a), _ptr(ids_b), _ptr(ttb), _ptr(E_byte), _ptr(out),
+                                       _stream(dev))
     L.check(rc, "mot_byte_pair_fwd")
 
 
-def byte_pair_backward_out(ids_a, ids_b, bpt: int, E_byte, grad_rows, col_offset: int, gE_byte, eps: float = FP32_EPS) -> None:
-    """mot_byte_pair_bwd: dense gE_byte from the byte columns of grad_rows [n, K]."""
-    dev = _require_cuda(ids_a, ids_b, E_byte, grad_rows, gE_byte)
-    need = int(L.lib().mot_byte_pair_workspace_bytes(E_byte.shape[0], E_byte.shape[1]))
-    ws = torch.empty(need, dtype=torch.uint8, device=dev)
+def pair_backward_out(desc: L.MotDesc, tok, ids_a, ids_b, ttb, E_byte, grad_rows, gE_byte) -> None:
+    """mot_byte_pair_bwd: dense gE_byte from the byte columns of grad_rows that desc locates."""
+    dev = _require_cuda(tok, ids_a, ids_b, ttb, E_byte, grad_rows, gE_byte)
+    ws = torch.empty(int(L.lib().mot_byte_pair_workspace_bytes(desc.byte_vocab, desc.byte_dim)), dtype=torch.uint8,
+                     device=dev)
     with _on_device(dev):
-        rc = L.lib().mot_byte_pair_bwd(_ptr(ids_a), _ptr(ids_b), 1 if ids_a.dtype == torch.int64 else 0, grad_rows.shape[0],
-                                       bpt, _ptr(E_byte), E_byte.shape[0], E_byte.shape[1], _DTYPE[E_byte.dtype], eps,
-                                       _ptr(grad_rows), grad_rows.stride(0), col_offset, _ptr(gE_byte), _ptr(ws),
-                                       ws.numel(), _stream(dev))
+        rc = L.lib().mot_byte_pair_bwd(desc, _ptr(tok), _ptr(ids_a), _ptr(ids_b), _ptr(ttb), _ptr(E_byte), _ptr(grad_rows),
+                                       _ptr(gE_byte), _ptr(ws), ws.numel(), _stream(dev))
     L.check(rc, "mot_byte_pair_bwd")
 
 
-_PAIR_PULL = L.F_TTB_PULL_LEFT | L.F_TTB_PULL_RIGHT | L.F_TTB_NEXT_TOK
+def byte_pair_forward_out(ids_a, ids_b, bpt: int, E_byte, out, col_offset: int, eps: float = FP32_EPS) -> None:
+    """pair_forward_out with explicit ids into the byte columns [col_offset, col_offset + bpt*bd) of the [n, K] operand
+    `out`."""
+    desc = _pair_desc(out.shape[0], bpt, E_byte, out.stride(0), col_offset, eps, ids=ids_a)
+    pair_forward_out(desc, None, ids_a, ids_b, None, E_byte, out)
 
 
-def byte_pair_ttb_forward_out(desc: L.MotDesc, tok, ttb, E_byte, out) -> None:
-    """mot_byte_pair_ttb_fwd: byte_pair_forward_out with ids_a = the padded and ids_b = the pulled ids of `tok`, both
-    derived from the ttb table inside the kernel.  desc: the bytes-only descriptor of the pair (_proj_descs), which holds
-    the rows of seq_len tokens, the pull flags and the byte columns of `out` (row_stride, col_offset)."""
-    dev = _require_cuda(tok, ttb, E_byte, out)
-    with _on_device(dev):
-        rc = L.lib().mot_byte_pair_ttb_fwd(_ptr(tok), _ptr(ttb), desc.tok_vocab, desc.ttb_dtype, desc.seq_len, desc.pad_id,
-                                           desc.eot_id, desc.n_tokens, desc.bpt, _ptr(E_byte), desc.byte_vocab,
-                                           desc.byte_dim, desc.dtype, desc.eps, _ptr(out), desc.row_stride,
-                                           desc.col_offset, desc.flags & _PAIR_PULL, _stream(dev))
-    L.check(rc, "mot_byte_pair_ttb_fwd")
-
-
-def byte_pair_ttb_backward_out(desc: L.MotDesc, tok, ttb, E_byte, grad_rows, gE_byte) -> None:
-    """mot_byte_pair_ttb_bwd: byte_pair_backward_out with both id sets derived from `tok` and the ttb table."""
-    dev = _require_cuda(tok, ttb, E_byte, grad_rows, gE_byte)
-    need = int(L.lib().mot_byte_pair_workspace_bytes(desc.byte_vocab, desc.byte_dim))
-    ws = torch.empty(need, dtype=torch.uint8, device=dev)
-    with _on_device(dev):
-        rc = L.lib().mot_byte_pair_ttb_bwd(_ptr(tok), _ptr(ttb), desc.tok_vocab, desc.ttb_dtype, desc.seq_len, desc.pad_id,
-                                           desc.eot_id, desc.n_tokens, desc.bpt, _ptr(E_byte), desc.byte_vocab,
-                                           desc.byte_dim, desc.dtype, desc.eps, _ptr(grad_rows), desc.row_stride,
-                                           desc.col_offset, _ptr(gE_byte), _ptr(ws), ws.numel(), desc.flags & _PAIR_PULL,
-                                           _stream(dev))
-    L.check(rc, "mot_byte_pair_ttb_bwd")
+def byte_pair_backward_out(ids_a, ids_b, bpt: int, E_byte, grad_rows, col_offset: int, gE_byte, eps: float = FP32_EPS) -> None:
+    """pair_backward_out with explicit ids: dense gE_byte from the byte columns of grad_rows [n, K]."""
+    desc = _pair_desc(grad_rows.shape[0], bpt, E_byte, grad_rows.stride(0), col_offset, eps, ids=ids_a)
+    pair_backward_out(desc, None, ids_a, ids_b, None, E_byte, grad_rows, gE_byte)
 
 
 def cast_out(w: torch.Tensor, dtype: torch.dtype) -> torch.Tensor:
@@ -962,9 +958,9 @@ def _proj_descs(spec: MixSpec, bpt: int, seq_len: int, tok, next_tok, ids, ids2,
                               ids, ttb, E_tok, E_byte)
         return tok, desc, None
     K = E_tok.shape[1] + bpt * E_byte.shape[1]
-    tok, desc_pair = _ids_desc(MixSpec(combine="bytes_only", byte_norm=True, out_norm=False, ttb_pull=True,
-                                       ttb_pull_side=spec.ttb_pull_side, eps=spec.eps),
-                               bpt, seq_len, tok, next_tok, ids, ttb, None, E_byte, row_stride=K, col_offset=E_tok.shape[1])
+    tok = _tok_next(tok, next_tok)
+    desc_pair = _pair_desc(tok.numel(), bpt, E_byte, K, E_tok.shape[1], spec.eps, ids=ids, ttb=ttb, seq_len=seq_len,
+                           pull_side=spec.ttb_pull_side, next_tok=next_tok is not None)
     desc = make_desc(MixSpec(combine="tok_only", tok_norm=spec.tok_norm, out_norm=False, eps=spec.eps), tok.numel(),
                      E_tok, None, 0, ids=None, ttb=None, has_lam=False, row_stride=K, col_offset=0)
     return tok, desc, desc_pair
@@ -975,10 +971,7 @@ def _gather_operand(desc: L.MotDesc, desc_pair: Optional[L.MotDesc], tok, ids, i
         embed_forward_out(desc, tok, ids, ttb, E_tok, E_byte, None, A)
     elif tok.numel() > 0:
         embed_forward_out(desc, tok, None, None, E_tok, None, None, A)
-        if ttb is not None:
-            byte_pair_ttb_forward_out(desc_pair, tok, ttb, E_byte, A)
-        else:
-            byte_pair_forward_out(ids, ids2, desc_pair.bpt, E_byte, A, desc_pair.col_offset, desc_pair.eps)
+        pair_forward_out(desc_pair, tok, ids, ids2, ttb, E_byte, A)
 
 
 def _scatter_operand(desc: L.MotDesc, desc_pair: Optional[L.MotDesc], tok, ids, ids2, ttb, E_tok, E_byte, dA, ws_buf,
@@ -991,10 +984,7 @@ def _scatter_operand(desc: L.MotDesc, desc_pair: Optional[L.MotDesc], tok, ids, 
     else:   # token columns through the sorted-stream scatter, byte columns through the pair kernel
         embed_backward_out(desc, tok, None, None, E_tok, None, None, dA, gE_tok, None, None, ws_buf,
                            plan_ready=plan_ready, ws_clean=ws_clean)
-        if ttb is not None:
-            byte_pair_ttb_backward_out(desc_pair, tok, ttb, E_byte, dA, gE_byte)
-        else:
-            byte_pair_backward_out(ids, ids2, desc_pair.bpt, E_byte, dA, desc_pair.col_offset, gE_byte, desc_pair.eps)
+        pair_backward_out(desc_pair, tok, ids, ids2, ttb, E_byte, dA, gE_byte)
     return gE_tok, gE_byte
 
 

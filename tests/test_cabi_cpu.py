@@ -55,14 +55,14 @@ def desc(**kw):
     return L.MotDesc(**base)
 
 
-def test_workspace_sizes_and_validation():
+def test_workspace_sizes_and_validation_v7():
     lib = L.lib()
     ws = lib.mot_embed_workspace_bytes(desc())
     assert 0 < ws < 64 << 20 and ws % 256 == 0
     assert lib.mot_embed_workspace_bytes(desc(n_tokens=1 << 20, tok_dim=1024, byte_dim=64, out_dim=1024)) < 256 << 20
     # inconsistent dims -> 0 bytes / error codes, all before any CUDA call
     assert lib.mot_embed_workspace_bytes(desc(out_dim=1024)) == 0
-    assert lib.mot_embed_workspace_bytes(desc(abi_version=7)) == 0
+    assert lib.mot_embed_workspace_bytes(desc(abi_version=L.ABI_VERSION + 1)) == 0
     null = None
     assert lib.mot_embed_fwd(desc(out_dim=1024), null, null, null, null, null, null, null, null) == L.ERR_BAD_ARG
     assert lib.mot_embed_fwd(desc(byte_dim=44, tok_dim=704, out_dim=704), null, null, null, null, null, null, null, null) == L.ERR_MISALIGNED
@@ -142,16 +142,17 @@ def test_saved_backward_query_needs_no_device():
     assert lib.mot_embed_bwd_uses_saved(desc(abi_version=9)) == 0
 
 
-def test_new_entry_points_validate_before_touching_the_device():
+def test_new_entry_points_validate_descriptors_before_touching_the_device():
     lib = L.lib()
     null = None
     # byte-pair kernels (spt/train_gpt.py:371-379): sizes, alignment and dtype are checked first
-    args = dict(ids_i64=1, n=4, bpt=16, Vb=458, bd=48, dtype=L.BF16, eps=1e-7, ld=256 + 16 * 48, col=256)
+    def pair_desc(n=4, bpt=16, bd=48, dtype=L.BF16, ld=256 + 16 * 48, col=256):
+        return L.MotDesc(abi_version=L.ABI_VERSION, dtype=dtype, n_tokens=n, byte_vocab=458, bpt=bpt, byte_dim=bd,
+                         out_dim=bpt * bd, combine=L.BYTES_ONLY, flags=L.F_BYTE_NORM | L.F_IDS_I64, eps=1e-7,
+                         row_stride=ld, col_offset=col)
 
     def pair_fwd(**kw):
-        a = {**args, **kw}
-        return lib.mot_byte_pair_fwd(null, null, a["ids_i64"], a["n"], a["bpt"], null, a["Vb"], a["bd"], a["dtype"], a["eps"], null,
-                                     a["ld"], a["col"], null)
+        return lib.mot_byte_pair_fwd(pair_desc(**kw), null, null, null, null, null, null, null)
     assert pair_fwd() == L.ERR_BAD_ARG                       # null pointers
     assert pair_fwd(n=0) == L.OK                             # empty batch: nothing to do
     assert pair_fwd(bd=44) == L.ERR_MISALIGNED
@@ -160,7 +161,7 @@ def test_new_entry_points_validate_before_touching_the_device():
     assert pair_fwd(bpt=33) == L.ERR_BAD_ARG
     assert pair_fwd(dtype=7) == L.ERR_UNSUPPORTED
     assert lib.mot_byte_pair_workspace_bytes(458, 48) == 16 * 458 * 48 * 4 and lib.mot_byte_pair_workspace_bytes(0, 48) == 0
-    assert lib.mot_byte_pair_bwd(null, null, 1, 4, 16, null, 458, 48, L.BF16, 1e-7, null, 1024, 256, null, null, 0, null) == L.ERR_BAD_ARG
+    assert lib.mot_byte_pair_bwd(pair_desc(), null, null, null, null, null, null, null, null, 0, null) == L.ERR_BAD_ARG
     # uint16 -> int32 widening of shard tokens
     assert lib.mot_tokens_widen_u16(null, 0, null, null) == L.OK
     assert lib.mot_tokens_widen_u16(null, 8, null, null) == L.ERR_BAD_ARG

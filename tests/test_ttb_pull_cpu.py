@@ -22,12 +22,12 @@ def _desc(side="left", **kw):
     return L.MotDesc(**base)
 
 
-def test_flag_and_abi():
-    assert L.ABI_VERSION == 6 and L.lib().mot_abi_version() == 6
+def test_flag_and_abi_v7():
+    assert L.ABI_VERSION == 7 and L.lib().mot_abi_version() == 7
     assert L.F_TTB_PULL_LEFT == 1 << 9
     names = [f[0] for f in L.MotDesc._fields_]
     assert names[-2:] == ["pad_id", "eot_id"]
-    for fn in ("mot_byte_pair_ttb_fwd", "mot_byte_pair_ttb_bwd"):
+    for fn in ("mot_byte_pair_fwd", "mot_byte_pair_bwd"):
         assert hasattr(L.lib(), fn)
 
 

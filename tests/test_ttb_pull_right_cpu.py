@@ -14,11 +14,12 @@ from mot_b200._library import pack_spec, unpack_spec
 from test_ttb_pull_cpu import BD, BPT, N, R, S, V, VB, _desc, _t, check_fake_shapes
 
 
-def test_flag_values_and_symbols():
+def test_flag_values_and_descriptor_symbols():
     assert L.F_TTB_PULL_RIGHT == 1 << 10 and L.F_TTB_NEXT_TOK == 1 << 11
-    assert L.ABI_VERSION == 6 and L.lib().mot_abi_version() == 6
-    for fn in ("mot_byte_pair_ttb_fwd", "mot_byte_pair_ttb_bwd"):   # the direction is their `flags` argument
-        assert hasattr(L.lib(), fn) and L._SIGNATURES[fn][1][-2] is L.C.c_int32
+    assert L.ABI_VERSION == 7 and L.lib().mot_abi_version() == 7
+    for fn in ("mot_byte_pair_fwd", "mot_byte_pair_bwd"):   # the direction is a flag of their descriptor
+        assert hasattr(L.lib(), fn) and L._SIGNATURES[fn][1][0] is L.C.POINTER(L.MotDesc)
+    assert not hasattr(L.lib(), "mot_byte_pair_ttb_fwd") and not hasattr(L.lib(), "mot_byte_pair_ttb_bwd")
 
 
 def test_validation_of_the_right_pull_flags():
@@ -35,14 +36,36 @@ def test_validation_of_the_right_pull_flags():
     assert ws(_desc("right", bpt=33, tok_dim=33 * 8, byte_dim=8, out_dim=33 * 8)) == 0
 
 
-def test_pair_ex_refuses_bad_flags():
-    # checked before anything else: no pointer is dereferenced, no device is needed
-    args = (None, None, 100, L.TTB_I16, 16, 456, 457, 64, 4, None, 458, 16, L.BF16, 1e-7)
-    fwd, bwd = L.lib().mot_byte_pair_ttb_fwd, L.lib().mot_byte_pair_ttb_bwd
-    for flags in (0, L.F_TTB_PULL_LEFT | L.F_TTB_PULL_RIGHT, L.F_TTB_PULL_LEFT | L.F_TTB_NEXT_TOK, L.F_TTB_NEXT_TOK,
-                  L.F_TTB_PULL_RIGHT | L.F_TTB_SCRAMBLE):
-        assert fwd(*args, None, 64, 0, flags, None) == L.ERR_BAD_ARG
-        assert bwd(*args, None, 64, 0, None, None, 0, flags, None) == L.ERR_BAD_ARG
+def _pair_desc(flags, **kw):
+    """A pair descriptor (bytes-only, per-byte norm, derived ids' fields set) with no positions; fields overridden by kw."""
+    base = dict(abi_version=L.ABI_VERSION, dtype=L.BF16, n_tokens=0, seq_len=16, tok_vocab=100, byte_vocab=458, bpt=4,
+                byte_dim=16, out_dim=64, combine=L.BYTES_ONLY, flags=flags, ttb_dtype=L.TTB_I16, eps=1e-7, row_stride=64,
+                pad_id=456, eot_id=457)
+    base.update(kw)
+    return L.MotDesc(**base)
+
+
+def test_pair_descriptor_refuses_bad_flags():
+    # checked before anything else: no pointer is dereferenced, no device is needed (no positions: accepted is MOT_OK)
+    fwd, bwd = L.lib().mot_byte_pair_fwd, L.lib().mot_byte_pair_bwd
+    norm, ttb = L.F_BYTE_NORM, L.F_BYTE_NORM | L.F_IDS_FROM_TTB
+    left, right, nxt = L.F_TTB_PULL_LEFT, L.F_TTB_PULL_RIGHT, L.F_TTB_NEXT_TOK
+    good = (norm, norm | L.F_IDS_I64, ttb | left, ttb | right, ttb | right | nxt)
+    for flags in good:
+        assert fwd(_pair_desc(flags), *[None] * 7) == L.OK
+    bad = [ttb | f for f in (0, left | right, left | nxt, nxt, right | L.F_TTB_SCRAMBLE)]   # the former `flags` argument
+    bad += [f | extra for f in good for extra in (L.F_TOK_NORM, L.F_OUT_NORM, L.F_BYTES_FIRST, L.F_SLOT_MAJOR,
+                                                  L.F_HAS_LAMBDAS, L.F_TTB_SCRAMBLE)]
+    bad += [norm | f for f in (left, right, right | nxt, nxt)]   # pulls without derived ids
+    bad += [f & ~L.F_BYTE_NORM for f in good] + [ttb | left | L.F_IDS_I64]
+    for flags in bad:
+        assert fwd(_pair_desc(flags), *[None] * 7) == L.ERR_BAD_ARG, hex(flags)
+        assert bwd(_pair_desc(flags), *[None] * 8, 0, None) == L.ERR_BAD_ARG, hex(flags)
+    # another combine, with a descriptor the fused kernels accept
+    for combine, tok_dim, out_dim in ((L.ADD, 64, 64), (L.CONCAT, 64, 128), (L.TOK_ONLY, 64, 64), (L.MEAN, 16, 16)):
+        d = _pair_desc(ttb | left, combine=combine, tok_dim=tok_dim, out_dim=out_dim, row_stride=out_dim)
+        assert L.lib().mot_embed_workspace_bytes(d) > 0
+        assert fwd(d, *[None] * 7) == L.ERR_BAD_ARG and bwd(d, *[None] * 8, 0, None) == L.ERR_BAD_ARG
 
 
 def test_make_desc_sets_the_right_flags():

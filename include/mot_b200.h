@@ -305,6 +305,26 @@ int mot_dp_exchange_rows(void* multicast_ptr, void* const* peer_ptrs_dev, void* 
                          int32_t rank, int32_t world, int64_t table_byte_offset, int32_t n_rows, int32_t row_bytes,
                          int64_t bitmap_byte_offset, int64_t dense_byte_offset, int64_t dense_bytes, int32_t dtype,
                          uint32_t epoch, int32_t algo, void* stream);
+/* Touched-rows exchange of several row tables.  Tables gathered with the same token ids (the front's token table and
+ * the value embeddings, runs/7:252,308) touch the same rows, so ONE bitmap describes them all; the kernel moves row v of
+ * every table for each row v of the union.  Tables may differ in width. */
+#define MOT_DP_MAX_ROW_TABLES 8
+typedef struct MotRowTable {
+  int64_t byte_offset;  /* row 0 of the table in the bucket */
+  int32_t row_bytes;
+  int32_t reserved;     /* 0 */
+} MotRowTable;
+/* mot_dp_exchange_rows for n_tables row tables of n_rows rows each, all indexed by the token ids the bitmap describes.
+ * `tables` is a HOST array read during the call.  Offsets and row_bytes are multiples of 16; the tables, the bitmap and
+ * the dense range must not overlap.  mot_dp_exchange_rows is this call with one table (same bits, same summation
+ * order).  Precondition as above, for every table: a row whose bit is clear in a rank's bitmap is all zeros in every
+ * table of that rank's copy.  Errors, all before any CUDA call: n_tables outside 1..MOT_DP_MAX_ROW_TABLES, a NULL
+ * `tables`, a nonzero `reserved` or overlapping ranges -> MOT_ERR_BAD_ARG; misaligned offsets or widths ->
+ * MOT_ERR_MISALIGNED; MOT_DP_P2P at a world other than 2 or 4 -> MOT_ERR_UNSUPPORTED. */
+int mot_dp_exchange_rows_multi(void* multicast_ptr, void* const* peer_ptrs_dev, void* const* signal_pads_dev,
+                               void* work_area, int32_t rank, int32_t world, const MotRowTable* tables, int32_t n_tables,
+                               int32_t n_rows, int64_t bitmap_byte_offset, int64_t dense_byte_offset, int64_t dense_bytes,
+                               int32_t dtype, uint32_t epoch, int32_t algo, void* stream);
 /* The whole bucket as one NVLS range with both barriers (= mot_dp_exchange(..., 0, n_bytes, ..., last = 1, MOT_DP_NVLS)):
  * `epoch` grows by 2 per call. */
 int mot_dp_allreduce_avg(void* multicast_ptr, void* const* signal_pads_dev, void* work_area, int32_t rank, int32_t world,

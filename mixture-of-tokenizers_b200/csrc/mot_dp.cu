@@ -224,13 +224,38 @@ static void launch_p2p(int unroll, dim3 g, dim3 b, cudaStream_t s, char* const* 
 // tokens touch 62 % of the vocabulary per rank (union 86 % at 2 ranks, ~100 % from 4 ranks on: no gain there); Zipf /
 // real text touches 20-30 % per rank.  Work unit: 64 rows (two bitmap words), handed out by the tile counter; a warp owns a
 // row, its lanes the row's 16-byte vectors.
+//
+// Several tables indexed by the same token ids (the front's token table and the value embeddings, runs/7:252,308) share
+// one bitmap: row v of every table is touched exactly when token v was gathered.  A warp moves row v of ALL tables, one
+// table after the other, with the same rows in flight.
 constexpr int kRowsPerTile = 64;
-constexpr int kMaxVecPerLane = 4;
-constexpr int kMaxRowWords = 2048; // bitmap words of one rank's rows held in shared memory (65536 rows per rank)   // rows up to 32 x 4 x 16 = 2048 bytes in one trip; wider rows loop
+constexpr int kMaxVecPerLane = 4;  // rows up to 32 x 4 x 16 = 2048 bytes in one trip; wider rows loop
+constexpr int kMaxRowWords = 2048; // bitmap words of one rank's rows held in shared memory (65536 rows per rank)
 
-template <bool BF16, bool NVLS, int WORLD>
+struct RowTables {                          // a kernel parameter: no device array, no copy
+  long long vec_off[MOT_DP_MAX_ROW_TABLES];  // bucket vector (16 bytes) of row 0 of table t
+  int row_vecs[MOT_DP_MAX_ROW_TABLES];       // vectors per row of table t
+  int n;
+};
+
+// Table t of the parameter struct, selected with compile-time indices (a run-time index would copy the struct to local
+// memory).  NT = the compile-time bound of the table count: NT = 1 is the one-table exchange, compiled to the code
+// (addresses, summation order, registers) of the single-table kernel it replaced.
+template <int NT>
+__device__ __forceinline__ void row_table(const RowTables& T, int t, long long& vec_off, int& row_vecs) {
+  vec_off = T.vec_off[0];
+  row_vecs = T.row_vecs[0];
+#pragma unroll
+  for (int k = 1; k < NT; ++k)
+    if (k == t) {
+      vec_off = T.vec_off[k];
+      row_vecs = T.row_vecs[k];
+    }
+}
+
+template <bool BF16, bool NVLS, int WORLD, int NT>
 __global__ void __launch_bounds__(NVLS ? 1024 : 512) rows_allreduce_avg_kernel(char* mc, char* const* peers, uint32_t* const* pads, int rank, int world,
-                                                                 long long tab_off, int n_rows, int row_vecs, long long bm_off,
+                                                                 const RowTables T, int n_rows, long long bm_off,
                                                                  long long dense_vec_lo, long long dense_vecs, uint32_t epoch,
                                                                  unsigned* work, int peer_bits, long long* trace) {
   pdl_launch_dependents();
@@ -285,7 +310,7 @@ __global__ void __launch_bounds__(NVLS ? 1024 : 512) rows_allreduce_avg_kernel(c
     // version ran at 250 GB/s)
     constexpr int RPW = NVLS ? 2 : (WORLD <= 2 ? 2 : 1);
     for (int rr0 = warp; rr0 < kRowsPerTile; rr0 += nw * RPW) {
-      long long vrow[RPW];
+      long long rows[RPW];
       bool act[RPW];
       uint32_t has[RPW];  // peer-to-peer: bit q = rank q gathered the row (its copy is read), else its copy is zeros
 #pragma unroll
@@ -293,7 +318,7 @@ __global__ void __launch_bounds__(NVLS ? 1024 : 512) rows_allreduce_avg_kernel(c
         const int rr = rr0 + q2 * nw;
         const long long row = row0 + rr;
         act[q2] = rr < kRowsPerTile && row < r_hi && ((bits_t[rr >> 5] >> (rr & 31)) & 1u);
-        vrow[q2] = tab_off / 16 + row * row_vecs;
+        rows[q2] = row;
         has[q2] = 0u;
         if (!NVLS && act[q2]) {
           const int wl = (int)((row0 - r_lo) >> 5) + (rr >> 5);
@@ -301,83 +326,91 @@ __global__ void __launch_bounds__(NVLS ? 1024 : 512) rows_allreduce_avg_kernel(c
           for (int q = 0; q < WORLD; ++q) has[q2] |= ((bits_rank[q][wl] >> (rr & 31)) & 1u) << q;
         }
       }
-      for (int j0 = 0; j0 < row_vecs; j0 += 32 * kMaxVecPerLane) {
-        if (NVLS) {
-          uint32_t r[RPW][kMaxVecPerLane][4];
-#pragma unroll
-          for (int q2 = 0; q2 < RPW; ++q2)
-#pragma unroll
-            for (int u = 0; u < kMaxVecPerLane; ++u) {
-              const int j = j0 + u * 32 + lane;
-              if (act[q2] && j < row_vecs) {
-                char* a = mc + (vrow[q2] + j) * 16;
-                if (BF16)
-                  asm volatile("multimem.ld_reduce.relaxed.sys.global.add.acc::f32.v4.bf16x2 {%0,%1,%2,%3}, [%4];"
-                               : "=r"(r[q2][u][0]), "=r"(r[q2][u][1]), "=r"(r[q2][u][2]), "=r"(r[q2][u][3]) : "l"(a) : "memory");
-                else
-                  asm volatile("multimem.ld_reduce.relaxed.sys.global.add.v4.f32 {%0,%1,%2,%3}, [%4];"
-                               : "=r"(r[q2][u][0]), "=r"(r[q2][u][1]), "=r"(r[q2][u][2]), "=r"(r[q2][u][3]) : "l"(a) : "memory");
-              }
-            }
-#pragma unroll
-          for (int q2 = 0; q2 < RPW; ++q2)
-#pragma unroll
-            for (int u = 0; u < kMaxVecPerLane; ++u) {
-              const int j = j0 + u * 32 + lane;
-              if (act[q2] && j < row_vecs) {
-                scale_vec(r[q2][u], inv, BF16);
-                asm volatile("multimem.st.relaxed.sys.global.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(mc + (vrow[q2] + j) * 16),
-                             "r"(r[q2][u][0]), "r"(r[q2][u][1]), "r"(r[q2][u][2]), "r"(r[q2][u][3]) : "memory");
-              }
-            }
-        } else {
-          uint32_t v[RPW][kMaxVecPerLane][WORLD][4];
-#pragma unroll
-          for (int q2 = 0; q2 < RPW; ++q2)
-#pragma unroll
-            for (int u = 0; u < kMaxVecPerLane; ++u) {
-              const int j = j0 + u * 32 + lane;
-              if (act[q2] && j < row_vecs) {
-#pragma unroll
-                for (int q = 0; q < WORLD; ++q) {
-                  if ((has[q2] >> q) & 1u) {
-                    ld_sys_16(P[q] + (vrow[q2] + j) * 16, v[q2][u][q]);
-                  } else {
-                    v[q2][u][q][0] = v[q2][u][q][1] = v[q2][u][q][2] = v[q2][u][q][3] = 0u;  // +0.0 in bf16x2 and fp32 alike
-                  }
+      for (int t = 0; t < (NT == 1 ? 1 : T.n); ++t) {
+        long long vec_off;
+        int row_vecs;
+        row_table<NT>(T, t, vec_off, row_vecs);
+        long long vrow[RPW];
+  #pragma unroll
+        for (int q2 = 0; q2 < RPW; ++q2) vrow[q2] = vec_off + rows[q2] * row_vecs;
+        for (int j0 = 0; j0 < row_vecs; j0 += 32 * kMaxVecPerLane) {
+          if (NVLS) {
+            uint32_t r[RPW][kMaxVecPerLane][4];
+  #pragma unroll
+            for (int q2 = 0; q2 < RPW; ++q2)
+  #pragma unroll
+              for (int u = 0; u < kMaxVecPerLane; ++u) {
+                const int j = j0 + u * 32 + lane;
+                if (act[q2] && j < row_vecs) {
+                  char* a = mc + (vrow[q2] + j) * 16;
+                  if (BF16)
+                    asm volatile("multimem.ld_reduce.relaxed.sys.global.add.acc::f32.v4.bf16x2 {%0,%1,%2,%3}, [%4];"
+                                 : "=r"(r[q2][u][0]), "=r"(r[q2][u][1]), "=r"(r[q2][u][2]), "=r"(r[q2][u][3]) : "l"(a) : "memory");
+                  else
+                    asm volatile("multimem.ld_reduce.relaxed.sys.global.add.v4.f32 {%0,%1,%2,%3}, [%4];"
+                                 : "=r"(r[q2][u][0]), "=r"(r[q2][u][1]), "=r"(r[q2][u][2]), "=r"(r[q2][u][3]) : "l"(a) : "memory");
                 }
               }
-            }
-#pragma unroll
-          for (int q2 = 0; q2 < RPW; ++q2)
-#pragma unroll
-            for (int u = 0; u < kMaxVecPerLane; ++u) {
-              const int j = j0 + u * 32 + lane;
-              if (act[q2] && j < row_vecs) {
-                uint32_t r[4];
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                  if (BF16) {
-                    float a = 0.f, b = 0.f;
-#pragma unroll
-                    for (int q = 0; q < WORLD; ++q) {
-                      float lo_f, hi_f;
-                      bf16x2_to_f32(v[q2][u][q][k], lo_f, hi_f);
-                      a += lo_f;
-                      b += hi_f;
+  #pragma unroll
+            for (int q2 = 0; q2 < RPW; ++q2)
+  #pragma unroll
+              for (int u = 0; u < kMaxVecPerLane; ++u) {
+                const int j = j0 + u * 32 + lane;
+                if (act[q2] && j < row_vecs) {
+                  scale_vec(r[q2][u], inv, BF16);
+                  asm volatile("multimem.st.relaxed.sys.global.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(mc + (vrow[q2] + j) * 16),
+                               "r"(r[q2][u][0]), "r"(r[q2][u][1]), "r"(r[q2][u][2]), "r"(r[q2][u][3]) : "memory");
+                }
+              }
+          } else {
+            uint32_t v[RPW][kMaxVecPerLane][WORLD][4];
+  #pragma unroll
+            for (int q2 = 0; q2 < RPW; ++q2)
+  #pragma unroll
+              for (int u = 0; u < kMaxVecPerLane; ++u) {
+                const int j = j0 + u * 32 + lane;
+                if (act[q2] && j < row_vecs) {
+  #pragma unroll
+                  for (int q = 0; q < WORLD; ++q) {
+                    if ((has[q2] >> q) & 1u) {
+                      ld_sys_16(P[q] + (vrow[q2] + j) * 16, v[q2][u][q]);
+                    } else {
+                      v[q2][u][q][0] = v[q2][u][q][1] = v[q2][u][q][2] = v[q2][u][q][3] = 0u;  // +0.0 in bf16x2 and fp32 alike
                     }
-                    r[k] = f32x2_to_bf16x2(a * inv, b * inv);
-                  } else {
-                    float a = 0.f;
-#pragma unroll
-                    for (int q = 0; q < WORLD; ++q) a += __uint_as_float(v[q2][u][q][k]);
-                    r[k] = __float_as_uint(a * inv);
                   }
                 }
-#pragma unroll
-                for (int q = 0; q < WORLD; ++q) st_sys_16(P[q] + (vrow[q2] + j) * 16, r);
               }
-            }
+  #pragma unroll
+            for (int q2 = 0; q2 < RPW; ++q2)
+  #pragma unroll
+              for (int u = 0; u < kMaxVecPerLane; ++u) {
+                const int j = j0 + u * 32 + lane;
+                if (act[q2] && j < row_vecs) {
+                  uint32_t r[4];
+  #pragma unroll
+                  for (int k = 0; k < 4; ++k) {
+                    if (BF16) {
+                      float a = 0.f, b = 0.f;
+  #pragma unroll
+                      for (int q = 0; q < WORLD; ++q) {
+                        float lo_f, hi_f;
+                        bf16x2_to_f32(v[q2][u][q][k], lo_f, hi_f);
+                        a += lo_f;
+                        b += hi_f;
+                      }
+                      r[k] = f32x2_to_bf16x2(a * inv, b * inv);
+                    } else {
+                      float a = 0.f;
+  #pragma unroll
+                      for (int q = 0; q < WORLD; ++q) a += __uint_as_float(v[q2][u][q][k]);
+                      r[k] = __float_as_uint(a * inv);
+                    }
+                  }
+  #pragma unroll
+                  for (int q = 0; q < WORLD; ++q) st_sys_16(P[q] + (vrow[q2] + j) * 16, r);
+                }
+              }
+          }
         }
       }
     }
@@ -511,12 +544,21 @@ extern "C" int mot_dp_allreduce_avg(void* multicast_ptr, void* const* signal_pad
                          stream);
 }
 
-extern "C" int mot_dp_exchange_rows(void* multicast_ptr, void* const* peer_ptrs_dev, void* const* signal_pads_dev, void* work_area,
-                                    int32_t rank, int32_t world, int64_t table_byte_offset, int32_t n_rows, int32_t row_bytes,
-                                    int64_t bitmap_byte_offset, int64_t dense_byte_offset, int64_t dense_bytes, int32_t dtype,
-                                    uint32_t epoch, int32_t algo, void* stream) {
-  if (!signal_pads_dev || !work_area || world < 1 || rank < 0 || rank >= world || n_rows < 0 || row_bytes <= 0 || dense_bytes < 0)
+static bool ranges_overlap(long long a_lo, long long a_n, long long b_lo, long long b_n) {
+  return a_n > 0 && b_n > 0 && a_lo < b_lo + b_n && b_lo < a_lo + a_n;
+}
+
+extern "C" int mot_dp_exchange_rows_multi(void* multicast_ptr, void* const* peer_ptrs_dev, void* const* signal_pads_dev,
+                                          void* work_area, int32_t rank, int32_t world, const MotRowTable* tables,
+                                          int32_t n_tables, int32_t n_rows, int64_t bitmap_byte_offset,
+                                          int64_t dense_byte_offset, int64_t dense_bytes, int32_t dtype, uint32_t epoch,
+                                          int32_t algo, void* stream) {
+  if (!signal_pads_dev || !work_area || world < 1 || rank < 0 || rank >= world || n_rows < 0 || dense_bytes < 0)
     return MOT_ERR_BAD_ARG;
+  if (!tables || n_tables < 1 || n_tables > MOT_DP_MAX_ROW_TABLES) return MOT_ERR_BAD_ARG;
+  for (int t = 0; t < n_tables; ++t)
+    if (tables[t].row_bytes <= 0 || tables[t].byte_offset < 0 || tables[t].reserved != 0) return MOT_ERR_BAD_ARG;
+  if (bitmap_byte_offset < 0 || dense_byte_offset < 0) return MOT_ERR_BAD_ARG;
   if (dtype != MOT_BF16 && dtype != MOT_F32) return MOT_ERR_UNSUPPORTED;
   if (algo == MOT_DP_NVLS && !multicast_ptr) return MOT_ERR_BAD_ARG;
   if (algo == MOT_DP_P2P && !peer_ptrs_dev) return MOT_ERR_BAD_ARG;
@@ -524,8 +566,23 @@ extern "C" int mot_dp_exchange_rows(void* multicast_ptr, void* const* peer_ptrs_
   if (algo == MOT_DP_P2P && world != 2 && world != 4) return MOT_ERR_UNSUPPORTED;
   if (world > 16) return MOT_ERR_UNSUPPORTED;
   if (((n_rows + world - 1) / world + 31) / 32 + 1 > kMaxRowWords) return MOT_ERR_UNSUPPORTED;
-  if ((row_bytes & 15) || (table_byte_offset & 15) || (bitmap_byte_offset & 3) || (dense_byte_offset & 15) || (dense_bytes & 15))
-    return MOT_ERR_MISALIGNED;
+  for (int t = 0; t < n_tables; ++t)
+    if ((tables[t].row_bytes & 15) || (tables[t].byte_offset & 15)) return MOT_ERR_MISALIGNED;
+  if ((bitmap_byte_offset & 3) || (dense_byte_offset & 15) || (dense_bytes & 15)) return MOT_ERR_MISALIGNED;
+  // the kernel reads the bitmap and rewrites the tables and the dense range in place: no byte may belong to two of them
+  const long long bm_bytes = ((long long)n_rows + 31) / 32 * 4;
+  RowTables T{};
+  T.n = n_tables;
+  for (int t = 0; t < n_tables; ++t) {
+    const long long lo = tables[t].byte_offset, nb = (long long)n_rows * tables[t].row_bytes;
+    if (ranges_overlap(lo, nb, dense_byte_offset, dense_bytes) || ranges_overlap(lo, nb, bitmap_byte_offset, bm_bytes))
+      return MOT_ERR_BAD_ARG;
+    for (int u = 0; u < t; ++u)
+      if (ranges_overlap(lo, nb, tables[u].byte_offset, (long long)n_rows * tables[u].row_bytes)) return MOT_ERR_BAD_ARG;
+    T.vec_off[t] = lo / 16;
+    T.row_vecs[t] = tables[t].row_bytes / 16;
+  }
+  if (ranges_overlap(bitmap_byte_offset, bm_bytes, dense_byte_offset, dense_bytes)) return MOT_ERR_BAD_ARG;
   int sms = 0, optin = 0;
   if (int rc = device_props(&sms, &optin)) return rc;
   const char* env_b = getenv("MOT_AR_BLOCKS");
@@ -542,20 +599,32 @@ extern "C" int mot_dp_exchange_rows(void* multicast_ptr, void* const* peer_ptrs_
   char* mc = reinterpret_cast<char*>(multicast_ptr);
   char* const* peers = reinterpret_cast<char* const*>(peer_ptrs_dev);
   const dim3 g((unsigned)blocks), b(algo == MOT_DP_NVLS ? 1024 : 512);
-  const int row_vecs = row_bytes / 16;
   const long long dlo = dense_byte_offset / 16, dn = dense_bytes / 16;
   const bool bf = dtype == MOT_BF16;
-#define MOT_ROWS_LAUNCH(BF, NV, WD)                                                                                         \
-  launch_pdl(rows_allreduce_avg_kernel<BF, NV, WD>, g, b, 0, s, mc, peers, pads, (int)rank, (int)world, (long long)table_byte_offset, \
-             (int)n_rows, row_vecs, (long long)bitmap_byte_offset, dlo, dn, epoch, work, peer_bits, trace)
+  // one table: the table loop compiled away (NT = 1); several: bounded by MOT_DP_MAX_ROW_TABLES, the count read at run time
+#define MOT_ROWS_LAUNCH(BF, NV, WD, NT)                                                                                       \
+  launch_pdl(rows_allreduce_avg_kernel<BF, NV, WD, NT>, g, b, 0, s, mc, peers, pads, (int)rank, (int)world, T, (int)n_rows,   \
+             (long long)bitmap_byte_offset, dlo, dn, epoch, work, peer_bits, trace)
+#define MOT_ROWS_LAUNCH_NT(BF, NV, WD) \
+  do { if (n_tables == 1) MOT_ROWS_LAUNCH(BF, NV, WD, 1); else MOT_ROWS_LAUNCH(BF, NV, WD, MOT_DP_MAX_ROW_TABLES); } while (0)
   if (algo == MOT_DP_NVLS) {
-    if (bf) MOT_ROWS_LAUNCH(true, true, 1); else MOT_ROWS_LAUNCH(false, true, 1);
+    if (bf) MOT_ROWS_LAUNCH_NT(true, true, 1); else MOT_ROWS_LAUNCH_NT(false, true, 1);
   } else if (world == 2) {
-    if (bf) MOT_ROWS_LAUNCH(true, false, 2); else MOT_ROWS_LAUNCH(false, false, 2);
+    if (bf) MOT_ROWS_LAUNCH_NT(true, false, 2); else MOT_ROWS_LAUNCH_NT(false, false, 2);
   } else {
-    if (bf) MOT_ROWS_LAUNCH(true, false, 4); else MOT_ROWS_LAUNCH(false, false, 4);
+    if (bf) MOT_ROWS_LAUNCH_NT(true, false, 4); else MOT_ROWS_LAUNCH_NT(false, false, 4);
   }
+#undef MOT_ROWS_LAUNCH_NT
 #undef MOT_ROWS_LAUNCH
   count_launch();
   return check_launch();
+}
+
+extern "C" int mot_dp_exchange_rows(void* multicast_ptr, void* const* peer_ptrs_dev, void* const* signal_pads_dev, void* work_area,
+                                    int32_t rank, int32_t world, int64_t table_byte_offset, int32_t n_rows, int32_t row_bytes,
+                                    int64_t bitmap_byte_offset, int64_t dense_byte_offset, int64_t dense_bytes, int32_t dtype,
+                                    uint32_t epoch, int32_t algo, void* stream) {
+  const MotRowTable table = {table_byte_offset, row_bytes, 0};
+  return mot_dp_exchange_rows_multi(multicast_ptr, peer_ptrs_dev, signal_pads_dev, work_area, rank, world, &table, 1, n_rows,
+                                    bitmap_byte_offset, dense_byte_offset, dense_bytes, dtype, epoch, algo, stream);
 }

@@ -24,6 +24,7 @@ F_SLOT_MAJOR, F_IDS_FROM_TTB, F_TTB_SCRAMBLE, F_IDS_I64, F_HAS_LAMBDAS = 16, 32,
 F_TTB_PULL_LEFT, F_TTB_PULL_RIGHT, F_TTB_NEXT_TOK = 512, 1024, 2048
 WS_PLAN_READY, WS_CLEAN, WS_PLAN_JOINED = 1, 2, 4
 DP_NVLS, DP_P2P = 0, 1
+DP_MAX_ROW_TABLES = 8
 
 
 class MotDesc(C.Structure):
@@ -37,6 +38,10 @@ class MotDesc(C.Structure):
         ("row_stride", C.c_int64), ("col_offset", C.c_int32), ("dp_slabs", C.c_int32),
         ("pad_id", C.c_int32), ("eot_id", C.c_int32),
     ]
+
+
+class MotRowTable(C.Structure):
+    _fields_ = [("byte_offset", C.c_int64), ("row_bytes", C.c_int32), ("reserved", C.c_int32)]
 
 
 _P = C.c_void_p
@@ -76,6 +81,8 @@ _SIGNATURES = {
     "mot_embed_touched_rows": (C.c_int, [C.POINTER(MotDesc), _P, C.c_size_t, _P, _P]),
     "mot_dp_exchange_rows": (C.c_int, [_P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int64,
                                        C.c_int64, C.c_int32, C.c_uint32, C.c_int32, _P]),
+    "mot_dp_exchange_rows_multi": (C.c_int, [_P, _P, _P, _P, C.c_int32, C.c_int32, C.POINTER(MotRowTable), C.c_int32, C.c_int32,
+                                             C.c_int64, C.c_int64, C.c_int64, C.c_int32, C.c_uint32, C.c_int32, _P]),
     "mot_dp_allreduce_avg": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_uint32, _P]),
     "mot_pull_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int64, C.c_int32]),
     "mot_pull": (C.c_int, [_P, _P, C.c_int64, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P,

@@ -85,12 +85,19 @@ class GradBucket:
     in-switch reduction or peer-to-peer two-shot) and can run as a PIPELINE beside the backward: the backward walks the
     vocabulary in `n_slabs` slabs (mot_embed_bwd_slab), `exchange_async(lo, hi, last)` averages the rows of a finished
     slab on a second stream while the next slab is computed, `wait()` joins.  This is the overlap the reference gets
-    from its asynchronous per-parameter all-reduces (runs/7:697-711), inside the path."""
+    from its asynchronous per-parameter all-reduces (runs/7:697-711), inside the path.
+
+    Touched-rows exchange: the first `row_tables` parameters are `[V, D_i]` tables gathered with the same token ids (the
+    front's token table and the value embeddings, runs/7:252,308).  The backwards publish the rows their batch gathered
+    (`mark_rows`) into one bitmap behind the bucket, and the exchange moves only the rows some rank gathered, in every
+    row table at once; the parameters after them are exchanged dense."""
 
     def __init__(self, params: Iterable[torch.nn.Parameter], dtype: Optional[torch.dtype] = None, symmetric="auto",
-                 group=None, n_slabs: Optional[int] = None, reserve_sms: int = 8, sparse_rows="auto"):
+                 group=None, n_slabs: Optional[int] = None, reserve_sms: int = 8, sparse_rows="auto", row_tables: int = 1):
         """symmetric=True / "auto" (CUDA, initialised process group with more than one rank): allocate the bucket in
-        symmetric memory so that the library's own exchange kernels apply; False: ordinary memory, NCCL."""
+        symmetric memory so that the library's own exchange kernels apply; False: ordinary memory, NCCL.
+        row_tables=k > 1: params[:k] are 2-D tables of one row count V, indexed by the same token ids, with rows of a
+        multiple of 16 bytes (ValueError otherwise); one bitmap of V bits covers all of them."""
         self.params: List[torch.nn.Parameter] = list(params)
         if not self.params:
             raise ValueError("GradBucket needs at least one parameter")
@@ -98,6 +105,18 @@ class GradBucket:
         dev = self.params[0].device
         esz = torch.empty(0, dtype=self.dtype).element_size()
         align = max(1, 16 // esz)
+        from ._lib import DP_MAX_ROW_TABLES
+        self.row_tables = int(row_tables)
+        if not 1 <= self.row_tables <= min(len(self.params), DP_MAX_ROW_TABLES):
+            raise ValueError(f"GradBucket: row_tables={row_tables} must be 1 .. min(len(params), {DP_MAX_ROW_TABLES})")
+        if self.row_tables > 1:
+            tabs = self.params[:self.row_tables]
+            if any(t.dim() != 2 for t in tabs):
+                raise ValueError("GradBucket: row tables must be 2-D [V, D] tables")
+            if len({t.shape[0] for t in tabs}) != 1:
+                raise ValueError("GradBucket: row tables must share their row count V (one bitmap of token ids)")
+            if any(t.shape[1] * esz % 16 for t in tabs):
+                raise ValueError("GradBucket: row-table rows must be a multiple of 16 bytes")
         self.offsets, n = [], 0
         for p in self.params:
             if p.device != dev:
@@ -111,11 +130,13 @@ class GradBucket:
         self.reserve_sms = int(reserve_sms)
         self._ev = None
         self._pending = False
-        self.sparse_rows = False          # touched-rows exchange of params[0] (a [V, D] table) available
+        self.sparse_rows = False          # touched-rows exchange of params[:row_tables] ([V, D_i] tables) available
         self.bitmap = None
-        self._rows_ready = False
+        self._rows_ready = False          # a mark since the last exchange: the bitmap holds this rank's rows
+        self._fresh = set()               # ids of the row tables a backward overwrote since the last exchange
+        self._bits_new = None             # the rows of a later mark, ORed into the bitmap
         n = (n + align - 1) // align * align
-        # room for the touched-rows bitmap of the first table behind the gradients (same symmetric allocation)
+        # room for the touched-rows bitmap of the row tables behind the gradients (same symmetric allocation)
         words = (self.params[0].shape[0] + 31) // 32 if self.params[0].dim() == 2 else 0
         extra = (words * 4 + 15) // 16 * 16 // esz
         self.flat = None
@@ -136,7 +157,8 @@ class GradBucket:
                     self._full = full
                     self.flat, self._symm, self.algo = full[:n], hdl, algo
                     want_sparse = sparse_rows if sparse_rows != "auto" else not os.environ.get("MOT_DP_DENSE")
-                    if want_sparse and words > 0 and (algo == "nvls" or world in (2, 4)) and self.params[0].is_contiguous():
+                    if want_sparse and words > 0 and (algo == "nvls" or world in (2, 4)) \
+                            and all(t.is_contiguous() for t in self.params[:self.row_tables]):
                         self.sparse_rows = True
                         self.bitmap = full[n:].view(torch.int32)[:words]
                         self._bitmap_off = n * esz
@@ -168,6 +190,12 @@ class GradBucket:
                 return o
         raise KeyError("parameter is not in this bucket")
 
+    def holds(self, param: torch.nn.Parameter) -> bool:
+        return any(p is param for p in self.params)
+
+    def is_row_table(self, param: torch.nn.Parameter) -> bool:
+        return any(p is param for p in self.params[:self.row_tables])
+
     def attach(self) -> None:
         """param.grad = its slice of the bucket (grads of a different dtype are copied in, e.g. an fp32 master-weight
         gradient into a bf16 bucket is NOT done silently: dtypes must match)."""
@@ -176,6 +204,7 @@ class GradBucket:
                 if p.grad.dtype != self.dtype:
                     raise TypeError("GradBucket: gradient dtype differs from the bucket dtype")
                 v.copy_(p.grad)
+                self._fresh.discard(id(p))      # rows no bitmap describes: the next exchange is dense
             p.grad = v
 
     # ------------------------------------------------------------------------------------------------ exchange
@@ -197,35 +226,62 @@ class GradBucket:
         L.check(rc, "mot_dp_exchange")
         self._epoch = (self._epoch + (2 if last else 1)) & 0xFFFFFFFF
 
-    def mark_rows(self, desc, ws_buf: torch.Tensor) -> None:
-        """Publish the rows of params[0] this rank's batch gathered (from the sort plan in `ws_buf`) for the touched-rows
-        exchange; call after the backward of the step, on its stream.  The next all_reduce_avg() then moves only the rows
-        some rank gathered (rows that are zero everywhere stay as they are)."""
+    def mark_rows(self, desc, ws_buf: torch.Tensor, fresh: Iterable[torch.nn.Parameter] = ()) -> None:
+        """Publish the rows of the row tables this rank's batch gathered (from the sort plan in `ws_buf`) for the
+        touched-rows exchange; call after a backward that produced a row table's gradient, on its stream.  The next
+        all_reduce_avg() then moves only the rows some rank gathered (rows that are zero everywhere stay as they are).
+        The first mark after an exchange writes the bitmap, later ones (micro-batches, several modules) are ORed into
+        it.  `fresh`: the row tables whose bucket view this backward overwrote.  A row table whose `.grad` is its view
+        and was not overwritten since the last exchange holds rows no bitmap describes: that exchange is dense."""
         if not self.sparse_rows:
             return
+        if desc.tok_vocab != self.params[0].shape[0]:
+            raise ValueError(f"GradBucket.mark_rows: a plan over {desc.tok_vocab} rows for row tables of "
+                             f"{self.params[0].shape[0]}")
         from . import _lib as L
         dev = self.flat.device
+        merge = self._rows_ready
+        if merge and self._bits_new is None:
+            self._bits_new = torch.empty_like(self.bitmap)
+        dst = self._bits_new if merge else self.bitmap
         with torch.cuda.device(dev):
-            rc = L.lib().mot_embed_touched_rows(desc, ws_buf.data_ptr(), ws_buf.numel(), self.bitmap.data_ptr(),
+            rc = L.lib().mot_embed_touched_rows(desc, ws_buf.data_ptr(), ws_buf.numel(), dst.data_ptr(),
                                                 torch.cuda.current_stream(dev).cuda_stream)
-        L.check(rc, "mot_embed_touched_rows")
+            L.check(rc, "mot_embed_touched_rows")
+            if merge:
+                self.bitmap.bitwise_or_(self._bits_new)
         self._rows_ready = True
+        self._fresh.update(id(p) for p in fresh)
+
+    def _rows_describe_bucket(self) -> bool:
+        """Every row table whose gradient is its bucket view was overwritten by a backward since the last exchange, so
+        its nonzero rows are all in this rank's bitmap (the precondition of the touched-rows exchange)."""
+        for p, v in zip(self.params[:self.row_tables], self._views):
+            if p.grad is not None and p.grad.data_ptr() == v.data_ptr() and id(p) not in self._fresh:
+                return False
+        return True
+
+    def rows_layout(self):
+        """Byte layout of the touched-rows exchange -> ([(byte offset, row bytes) per row table], dense byte offset,
+        dense bytes): the row tables lead the bucket, everything from params[row_tables] on is exchanged dense."""
+        esz, k = self.flat.element_size(), self.row_tables
+        tabs = [(o * esz, p.shape[1] * esz) for o, p in zip(self.offsets[:k], self.params[:k])]
+        dense_lo = self.offsets[k] if len(self.offsets) > k else self.flat.numel()
+        return tabs, dense_lo * esz, (self.flat.numel() - dense_lo) * esz
 
     def _exchange_rows(self, stream: int) -> None:
         from . import _lib as L
         h = self._symm
-        esz = self.flat.element_size()
-        V, D = self.params[0].shape
-        dense_lo = self.offsets[1] if len(self.offsets) > 1 else self.flat.numel()
-        rc = L.lib().mot_dp_exchange_rows(h.multicast_ptr if self.algo == "nvls" else None,
-                                          h.buffer_ptrs_dev if self.algo == "p2p" else None, h.signal_pad_ptrs_dev,
-                                          self._work.data_ptr(), h.rank, h.world_size, self.offsets[0] * esz, V, D * esz,
-                                          self._bitmap_off, dense_lo * esz, (self.flat.numel() - dense_lo) * esz,
-                                          L.BF16 if self.dtype == torch.bfloat16 else L.F32, self._epoch,
-                                          L.DP_NVLS if self.algo == "nvls" else L.DP_P2P, stream)
-        L.check(rc, "mot_dp_exchange_rows")
+        tabs, dense_lo, dense_bytes = self.rows_layout()
+        tables = (L.MotRowTable * len(tabs))(*[L.MotRowTable(o, rb, 0) for o, rb in tabs])
+        rc = L.lib().mot_dp_exchange_rows_multi(h.multicast_ptr if self.algo == "nvls" else None,
+                                                h.buffer_ptrs_dev if self.algo == "p2p" else None, h.signal_pad_ptrs_dev,
+                                                self._work.data_ptr(), h.rank, h.world_size, tables, len(tabs),
+                                                self.params[0].shape[0], self._bitmap_off, dense_lo, dense_bytes,
+                                                L.BF16 if self.dtype == torch.bfloat16 else L.F32, self._epoch,
+                                                L.DP_NVLS if self.algo == "nvls" else L.DP_P2P, stream)
+        L.check(rc, "mot_dp_exchange_rows_multi")
         self._epoch = (self._epoch + 2) & 0xFFFFFFFF
-        self._rows_ready = False
 
     def exchange_async(self, lo: int, hi: int, last: bool) -> None:
         """Average elements [lo, hi) of the bucket (multiples of 16 bytes) across ranks on the exchange stream, ordered
@@ -259,12 +315,15 @@ class GradBucket:
             if async_op or group is not None:
                 raise NotImplementedError("GradBucket: the symmetric-memory exchange is stream-ordered on the whole world "
                                           "(async_op / sub-groups are NCCL features: build the bucket with symmetric=False)")
+            rows = self._rows_ready and self._rows_describe_bucket()
+            self._rows_ready = False
+            self._fresh.clear()
             if self._pending:          # the slabs are already in flight on the exchange stream
                 self.wait()
                 return None
             dev = self.flat.device
             with torch.cuda.device(dev):
-                if self._rows_ready:       # the backward published its row bitmap: move only the rows of the union
+                if rows:                   # the backwards published their row bitmap: move only the rows of the union
                     self._exchange_rows(torch.cuda.current_stream(dev).cuda_stream)
                 else:
                     self._exchange(0, self.flat.numel(), True, torch.cuda.current_stream(dev).cuda_stream)

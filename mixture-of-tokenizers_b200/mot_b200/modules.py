@@ -60,7 +60,9 @@ class MoTEmbedding(nn.Module):
     def attach_grad_bucket(self, bucket=None):
         """Data parallelism: let the backward kernels write `embed_tokens.weight.grad` / `embed_bytes.weight.grad`
         straight into one flat bucket, so the per-parameter all-reduces of the reference (runs/7:697-700) become a
-        single `bucket.all_reduce_avg()`.  Call after the module is on its device and in its final dtype."""
+        single `bucket.all_reduce_avg()`.  The bucket may hold more tables (the value embeddings: see
+        TokenValueEmbeddings.attach_grad_bucket); the rows of the batch are marked whenever the token table is one of
+        its row tables.  Call after the module is on its device and in its final dtype."""
         from .dp import GradBucket
         tables = [m.weight for m in (self.embed_tokens, self.embed_bytes) if m is not None]
         self.grad_bucket = bucket if bucket is not None else GradBucket(tables, symmetric="auto")
@@ -199,9 +201,22 @@ class TokenValueEmbeddings(nn.Module):
     def __init__(self, vocab_size: int, model_dim: int, n_tables: int = 3):
         super().__init__()
         self.value_embeds = nn.ModuleList([nn.Embedding(vocab_size, model_dim) for _ in range(n_tables)])
+        self.grad_bucket = None
+
+    def attach_grad_bucket(self, bucket=None):
+        """Data parallelism: the backward writes the dense gradients of the tables straight into `bucket` (default: a
+        bucket of these tables, all of them row tables) and marks the gathered rows, so that the per-table all-reduces
+        of the reference (runs/7:697-700) become one `bucket.all_reduce_avg()` that moves only the rows some rank
+        gathered.  A bucket shared with the front lists its token table and these tables as its row tables:
+        `GradBucket([front.embed_tokens.weight, *(m.weight for m in ve.value_embeds), front.embed_bytes.weight],
+        row_tables=4)`.  Call after the module is on its device and in its final dtype."""
+        from .dp import GradBucket
+        tables = [m.weight for m in self.value_embeds]
+        self.grad_bucket = bucket if bucket is not None else GradBucket(tables, symmetric="auto", row_tables=len(tables))
+        return self.grad_bucket
 
     def forward(self, token_inputs: torch.Tensor):
-        outs = tok_gather(token_inputs, *[m.weight for m in self.value_embeds])
+        outs = tok_gather(token_inputs, *[m.weight for m in self.value_embeds], grad_bucket=self.grad_bucket)
         return [o.view(*token_inputs.shape, -1) for o in outs]
 
 

@@ -608,10 +608,12 @@ class _MotEmbedFn(torch.autograd.Function):
             embed_backward_out(desc, tok, ids, ttb, E_tok, E_byte, lam, g, gE_tok, gE_byte, g_lam, ws.buf,
                                plan_ready=planned, ws_clean=clean, stream=st, out_saved=out_saved, rstd=rstd,
                                plan_joined=planned)
-        if ctx.grad_bufs is not None and len(ctx.grad_bufs) > 2 and direct[0] is not None and tok is not None:
-            bk = ctx.grad_bufs[2]
-            if bk is not None and bk.sparse_rows and bk.params[0] is direct[0][0] and not bk._pending:
-                bk.mark_rows(desc, ws.buf)      # the rows this batch gathered: the exchange moves only the union
+        if ctx.grad_bufs is not None and len(ctx.grad_bufs) > 2 and ctx.grad_bufs[0] is not None and tok is not None:
+            bk, p_tok = ctx.grad_bufs[2], ctx.grad_bufs[0][0]
+            if bk is not None and bk.sparse_rows and bk.is_row_table(p_tok) and not bk._pending:
+                # the rows this batch gathered, also when autograd adds this gradient to an existing one: the exchange
+                # moves only the union of every backward since the last exchange
+                bk.mark_rows(desc, ws.buf, fresh=(p_tok,) if direct[0] is not None else ())
         ctx.ws = None
         _return_workspace(ws)
         if g_lam is not None:
@@ -679,16 +681,17 @@ def _gather_forward(desc: L.MotDesc, tok, tables, dev, stream: Optional[int] = N
 
 
 def _gather_backward(desc: L.MotDesc, tok, tables, grads, want, ws_buf, plan_ready: bool, ws_clean: bool,
-                     stream: Optional[int] = None):
+                     stream: Optional[int] = None, outs=None):
     """Dense gradients of the tables whose `want` entry is true (None for the others), one scatter launch each; the
-    first one finds the plan in place or builds it, and every one leaves the accumulators zeroed."""
+    first one finds the plan in place or builds it, and every one leaves the accumulators zeroed.  outs[i], where given,
+    is the tensor table i's gradient is written into (a gradient-bucket view), else a new one."""
     gEs = []
-    for E, g, w in zip(tables, grads, want):
+    for i, (E, g, w) in enumerate(zip(tables, grads, want)):
         if not w:
             gEs.append(None)
             continue
         g = g.reshape(-1, E.shape[1]).to(E.dtype).contiguous()
-        gE = torch.empty_like(E)
+        gE = outs[i] if outs is not None and outs[i] is not None else torch.empty_like(E)
         embed_backward_out(desc, tok, None, None, E, None, None, g, gE, None, None, ws_buf,
                            plan_ready=plan_ready, ws_clean=ws_clean, stream=stream)
         plan_ready, ws_clean = True, True
@@ -699,16 +702,20 @@ def _gather_backward(desc: L.MotDesc, tok, tables, grads, want, ws_buf, plan_rea
 class _TokGatherFn(torch.autograd.Function):
     """outs[i] = tables[i][tokens]: plain gathers (no norm) of same-shaped tables.  The backward needs the positions
     grouped by token id once for all tables: one sort plan (started beside the first forward gather), one scatter
-    launch per table reusing it (MOT_WS_PLAN_READY); the dense gradients need no token rows (R = 0)."""
+    launch per table reusing it (MOT_WS_PLAN_READY); the dense gradients need no token rows (R = 0).
+    grad_bucket = optional (dp.GradBucket, the table parameters): the gradient of a table the bucket holds is written
+    into its bucket view, which becomes param.grad, and the rows of the batch are marked for the touched-rows exchange."""
 
     @staticmethod
-    def forward(ctx, dev, tok, *tables):
+    def forward(ctx, dev, tok, grad_bucket, *tables):
+        if grad_bucket is not None:      # an output without gradient leaves its table's grad None, not a view of zeros
+            ctx.set_materialize_grads(False)
         desc = _gather_desc(tok, tables[0])
         st = _stream(dev)
-        ctx.ws = _planned_workspace(desc, tok, dev, st) if any(ctx.needs_input_grad[2:]) and tok.numel() > 0 else None
+        ctx.ws = _planned_workspace(desc, tok, dev, st) if any(ctx.needs_input_grad[3:]) and tok.numel() > 0 else None
         outs = _gather_forward(desc, tok, tables, dev, st)
         embed_plan_join_if_capturing(ctx.ws, dev, st)
-        ctx.desc, ctx.dev = desc, dev
+        ctx.desc, ctx.dev, ctx.grad_bucket = desc, dev, grad_bucket
         ctx.save_for_backward(tok, *tables)
         return tuple(outs)
 
@@ -717,21 +724,44 @@ class _TokGatherFn(torch.autograd.Function):
         tok, *Es = ctx.saved_tensors
         st = _stream(ctx.dev)
         ws, planned, clean = _take_workspace(ctx.ws, ctx.desc, ctx.dev, st)
-        want = [g is not None and ctx.needs_input_grad[2 + i] for i, g in enumerate(grad_outs)]
-        grads = _gather_backward(ctx.desc, tok, Es, grad_outs, want, ws.buf, planned, clean, st)
+        want = [g is not None and ctx.needs_input_grad[3 + i] for i, g in enumerate(grad_outs)]
+        direct = [None] * len(Es)
+        if ctx.grad_bucket is not None:
+            # as in _MotEmbedFn: the scatter overwrites every row, so it writes straight into the bucket; with a
+            # gradient already on the parameter the normal path is taken and autograd adds to it
+            bk, params = ctx.grad_bucket
+            for i, (p, E) in enumerate(zip(params, Es)):
+                if want[i] and p.grad is None and bk.holds(p):
+                    view = bk.view_of(p)
+                    if view.dtype != E.dtype or view.shape != E.shape or not view.is_contiguous() or view.device != E.device:
+                        raise TypeError("mot_b200: the gradient-bucket view of a table must match its dtype, shape and "
+                                        f"device and be contiguous (table {tuple(E.shape)} {E.dtype}, view "
+                                        f"{tuple(view.shape)} {view.dtype})")
+                    direct[i] = view
+        grads = _gather_backward(ctx.desc, tok, Es, grad_outs, want, ws.buf, planned, clean, st, outs=direct)
+        if ctx.grad_bucket is not None:
+            bk, params = ctx.grad_bucket
+            if bk.sparse_rows and not bk._pending and tok.numel() > 0 \
+                    and any(w and bk.is_row_table(p) for w, p in zip(want, params)):
+                bk.mark_rows(ctx.desc, ws.buf,
+                             fresh=[p for p, d in zip(params, direct) if d is not None and bk.is_row_table(p)])
+            for i, p in enumerate(params):
+                if direct[i] is not None:
+                    p.grad, grads[i] = direct[i], None
         ctx.ws = None
         _return_workspace(ws)
-        return (None, None, *grads)
+        return (None, None, None, *grads)
 
 
-def tok_gather(tokens: torch.Tensor, *tables: torch.Tensor):
+def tok_gather(tokens: torch.Tensor, *tables: torch.Tensor, grad_bucket=None):
     """`[E(tokens) for E in tables]` (the value embeddings of runs/7:308 / spt/train_gpt.py:600): returns a tuple of
-    [n_tokens, D] tensors; dense gradients, one token sort shared by every table."""
+    [n_tokens, D] tensors; dense gradients, one token sort shared by every table.  grad_bucket = optional
+    dp.GradBucket holding the tables: the backward writes their gradients into it and marks the gathered rows."""
     dev, tok, Es = _gather_args(tokens, tables)
-    if _custom_ops_wanted():
+    if grad_bucket is None and _custom_ops_wanted():
         need = torch.is_grad_enabled() and any(E.requires_grad for E in tables)
         return tuple(torch.ops.mot_b200.tok_gather(tok, Es, need)[:-1])
-    return _TokGatherFn.apply(dev, tok, *Es)
+    return _TokGatherFn.apply(dev, tok, (grad_bucket, tables) if grad_bucket is not None else None, *Es)
 
 
 # ------------------------------------------------------------------------------------------------------------

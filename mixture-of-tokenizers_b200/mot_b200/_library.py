@@ -62,24 +62,21 @@ def unpack_spec(code: int, eps: float):
                      ttb_pull_side="right" if code & 2048 else "left")
 
 
-_PLANNERS: dict = {}
+def _plan_beside(desc, tok: Tensor, dev):
+    """A fresh workspace (O.fresh_workspace) with the sort plan of `tok`, started on the side stream (fork after
+    everything queued on the current stream; the library zeroes the head of the fresh buffer there first).  The caller
+    launches its forward kernels and then returns _rejoin(ws, dev)."""
+    ws = O.fresh_workspace(desc, dev)
+    O.embed_plan_async(desc, tok, ws, dev)         # ws.clean is False: the plan clears the fresh buffer
+    return ws
 
 
-def _plan_beside(desc, tok: Tensor, dev) -> Tensor:
-    """A fresh workspace with the sort plan of `tok`, started on the side stream (fork after everything queued on the
-    current stream; the library zeroes the head of the fresh buffer there first).  The caller launches its forward
-    kernels and then calls _rejoin()."""
-    ws = _PLANNERS.get(dev.index)
-    if ws is None:   # one per device; the operators share its fork / join events, never its buffer
-        ws = _PLANNERS[dev.index] = O.Workspace(None, dev)
-    ws.buf = torch.empty(O.embed_workspace_bytes(desc), dtype=torch.uint8, device=dev)
-    O.embed_plan_async(desc, tok, ws, dev)         # ws.clean stays False: the plan clears the fresh buffer
-    buf, ws.buf = ws.buf, None
-    return buf
-
-
-def _rejoin(dev) -> None:
-    O.embed_plan_join(_PLANNERS[dev.index], dev)
+def _rejoin(ws, dev) -> Tensor:
+    """The workspace tensor an operator returns: the plan joined to the current stream, or [0] without a plan."""
+    if ws is None:
+        return _empty(dev)
+    O.embed_plan_join(ws, dev)
+    return ws.buf
 
 
 def _bwd_workspace(ws: Tensor, desc, dev) -> Tuple[Tensor, bool]:
@@ -106,13 +103,11 @@ def embed_op(tok: Optional[Tensor], ids: Optional[Tensor], ttb: Optional[Tensor]
     dev = ref.device
     out = torch.empty((n, desc.out_dim), dtype=ref.dtype, device=dev)
     planned = plan and tok is not None and n > 0
-    ws = _plan_beside(desc, tok, dev) if planned else _empty(dev)
+    ws = _plan_beside(desc, tok, dev) if planned else None
     keep = plan and n > 0 and O.embed_bwd_uses_saved(desc)
     rstd = torch.empty(n if keep else 0, dtype=torch.float32, device=dev)
     O.embed_forward_out(desc, tok, ids, ttb, E_tok, E_byte, lam, out, rstd=rstd if keep else None)
-    if planned:
-        _rejoin(dev)
-    return out, rstd, ws
+    return out, rstd, _rejoin(ws, dev)
 
 
 @embed_op.register_fake
@@ -182,11 +177,9 @@ def tok_gather_op(tok: Tensor, tables: List[Tensor], plan: bool) -> List[Tensor]
     dev = tok.device
     desc = O._gather_desc(tok, tables[0])
     planned = plan and tok.numel() > 0
-    ws = _plan_beside(desc, tok, dev) if planned else _empty(dev)
+    ws = _plan_beside(desc, tok, dev) if planned else None
     outs = O._gather_forward(desc, tok, tables, dev)
-    if planned:
-        _rejoin(dev)
-    return outs + [ws]
+    return outs + [_rejoin(ws, dev)]
 
 
 @tok_gather_op.register_fake
@@ -250,10 +243,9 @@ def embed_proj_op(tok: Tensor, ids: Optional[Tensor], ids2: Optional[Tensor], E_
     tok, desc, desc_pair = O._proj_descs(sp, bpt, seq_len, tok, next_tok, ids, ids2, ttb, ttb_pair, E_tok, E_byte)
     w_c = W if W.dtype == cdt else O.cast_out(W, cdt)
     planned = plan and tok.numel() > 0
-    ws = _plan_beside(desc, tok, dev) if planned else _empty(dev)
+    ws = _plan_beside(desc, tok, dev) if planned else None
     out, Y, _ = O._proj_forward(sp, desc, desc_pair, tok, ids, ids2, ttb, E_tok, E_byte, w_c, bias, False)
-    if planned:
-        _rejoin(dev)
+    ws = _rejoin(ws, dev)
     return out, (Y if sp.out_norm else _empty(dev, cdt)), (w_c if w_c is not W else _empty(dev, cdt)), ws
 
 
@@ -325,11 +317,9 @@ def embed_byte_fc_op(tok: Tensor, ids: Optional[Tensor], E_tok: Tensor, E_byte: 
     tok, desc_b, desc_t = O._fc_descs(unpack_spec(spec_b, eps), bpt, seq_len, tok, next_tok, ids, ttb, E_tok, E_byte)
     w_c = W if W.dtype == cdt else O.cast_out(W, cdt)
     planned = plan and tok.numel() > 0
-    ws = _plan_beside(desc_t, tok, dev) if planned else _empty(dev)
+    ws = _plan_beside(desc_t, tok, dev) if planned else None
     out, Y = O._byte_fc_forward(desc_b, desc_t, tok, ids, E_tok, E_byte, w_c, ttb)
-    if planned:
-        _rejoin(dev)
-    return out, Y, (w_c if w_c is not W else _empty(dev, cdt)), ws
+    return out, Y, (w_c if w_c is not W else _empty(dev, cdt)), _rejoin(ws, dev)
 
 
 @embed_byte_fc_op.register_fake

@@ -324,19 +324,25 @@ def slab_rows(tok_vocab: int, slab: int, n_slabs: int):
     return lo.value, hi.value
 
 
+def _event_pair(dev):
+    """Fork / join events of a plan on the side stream, their cudaEvent_t handles materialised."""
+    pair = (torch.cuda.Event(), torch.cuda.Event())
+    cur = torch.cuda.current_stream(dev)
+    for ev in pair:
+        ev.record(cur)
+    return pair
+
+
 class Workspace:
     """A backward workspace that remembers whether the library left it clean (so the steady-state step needs no
     memset), plus the fork / join events of the plan that runs on the side stream.  Instances are recycled through a
-    pool per (device, table geometry)."""
+    pool per (device, table geometry); one with key None (fresh_workspace) is never pooled."""
 
-    def __init__(self, key, dev):
+    def __init__(self, key, dev, events=None):
         self.key = key
         self.buf: Optional[torch.Tensor] = None
         self.clean = False
-        self.ev_fork, self.ev_join = torch.cuda.Event(), torch.cuda.Event()
-        cur = torch.cuda.current_stream(dev)
-        self.ev_fork.record(cur)   # materialise the cudaEvent_t handles
-        self.ev_join.record(cur)
+        self.ev_fork, self.ev_join = events if events is not None else _event_pair(dev)
         self.pending = False       # a plan was launched on the side stream and no backward has consumed it yet
 
     def reserve(self, desc: L.MotDesc, dev) -> torch.Tensor:
@@ -361,9 +367,27 @@ class Workspace:
 
 _WS_POOL: dict = {}
 _SIDE_STREAMS: dict = {}
+_FRESH_EVENTS: dict = {}
+
+
+def fresh_workspace(desc: L.MotDesc, dev) -> Workspace:
+    """A workspace of its own that is never pooled: a fresh buffer whose head is dirty (a plan or a backward on it
+    clears it first).  Whoever plans in it rejoins before the next such plan starts, so one pair of fork / join events
+    per device serves all of them."""
+    events = _FRESH_EVENTS.get(dev.index)
+    if events is None:
+        events = _FRESH_EVENTS[dev.index] = _event_pair(dev)
+    ws = Workspace(None, dev, events)
+    ws.buf = torch.empty(embed_workspace_bytes(desc), dtype=torch.uint8, device=dev)
+    return ws
 
 
 def acquire_workspace(desc: L.MotDesc, dev) -> Workspace:
+    if torch.cuda.is_current_stream_capturing():
+        # a captured step owns its workspaces (from the capture's memory pool, the clearing memset captured with the
+        # plan): a pooled one would be shared with eager calls and other graphs of the same shapes, whose plans would
+        # then overwrite the graph's between its forward and its backward
+        return fresh_workspace(desc, dev)
     # the zeroed head of the workspace (histogram | byte accumulators | one fp32 slot per stream chunk) is laid out by the
     # table geometry AND by (n_tokens, tok_dim): a buffer is only "clean" for the exact layout it was last used with
     key = (dev.index, desc.tok_vocab, desc.byte_vocab, desc.byte_dim, desc.combine, desc.n_tokens, desc.tok_dim, desc.dp_slabs)
@@ -376,6 +400,8 @@ def acquire_workspace(desc: L.MotDesc, dev) -> Workspace:
 
 
 def release_workspace(ws: Workspace) -> None:
+    if ws.key is None:        # fresh_workspace: never handed to another call
+        return
     free = _WS_POOL.setdefault(ws.key, [])
     if len(free) < 4:
         free.append(ws)
@@ -415,7 +441,8 @@ def embed_plan_join(ws: Workspace, dev, stream: Optional[int] = None) -> None:
 
 
 def _planned_workspace(desc: L.MotDesc, tok, dev, stream: Optional[int] = None) -> Workspace:
-    """A pooled workspace with the backward's sort plan of `tok` started on the side stream, beside the forward."""
+    """A pooled workspace (under capture the graph's own, see acquire_workspace) with the backward's sort plan of `tok`
+    started on the side stream, beside the forward."""
     ws = acquire_workspace(desc, dev)
     embed_plan_async(desc, tok, ws, dev, stream)
     return ws

@@ -250,6 +250,25 @@ int mot_embed_slab_rows(int32_t tok_vocab, int32_t slab, int32_t n_slabs, int32_
  * (beyond that the token rows of the recompute kernel are L2 hits and it is the faster one). */
 int mot_embed_bwd_uses_saved(const MotDesc* d);
 
+/* ---- split residual (runs/71081:302-304,315, V3g) ----------------------------------------------------------------
+ * One gather, three outputs ([n_tokens, out_dim] each, table dtype, 16-byte aligned):
+ *   x0t = rms_norm(E_tok[tok]),  x0b = the per-byte-normed byte rows C'_n,  x = lam[0] * x0t + lam[1] * x0b,
+ * every element bit-identical to the separate tok-only / bytes-only / MOT_ADD launches.  d must be the V3c descriptor:
+ * MOT_ADD with MOT_F_TOK_NORM | MOT_F_BYTE_NORM | MOT_F_HAS_LAMBDAS, no MOT_F_OUT_NORM / MOT_F_TTB_PULL_RIGHT, no
+ * row_stride / col_offset / dp_slabs (else MOT_ERR_BAD_ARG); ids explicit, or from the ttb table (scramble, left pull).
+ * out_dim 512 or 1024 (else MOT_ERR_UNSUPPORTED).
+ * The backward forms g_nt = lam[0] * gx + gx0t and g_nb = lam[1] * gx + gx0b in fp32 and runs the per-input norm
+ * backwards from them: one sort plan, one token-row gather per occurrence, one dense write of each table; g_lam =
+ * (sum gx . x0t, sum gx . x0b).  gx0t / gx0b may be NULL (zero: the output was not used).  Workspace, plan and
+ * ws_flags as for mot_embed_bwd (mot_embed_workspace_bytes(d), mot_embed_plan(_async)). */
+int mot_split_residual_fwd(const MotDesc* d, const int32_t* tok, const void* byte_ids, const void* ttb,
+                           const void* E_tok, const void* E_byte, const float* lam, void* x, void* x0t, void* x0b,
+                           void* stream);
+int mot_split_residual_bwd(const MotDesc* d, const int32_t* tok, const void* byte_ids, const void* ttb,
+                           const void* E_tok, const void* E_byte, const float* lam, const void* gx, const void* gx0t,
+                           const void* gx0b, void* gE_tok, void* gE_byte, float* g_lam, void* workspace, size_t ws_bytes,
+                           int32_t ws_flags, void* stream);
+
 /* ---- byte half of `--add-padded-and-pulled` (spt/train_gpt.py:371-379) ----------------------------------------
  * rows[pos, col_offset + k*byte_dim : +byte_dim] = rms_norm(E_byte[ids_a[pos,k]] + E_byte[ids_b[pos,k]]) for k < bpt:
  * two gathers summed BEFORE the per-byte norm (`norm(self.embed_bytes(byte_tensor) + self.embed_bytes(byte_tensor_pulled))`).

@@ -432,11 +432,21 @@ extern "C" int mot_embed_bwd(const MotDesc* d, const int32_t* tok, const void* b
                           g_lam, nullptr, workspace, ws_bytes, ws_flags, stream);
 }
 
+// The split residual (runs/71081) runs on the V3c descriptor: ADD, per-input norms, lambdas, no output norm, whole rows,
+// left pulls only.
+static bool split_residual_desc(const MotDesc* d) {
+  const int f = d->flags & (MOT_F_TOK_NORM | MOT_F_BYTE_NORM | MOT_F_OUT_NORM | MOT_F_BYTES_FIRST | MOT_F_HAS_LAMBDAS);
+  return d->combine == MOT_ADD && f == (MOT_F_TOK_NORM | MOT_F_BYTE_NORM | MOT_F_HAS_LAMBDAS) &&
+         !(d->flags & MOT_F_TTB_PULL_RIGHT) && d->row_stride == 0 && d->col_offset == 0 && d->dp_slabs <= 1;
+}
+
+// split: the split-residual backward, gx0t / gx0b the gradients of x0t / x0b (nullptr = zero)
 static int embed_bwd_impl(const MotDesc* d, const int32_t* tok, const void* byte_ids, const void* ttb,
                           const void* E_tok, const void* E_byte, const float* lam, const void* addend,
                           const void* grad_out, const void* out_saved, const float* rstd_saved, void* gE_tok,
                           void* gE_byte, float* g_lam, void* d_addend, void* workspace, size_t ws_bytes,
-                          int32_t ws_flags, int slab, int n_slabs, int reserve_sms, void* stream) {
+                          int32_t ws_flags, int slab, int n_slabs, int reserve_sms, void* stream, bool split = false,
+                          const void* gx0t = nullptr, const void* gx0b = nullptr) {
   const bool plan_ready = (ws_flags & MOT_WS_PLAN_READY) != 0, ws_clean = (ws_flags & MOT_WS_CLEAN) != 0;
   if (int rc = validate(d)) return rc;
   const bool slabbed = n_slabs > 1;
@@ -450,6 +460,8 @@ static int embed_bwd_impl(const MotDesc* d, const int32_t* tok, const void* byte
   if (d_addend && (d->flags & MOT_F_OUT_NORM) && !addend) return MOT_ERR_BAD_ARG;  // d z needs z: the addend itself
   if (!aligned16(addend) || !aligned16(d_addend)) return MOT_ERR_MISALIGNED;
   if (!aligned16(gE_tok) || !aligned16(gE_byte)) return MOT_ERR_MISALIGNED;
+  if (split && (!split_residual_desc(d) || !g_lam)) return MOT_ERR_BAD_ARG;
+  if (!aligned16(gx0t) || !aligned16(gx0b)) return MOT_ERR_MISALIGNED;
   if (d->n_tokens == 0) {  // nothing gathered: dense zero grads
     cudaStream_t s0 = reinterpret_cast<cudaStream_t>(stream);
     const size_t esz0 = d->dtype == MOT_BF16 ? 2 : 4;
@@ -477,6 +489,7 @@ static int embed_bwd_impl(const MotDesc* d, const int32_t* tok, const void* byte
   p.tok = tok; p.ids = byte_ids; p.ttb = ttb; p.E_tok = E_tok; p.E_byte = E_byte; p.lam = lam;
   p.gout = grad_out; p.gE_tok = gE_tok; p.gE_byte = gE_byte; p.g_lam = g_lam;
   p.addend = addend; p.d_addend = d_addend;
+  p.gout_tok = gx0t; p.gout_byte = gx0b;
   p.plan_early = (plan_ready && (ws_flags & MOT_WS_PLAN_JOINED)) ? 1 : 0;
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   if (slabbed) {
@@ -505,6 +518,8 @@ static int embed_bwd_impl(const MotDesc* d, const int32_t* tok, const void* byte
       q->R = p.R;  // one stream chunking for both halves and the finalize pass
       if ((rc = d->dtype == MOT_BF16 ? dispatch_bwd_bf16(*q, s) : dispatch_bwd_f32(*q, s))) return rc;
     }
+  } else if (split) {
+    if ((rc = d->dtype == MOT_BF16 ? dispatch_bwd_resid_bf16(p, s) : dispatch_bwd_resid_f32(p, s))) return rc;
   } else {
     // the MoT-sum variant with the forward result kept: the saved-output kernel (mot_embed_bwd_sum.cuh); every other
     // case recomputes the mixed row
@@ -532,7 +547,11 @@ static int embed_bwd_impl(const MotDesc* d, const int32_t* tok, const void* byte
     if (fb > 8LL * sms) fb = 8LL * sms;
     if (fb < 1) fb = 1;
     p.trace = g_trace ? g_trace + 2 * 4096 * 64 : nullptr;
-    rc = d->dtype == MOT_BF16 ? launch_finalize_bf16(p, (int)fb, s) : launch_finalize_f32(p, (int)fb, s);
+    EmbedParams pf = p;
+    // the split residual's row sums already carry lam_tok (g_nt = lam_t * gx + gx0t) and its d lam_tok is complete: the
+    // finalize pass sees a variant without lambdas (pure per-input norm backward)
+    if (split) pf.flags &= ~MOT_F_HAS_LAMBDAS;
+    rc = d->dtype == MOT_BF16 ? launch_finalize_bf16(pf, (int)fb, s) : launch_finalize_f32(pf, (int)fb, s);
   }
   if (rc) return rc;
   if ((d->flags & MOT_F_HAS_LAMBDAS) && g_lam && p.last_slab) {
@@ -581,4 +600,32 @@ extern "C" int mot_embed_touched_rows(const MotDesc* d, const void* workspace, s
              (const int*)p.off, (int)p.V, bitmap);
   count_launch();
   return check_launch();
+}
+
+extern "C" int mot_split_residual_fwd(const MotDesc* d, const int32_t* tok, const void* byte_ids, const void* ttb,
+                                      const void* E_tok, const void* E_byte, const float* lam, void* x, void* x0t, void* x0b,
+                                      void* stream) {
+  if (int rc = validate(d)) return rc;
+  if (!split_residual_desc(d)) return MOT_ERR_BAD_ARG;
+  if (d->n_tokens == 0) return MOT_OK;
+  if (!x || !x0t || !x0b || !tok || !E_tok || !E_byte || !lam) return MOT_ERR_BAD_ARG;
+  if (d->flags & MOT_F_IDS_FROM_TTB) { if (!ttb) return MOT_ERR_BAD_ARG; }
+  else if (!byte_ids) return MOT_ERR_BAD_ARG;
+  if (!aligned16(x) || !aligned16(x0t) || !aligned16(x0b) || !aligned16(E_tok) || !aligned16(E_byte)) return MOT_ERR_MISALIGNED;
+  EmbedParams p;
+  fill_params(d, p);
+  p.tok = tok; p.ids = byte_ids; p.ttb = ttb; p.E_tok = E_tok; p.E_byte = E_byte; p.lam = lam;
+  p.out = x; p.out_tok = x0t; p.out_byte = x0b;
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  return d->dtype == MOT_BF16 ? dispatch_fwd_resid_bf16(p, s) : dispatch_fwd_resid_f32(p, s);
+}
+
+extern "C" int mot_split_residual_bwd(const MotDesc* d, const int32_t* tok, const void* byte_ids, const void* ttb,
+                                      const void* E_tok, const void* E_byte, const float* lam, const void* gx,
+                                      const void* gx0t, const void* gx0b, void* gE_tok, void* gE_byte, float* g_lam,
+                                      void* workspace, size_t ws_bytes, int32_t ws_flags, void* stream) {
+  if (int rc = validate(d)) return rc;
+  if (!split_residual_desc(d)) return MOT_ERR_BAD_ARG;
+  return embed_bwd_impl(d, tok, byte_ids, ttb, E_tok, E_byte, lam, nullptr, gx, nullptr, nullptr, gE_tok, gE_byte, g_lam,
+                        nullptr, workspace, ws_bytes, ws_flags, 0, 1, 0, stream, true, gx0t, gx0b);
 }

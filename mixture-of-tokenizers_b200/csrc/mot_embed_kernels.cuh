@@ -82,6 +82,12 @@ struct EmbedParams {
   long long* chk;    // MOT_CHECK builds: violation record
   int n_slots;       // fp32 slots of `partial` (MOT_CHECK builds verify every slot index against it)
   int pad_eot;      // MOT_F_TTB_PULL_LEFT / _RIGHT: pad byte | end-of-text byte << 16 (int16 each; fits the struct's tail padding)
+  // split residual (MOT_SPLIT modes, runs/71081): the forward also stores x0t = nrm(t) and x0b = C'_n ([N, Do] each); the
+  // backward reads their upstream gradients (nullptr: zero).  Appended last: the fields above keep their offsets.
+  void* out_tok;
+  void* out_byte;
+  const void* gout_tok;
+  const void* gout_byte;
 };
 
 struct ChunkMap {
@@ -365,7 +371,8 @@ __device__ __forceinline__ int pulled_lane_id(const EmbedParams& p, int pos, boo
 //   over the mixed row, so the backward needs no reduction and keeps nothing of the row in registers).
 // MODE 0 and MODE 4 decide every variant flag at run time; MODE 4 additionally handles the dense addend (kept out of
 // MODE 0 so that the common kernels do not carry its registers)
-#define MOT_RT(M) ((M) == 0 || (M) == 4)
+// MODE 7: MODE 0 plus the split residual (below), the fp32 forward of runs/71081
+#define MOT_RT(M) ((M) == 0 || (M) == 4 || (M) == 7)
 // MODE 5: plain token gather (no norm, no lambdas): the value embeddings (runs/7:308);
 // MODE 6: pure concat with the output norm only (runs/711:224-232), token / byte columns decided per chunk;
 // MODE 16 + f: the ADD family with its flags fixed at compile time, f = tok_norm | byte_norm << 1 | out_norm << 2 |
@@ -374,6 +381,13 @@ __device__ __forceinline__ int pulled_lane_id(const EmbedParams& p, int pos, boo
 //   1024 columns, profiles/r1_bwd_generic_ncu.txt).
 #define MOT_ADDFAM(M) ((M) >= 16)
 #define MOT_ADDFLAG(M, bit) (MOT_ADDFAM(M) && (((M) - 16) & (bit)) != 0)
+// f bit 16 = split residual (runs/71081, V3g): the V3c kernel (f = 11) that also writes x0t = nrm(t) and x0b = C'_n, and
+// whose backward takes their gradients: g_nt = lam_t * gx + gx0t, g_nb = lam_b * gx + gx0b.  Only kModeSplitResidual,
+// and kModeSplitResidualRT for the fp32 forward: x is bit-identical to the V3c launch only from the kernel family that
+// launch runs (the static ADD family for bf16, the run-time-flag kernel for fp32: nvcc contracts x * tscale + bs * b
+// differently in the two).
+#define MOT_SPLIT(M) ((M) == 7 || MOT_ADDFLAG(M, 16))
+constexpr int kModeSplitResidual = 16 + 11 + 16, kModeSplitResidualRT = 7;
 template <int MODE>
 struct Cfg {
   __device__ __forceinline__ static bool tok_norm(const EmbedParams& p) {
@@ -475,7 +489,8 @@ __host__ __device__ inline size_t align_up(size_t x, size_t a) { return (x + a -
 struct SmemLayout {
   size_t rs, tab, bars, ring, stage_bytes, g_bytes, total;
 };
-__host__ __device__ inline SmemLayout smem_layout(const EmbedParams& p, size_t esz, int warps, bool backward) {
+// g_rows: upstream-gradient rows per backward stage (3 for the split residual: gx, gx0t, gx0b)
+__host__ __device__ inline SmemLayout smem_layout(const EmbedParams& p, size_t esz, int warps, bool backward, int g_rows = 1) {
   SmemLayout L{};
   const bool has_bytes = p.combine != MOT_TOK_ONLY, has_tok = p.combine != MOT_BYTES_ONLY;
   size_t o = 0;
@@ -486,7 +501,7 @@ __host__ __device__ inline SmemLayout smem_layout(const EmbedParams& p, size_t e
   L.bars = o;
   o += align_up((size_t)warps * p.stages * 8, 128);
   L.ring = o;
-  L.g_bytes = backward ? align_up((size_t)p.Do * esz, 128) : 0;
+  L.g_bytes = backward ? (size_t)g_rows * align_up((size_t)p.Do * esz, 128) : 0;
   L.stage_bytes = L.g_bytes + (has_tok ? align_up((size_t)p.Dt * esz, 128) : 0);
   o += (size_t)warps * p.stages * L.stage_bytes;
   L.total = o;
@@ -623,13 +638,25 @@ __global__ void __launch_bounds__(NT, 1) mot_fwd_kernel(const EmbedParams p) {
         for (int e = 0; e < 8; ++e) x[it][e] = 0.f;
     }
     float tscale = lam_t;
+    float r_t = 1.f;  // split residual: the token norm alone, x0t = t * r_t (what a tok-only launch computes)
     if (tok_norm) {
       ss_t = warp_sum(ss_t);
-      tscale *= rsqrtf(ss_t * inv_Dt + p.eps);
+      if constexpr (MOT_SPLIT(MODE)) {
+        r_t = rsqrtf(ss_t * inv_Dt + p.eps);
+        tscale *= r_t;
+      } else {
+        tscale *= rsqrtf(ss_t * inv_Dt + p.eps);
+      }
     }
     float ss = 0.f;
 #pragma unroll
     for (int it = 0; it < CPL; ++it) {
+      if constexpr (MOT_SPLIT(MODE)) {
+        float y[8];
+#pragma unroll
+        for (int e = 0; e < 8; ++e) y[e] = x[it][e] * r_t;
+        Vec8<T>::stg(reinterpret_cast<T*>(p.out_tok) + mul_u32(pos, p.Do) + (size_t)(it * 32 + lane) * kChunk, y);
+      }
       if (C::kTokScaled) {
 #pragma unroll
         for (int e = 0; e < 8; ++e) x[it][e] *= tscale;
@@ -653,6 +680,12 @@ __global__ void __launch_bounds__(NT, 1) mot_fwd_kernel(const EmbedParams p) {
             Vec8<T>::unpack(tab_load<T, MODE>(p, tab, (unsigned)(id * p.bd + cm[it].boff)), b);
             if (byte_scale) {
               const float bs = lam_b * rs[id];
+              if constexpr (MOT_SPLIT(MODE)) {  // x0b = C'_n as a bytes-only launch computes it: 0 + rs * b
+                float y[8];
+#pragma unroll
+                for (int e = 0; e < 8; ++e) y[e] = fmaf(rs[id], b[e], 0.f);
+                Vec8<T>::stg(reinterpret_cast<T*>(p.out_byte) + mul_u32(pos, p.Do) + (size_t)(it * 32 + lane) * kChunk, y);
+              }
 #pragma unroll
               for (int e = 0; e < 8; ++e) x[it][e] += bs * b[e];
             } else {
@@ -781,8 +814,12 @@ struct Batch {
 #ifndef MOT_WIDE_STATIC_THREADS
 #define MOT_WIDE_STATIC_THREADS 256
 #endif
+// The split residual stages three gradient rows per occurrence: 8 warps at most (the launcher takes fewer where the stages
+// and the byte table do not fit shared memory).
 template <int CPL, int MODE>
-constexpr int bwd_threads() { return (MOT_ADDFLAG(MODE, 4) && CPL >= 8) ? MOT_WIDE_STATIC_THREADS : kBwdThreads; }
+constexpr int bwd_threads() {
+  return MOT_SPLIT(MODE) ? 256 : (MOT_ADDFLAG(MODE, 4) && CPL >= 8) ? MOT_WIDE_STATIC_THREADS : kBwdThreads;
+}
 
 template <typename T, int CPL, int MODE, int PULL>
 __global__ void __launch_bounds__((bwd_threads<CPL, MODE>()), 1) mot_bwd_kernel(const EmbedParams p) {
@@ -794,7 +831,7 @@ __global__ void __launch_bounds__((bwd_threads<CPL, MODE>()), 1) mot_bwd_kernel(
   const int lane = lane_id();
   const int warp = threadIdx.x >> 5;
   const int nw = blockDim.x >> 5;
-  const SmemLayout L = smem_layout(p, sizeof(T), nw, true);
+  const SmemLayout L = smem_layout(p, sizeof(T), nw, true, MOT_SPLIT(MODE) ? 3 : 1);
   float* rs = reinterpret_cast<float*>(smem_raw + L.rs);
   T* tab = reinterpret_cast<T*>(smem_raw + L.tab);
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + L.bars) + warp * p.stages;
@@ -819,6 +856,9 @@ __global__ void __launch_bounds__((bwd_threads<CPL, MODE>()), 1) mot_bwd_kernel(
   // value embeddings of runs/7:308, has d E[v] = sum of the upstream rows: R = 0 in SURVEY 8d's byte count)
   const bool need_trow = has_tok && (C::tok_norm(p) || C::out_norm(p) || C::has_lam(p));
   const uint32_t t_bytes = need_trow ? (uint32_t)p.Dt * sizeof(T) : 0u;
+  // split residual: the stage holds [gx | gx0t | gx0b | t], the two extra rows only when their gradient exists
+  const uint32_t g_row = (uint32_t)align_up((size_t)p.Do * sizeof(T), 128);
+  const bool has_gt = MOT_SPLIT(MODE) && p.gout_tok != nullptr, has_gb = MOT_SPLIT(MODE) && p.gout_byte != nullptr;
 
   // ---- the warp's share of the token-sorted stream: chunks gw, gw+W, ... of R entries (gw is interleaved over the
   //      CTAs, so every SM gets the same number of chunks +-1), walked in batches of 32 entries (one per lane) ----
@@ -876,9 +916,17 @@ __global__ void __launch_bounds__((bwd_threads<CPL, MODE>()), 1) mot_bwd_kernel(
     if (lane == ik) {  // the lane that holds entry ik of the batch issues its two row copies (no broadcast needed)
       const int pos = iw ? B.pos : A.pos, v = iw ? B.v : A.v;
       unsigned char* st = ring + (size_t)is * L.stage_bytes;
-      mbar_expect_tx(bars + is, g_bytes + t_bytes);
-      bulk_g2s(st, gout + mul_u32(pos, (int)p.io_ld) + p.io_col, g_bytes, bars + is);
-      if (need_trow) bulk_g2s(st + L.g_bytes, E_tok + mul_u32(v, p.Dt), t_bytes, bars + is);
+      if constexpr (MOT_SPLIT(MODE)) {
+        mbar_expect_tx(bars + is, g_bytes * (1u + has_gt + has_gb) + t_bytes);
+        bulk_g2s(st, gout + mul_u32(pos, p.Do), g_bytes, bars + is);
+        if (has_gt) bulk_g2s(st + g_row, reinterpret_cast<const T*>(p.gout_tok) + mul_u32(pos, p.Do), g_bytes, bars + is);
+        if (has_gb) bulk_g2s(st + 2 * g_row, reinterpret_cast<const T*>(p.gout_byte) + mul_u32(pos, p.Do), g_bytes, bars + is);
+        bulk_g2s(st + L.g_bytes, E_tok + mul_u32(v, p.Dt), t_bytes, bars + is);
+      } else {
+        mbar_expect_tx(bars + is, g_bytes + t_bytes);
+        bulk_g2s(st, gout + mul_u32(pos, (int)p.io_ld) + p.io_col, g_bytes, bars + is);
+        if (need_trow) bulk_g2s(st + L.g_bytes, E_tok + mul_u32(v, p.Dt), t_bytes, bars + is);
+      }
     }
     ++issued;
     if (++is == D) is = 0;
@@ -940,8 +988,9 @@ __global__ void __launch_bounds__((bwd_threads<CPL, MODE>()), 1) mot_bwd_kernel(
   auto flush = [&](bool trail) {
     const T* trow = reinterpret_cast<const T*>(ring + (size_t)ps * L.stage_bytes + L.g_bytes);
     if (!seg_lead && !trail) {
-      const float d = finish_tok_row<T, CPL, MODE>(p, cm, cur_v, Du, trow, lam_t);
-      if (lane == 0) dlam_t += d;
+      // split residual: Du already carries lam_t (g_nt = lam_t * gx + gx0t) and d lam_tok is summed per occurrence
+      const float d = finish_tok_row<T, CPL, MODE>(p, cm, cur_v, Du, trow, MOT_SPLIT(MODE) ? 1.f : lam_t);
+      if (!MOT_SPLIT(MODE) && lane == 0) dlam_t += d;
     } else {
       // the row continues in another chunk: add this segment into the fp32 slot of the row's FIRST chunk (a chunk is
       // the first chunk of at most one such row: its last one).  Hot rows spread over many chunks meet there through
@@ -1010,7 +1059,7 @@ __global__ void __launch_bounds__((bwd_threads<CPL, MODE>()), 1) mot_bwd_kernel(
           }
         }
         ss_t = warp_sum(ss_t);
-        tscale = lam_t * rsqrtf(ss_t * inv_Dt + p.eps);
+        tscale = (MOT_SPLIT(MODE) ? 1.f : lam_t) * rsqrtf(ss_t * inv_Dt + p.eps);  // split residual: r_t alone
       }
 
       int idv[CPL];  // byte id of this lane's slot per chunk (warp collective: outside lane-dependent branches)
@@ -1083,6 +1132,7 @@ __global__ void __launch_bounds__((bwd_threads<CPL, MODE>()), 1) mot_bwd_kernel(
         r_o = rsqrtf(ss * inv_Do + p.eps);
         coef = r_o * r_o * r_o * gz * inv_Do;
       }
+      float gx_t = 0.f;  // split residual: this lane's part of <gx, t> (d lam_tok += r_t * <gx, t>)
 #pragma unroll
       for (int it = 0; it < CPL; ++it) {
         const bool valid = MOT_CHUNK_OK(it);  // lane-dependent: no warp collectives under it
@@ -1096,7 +1146,16 @@ __global__ void __launch_bounds__((bwd_threads<CPL, MODE>()), 1) mot_bwd_kernel(
           } else {  // no norm over the mixed row: dz is the upstream gradient itself
             V::unpack(V::lds_raw(grow + (size_t)(it * 32 + lane) * CW), dz);
           }
-          if (MOT_TOK_OK(it)) {
+          if constexpr (MOT_SPLIT(MODE)) {
+            float tv[CW], gt[CW] = {0.f, 0.f, 0.f, 0.f};
+            V::unpack(V::lds_raw(trow + MOT_TOFF(it)), tv);
+            if (has_gt) V::unpack(V::lds_raw(grow + g_row / sizeof(T) + (size_t)(it * 32 + lane) * CW), gt);
+#pragma unroll
+            for (int e = 0; e < CW; ++e) {
+              gx_t += dz[e] * tv[e];
+              Du[it][e] += fmaf(lam_t, dz[e], gt[e]);
+            }
+          } else if (MOT_TOK_OK(it)) {
 #pragma unroll
             for (int e = 0; e < CW; ++e) Du[it][e] += dz[e];
           }
@@ -1133,7 +1192,12 @@ __global__ void __launch_bounds__((bwd_threads<CPL, MODE>()), 1) mot_bwd_kernel(
 #pragma unroll
               for (int e = 0; e < CW; ++e) dlam_b += dz[e] * r * b[e];
             }
-            if (C::kLam) {
+            if constexpr (MOT_SPLIT(MODE)) {
+              float gb[CW] = {0.f, 0.f, 0.f, 0.f};
+              if (has_gb) V::unpack(V::lds_raw(grow + 2 * (g_row / sizeof(T)) + (size_t)(it * 32 + lane) * CW), gb);
+#pragma unroll
+              for (int e = 0; e < CW; ++e) dz[e] = fmaf(lam_b_eff, dz[e], gb[e]);
+            } else if (C::kLam) {
 #pragma unroll
               for (int e = 0; e < CW; ++e) dz[e] *= lam_b_eff;
             }
@@ -1141,6 +1205,7 @@ __global__ void __launch_bounds__((bwd_threads<CPL, MODE>()), 1) mot_bwd_kernel(
           }
         }
       }
+      if constexpr (MOT_SPLIT(MODE)) dlam_t += tscale * gx_t;
       __syncwarp();  // shared-memory reads of this stage are done (values consumed above)
     }
     // at the end of a chunk the open row segment is flushed
@@ -1359,7 +1424,7 @@ __global__ void __launch_bounds__(256) mot_bwd_finalize_kernel(const EmbedParams
 // Launchers
 // ======================================================================================
 // Pick the ring depth and whether the byte table fits next to it; returns dynamic smem bytes or 0.
-inline size_t plan_smem(EmbedParams& p, size_t esz, int warps, bool backward, int optin) {
+inline size_t plan_smem(EmbedParams& p, size_t esz, int warps, bool backward, int optin, int g_rows = 1) {
   static const char* env_st = getenv("MOT_STAGES");  // debug knob
   const int want = env_st ? atoi(env_st) : 2;  // measured: 2 stages per warp are as fast as 4 (profiles/r1_experiments.md)
   p.tab_smem = 1;
@@ -1367,7 +1432,7 @@ inline size_t plan_smem(EmbedParams& p, size_t esz, int warps, bool backward, in
     p.tab_smem = tab;
     for (int st = want; st >= 2; --st) {
       p.stages = st;
-      const SmemLayout L = smem_layout(p, esz, warps, backward);
+      const SmemLayout L = smem_layout(p, esz, warps, backward, g_rows);
       if (L.total + 1024 <= (size_t)optin) return L.total;
     }
   }
@@ -1376,7 +1441,9 @@ inline size_t plan_smem(EmbedParams& p, size_t esz, int warps, bool backward, in
 
 template <typename T, int CPL, int MODE, int PULL = kNoPull>
 static int launch_fwd(const EmbedParams& p_in, cudaStream_t s) {
-  if constexpr (PULL == kNoPull && MODE != 2 && MODE != 5) {
+  if constexpr (PULL == kNoPull && MOT_SPLIT(MODE)) {  // the split residual has left pulls only (runs/71081)
+    if (const int k = ids_pulled(p_in)) return k == kPullLeft ? launch_fwd<T, CPL, MODE, kPullLeft>(p_in, s) : MOT_ERR_UNSUPPORTED;
+  } else if constexpr (PULL == kNoPull && MODE != 2 && MODE != 5) {
     if (const int k = ids_pulled(p_in))
       return k == kPullLeft ? launch_fwd<T, CPL, MODE, kPullLeft>(p_in, s) : launch_fwd<T, CPL, MODE, kPullRight>(p_in, s);
   }
@@ -1394,8 +1461,9 @@ static int launch_fwd(const EmbedParams& p_in, cudaStream_t s) {
     smem = plan_smem(p, sizeof(T), threads / 32, false, optin);
     if (smem != 0 && (p.tab_smem || p.combine == MOT_TOK_ONLY || threads == 256)) break;
   }
-  if (smem == 0) return MOT_ERR_UNSUPPORTED;
-  if ((MODE == 1 || MOT_ADDFAM(MODE)) && !p.tab_smem) return launch_fwd<T, CPL, 0, PULL>(p_in, s);  // fast paths assume the table in smem
+  if (smem == 0 || (MOT_SPLIT(MODE) && !p.tab_smem)) return MOT_ERR_UNSUPPORTED;  // the split residual has no run-time-flag kernel
+  if constexpr (!MOT_SPLIT(MODE))
+    if ((MODE == 1 || MOT_ADDFAM(MODE)) && !p.tab_smem) return launch_fwd<T, CPL, 0, PULL>(p_in, s);  // fast paths assume the table in smem
   p.trace = g_trace;
   auto kern = mot_fwd_kernel<T, CPL, MODE, NT, PULL>;
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return check_launch();
@@ -1412,7 +1480,9 @@ static int launch_fwd(const EmbedParams& p_in, cudaStream_t s) {
 
 template <typename T, int CPL, int MODE, int PULL = kNoPull>
 static int launch_bwd(const EmbedParams& p_in, cudaStream_t s) {
-  if constexpr (PULL == kNoPull && MODE != 2 && MODE != 5) {
+  if constexpr (PULL == kNoPull && MOT_SPLIT(MODE)) {
+    if (const int k = ids_pulled(p_in)) return k == kPullLeft ? launch_bwd<T, CPL, MODE, kPullLeft>(p_in, s) : MOT_ERR_UNSUPPORTED;
+  } else if constexpr (PULL == kNoPull && MODE != 2 && MODE != 5) {
     if (const int k = ids_pulled(p_in))
       return k == kPullLeft ? launch_bwd<T, CPL, MODE, kPullLeft>(p_in, s) : launch_bwd<T, CPL, MODE, kPullRight>(p_in, s);
   }
@@ -1420,13 +1490,22 @@ static int launch_bwd(const EmbedParams& p_in, cudaStream_t s) {
   if (int rc = device_props(&sms, &optin)) return rc;
   EmbedParams p = p_in;
   constexpr int NT = bwd_threads<CPL, MODE>();
-  const size_t smem = plan_smem(p, sizeof(T), NT / 32, true, optin);
+  int threads = NT;
+  size_t smem = plan_smem(p, sizeof(T), NT / 32, true, optin);
+  if constexpr (MOT_SPLIT(MODE)) {  // three gradient rows per stage: halve the warps until stages and byte table fit
+    for (; threads >= 32; threads >>= 1) {
+      smem = plan_smem(p, sizeof(T), threads / 32, true, optin, 3);
+      if (smem != 0 && p.tab_smem) break;
+    }
+    if (threads < 32) return MOT_ERR_UNSUPPORTED;
+  }
   if (smem == 0) return MOT_ERR_UNSUPPORTED;
-  if ((MODE == 1 || MODE == 3 || MODE == 6 || MOT_ADDFAM(MODE)) && !p.tab_smem) return launch_bwd<T, CPL, 0, PULL>(p_in, s);  // fast paths assume the table in smem
+  if constexpr (!MOT_SPLIT(MODE))  // (the split residual's loop above left the table in smem)
+    if ((MODE == 1 || MODE == 3 || MODE == 6 || MOT_ADDFAM(MODE)) && !p.tab_smem) return launch_bwd<T, CPL, 0, PULL>(p_in, s);  // fast paths assume the table in smem
   auto kern = mot_bwd_kernel<T, CPL, MODE, PULL>;
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return check_launch();
   if (g_prof_start) cudaEventRecord(g_prof_start, s);
-  launch_pdl(kern, dim3((unsigned)sms), dim3(NT), smem, s, p);
+  launch_pdl(kern, dim3((unsigned)sms), dim3(threads), smem, s, p);
   if (g_prof_stop) cudaEventRecord(g_prof_stop, s);
   count_launch();
   return check_launch();
@@ -1448,6 +1527,10 @@ int dispatch_fwd_addend_bf16(const EmbedParams& p, cudaStream_t s);  // MODE 4 i
 int dispatch_fwd_addend_f32(const EmbedParams& p, cudaStream_t s);
 int dispatch_bwd_addend_bf16(const EmbedParams& p, cudaStream_t s);
 int dispatch_bwd_addend_f32(const EmbedParams& p, cudaStream_t s);
+int dispatch_fwd_resid_bf16(const EmbedParams& p, cudaStream_t s);  // split residual (kModeSplitResidual)
+int dispatch_fwd_resid_f32(const EmbedParams& p, cudaStream_t s);
+int dispatch_bwd_resid_bf16(const EmbedParams& p, cudaStream_t s);
+int dispatch_bwd_resid_f32(const EmbedParams& p, cudaStream_t s);
 int launch_finalize_bf16(const EmbedParams& p, int blocks, cudaStream_t s);
 int launch_finalize_f32(const EmbedParams& p, int blocks, cudaStream_t s);
 

@@ -73,6 +73,9 @@ _SIGNATURES = {
     "mot_embed_slab_rows": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "mot_tokens_widen_u16": (C.c_int, [_P, C.c_int64, _P, _P]),
     "mot_embed_bwd_uses_saved": (C.c_int, [C.POINTER(MotDesc)]),
+    "mot_split_residual_fwd": (C.c_int, [C.POINTER(MotDesc), _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "mot_split_residual_bwd": (C.c_int, [C.POINTER(MotDesc), _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.c_size_t,
+                                         C.c_int32, _P]),
     "mot_byte_pair_fwd": (C.c_int, [C.POINTER(MotDesc), _P, _P, _P, _P, _P, _P, _P]),
     "mot_byte_pair_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32]),
     "mot_byte_pair_bwd": (C.c_int, [C.POINTER(MotDesc), _P, _P, _P, _P, _P, _P, _P, _P, C.c_size_t, _P]),

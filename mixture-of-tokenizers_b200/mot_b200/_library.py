@@ -169,6 +169,64 @@ embed_op.register_autograd(_embed_backward, setup_context=_embed_setup)
 
 
 # ---------------------------------------------------------------------------------------------------------------
+# mot_b200::split_residual  (runs/71081: x, x0t, x0b from one gather; one backward for the three uses)
+# ---------------------------------------------------------------------------------------------------------------
+@torch.library.custom_op("mot_b200::split_residual", mutates_args=(), device_types="cuda")
+def split_residual_op(tok: Tensor, ids: Optional[Tensor], ttb: Optional[Tensor], E_tok: Tensor, E_byte: Tensor,
+                      lam: Tensor, spec: int, bpt: int, seq_len: int, eps: float,
+                      plan: bool) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """-> (x, x0t, x0b [n, D], workspace uint8 or [0]).  lam: fp32 [2] = (lam_tok, lam_byte)."""
+    tok, desc = O._ids_desc(unpack_spec(spec, eps), bpt, seq_len, tok, None, ids, ttb, E_tok, E_byte, True)
+    dev = E_tok.device
+    ws = _plan_beside(desc, tok, dev) if plan and desc.n_tokens > 0 else None
+    x, x0t, x0b = O._split_residual_forward(desc, tok, ids, ttb, E_tok, E_byte, lam, dev)
+    return x, x0t, x0b, _rejoin(ws, dev)
+
+
+@split_residual_op.register_fake
+def _(tok, ids, ttb, E_tok, E_byte, lam, spec, bpt, seq_len, eps, plan):
+    tok, desc = O._ids_desc(unpack_spec(spec, eps), bpt, seq_len, tok, None, ids, ttb, E_tok, E_byte, True)
+    n, D = desc.n_tokens, desc.out_dim
+    return (E_tok.new_empty((n, D)), E_tok.new_empty((n, D)), E_tok.new_empty((n, D)),
+            E_tok.new_empty((O.embed_workspace_bytes(desc) if plan and n > 0 else 0,), dtype=torch.uint8))
+
+
+@torch.library.custom_op("mot_b200::split_residual_bwd", mutates_args=(), device_types="cuda")
+def split_residual_bwd_op(gx: Optional[Tensor], gx0t: Optional[Tensor], gx0b: Optional[Tensor], tok: Tensor,
+                          ids: Optional[Tensor], ttb: Optional[Tensor], E_tok: Tensor, E_byte: Tensor, lam: Tensor,
+                          ws: Tensor, spec: int, bpt: int, seq_len: int, eps: float) -> Tuple[Tensor, Tensor, Tensor]:
+    """-> (gE_tok, gE_byte dense, g_lam fp32 [2]) from the gradients of (x, x0t, x0b); None: that output was unused."""
+    tok, desc = O._ids_desc(unpack_spec(spec, eps), bpt, seq_len, tok, None, ids, ttb, E_tok, E_byte, True)
+    dev = E_tok.device
+    gE_tok, gE_byte = torch.empty_like(E_tok), torch.empty_like(E_byte)
+    g_lam = torch.empty(2, dtype=torch.float32, device=dev)
+    ws, planned = _bwd_workspace(ws, desc, dev)
+    O._split_residual_backward(desc, tok, ids, ttb, E_tok, E_byte, lam, (gx, gx0t, gx0b), gE_tok, gE_byte, g_lam, ws,
+                               planned, planned, plan_joined=planned)
+    return gE_tok, gE_byte, g_lam
+
+
+@split_residual_bwd_op.register_fake
+def _(gx, gx0t, gx0b, tok, ids, ttb, E_tok, E_byte, lam, ws, spec, bpt, seq_len, eps):
+    return torch.empty_like(E_tok), torch.empty_like(E_byte), lam.new_empty((2,), dtype=torch.float32)
+
+
+def _split_residual_setup(ctx, inputs, output):
+    tok, ids, ttb, E_tok, E_byte, lam, spec, bpt, seq_len, eps, plan = inputs
+    ctx.save_for_backward(tok, ids, ttb, E_tok, E_byte, lam, output[3])
+    ctx.cfg = (spec, bpt, seq_len, eps)
+
+
+def _split_residual_backward(ctx, gx, gx0t, gx0b, g_ws):
+    tok, ids, ttb, E_tok, E_byte, lam, ws = ctx.saved_tensors
+    gt, gb, gl = torch.ops.mot_b200.split_residual_bwd(gx, gx0t, gx0b, tok, ids, ttb, E_tok, E_byte, lam, ws, *ctx.cfg)
+    return None, None, None, gt, gb, gl, None, None, None, None, None
+
+
+split_residual_op.register_autograd(_split_residual_backward, setup_context=_split_residual_setup)
+
+
+# ---------------------------------------------------------------------------------------------------------------
 # mot_b200::tok_gather  (several tables gathered with the same token ids: the value embeddings)
 # ---------------------------------------------------------------------------------------------------------------
 @torch.library.custom_op("mot_b200::tok_gather", mutates_args=(), device_types="cuda")

@@ -16,7 +16,7 @@ from typing import Optional
 import torch
 from torch import nn
 
-from .ops import MixSpec, mot_embed, mot_embed_byte_fc, mot_embed_proj, tok_gather
+from .ops import _TTB_DTYPE, MixSpec, mot_embed, mot_embed_byte_fc, mot_embed_proj, split_residual, tok_gather
 
 # variant name -> MixSpec kwargs (SURVEY.md 2.4; `slot_major` is the `.view(bpt,-1)` id layout of the sum runs)
 RUN_VARIANTS = {
@@ -169,26 +169,47 @@ class MoTSplitResidualEmbedding(nn.Module):
     forward(token_inputs [T], byte_inputs [bpt, T]) -> (x, x0t, x0b), each [1, T, model_dim], with
     x0t = norm(embed_tokens(tok)), x0b = the per-byte-normed bytes concatenated in the `.view(bpt,-1)` order and
     x = lam_tok * x0t + lam_byte * x0b.  Parameters `embed_tokens.weight`, `embed_bytes.weight`, `lambdas` ([byte,
-    token] = the reference's scalars[-2], scalars[-1]).  Three launches of the fused kernel (V3c, token half, byte
-    half); autograd adds the dense gradients of the three uses."""
+    token] = the reference's scalars[-2], scalars[-1]).  One fused kernel writes the three outputs and one backward
+    takes the gradients of all three uses (model_dim 512 or 1024).  With byte_inputs=None and a ttb table the byte ids
+    are derived inside the kernels: the padded ids, or with pull_in=True the pulled ids of pull_from_left over the T
+    tokens."""
 
-    def __init__(self, token_vocab_size: int, byte_vocab_size: int, model_dim: int, byte_dim: int, bytes_per_token: int = 16):
+    def __init__(self, token_vocab_size: int, byte_vocab_size: int, model_dim: int, byte_dim: int, bytes_per_token: int = 16,
+                 ttb: Optional[torch.Tensor] = None, pull_in: bool = False):
         super().__init__()
         if byte_dim * bytes_per_token != model_dim:
             raise ValueError("MoTSplitResidualEmbedding: bytes_per_token * byte_dim must equal model_dim (runs/71081:500-501)")
-        self.bpt = bytes_per_token
+        if ttb is not None and (ttb.dim() != 2 or ttb.shape[1] != bytes_per_token or ttb.dtype not in _TTB_DTYPE):
+            raise ValueError(f"MoTSplitResidualEmbedding: ttb must be a [V, {bytes_per_token}] int16 / float32 / bfloat16 "
+                             f"table, got {tuple(ttb.shape)} {ttb.dtype}")
+        if pull_in and ttb is None:
+            raise ValueError("MoTSplitResidualEmbedding: pull_in=True derives the pulled ids from a ttb table: pass ttb=")
+        self.bpt, self.pull_in = bytes_per_token, pull_in
         self.embed_tokens = nn.Embedding(token_vocab_size, model_dim)
         self.embed_bytes = nn.Embedding(byte_vocab_size, byte_dim)
         self.lambdas = nn.Parameter(torch.tensor([0.5, 0.5]))
+        self.register_buffer("ttb", ttb, persistent=False)
+        self.grad_bucket = None
 
-    def forward(self, token_inputs: torch.Tensor, byte_inputs: torch.Tensor):
+    def attach_grad_bucket(self, bucket=None):
+        """Data parallelism, as MoTEmbedding.attach_grad_bucket: the backward writes `embed_tokens.weight.grad` and
+        `embed_bytes.weight.grad` straight into one flat bucket (default: a bucket of these two tables) and marks the
+        rows of the batch when the token table is one of its row tables, so one `bucket.all_reduce_avg()` moves only the
+        rows some rank gathered.  Call after the module is on its device and in its final dtype."""
+        from .dp import GradBucket
+        self.grad_bucket = bucket if bucket is not None else \
+            GradBucket([self.embed_tokens.weight, self.embed_bytes.weight], symmetric="auto")
+        return self.grad_bucket
+
+    def forward(self, token_inputs: torch.Tensor, byte_inputs: Optional[torch.Tensor] = None):
         assert token_inputs.ndim == 1
-        Et, Eb = self.embed_tokens.weight, self.embed_bytes.weight
-        x0t = mot_embed(token_inputs, None, Et, None, MixSpec(combine="tok_only", tok_norm=True, out_norm=False))
-        x0b = mot_embed(None, byte_inputs, None, Eb,
-                        MixSpec(combine="bytes_only", byte_norm=True, out_norm=False, slot_major=True), bpt=self.bpt)
-        x = mot_embed(token_inputs, byte_inputs, Et, Eb, MixSpec(**RUN_VARIANTS["V3c"]), bpt=self.bpt,
-                      lam=self.lambdas.flip(0))
+        if byte_inputs is None and self.ttb is None:
+            raise RuntimeError("MoTSplitResidualEmbedding: byte_inputs=None derives the ids from a ttb table: pass ttb=")
+        Et, Eb, b = self.embed_tokens.weight, self.embed_bytes.weight, self.grad_bucket
+        x, x0t, x0b = split_residual(token_inputs, byte_inputs, Et, Eb, self.lambdas.flip(0), bpt=self.bpt,
+                                     ttb=self.ttb if byte_inputs is None else None, seq_len=token_inputs.numel(),
+                                     pull=self.pull_in, grad_bufs=((Et, b.view_of(Et)), (Eb, b.view_of(Eb)), b)
+                                     if b is not None else None)
         return x[None], x0t[None], x0b[None]
 
 

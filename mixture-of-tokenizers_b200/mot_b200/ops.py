@@ -557,6 +557,34 @@ def _embed_args(spec: MixSpec, bpt: int, tokens, byte_ids, ttb, E_tok, E_byte, l
     return dev, tok, ids, ttb, E_tok, E_byte, nxt
 
 
+def _bucket_direct(grad_bufs, tables):
+    """The gradient-bucket views the backward writes straight into, one per table (None: the normal path).  The kernels
+    overwrite every row, so the view becomes param.grad (autograd would clone a view); a parameter that already holds a
+    gradient takes the normal path and autograd adds to it."""
+    direct = [None] * len(tables)
+    if grad_bufs is None:
+        return direct
+    for i, (pv, E) in enumerate(zip(grad_bufs, tables)):
+        if pv is not None and E is not None and pv[0].grad is None:
+            view = pv[1]
+            if view.dtype != E.dtype or view.shape != E.shape or not view.is_contiguous() or view.device != E.device:
+                raise TypeError("mot_b200: the gradient-bucket view of a table must match its dtype, shape and "
+                                f"device and be contiguous (table {tuple(E.shape)} {E.dtype}, view "
+                                f"{tuple(view.shape)} {view.dtype})")
+            direct[i] = pv
+    return direct
+
+
+def _bucket_mark_rows(grad_bufs, desc: L.MotDesc, ws_buf, tok, direct_tok) -> None:
+    """After a backward that produced the token table's gradient: the rows this batch gathered, also when autograd adds
+    this gradient to an existing one (the exchange moves only the union of every backward since the last exchange)."""
+    if grad_bufs is None or len(grad_bufs) <= 2 or grad_bufs[0] is None or tok is None:
+        return
+    bk, p_tok = grad_bufs[2], grad_bufs[0][0]
+    if bk is not None and bk.sparse_rows and bk.is_row_table(p_tok) and not bk._pending:
+        bk.mark_rows(desc, ws_buf, fresh=(p_tok,) if direct_tok is not None else ())
+
+
 class _MotEmbedFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, desc: L.MotDesc, dev, tok, ids, ttb, E_tok, E_byte, lam, grad_bufs=None):
@@ -601,19 +629,7 @@ class _MotEmbedFn(torch.autograd.Function):
         g = grad_out.contiguous()
         if g.dtype != (E_tok if E_tok is not None else E_byte).dtype:
             g = g.to((E_tok if E_tok is not None else E_byte).dtype)
-        direct = [None, None]
-        if ctx.grad_bufs is not None:
-            # the kernels overwrite every row, so they can write straight into the caller's flat bucket; the view is
-            # installed as param.grad here (autograd would clone a view).  With a gradient already accumulated on the
-            # parameter the normal path is taken and autograd adds to it.
-            for i, (pv, E) in enumerate(zip(ctx.grad_bufs, (E_tok, E_byte))):
-                if pv is not None and E is not None and pv[0].grad is None:
-                    view = pv[1]
-                    if view.dtype != E.dtype or view.shape != E.shape or not view.is_contiguous() or view.device != E.device:
-                        raise TypeError("mot_b200: the gradient-bucket view of a table must match its dtype, shape and "
-                                        f"device and be contiguous (table {tuple(E.shape)} {E.dtype}, view "
-                                        f"{tuple(view.shape)} {view.dtype})")
-                    direct[i] = pv
+        direct = _bucket_direct(ctx.grad_bufs, (E_tok, E_byte))
         gE_tok = direct[0][1] if direct[0] is not None else (torch.empty_like(E_tok) if E_tok is not None else None)
         gE_byte = direct[1][1] if direct[1] is not None else (torch.empty_like(E_byte) if E_byte is not None else None)
         g_lam = torch.empty(2, dtype=torch.float32, device=dev) if lam is not None else None
@@ -635,12 +651,7 @@ class _MotEmbedFn(torch.autograd.Function):
             embed_backward_out(desc, tok, ids, ttb, E_tok, E_byte, lam, g, gE_tok, gE_byte, g_lam, ws.buf,
                                plan_ready=planned, ws_clean=clean, stream=st, out_saved=out_saved, rstd=rstd,
                                plan_joined=planned)
-        if ctx.grad_bufs is not None and len(ctx.grad_bufs) > 2 and ctx.grad_bufs[0] is not None and tok is not None:
-            bk, p_tok = ctx.grad_bufs[2], ctx.grad_bufs[0][0]
-            if bk is not None and bk.sparse_rows and bk.is_row_table(p_tok) and not bk._pending:
-                # the rows this batch gathered, also when autograd adds this gradient to an existing one: the exchange
-                # moves only the union of every backward since the last exchange
-                bk.mark_rows(desc, ws.buf, fresh=(p_tok,) if direct[0] is not None else ())
+        _bucket_mark_rows(ctx.grad_bufs, desc, ws.buf, tok, direct[0])
         ctx.ws = None
         _return_workspace(ws)
         if g_lam is not None:
@@ -674,6 +685,110 @@ def mot_embed(tokens: Optional[torch.Tensor], byte_ids: Optional[torch.Tensor], 
                                         float(spec.eps), need, nxt)[0]
     tok, desc = _ids_desc(spec, bpt, seq_len, tok, nxt, ids, ttb_c, E_tok_c, E_byte_c, has_lam=lam is not None)
     return _MotEmbedFn.apply(desc, dev, tok, ids, ttb_c, E_tok_c, E_byte_c, lam, grad_bufs)
+
+
+# ------------------------------------------------------------------------------------------------------------
+# the split residual (runs/71081:302-304,315, V3g): x, x0t, x0b from one gather, one backward for the three uses
+# ------------------------------------------------------------------------------------------------------------
+def _resid_spec(derive: bool, pull: bool, eps: float) -> MixSpec:
+    """The V3c spec of the split residual: `[bpt, T]` ids, or derived from the ttb table in the `.view(bpt,-1)` order
+    (the pulled ids of pull_from_left with `pull`)."""
+    return MixSpec(combine="add", tok_norm=True, byte_norm=True, out_norm=False, slot_major=not derive,
+                   ttb_scramble=derive, ttb_pull=derive and pull, eps=eps)
+
+
+def _split_residual_forward(desc: L.MotDesc, tok, ids, ttb, E_tok, E_byte, lam32, dev, stream: Optional[int] = None):
+    """mot_split_residual_fwd into new tensors -> [x, x0t, x0b], each [n_tokens, D]."""
+    outs = [torch.empty((desc.n_tokens, desc.out_dim), dtype=E_tok.dtype, device=dev) for _ in range(3)]
+    with _on_device(dev):
+        rc = L.lib().mot_split_residual_fwd(desc, _ptr(tok), _ptr(ids), _ptr(ttb), _ptr(E_tok), _ptr(E_byte), _ptr(lam32),
+                                            *[_ptr(o) for o in outs], _stream(dev) if stream is None else stream)
+    L.check(rc, "mot_split_residual_fwd")
+    return outs
+
+
+def _split_residual_backward(desc: L.MotDesc, tok, ids, ttb, E_tok, E_byte, lam32, grads, gE_tok, gE_byte, g_lam, ws_buf,
+                             plan_ready: bool, ws_clean: bool, plan_joined: bool = False,
+                             stream: Optional[int] = None) -> None:
+    """mot_split_residual_bwd: dense gE_tok, gE_byte and g_lam (fp32 [2]) from the gradients (gx, gx0t, gx0b) of the
+    three outputs; None for an output that received none (gx0t / gx0b are passed as NULL, a missing gx as zeros)."""
+    dev, dt = E_tok.device, E_tok.dtype
+    gs = [g.reshape(desc.n_tokens, desc.out_dim).to(dt).contiguous() if g is not None else None for g in grads]
+    if gs[0] is None:
+        gs[0] = torch.zeros((desc.n_tokens, desc.out_dim), dtype=dt, device=dev)
+    flags = (L.WS_PLAN_READY if plan_ready else 0) | (L.WS_CLEAN if ws_clean else 0) | \
+        (L.WS_PLAN_JOINED if plan_ready and plan_joined else 0)
+    with _on_device(dev):
+        rc = L.lib().mot_split_residual_bwd(desc, _ptr(tok), _ptr(ids), _ptr(ttb), _ptr(E_tok), _ptr(E_byte), _ptr(lam32),
+                                            *[_ptr(g) for g in gs], _ptr(gE_tok), _ptr(gE_byte), _ptr(g_lam), _ptr(ws_buf),
+                                            ws_buf.numel(), flags, _stream(dev) if stream is None else stream)
+    L.check(rc, "mot_split_residual_bwd")
+
+
+class _SplitResidualFn(torch.autograd.Function):
+    """(x, x0t, x0b) = (lam_t * nrm(t) + lam_b * C'_n, nrm(t), C'_n): one fused gather writes all three; the backward
+    runs one sort plan (started beside the forward) and one recompute backward from the three upstream gradients, an
+    unused output's being None.  grad_bufs as for _MotEmbedFn: the table gradients go straight into a gradient bucket."""
+
+    @staticmethod
+    def forward(ctx, desc: L.MotDesc, dev, tok, ids, ttb, E_tok, E_byte, lam, grad_bufs=None):
+        ctx.set_materialize_grads(False)
+        lam_c = lam.detach().to(torch.float32).contiguous()
+        st = _stream(dev)
+        needs_grad = any(ctx.needs_input_grad[5:8])
+        ctx.ws = _planned_workspace(desc, tok, dev, st) if needs_grad and desc.n_tokens > 0 else None
+        outs = _split_residual_forward(desc, tok, ids, ttb, E_tok, E_byte, lam_c, dev, st)
+        embed_plan_join_if_capturing(ctx.ws, dev, st)
+        ctx.desc, ctx.dev, ctx.grad_bufs, ctx.lam_dtype = desc, dev, grad_bufs, lam.dtype
+        ctx.present = (ids is not None, ttb is not None)
+        ctx.save_for_backward(tok, ids if ids is not None else _ABSENT, ttb if ttb is not None else _ABSENT,
+                              E_tok, E_byte, lam_c)
+        return tuple(outs)
+
+    @staticmethod
+    def backward(ctx, gx, gx0t, gx0b):
+        tok, ids, ttb, E_tok, E_byte, lam = ctx.saved_tensors
+        ids, ttb = [t if ok else None for t, ok in zip((ids, ttb), ctx.present)]
+        desc, dev = ctx.desc, ctx.dev
+        direct = _bucket_direct(ctx.grad_bufs, (E_tok, E_byte))
+        gE_tok = direct[0][1] if direct[0] is not None else torch.empty_like(E_tok)
+        gE_byte = direct[1][1] if direct[1] is not None else torch.empty_like(E_byte)
+        g_lam = torch.empty(2, dtype=torch.float32, device=dev)
+        st = _stream(dev)
+        ws, planned, clean = _take_workspace(ctx.ws, desc, dev, st)
+        _split_residual_backward(desc, tok, ids, ttb, E_tok, E_byte, lam, (gx, gx0t, gx0b), gE_tok, gE_byte, g_lam, ws.buf,
+                                 planned, clean, plan_joined=planned, stream=st)
+        _bucket_mark_rows(ctx.grad_bufs, desc, ws.buf, tok, direct[0])
+        ctx.ws = None
+        _return_workspace(ws)
+        if direct[0] is not None:
+            direct[0][0].grad, gE_tok = gE_tok, None
+        if direct[1] is not None:
+            direct[1][0].grad, gE_byte = gE_byte, None
+        return None, None, None, None, None, gE_tok, gE_byte, g_lam.to(ctx.lam_dtype), None
+
+
+def split_residual(tokens: torch.Tensor, byte_ids: Optional[torch.Tensor], E_tok: torch.Tensor, E_byte: torch.Tensor,
+                   lam: torch.Tensor, *, bpt: int = 16, ttb: Optional[torch.Tensor] = None, seq_len: int = 0,
+                   pull: bool = False, eps: float = FP32_EPS, grad_bufs=None):
+    """The split residual of runs/71081:302-304,315 -> (x, x0t, x0b), each [n_tokens, D] in the table dtype:
+    x0t = rms_norm(E_tok[tokens]), x0b = the per-byte-normed byte rows in the `.view(bpt,-1)` order, x = lam[0] * x0t +
+    lam[1] * x0b (lam = (lam_tok, lam_byte) float [2]).  byte_ids int32/int64 [bpt, T]; byte_ids=None derives them from
+    `ttb` inside the kernels over rows of seq_len tokens (the pulled ids of pull_from_left with pull=True).  D = bpt *
+    byte_dim must be 512 or 1024.  grad_bufs: as for mot_embed."""
+    spec = _resid_spec(byte_ids is None, pull, eps)
+    dev, tok, ids, ttb_c, E_tok_c, E_byte_c, _ = _embed_args(spec, bpt, tokens, byte_ids, ttb, E_tok, E_byte, lam, seq_len,
+                                                             None)
+    if E_tok_c is None or E_byte_c is None or lam is None:
+        raise RuntimeError("mot_b200.split_residual: needs both tables and the two lambdas")
+    if grad_bufs is None and _custom_ops_wanted():
+        need = torch.is_grad_enabled() and any(t.requires_grad for t in (E_tok, E_byte, lam))
+        x, x0t, x0b, _ = torch.ops.mot_b200.split_residual(tok, ids, ttb_c, E_tok_c, E_byte_c,
+                                                           lam.to(torch.float32).contiguous(), pack_spec(spec), bpt,
+                                                           seq_len, float(eps), need)
+        return x, x0t, x0b
+    tok, desc = _ids_desc(spec, bpt, seq_len, tok, None, ids, ttb_c, E_tok_c, E_byte_c, has_lam=True)
+    return _SplitResidualFn.apply(desc, dev, tok, ids, ttb_c, E_tok_c, E_byte_c, lam, grad_bufs)
 
 
 # ------------------------------------------------------------------------------------------------------------
